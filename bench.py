@@ -2,7 +2,7 @@
 """bench.py -- LAS forward hot path on B200: audio-seconds per second (RTFx) + microseconds per decoder step.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|reference-gpu] [--precision bf16|fp16|fp32]
-                    [--workload c3|c2|c4|c5|yaml]
+                    [--workload c3|c2|c4|c5|yaml] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (Listener pBLSTM encoder + Speller greedy attention-decoder loop) over one
 synthetic batch.  Workloads are BASELINE.json configs (SURVEY.md section 8):
@@ -24,6 +24,9 @@ reference's torch op sequence) timed on this box's host cores on a bounded sampl
 `--impl reference` times that CPU path alone (rank 0 only); `--impl reference-gpu` times the same op sequence on cuda:0
 (torch -> cuDNN RNN / cuBLAS, the reference with use_gpu=True; SURVEY.md 2.1), which the default line also carries as
 `gpu_baseline`.  `parity` compares this run's GPU token stream / log-probs with the CPU arm's on the same inputs.
+`--dump-outputs DIR` writes what the timed path returned in its last timed step (tokens, log-probs, attention; c2 also
+the teacher-forced loss) as DIR/<name>.npy in float32.  Inputs and weights are seeded, so two builds run with the same
+arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -51,6 +54,7 @@ WORKLOADS = {
                desc="paper LAS, global batch 512 x 1600 frames sharded 512/N per GPU, 300-char greedy decode"),
 }
 FRAME_SEC = 0.01  # 10 ms frame hop (BASELINE.md: 3000 frames = 30 s)
+DUMP_BYTES = 64_000_000
 
 
 def measured_peaks():
@@ -145,6 +149,24 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm), "source": "nvidia-smi"}
 
 
+def dump_outputs(dirname, outs):
+    """Writes each of `outs` (name -> tensor with the utterances on axis 1, or a scalar) as <dirname>/<name>.npy in float32.
+    Above DUMP_BYTES in all, a fixed seeded sample of the utterances is kept (the same in every run), listed in
+    utterance_index.npy."""
+    import numpy as np
+
+    arrs = {k: v.detach().float().cpu().numpy() for k, v in outs.items()}
+    batch = max(a.shape[1] for a in arrs.values() if a.ndim > 1)
+    if sum(a.nbytes for a in arrs.values()) > DUMP_BYTES:
+        per_utt = sum(a.nbytes for a in arrs.values() if a.ndim > 1) / batch
+        keep = np.sort(np.random.default_rng(0).choice(batch, int((DUMP_BYTES - (1 << 16)) // per_utt), replace=False))
+        arrs = {k: (a[:, keep] if a.ndim > 1 else a) for k, a in arrs.items()}
+        arrs["utterance_index"] = keep.astype(np.float32)
+    os.makedirs(dirname, exist_ok=True)
+    for k, a in arrs.items():
+        np.save(os.path.join(dirname, k + ".npy"), a)
+
+
 def shared_config(args, wl, world):
     """`config` is the SAME dict in both arms (the driver compares them): it names the workload and says, per arm, what differs."""
     per_gpu = wl["B"] // world if wl.get("strong") else wl["B"]
@@ -185,7 +207,7 @@ def reference_arm(wl, sample_B, steps, warmup, device="cpu", seed=17, x=None):
         if cuda:
             torch.cuda.synchronize()
         t1 = time.perf_counter()
-        logp, _ = m.speller(enc, wl["S"], None, 1)
+        logp, attn = m.speller(enc, wl["S"], None, 1)
         if cuda:
             torch.cuda.synchronize()
         t2 = time.perf_counter()
@@ -197,7 +219,7 @@ def reference_arm(wl, sample_B, steps, warmup, device="cpu", seed=17, x=None):
                 sample=f"{sample_B} of the workload's {wl['B']} utterances x {wl['T']} frames, full {wl['S']}-step greedy decode, "
                 f"{len(times)} timed runs after {warmup} warm-up", ms_per_step=1e3 * tot / len(times),
                 listener_ms=1e3 * sum(lis_t) / len(times), us_per_decoder_step=1e6 * (tot - sum(lis_t)) / len(times) / wl["S"],
-                model=m, enc=enc, logp=logp, tokens=logp.argmax(-1), c=c)
+                model=m, enc=enc, logp=logp, attn=attn, tokens=logp.argmax(-1), c=c)
     return audio / tot, info
 
 
@@ -213,7 +235,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-baseline", action="store_true")
     ap.add_argument("--no-pipeline", action="store_true", help="time LAS.forward batch by batch instead of the cross-batch serving pipeline")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
@@ -233,10 +258,10 @@ def main():
         if rank != 0:
             return
         on_gpu = args.impl == "reference-gpu"
-        # one step = a whole 64-utterance batch through the reference's op sequence (1-20 s on the host cores): the run is bounded to
-        # 10 timed steps and 1 warm-up, and the line reports the steps it RAN
-        n_steps, n_warm = min(args.steps, 10), min(args.warmup, 1)
-        val, info = reference_arm(wl, cpu_sample, n_steps, n_warm, device="cuda:0" if on_gpu else "cpu")
+        # one step = a whole 64-utterance batch through the reference's op sequence (1-20 s on the host cores): one warm-up step
+        val, info = reference_arm(wl, cpu_sample, args.steps, min(args.warmup, 1), device="cuda:0" if on_gpu else "cpu")
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"tokens": info["tokens"], "logp": info["logp"], "attn": info["attn"]})
         out = dict(base, impl=args.impl, steps=info["steps_run"], warmup=info["warmup_run"], steps_requested=args.steps, value=val,
                    ms_per_step=info["ms_per_step"], dtype="f32",
                    cpu_baseline={"value": val, "unit": "audio-s/s", "cores": info["cores"], "kind": "port", "sample": info["sample"],
@@ -310,19 +335,19 @@ def main():
                 one_step.loss = las.speller.last_nll_terms.sum() / float(labels_dev.numel())
                 if not serial:
                     one_step.join.record(one_step.side)
-            las.speller(enc, None, 0.0)
+            one_step.result = las.speller(enc, None, 0.0)
             if not serial:
                 cur.wait_event(one_step.join)
                 enc.record_stream(one_step.side)
             return las.speller.last_tokens
-        las.speller(enc, None, 0.0)
+        one_step.result = las.speller(enc, None, 0.0)
         return las.speller.last_tokens
 
     one_step.side, one_step.fork, one_step.join = torch.cuda.Stream(device=dev), torch.cuda.Event(), torch.cuda.Event()
 
     if not tf_leg and not use_pipeline:
         def one_step(x):  # noqa: F811 -- plain LAS.forward (batches beyond one decoder launch group are chunk-pipelined inside it)
-            las(x, None, 0.0, is_training=False)
+            one_step.result = las(x, None, 0.0, is_training=False)
             return las.speller.last_tokens
 
     pipe = las.serve() if use_pipeline else None
@@ -331,7 +356,7 @@ def main():
         """What the timed loop calls: through the serving pipeline the call returns the PREVIOUS batch's outputs (None first)."""
         if pipe is None:
             return one_step(x)
-        out = pipe.submit(x)
+        out = timed_step.result = pipe.submit(x)
         return None if out is None else out.tokens
 
     for _ in range(args.warmup):
@@ -398,6 +423,15 @@ def main():
         ctypes_buf = ctypes.create_string_buffer(1 << 20)
         _cabi.check(lib.las_prof_report(ctypes_buf, len(ctypes_buf)))
         lib.las_prof_enable(0)
+    # what the last timed step returned (device tensors; the untimed passes below produce new ones); one attention head
+    if pipe is None:
+        preds, attns = one_step.result
+        final = {"tokens": tokens, "logp": torch.stack(preds), "attn": torch.stack([a[0] for a in attns])}
+        if tf_leg:
+            final["teacher_forced_loss"] = one_step.loss
+    else:
+        r = timed_step.result
+        final = {"tokens": r.tokens, "logp": r.logp, "attn": r.attn}
     groups = {}
     if os.environ.get("LAS_BENCH_DEBUG"):
         sys.stderr.write("PROF-RAW\n" + ctypes_buf.value.decode() + "\n")
@@ -540,6 +574,8 @@ def main():
     if dist is not None:
         dist.all_reduce(t_e2e, op=dist.ReduceOp.MAX)
     e2e_value = audio_per_step * args.steps / float(t_e2e)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, final)
 
     if rank != 0:
         if dist is not None:

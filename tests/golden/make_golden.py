@@ -1,15 +1,14 @@
-"""Generates tests/golden/*.npz by running the UNMODIFIED reference (/root/reference) on CPU.
+"""Generates tests/golden/*.npz by running the UNMODIFIED reference (a checkout of jiwidi/las-pytorch) on CPU:
 
-Run in the build container only (the GPU box has no /root/reference):
-
-    python tests/golden/make_golden.py
+    LAS_REFERENCE_ROOT=<reference checkout> python tests/golden/make_golden.py
 
 The reference is imported as-is; only three data-prep-only third-party modules that `utils/functions.py`
 imports at module top level are stubbed (SURVEY.md B.1) -- none is reachable from any `forward`.
 Each case stores inputs, (for the tiny configs) the full state_dict, and the reference's fp32 and fp64 outputs.
 For the larger configs the weights are reproduced from the seed by `las_pytorch_b200`'s own parameter
 containers; this script asserts that those are bit-identical to the reference's freshly constructed weights and
-stores a fingerprint.
+stores a fingerprint.  Those cases are stored compactly (`compact`) so that every file stays under 1 MB;
+tests/las_testlib.py `load_golden` restores them.
 """
 from __future__ import annotations
 
@@ -26,15 +25,34 @@ ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 sys.path.insert(0, ROOT)
 
-REF_ROOT = os.environ.get("LAS_REFERENCE_ROOT", "/root/reference")
+
+def compact(out):
+    """Seeded cases: the input is regenerated from the seed (SHA-256 kept to check it), and each fp64 output is kept as a
+    float32 difference from the fp32 one where that difference restores it to 1e-13 (not so in the chaotic gain-6 case,
+    whose fp32 and fp64 runs are far apart: there the fp64 output is kept as it is)."""
+    import hashlib
+
+    x = out.pop("x")
+    out["x_shape"] = np.asarray(x.shape, dtype=np.int64)
+    out["x_sha256"] = hashlib.sha256(np.ascontiguousarray(x, dtype=np.float32).tobytes()).hexdigest()
+    for k in ("enc", "logp", "attn"):
+        f32, f64 = out[f"{k}_f32"], out[f"{k}_f64"]
+        diff = (f64 - f32).astype(np.float32)
+        if np.abs(f32.astype(np.float64) + diff - f64).max() <= 1e-13:
+            del out[f"{k}_f64"]
+            out[f"{k}_f64_minus_f32"] = diff
+    return out
 
 
 def import_reference():
+    ref_root = os.environ.get("LAS_REFERENCE_ROOT")
+    if not ref_root:
+        raise SystemExit("set LAS_REFERENCE_ROOT to a checkout of the reference (jiwidi/las-pytorch)")
     for name in ("pydub", "editdistance", "python_speech_features"):
         sys.modules.setdefault(name, types.ModuleType(name))
     sys.modules["pydub"].AudioSegment = object
     sys.modules["python_speech_features"].logfbank = None
-    sys.path.insert(0, REF_ROOT)
+    sys.path.insert(0, ref_root)
     import model.las_model as ref  # noqa
 
     return ref
@@ -170,16 +188,18 @@ def main():
         for dt, tag in ((torch.float32, "f32"), (torch.float64, "f64")):
             enc, logp, attn = run_reference(ref_las, x, gt, mode == "tf", dt)
             out[f"enc_{tag}"], out[f"logp_{tag}"], out[f"attn_{tag}"] = enc, logp, attn
+        d32 = np.abs(out["logp_f32"] - out["logp_f64"]).max()
+        agree = (out["logp_f32"].argmax(-1) == out["logp_f64"].argmax(-1)).mean()
+        tokens = len(np.unique(out["logp_f64"].argmax(-1)))
         if store_w:
             for k, v in sd_ref.items():
                 out["w:" + k] = v
+        else:
+            out = compact(out)
         path = os.path.join(HERE, name + ".npz")
         np.savez_compressed(path, **out)
-        d32 = np.abs(out["logp_f32"] - out["logp_f64"]).max()
-        agree = (out["logp_f32"].argmax(-1) == out["logp_f64"].argmax(-1)).mean()
         print(f"{name:18s} enc{out['enc_f32'].shape} logp{out['logp_f32'].shape} fp32-vs-fp64 logp {d32:.2e} "
-              f"argmax agree {agree:.3f} distinct tokens {len(np.unique(out['logp_f64'].argmax(-1)))} "
-              f"-> {os.path.getsize(path) / 1024:.0f} KiB")
+              f"argmax agree {agree:.3f} distinct tokens {tokens} -> {os.path.getsize(path) / 1024:.0f} KiB")
 
 
 if __name__ == "__main__":

@@ -20,6 +20,29 @@ def golden_cases():
 
     return sorted(os.path.basename(p)[:-4] for p in glob.glob(os.path.join(GOLDEN_DIR, "*.npz")) if not os.path.basename(p).startswith("ref_"))
 
+
+def load_golden(name):
+    """tests/golden/<name>.npz as a dict of arrays.  A case whose weights are reproduced from the seed may be stored compactly
+    (tests/golden/make_golden.py `compact`) to keep the file under 1 MB: its input `x` is then regenerated from the seed as
+    well (checked by SHA-256), and an fp64 output may be stored as a float32 difference from the fp32 one.  That restores
+    the fp64 output to within 1e-13, below the tightest tolerance any test applies to it (1e-12)."""
+    import hashlib
+
+    g = dict(np.load(os.path.join(GOLDEN_DIR, name + ".npz"), allow_pickle=False))
+    if "x" not in g:
+        c = CONFIGS[str(g["cfg"])]
+        B, T, _ = (int(n) for n in g["x_shape"])
+        x, labels = make_inputs(B, T, c["F"], g["labels"].shape[1], c["V"], seed=int(g["seed"]))
+        x = x.numpy()
+        assert hashlib.sha256(x.tobytes()).hexdigest() == str(g["x_sha256"]), f"{name}: seeded input differs from the golden run's"
+        assert np.array_equal(labels.numpy(), g["labels"])
+        g["x"] = x
+    for k in ("enc", "logp", "attn"):
+        if f"{k}_f64" not in g:
+            g[f"{k}_f64"] = g[f"{k}_f32"].astype(np.float64) + g.pop(f"{k}_f64_minus_f32")
+    return g
+
+
 # name -> (listener kwargs, speller kwargs).  V=30, D=64 from config/librispeech-config.yaml:12,31.
 CONFIGS = {
     # tiny shapes whose weights are stored inside the golden files

@@ -1,6 +1,5 @@
 """Pins both CPU restatements (oracle/) against outputs of the reference itself (tests/golden/*.npz)."""
 import glob
-import os
 
 import numpy as np
 import pytest
@@ -14,9 +13,9 @@ CASES = tl.golden_cases()
 
 
 def load_case(name):
-    g = np.load(os.path.join(tl.GOLDEN_DIR, name + ".npz"), allow_pickle=False)
+    g = tl.load_golden(name)
     cfg = tl.CONFIGS[str(g["cfg"])]
-    sd = {k[2:]: g[k] for k in g.files if k.startswith("w:")}
+    sd = {k[2:]: g[k] for k in g if k.startswith("w:")}
     if not sd:  # weights reproduced from the seed by our own parameter containers
         S = g["logp_f32"].shape[0]
         las = tl.build_model(str(g["cfg"]), max_label_len=S, seed=int(g["seed"]), gain=float(g["gain"]))

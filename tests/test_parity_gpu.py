@@ -33,13 +33,13 @@ def precisions():
 
 
 def load_case(name, precision):
-    g = np.load(os.path.join(tl.GOLDEN_DIR, name + ".npz"), allow_pickle=False)
+    g = tl.load_golden(name)
     cfg = str(g["cfg"])
     mode = str(g["mode"])
     S = g["logp_f64"].shape[0]
     las = tl.build_model(cfg, max_label_len=S, decode_mode=0 if mode == "raw" else 1, seed=int(g["seed"]),
                          gain=float(g["gain"]), precision=precision)
-    sd = {k[2:]: torch.from_numpy(g[k]) for k in g.files if k.startswith("w:")}
+    sd = {k[2:]: torch.from_numpy(g[k]) for k in g if k.startswith("w:")}
     if sd:
         las.load_state_dict(sd, strict=True)
     else:

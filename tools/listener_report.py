@@ -26,20 +26,20 @@ def phases(lib):
 
 def main():
     lib = _cabi.load_library()
-    for path in (os.path.join(tl.GOLDEN_DIR, n + ".npz") for n in tl.golden_cases()):
-        g = np.load(path)
+    for name in tl.golden_cases():
+        g = tl.load_golden(name)
         cfg = str(g["cfg"])
         if cfg in ("tiny_mh", "tiny_nomlp", "tiny_gru", "tiny_rnn"):  # attention variants run in the fp32 mode only
             continue
         las = tl.build_model(cfg, max_label_len=4, seed=int(g["seed"]), gain=float(g["gain"]), precision="bf16")
-        sd = {k[2:]: torch.from_numpy(g[k]) for k in g.files if k.startswith("w:")}
+        sd = {k[2:]: torch.from_numpy(g[k]) for k in g if k.startswith("w:")}
         if sd:
             las.load_state_dict(sd)
         lis = las.listener.cuda()
         enc = lis(torch.from_numpy(g["x"]).cuda())
         torch.cuda.synchronize()
         err = float(np.abs(enc.cpu().numpy() - g["enc_f64"]).max())
-        print(f"{os.path.basename(path):24s} bf16 listener max-abs err vs fp64 reference = {err:.3e}", flush=True)
+        print(f"{name + '.npz':24s} bf16 listener max-abs err vs fp64 reference = {err:.3e}", flush=True)
     for cfgname, B, T in (("paper", 64, 1600), ("small", 32, 1600), ("paper", 16, 3000)):
         c = tl.CONFIGS[cfgname]
         x, _ = tl.make_inputs(B, T, c["F"], 4, c["V"], seed=17)

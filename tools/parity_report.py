@@ -14,8 +14,8 @@ import las_testlib as tl  # noqa: E402
 
 def main():
     print(f"{'case':18s} {'prec':5s} {'enc':>10s} {'logp':>10s} {'attn':>10s} {'argmax agree':>13s}  (vs the reference's fp64 run)")
-    for path in (os.path.join(tl.GOLDEN_DIR, n + ".npz") for n in tl.golden_cases()):
-        g = np.load(path)
+    for name in tl.golden_cases():
+        g = tl.load_golden(name)
         cfg, mode = str(g["cfg"]), str(g["mode"])
         c = tl.CONFIGS[cfg]
         S = g["logp_f64"].shape[0]
@@ -23,7 +23,7 @@ def main():
             if prec == "bf16" and (c.get("heads", 1) > 1 or not c.get("use_mlp", True) or c.get("unit", "LSTM") != "LSTM"):
                 continue  # attention variants run in the fp32 mode only
             las = tl.build_model(cfg, max_label_len=S, decode_mode=0 if mode == "raw" else 1, seed=int(g["seed"]), gain=float(g["gain"]), precision=prec)
-            sd = {k[2:]: torch.from_numpy(g[k]) for k in g.files if k.startswith("w:")}
+            sd = {k[2:]: torch.from_numpy(g[k]) for k in g if k.startswith("w:")}
             if sd:
                 las.load_state_dict(sd)
             las = las.cuda()
@@ -35,7 +35,7 @@ def main():
             logp = torch.stack(preds).cpu().numpy()
             attn = (torch.stack([a[0] for a in attns]) if len(attns[0]) == 1 else torch.stack([torch.stack(list(a)) for a in attns])).cpu().numpy()
             agree = (logp.argmax(-1) == g["logp_f64"].argmax(-1)).mean()
-            print(f"{os.path.basename(path)[:-4]:18s} {prec:5s} {np.abs(enc - g['enc_f64']).max():10.3e} {np.abs(logp - g['logp_f64']).max():10.3e} "
+            print(f"{name:18s} {prec:5s} {np.abs(enc - g['enc_f64']).max():10.3e} {np.abs(logp - g['logp_f64']).max():10.3e} "
                   f"{np.abs(attn - g['attn_f64']).max():10.3e} {agree:13.3f}", flush=True)
 
 
