@@ -14,8 +14,10 @@
  *   - every function returns LAS_OK (0) or a negative LAS_E* code; `las_last_error()` returns a thread-local
  *     message.  The library never aborts and never falls back to the CPU: on a device that is not sm_100 the
  *     compute entry points return LAS_EDEVICE;
- *   - entry points are re-entrant; the library keeps no mutable global state except per-device constant
- *     lookups (SM count), so one thread per GPU replica (nn.DataParallel, train.py:76-78) is safe.
+ *   - entry points are re-entrant and one thread per GPU replica (nn.DataParallel, train.py:76-78) is safe.  The
+ *     library's mutable global state is per-device constant lookups (SM count) and the test hooks at the end of this
+ *     header: the las_debug_set_option switches and the las_debug_set_trace buffer are process-wide and unsynchronised;
+ *     set them while no other thread calls into the library.
  */
 #ifndef LAS_B200_H_
 #define LAS_B200_H_
@@ -274,19 +276,22 @@ int las_debug_umma_probe(const void* a_bf16, const void* b_bf16, float* d, int N
 
 /* Device buffer of 64*8 int64 that the layer-0 recurrence kernel fills with clock64 stamps (NULL disables). */
 int las_debug_set_trace(void* dev_buf);
-/* Kernel variant switches for A/B tests.  key 1: recurrence keeps W_hh in tensor memory (1, default) or shared memory (0);
- * key 2: decoder context through tensor memory (1, default: all feature tiles when they fit, otherwise as many as fit + the rest on the
- * CUDA cores), CUDA cores only (0), tensor memory only when everything fits (2); key 4: recurrence accumulator chains (0 = default);
- * key 5: decoder A/B flags (bit 0: W_phi from shared memory instead of registers; bit 2: one 2-D TMA copy per 64-column atom of an
- * activation part instead of one 3-D copy); key 6: listener input-projection GEMM concurrent with the recurrence (1, default) or in
- * front of it (0); key 7: persistent CTAs of that concurrent GEMM (0 = auto); key 8: tcgen05 GEMM epilogue with row-per-thread
- * global stores (1) instead of shared-memory staging + TMA stores (0, default); key 9: batch chunk per recurrence cluster (16 / 32 /
- * 64; 0 = automatic); key 12: generic tensor-core decoder step fused (1, default: one launch per stacked-cell layer + a cluster of CTAs
- * per utterance for the attention) or as separate GEMM / cell / operand kernels with one attention CTA per utterance (0); key 13: CTAs per
- * utterance of that attention cluster (1 / 2 / 4 / 8; 0 = by batch size); key 15: M = 64 (1, default) or M = 128 (0) MMAs in the fused cell
- * kernel; key 16: programmatic dependent launch between the fused step's kernels (1, default) or plain stream order (0); key 18: the last
- * layer's kernel triggers the attention kernel at its start (1, default) or after its own dependency (0); key 19: two utterance groups
- * pipelined through the persistent decoder's LSTM CTAs (1, default) or the whole batch in lockstep (0); keys 20 + l: decoder steps of the serving pipeline's segment l (0 = proportional to the layer's time steps). */
+/* Process-wide switches for tests and measurements.  Returns LAS_EINVAL (las_last_error names the key) for a key not listed
+ * here or a value outside the key's set.
+ *   key 2:  decoder context through tensor memory (1, default: all feature tiles when they fit, otherwise as many as fit + the rest
+ *           on the CUDA cores) or on the CUDA cores only (0);
+ *   key 5:  persistent decoder LSTM CTAs in the weights-stationary form with one 3-D TMA copy per activation part (0, default where
+ *           Hs is a multiple of 64) or with shared-memory operands and one 2-D copy per 64-column atom (1);
+ *   key 6:  listener input-projection GEMM concurrent with the recurrence (1, default) or in front of it (0);
+ *   key 8:  tcgen05 GEMM epilogue with row-per-thread global stores (1) instead of shared-memory staging + TMA stores (0, default);
+ *   key 9:  batch chunk per recurrence cluster (16 / 32 / 64; 0 = automatic);
+ *   key 11: long encoders attended by a cluster of two CTAs per utterance where one CTA's tensor memory cannot hold enc[b]^T (1,
+ *           default) or never (0);
+ *   key 12: generic tensor-core decoder step fused (1, default: one launch per stacked-cell layer + a cluster of CTAs per utterance
+ *           for the attention) or as separate GEMM / cell / operand kernels with one attention CTA per utterance (0);
+ *   key 13: CTAs per utterance of that attention cluster (1 / 2 / 4 / 8; 0 = by batch size);
+ *   key 19: two utterance groups pipelined through the persistent decoder's LSTM CTAs (1, default) or the whole batch in lockstep (0);
+ *   keys 20 + l (l < 8): decoder steps of the serving pipeline's segment l (>= 0; 0 = proportional to the layer's time steps). */
 int las_debug_set_option(int key, int value);
 
 #ifdef __cplusplus

@@ -297,8 +297,10 @@ bool tma_store_ok(const float* C, long long ldc, int N, const uint32_t* flags) {
 
 }  // namespace
 
-void fast_set_option_gemm(int key, int value) {
-  if (key == 8) g_gemm_direct_store = value;
+bool fast_set_option_gemm(int key, int value) {
+  if (key != 8 || (value != 0 && value != 1)) return false;
+  g_gemm_direct_store = value;
+  return true;
 }
 
 int make_tmap_bf16_box(CUtensorMap* tm, const void* base, long long rows, long long cols, long long ld, int box_rows) {

@@ -4,7 +4,7 @@
 //   * one thread-block CLUSTER per (direction, batch chunk of Bc utterances); forward and backward directions and
 //     all batch chunks run concurrently in one launch;
 //   * the cluster's CS CTAs split the hidden units 32 per CTA; each CTA keeps its [4 gates x 32 units, H] slice of
-//     W_hh (bf16) resident in shared memory for the whole sequence, as the A operand of a "swap-AB" UMMA:
+//     W_hh (bf16) resident in tensor memory for the whole sequence, as the A operand of a "swap-AB" UMMA:
 //         D[128 gate rows, Bc] (TMEM, fp32) = W_slice[128, H] . h_{t-1}^T[H, Bc]
 //   * h_{t-1} (bf16, the B operand) lives in every CTA's shared memory; after the gate math each CTA pushes its
 //     32-unit slice of h_t into all CS CTAs' buffers with st.shared::cluster (DSMEM) and arrives on their mbarriers;
@@ -35,12 +35,11 @@ struct RecParams {
   const float* P;               // [Tl*Bp, NP] fp32, time-major: row = t*Bp + b; column = dir*4Hp + r*128 + jj*4 + gate
   const uint32_t* gemm_flags;   // nullable [m_tiles * n_tiles]: the GEMM's per-tile completion counters (4 = tile stored)
   int Bp, n_tiles;              // padded batch (rows per time step of P); column tiles of the GEMM
-  const uint8_t* whh_img;       // [2][CS] shared-memory images of the W_hh slices (128 x Hp bf16, INTERLEAVE layout)
+  const uint8_t* whh_img;       // [2][CS] images of the W_hh slices (128 x Hp bf16, INTERLEAVE layout), copied to tensor memory
   float* out_f32;               // nullable [B, Tl, 2H]
   __nv_bfloat16* out_bf16;      // nullable [B, Tl, 2H]
   const int32_t* lengths;       // nullable [B]: valid steps of this layer (length-mask extension)
   int B, Tl, H, Hp, CS, nchunks;
-  int a_tmem;                   // 1: W_hh slice lives in tensor memory (UMMA .ts form); 0: in shared memory
   long long* trace;             // nullable test hook: [64 steps][8] clock64 stamps from CTA 0
   // Fused input projection (layer 0, template FX): the K = 2F projection X.W_ih^T is never materialised.  Each step's folded frames
   // x_t [BC, Kx] arrive by TMA straight in the B-operand layout, W_ih's slice sits in tensor memory next to W_hh's, and the Kx/16
@@ -71,32 +70,27 @@ __host__ __device__ inline UmmaLayout whh_layout() { return UmmaLayout{0, 2048, 
 // h operand: Bc rows x Hp, INTERLEAVE: [coreK][coreN][8 rows][16 B]
 __host__ __device__ inline UmmaLayout h_layout(int Bc) { return UmmaLayout{0, (uint32_t)Bc * 16u, 128, 0}; }
 
-__host__ __device__ inline uint32_t rec_tmem_cols(int Hp, int BC, int a_tmem, int Kx = 0) {
+__host__ __device__ inline uint32_t rec_tmem_cols(int Hp, int BC, int Kx = 0) {
   // Kx > 0 (fused input projection): W_ih slice behind W_hh, and two accumulator sets (step s+1's input part is issued while the
   // epilogue still reads step s's)
-  uint32_t need = (uint32_t)BC * (Kx > 0 ? 2u : 1u) + (a_tmem ? (uint32_t)Hp / 2 : 0u) + (uint32_t)Kx / 2, c = 32;
+  uint32_t need = (uint32_t)BC * (Kx > 0 ? 2u : 1u) + (uint32_t)Hp / 2 + (uint32_t)Kx / 2, c = 32;
   while (c < need) c <<= 1;
   return c;
 }
 
 constexpr int XSLOTS = 4;  // ring of x_t tiles (fused input projection)
 
-template <int BC, int NACC, bool FX>
+template <int BC, bool FX>
 __global__ void __launch_bounds__(RecCfg<BC>::THREADS, 1) lstm_recurrence_cluster_kernel(const __grid_constant__ RecParams p) {
   constexpr int EPW = RecCfg<BC>::EPW;
   constexpr int REC_MMA_WARP = 4 * EPW, REC_POLL_WARP = 4 * EPW + 1, REC_EPI_THREADS = 4 * EPW * 32;
   constexpr int HB = BC / EPW;  // batch columns per epilogue warp (EPW warps share a TMEM lane quadrant)
   constexpr int NB = HB / 4;    // cells per epilogue thread
-  // The K loop can be spread round-robin over NACC independent accumulators that the epilogue sums (test hook:
-  // las_debug_set_option(4, n)).  tools/microbench.cu: a tcgen05.mma with the A operand in TMEM issues every ~33 cycles
-  // whatever N is and whether or not consecutive instructions share an accumulator, so NACC = 1 is the default.
   extern __shared__ uint8_t smem_raw[];
   uint8_t* base = smem_raw + ((1024u - (ptx::smem_u32(smem_raw) & 1023u)) & 1023u);  // offset from the __shared__ symbol keeps the address space
   const int Hp = p.Hp;
   const uint32_t a_bytes = 128u * Hp * 2u, h_bytes = (uint32_t)BC * Hp * 2u;
-  const uint32_t a_smem_bytes = p.a_tmem ? 0u : a_bytes;
-  uint8_t* sA = base;
-  uint8_t* sH0 = base + a_smem_bytes;                         // two h buffers of h_bytes each
+  uint8_t* sH0 = base;                                        // two h buffers of h_bytes each
   uint8_t* sStage = sH0 + 2 * h_bytes;                        // [2 parities] x (4 coreK x BC x 16 bytes)
   const uint32_t x_bytes = FX ? (uint32_t)BC * p.Kx * 2u : 0u;  // one x_t tile: [Kx/8][BC][8] bf16
   uint8_t* sX = sStage + 2 * 4 * BC * 16;                     // XSLOTS tiles (FX)
@@ -113,7 +107,7 @@ __global__ void __launch_bounds__(RecCfg<BC>::THREADS, 1) lstm_recurrence_cluste
   const int cluster_id = blockIdx.x / CS;
   const int dir = cluster_id / p.nchunks, chunk = cluster_id % p.nchunks;
   const int b_base = chunk * BC;
-  const uint32_t tcols = rec_tmem_cols(Hp, BC * NACC, p.a_tmem, FX ? p.Kx : 0);
+  const uint32_t tcols = rec_tmem_cols(Hp, BC, FX ? p.Kx : 0);
   const uint8_t* w_img = p.whh_img + ((size_t)dir * CS + r) * a_bytes;
 
   // ---- one-time setup: barriers, TMEM, resident W_hh slice
@@ -131,18 +125,13 @@ __global__ void __launch_bounds__(RecCfg<BC>::THREADS, 1) lstm_recurrence_cluste
     if (p.Tl > 2) ptx::mbar_arrive_expect_tx(&h_full[0], h_bytes);
   }
   if (warp == REC_MMA_WARP) ptx::tmem_alloc(tmem_slot, tcols);
-  if (!p.a_tmem) {
-    const uint4* src = reinterpret_cast<const uint4*>(w_img);
-    uint4* dst = reinterpret_cast<uint4*>(sA);
-    for (uint32_t i = threadIdx.x; i < a_bytes / 16; i += blockDim.x) dst[i] = src[i];
-  }
   ptx::fence_proxy_async();
   ptx::tc_fence_before();
   __syncthreads();
   ptx::tc_fence_after();
   const uint32_t tmem = *tmem_slot;
   // TMEM map: A operand (W_hh slice, lane = gate row, 2 bf16 per column) in columns [0, Hp/2), accumulator behind it
-  const uint32_t x_col = p.a_tmem ? (uint32_t)Hp / 2 : 0u;       // W_ih slice (FX): Kx/2 columns
+  const uint32_t x_col = (uint32_t)Hp / 2;                       // W_ih slice (FX): Kx/2 columns
   const uint32_t d_col = x_col + (FX ? (uint32_t)p.Kx / 2 : 0u);
   if (FX && warp < 4) {
     const __nv_bfloat16* wx = p.wih_img + ((size_t)(dir * CS + r) * 128 + threadIdx.x) * p.Kx;  // this lane's gate row
@@ -153,7 +142,7 @@ __global__ void __launch_bounds__(RecCfg<BC>::THREADS, 1) lstm_recurrence_cluste
     }
     ptx::tmem_st_wait();
   }
-  if (p.a_tmem && warp < 4) {
+  if (warp < 4) {
     const UmmaLayout la = whh_layout();
     const int row = threadIdx.x;
     for (int k0 = 0; k0 < Hp; k0 += 16) {
@@ -174,9 +163,8 @@ __global__ void __launch_bounds__(RecCfg<BC>::THREADS, 1) lstm_recurrence_cluste
     // ================================ MMA issuer ================================
     // The whole warp walks the loop with warp-uniform values (descriptors end up in uniform registers); only the
     // tcgen05 / mbarrier-arrive instructions are predicated on one elected lane.
-    const UmmaLayout la = whh_layout(), lb = h_layout(BC);
+    const UmmaLayout lb = h_layout(BC);
     const uint32_t idesc = umma_idesc_bf16(128, BC, p.f16);
-    const uint32_t a_addr = ptx::smem_u32(sA);
     const uint32_t h0_addr = ptx::smem_u32(sH0);
     const uint32_t x0_addr = ptx::smem_u32(sX);
     // x_t tile of processing step `st` -> ring slot st % XSLOTS (all CTAs of the cluster read the same tile; it stays in L2)
@@ -198,7 +186,7 @@ __global__ void __launch_bounds__(RecCfg<BC>::THREADS, 1) lstm_recurrence_cluste
     }
     __syncwarp();
     for (int s = FX ? 0 : 1; s < Tl; ++s) {
-      const uint32_t acc = tmem + d_col + (FX ? (uint32_t)(s & 1) * (BC * NACC) : 0u);
+      const uint32_t acc = tmem + d_col + (FX ? (uint32_t)(s & 1) * BC : 0u);
       if (FX) {
         // input part of step s: x_t . W_ih^T into a fresh accumulator, issued before h_{s-1} is here
         ptx::mbar_wait(&x_full[s % XSLOTS], (uint32_t)((s / XSLOTS) & 1));
@@ -224,32 +212,19 @@ __global__ void __launch_bounds__(RecCfg<BC>::THREADS, 1) lstm_recurrence_cluste
       const uint32_t b_addr = h0_addr + (uint32_t)(s & 1) * h_bytes;
       if (ptx::elect_one()) {
         if (s + 2 < Tl) ptx::mbar_arrive_expect_tx(&h_full[s & 1], h_bytes);  // re-arm for step s+2
-        if (p.a_tmem) {
-          if constexpr (NACC == 1) {
-            // Lean issue loop: the issuing thread's own instructions between two tcgen05.mma pace the chain (~40 cycles per
-            // instruction with the descriptor rebuilt each time, ~27 in tools/microbench_mma_insitu.cu's lean loop).  Consecutive K
-            // steps are 8 tensor-memory columns and two core-matrix columns (2 * BC * 16 bytes) apart, so both operands advance by
-            // constants (the descriptor's 14-bit address field cannot carry: shared memory ends below 256 KB).
-            uint64_t bd = umma_smem_desc(lb, b_addr, 0);
-            uint32_t a = tmem;
-            ptx::umma_bf16_ts(acc, a, bd, idesc, FX ? 1u : 0u);
+        // Lean issue loop, one accumulator chain: the issuing thread's own instructions between two tcgen05.mma pace the chain (~40
+        // cycles per instruction with the descriptor rebuilt each time, ~27 in tools/microbench_mma_insitu.cu's lean loop).  Consecutive
+        // K steps are 8 tensor-memory columns and two core-matrix columns (2 * BC * 16 bytes) apart, so both operands advance by
+        // constants (the descriptor's 14-bit address field cannot carry: shared memory ends below 256 KB).  Every chunk size BC
+        // accumulates in this one order, so an utterance's result does not depend on how its batch is sharded.
+        uint64_t bd = umma_smem_desc(lb, b_addr, 0);
+        uint32_t a = tmem;
+        ptx::umma_bf16_ts(acc, a, bd, idesc, FX ? 1u : 0u);
 #pragma unroll 4
-            for (int ki = 1; ki < Hp / 16; ++ki) {
-              a += 8;
-              bd += 2 * BC;
-              ptx::umma_bf16_ts(acc, a, bd, idesc, 1u);
-            }
-          } else {
-#pragma unroll 4
-            for (int ki = 0; ki < Hp / 16; ++ki)
-              ptx::umma_bf16_ts(acc + (ki % NACC) * BC, tmem + ki * 8, umma_smem_desc(lb, b_addr, ki * 16), idesc,
-                                (FX && (ki % NACC) == 0) ? 1u : (uint32_t)(ki >= NACC));
-          }
-        } else {
-#pragma unroll 4
-          for (int ki = 0; ki < Hp / 16; ++ki)
-            ptx::umma_bf16(acc + (ki % NACC) * BC, umma_smem_desc(la, a_addr, ki * 16), umma_smem_desc(lb, b_addr, ki * 16), idesc,
-                           (FX && (ki % NACC) == 0) ? 1u : (uint32_t)(ki >= NACC));
+        for (int ki = 1; ki < Hp / 16; ++ki) {
+          a += 8;
+          bd += 2 * BC;
+          ptx::umma_bf16_ts(acc, a, bd, idesc, 1u);
         }
         ptx::umma_commit(mma_done);
         // the MMAs of step s-1 are complete (h_s could not have arrived otherwise): its x slot takes the tile of step s + XSLOTS - 1
@@ -359,19 +334,11 @@ __global__ void __launch_bounds__(RecCfg<BC>::THREADS, 1) lstm_recurrence_cluste
         ptx::tc_fence_after();
         constexpr int LDW = HB < 16 ? HB : 16;  // columns per tcgen05.ld
 #pragma unroll
-        for (int a = 0; a < NACC; ++a) {
-          if (a == 0 || (a < Hp / 16 && s > 0)) {  // accumulator `a` was written this step (Hp = 32 has only two K steps; FX step 0: only a = 0)
-#pragma unroll
-            for (int c0 = 0; c0 < HB; c0 += LDW) {
-              uint32_t t[LDW];
-              const uint32_t addr = tmem + ((uint32_t)(wq * 32) << 16) + d_col + (FX ? (uint32_t)(s & 1) * (BC * NACC) : 0u) + a * BC + hb * HB + c0;
-              if constexpr (LDW == 16) ptx::tmem_ld_32x32b_x16(addr, *reinterpret_cast<uint32_t(*)[16]>(t));
-              else ptx::tmem_ld_32x32b_x8(addr, *reinterpret_cast<uint32_t(*)[8]>(t));
-              ptx::tmem_ld_wait();
-#pragma unroll
-              for (int i = 0; i < LDW; ++i) v[c0 + i] = (a == 0) ? t[i] : __float_as_uint(__uint_as_float(v[c0 + i]) + __uint_as_float(t[i]));
-            }
-          }
+        for (int c0 = 0; c0 < HB; c0 += LDW) {
+          const uint32_t addr = tmem + ((uint32_t)(wq * 32) << 16) + d_col + (FX ? (uint32_t)(s & 1) * BC : 0u) + hb * HB + c0;
+          if constexpr (LDW == 16) ptx::tmem_ld_32x32b_x16(addr, *reinterpret_cast<uint32_t(*)[16]>(v + c0));
+          else ptx::tmem_ld_32x32b_x8(addr, *reinterpret_cast<uint32_t(*)[8]>(v + c0));
+          ptx::tmem_ld_wait();
         }
         ptx::tc_fence_before();
       } else {
@@ -493,7 +460,6 @@ __global__ void pack_whh_kernel(const float* w_fwd, const float* w_rev, uint8_t*
 }
 
 long long* g_rec_trace = nullptr;  // set through las_debug_set_trace (test hook)
-int g_rec_gemm_ctas = 0;           // las_debug_set_option(7, v): persistent CTAs of the overlapped GEMM (0 = all SMs the recurrence leaves free)
 int g_rec_overlap = 1;             // las_debug_set_option(6, v): run each layer's input-projection GEMM concurrently with its recurrence
 
 // Side stream on which a layer's input-projection GEMM runs while the recurrence consumes its tiles on the caller's
@@ -523,10 +489,7 @@ int side_stream(SideStream** out) {
   *out = &g_side;
   return LAS_OK;
 }
-int g_rec_a_tmem = 1;              // las_debug_set_option(1, v)
-int g_rec_fuse_x = 1;              // las_debug_set_option(10, v): layer 0's input projection fused into its recurrence (1, default) or a GEMM (0)
 int g_rec_force_bc = 0;            // las_debug_set_option(9, v): batch chunk per recurrence cluster (0 = pick_bc)
-int g_rec_nacc = 0;                // las_debug_set_option(4, v): independent accumulators the K loop is spread over (0 = default)
 
 struct Geo {
   int Hp, CS;
@@ -600,15 +563,15 @@ int shape_ok(const las_listener_dims* d) {
   return LAS_OK;
 }
 
-template <int BC, int NACC, bool FX>
+template <int BC, bool FX>
 int launch_rec(const RecParams& p, cudaStream_t st, bool exclusive_sm) {
-  size_t smem = 1024 + (p.a_tmem ? 0u : 128u * p.Hp * 2) + 2u * BC * p.Hp * 2 + 2 * 4 * BC * 16 + (FX ? XSLOTS * (size_t)BC * p.Kx * 2 : 0) + 128;
+  size_t smem = 1024 + 2u * BC * p.Hp * 2 + 2 * 4 * BC * 16 + (FX ? XSLOTS * (size_t)BC * p.Kx * 2 : 0) + 128;
   // While the GEMM runs concurrently, a GEMM CTA (197 KB of shared memory, all 512 TMEM columns) must never land on an SM that
   // hosts a recurrence CTA (it would wait for tensor memory held by a CTA that waits for the GEMM's tiles): ask for enough
   // shared memory that the two cannot be co-resident.
   if (exclusive_sm && smem < 48 * 1024) smem = 48 * 1024;
-  LAS_CUDA_OK(cudaFuncSetAttribute(lstm_recurrence_cluster_kernel<BC, NACC, FX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  if (p.CS > 8) LAS_CUDA_OK(cudaFuncSetAttribute(lstm_recurrence_cluster_kernel<BC, NACC, FX>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+  LAS_CUDA_OK(cudaFuncSetAttribute(lstm_recurrence_cluster_kernel<BC, FX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  if (p.CS > 8) LAS_CUDA_OK(cudaFuncSetAttribute(lstm_recurrence_cluster_kernel<BC, FX>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(p.CS * 2 * p.nchunks);
   cfg.blockDim = dim3(p.gemm_flags ? RecCfg<BC>::THREADS : RecCfg<BC>::THREADS - 32);  // the watcher warp exists only next to a concurrent GEMM
@@ -621,7 +584,7 @@ int launch_rec(const RecParams& p, cudaStream_t st, bool exclusive_sm) {
   at[0].val.clusterDim.z = 1;
   cfg.attrs = at;
   cfg.numAttrs = 1;
-  LAS_CUDA_OK(cudaLaunchKernelEx(&cfg, lstm_recurrence_cluster_kernel<BC, NACC, FX>, p));
+  LAS_CUDA_OK(cudaLaunchKernelEx(&cfg, lstm_recurrence_cluster_kernel<BC, FX>, p));
   count_launch();
   return LAS_OK;
 }
@@ -632,19 +595,14 @@ int launch_rec(const RecParams& p, cudaStream_t st, bool exclusive_sm) {
 
 void fast_set_trace(long long* p) { g_rec_trace = p; }
 long long* fast_get_trace() { return g_rec_trace; }
-void fast_set_option_speller(int key, int value);
-void fast_set_option_gemm(int key, int value);  // fast_gemm.cu: 8 = direct-store epilogue
-void fast_set_option(int key, int value) {
-  if (key == 1) g_rec_a_tmem = value;
-  if (key == 4) g_rec_nacc = value;
-  if (key == 6) g_rec_overlap = value;
-  if (key == 7) g_rec_gemm_ctas = value;
-  if (key == 9) g_rec_force_bc = value;
-  if (key == 10) g_rec_fuse_x = value;
-  fast_set_option_speller(key, value);
-  fast_set_option_gemm(key, value);
-  fast_set_option_pipeline(key, value);
-  fast_set_option_gen(key, value);
+bool fast_set_option_speller(int key, int value);
+bool fast_set_option_gemm(int key, int value);  // fast_gemm.cu: 8 = direct-store epilogue
+bool fast_set_option(int key, int value) {
+  if (key == 6 && (value == 0 || value == 1)) g_rec_overlap = value;
+  else if (key == 9 && (value == 0 || value == 16 || value == 32 || value == 64)) g_rec_force_bc = value;
+  else return fast_set_option_speller(key, value) || fast_set_option_gemm(key, value) || fast_set_option_pipeline(key, value) ||
+              fast_set_option_gen(key, value);
+  return true;
 }
 
 // Does the cluster-resident recurrence cover this model?  (Otherwise las_api.cu runs the generic path: tensor-core input projection,
@@ -704,7 +662,6 @@ static RecParams rec_params(const las_listener_dims* d, const Geo& g, const List
   rp.lengths = len_l;
   rp.B = d->B; rp.Tl = q.Tl; rp.H = d->H; rp.Hp = g.Hp; rp.CS = g.CS;
   rp.trace = (l == 0) ? g_rec_trace : nullptr;
-  rp.a_tmem = g_rec_a_tmem;
   rp.nchunks = (d->B + bc - 1) / bc;
   rp.resident = nullptr;
   rp.f16 = op_f16();
@@ -724,24 +681,17 @@ static int rec_fuse(RecParams& rp, const las_listener_dims* d, const ListenerPac
 }
 static int launch_rec_bc(const RecParams& rp, int bc, cudaStream_t st, bool exclusive) {
   if (rp.Kx > 0) {  // fused input projection (layer 0)
-    if (bc == 16) return launch_rec<16, 1, true>(rp, st, exclusive);
-    if (bc == 32) return launch_rec<32, 1, true>(rp, st, exclusive);
-    return launch_rec<64, 1, true>(rp, st, exclusive);
+    if (bc == 16) return launch_rec<16, true>(rp, st, exclusive);
+    if (bc == 32) return launch_rec<32, true>(rp, st, exclusive);
+    return launch_rec<64, true>(rp, st, exclusive);
   }
-  if (bc == 16) {
-    const int nacc = g_rec_nacc ? g_rec_nacc : 1;  // measured: one accumulator chain is fastest with the A operand in TMEM
-    if (nacc == 1) return launch_rec<16, 1, false>(rp, st, exclusive);
-    if (nacc == 2) return launch_rec<16, 2, false>(rp, st, exclusive);
-    return launch_rec<16, 4, false>(rp, st, exclusive);
-  }
-  // one accumulator chain for every chunk size: an utterance's result must not depend on how its batch is sharded (the chunk size
-  // follows the batch size), so all variants accumulate in the same order
-  if (bc == 32) return launch_rec<32, 1, false>(rp, st, exclusive);
-  return launch_rec<64, 1, false>(rp, st, exclusive);
+  if (bc == 16) return launch_rec<16, false>(rp, st, exclusive);
+  if (bc == 32) return launch_rec<32, false>(rp, st, exclusive);
+  return launch_rec<64, false>(rp, st, exclusive);
 }
 
-// layer l's input projection can be fused when the A operand is in tensor memory and K = 2F splits into 16-wide MMA steps
-static bool fuse_x(const las_listener_dims* d, int l) { return l == 0 && g_rec_fuse_x && g_rec_a_tmem && (2 * d->F) % 16 == 0 && 2 * d->F <= 256; }
+// layer l's input projection can be fused when K = 2F splits into 16-wide MMA steps
+static bool fuse_x(const las_listener_dims* d, int l) { return l == 0 && (2 * d->F) % 16 == 0 && 2 * d->F <= 256; }
 
 // CTAs the recurrence of this model occupies with batch chunk `bc`
 int fast_listener_rec_ctas(const las_listener_dims* d, int bc) {
@@ -819,7 +769,7 @@ int fast_listener_forward(const float* x, const int32_t* x_lengths, const void* 
       continue;
     }
     const int rec_ctas = 2 * rp.nchunks * g.CS;
-    const int gemm_ctas = g_rec_gemm_ctas > 0 ? g_rec_gemm_ctas : sm_count() - rec_ctas - 4;
+    const int gemm_ctas = sm_count() - rec_ctas - 4;
     const bool overlap = g_rec_overlap && ((q.NP / 2) % 256 == 0) && gemm_ctas >= 32;
     SideStream* side = nullptr;
     if (overlap) LAS_TRY(side_stream(&side));

@@ -65,8 +65,10 @@ int g_pipe_split[8] = {0};  // las_debug_set_option(20 + l, steps): decoder step
 
 }  // namespace
 
-void fast_set_option_pipeline(int key, int value) {
-  if (key >= 20 && key < 28) g_pipe_split[key - 20] = value;
+bool fast_set_option_pipeline(int key, int value) {
+  if (key < 20 || key >= 28 || value < 0) return false;
+  g_pipe_split[key - 20] = value;
+  return true;
 }
 
 // Can the listener of `ld` run next to the decoder of `sd`?  Returns the recurrence's batch chunk (16 / 32 / 64) or 0.

@@ -52,9 +52,8 @@ struct DecParams {
   CUtensorMap tm_h[MAX_SL][2];  // hbuf[l][parity]  bf16 [B, Hs]
   CUtensorMap tm_x[2];          // xbuf[parity]     bf16 [B, E]   the context fed to layer 0 (same pitch as an h buffer)
   CUtensorMap tm_w[2];          // wbuf[parity]     bf16 [B, VP]  the dense word fed to layer 0 (one atom)
-  CUtensorMap tm_h3[MAX_SL][2]; // the same buffers as {64 k, B, atoms}: one copy brings a whole activation part (tma3d)
+  CUtensorMap tm_h3[MAX_SL][2]; // the same buffers as {64 k, B, atoms}: one copy brings a whole activation part (lstm_role_ts)
   CUtensorMap tm_x3[2];
-  int tma3d;                    // 1: Hs and E are multiples of 64, every part is ONE 3-D copy completing on full[0]
   const uint8_t* w_img[MAX_SL]; // [ncl][atoms_l] swizzled 64x64 bf16 atoms: h part, (layer 0: word atom), input part
   const float* bias[MAX_SL];    // [ncl*64] b_ih + b_hh in CTA column order
   __nv_bfloat16* hbuf[MAX_SL][2];
@@ -95,11 +94,10 @@ struct DecParams {
   int b0;
   int U, E, Hs, sl, V, D, steps, decode_mode, relu, gt_steps, ncl, k_in_smem;
   int wreg;  // 1: every attention thread keeps its chunks of W_phi in registers (D <= 64, Hs <= 512); no shared-memory copy
-  int ab_flags;     // test hook (las_debug_set_option(5, v)): bit 0 = W_phi from shared memory instead of registers; bit 2 (value 4) = eight 2-D copies per activation part instead of one 3-D copy; bit 5 (value 32) = query GEMV after a CTA-wide barrier (8 lanes per output) instead of per-warp partials; bit 6 (value 64) = LSTM epilogue stores one row per thread from the registers instead of staging + coalesced rows; bit 9 (value 512) = context UMMA descriptors rebuilt per instruction instead of advanced by constants
   unsigned long long sample_seed;  // LAS_DECODE_SAMPLE
   int word_gather;  // 1: the fed-back word is an index (greedy argmax / gt_index); 0: a dense vector (part 1b)
   int f16;          // GEMM operand format: 0 = bf16 (LAS_MODE_BF16), 1 = IEEE fp16 (LAS_MODE_F16)
-  int lstm_ts;      // 1: LSTM CTAs use the weights-stationary operand roles (lstm_role_ts); 0: lstm_role
+  int lstm_ts;      // 1: LSTM CTAs use the weights-stationary operand roles and one 3-D copy per part (lstm_role_ts); 0: lstm_role
   int att_split;    // 2: every utterance is attended by a CLUSTER of two CTAs, each holding half of the encoder steps (long encoders:
                     // all of enc[b]^T stays in tensor memory; partial softmax / context combined through DSMEM); 1: one CTA
   int ctx_tmem;     // > 0: enc[b]^T is resident in the attention CTA's tensor memory and the context is a UMMA
@@ -264,25 +262,17 @@ __device__ void lstm_role(const DecParams& p, uint8_t* smem, int l, int nb) {
       __syncwarp();
       fence_proxy_async_global();  // other SMs' generic-proxy stores (acquired above) -> this warp's TMA reads
       if (ptx::elect_one()) {
-        if (p.tma3d) {
-          ptx::mbar_arrive_expect_tx(&full[0], nh * STAGE_BYTES);
-          ptx::tma_load_3d(abuf, &p.tm_h3[l][par], &full[0], 0, 0, 0);
-        } else {
-          for (int i = 0; i < nh; ++i) {
-            ptx::mbar_arrive_expect_tx(&full[i], STAGE_BYTES);
-            ptx::tma_load_2d(abuf + (size_t)i * STAGE_BYTES, &p.tm_h[l][par], &full[i], i * 64, 0);
-          }
+        for (int i = 0; i < nh; ++i) {
+          ptx::mbar_arrive_expect_tx(&full[i], STAGE_BYTES);
+          ptx::tma_load_2d(abuf + (size_t)i * STAGE_BYTES, &p.tm_h[l][par], &full[i], i * 64, 0);
         }
       }
       __syncwarp();
       // ---- part 1a: context of step s-1 (layer 0) / the lower layer's h of THIS step
       ptx::mbar_wait(part_empty, (uint32_t)((n - 1) & 1));
       ++n;
-      if (ptx::elect_one()) {  // slots are free: arm their barriers now, so that only the copies are left to issue once the input is there
-        if (p.tma3d) ptx::mbar_arrive_expect_tx(&full[0], nc * STAGE_BYTES);
-        else
-          for (int i = 0; i < nc; ++i) ptx::mbar_arrive_expect_tx(&full[i], STAGE_BYTES);
-      }
+      if (ptx::elect_one())  // slots are free: arm their barriers now, so that only the copies are left to issue once the input is there
+        for (int i = 0; i < nc; ++i) ptx::mbar_arrive_expect_tx(&full[i], STAGE_BYTES);
       __syncwarp();
       if (lane == 0) {
         wait_counter(in_ctr, first ? (uint32_t)s * p.B : (uint32_t)(s + 1) * p.ncl);
@@ -294,13 +284,8 @@ __device__ void lstm_role(const DecParams& p, uint8_t* smem, int l, int nb) {
       if (lane == 0 && trole >= 0) DEC_TRACE(4, 6 + trole);
       {
         const CUtensorMap* tm = first ? &p.tm_x[par] : &p.tm_h[l - 1][par ^ 1];
-        const CUtensorMap* tm3 = first ? &p.tm_x3[par] : &p.tm_h3[l - 1][par ^ 1];
-        if (ptx::elect_one()) {
-          // one instruction for the whole part: issuing eight 2-D copies took ~0.55 us (~68 ns each), all of it on the critical path
-          if (p.tma3d) ptx::tma_load_3d(abuf, tm3, &full[0], 0, 0, 0);
-          else
-            for (int i = 0; i < nc; ++i) ptx::tma_load_2d(abuf + (size_t)i * STAGE_BYTES, tm, &full[i], i * 64, 0);
-        }
+        if (ptx::elect_one())
+          for (int i = 0; i < nc; ++i) ptx::tma_load_2d(abuf + (size_t)i * STAGE_BYTES, tm, &full[i], i * 64, 0);
         __syncwarp();
       }
       if (lane == 0 && trole >= 0) DEC_TRACE(trole, 1);
@@ -333,9 +318,8 @@ __device__ void lstm_role(const DecParams& p, uint8_t* smem, int l, int nb) {
         // rate the tensor pipe accepts).  Issuing box by box as they land is slower: MMAs issued while later boxes are
         // still being written into shared memory slow both down (measured per group size 1 / 2 / 4 / all boxes:
         // 15.3 / 14.8 / 14.3 / 14.2 us per step, profiles/r01_decoder_issue_groups.log).
-        const int nwait = p.tma3d ? 1 : na;
-        for (int i = 0; i < nwait; ++i) ptx::mbar_wait(&full[i], (phase_bits >> i) & 1u);
-        phase_bits ^= (1u << nwait) - 1u;
+        for (int i = 0; i < na; ++i) ptx::mbar_wait(&full[i], (phase_bits >> i) & 1u);
+        phase_bits ^= (1u << na) - 1u;
         ptx::tc_fence_after();
         if (part == 1 && lane == 0 && trole >= 0) DEC_TRACE(4, 3 + 2 * trole);  // critical part landed
         if (ptx::elect_one()) {
@@ -430,59 +414,44 @@ __device__ void lstm_role(const DecParams& p, uint8_t* smem, int l, int nb) {
       ptx::tc_fence_before();
       ptx::mbar_arrive(tmem_empty);
       const int np = (s + 1) & 1;
-      if (!(p.ab_flags & 64)) {
-        // Coalesced hand-off stores.  A thread owns one batch row, so a warp-wide store of its values touches 32 different
-        // rows of the row-major hand-off buffers (32 partial sectors per instruction; the top layer's flag-in-data slots took
-        // up to ~1.4 us to become visible).  The 64 x 16 block goes through shared memory instead (rows padded to 20 floats:
-        // conflict-free 16-byte writes) and every warp writes 8 whole rows: full 128-byte lines of {h, tag} slots for the
-        // attention CTAs, full 32-byte sectors of the bf16 operand copy.
-        if (warp_live) *reinterpret_cast<float4*>(s_st + b * 20 + cs * 4) = make_float4(h[0], h[1], h[2], h[3]);
-        asm volatile("bar.sync 1, 256;" ::: "memory");
-        const int r0 = (cs * 2 + q) * 8;  // this warp's 8 rows
-        if (top) {
-          const uint32_t tag = (uint32_t)(s + 1);
+      // Coalesced hand-off stores.  A thread owns one batch row, so a warp-wide store of its values touches 32 different
+      // rows of the row-major hand-off buffers (32 partial sectors per instruction; the top layer's flag-in-data slots took
+      // up to ~1.4 us to become visible).  The 64 x 16 block goes through shared memory instead (rows padded to 20 floats:
+      // conflict-free 16-byte writes) and every warp writes 8 whole rows: full 128-byte lines of {h, tag} slots for the
+      // attention CTAs, full 32-byte sectors of the bf16 operand copy.
+      if (warp_live) *reinterpret_cast<float4*>(s_st + b * 20 + cs * 4) = make_float4(h[0], h[1], h[2], h[3]);
+      asm volatile("bar.sync 1, 256;" ::: "memory");
+      const int r0 = (cs * 2 + q) * 8;  // this warp's 8 rows
+      if (top) {
+        const uint32_t tag = (uint32_t)(s + 1);
 #pragma unroll
-          for (int hf = 0; hf < 2; ++hf) {
-            const int row = r0 + hf * 4 + (lane >> 3), piece = lane & 7;
-            if (row < p.B) {
-              const float2 v = *reinterpret_cast<const float2*>(s_st + row * 20 + piece * 2);
-              ll_store2(p.h_ll + (size_t)row * p.Hs + nb * DEC_UNITS + piece * 2, ll_pack(__float_as_uint(v.x), tag), ll_pack(__float_as_uint(v.y), tag));
-            }
-          }
-        }
-        if (lane < 16) {
-          const int row = r0 + (lane >> 1), hf = lane & 1;
+        for (int hf = 0; hf < 2; ++hf) {
+          const int row = r0 + hf * 4 + (lane >> 3), piece = lane & 7;
           if (row < p.B) {
-            const float4 x0 = *reinterpret_cast<const float4*>(s_st + row * 20 + hf * 8), x1 = *reinterpret_cast<const float4*>(s_st + row * 20 + hf * 8 + 4);
-            const __nv_bfloat162 t0 = op2_from_f32(x0.x, x0.y, F16), t1 = op2_from_f32(x0.z, x0.w, F16);
-            const __nv_bfloat162 t2 = op2_from_f32(x1.x, x1.y, F16), t3 = op2_from_f32(x1.z, x1.w, F16);
-            *reinterpret_cast<uint4*>(p.hbuf[l][np] + (size_t)row * p.Hs + nb * DEC_UNITS + hf * 8) =
-                make_uint4(*reinterpret_cast<const uint32_t*>(&t0), *reinterpret_cast<const uint32_t*>(&t1),
-                           *reinterpret_cast<const uint32_t*>(&t2), *reinterpret_cast<const uint32_t*>(&t3));
+            const float2 v = *reinterpret_cast<const float2*>(s_st + row * 20 + piece * 2);
+            ll_store2(p.h_ll + (size_t)row * p.Hs + nb * DEC_UNITS + piece * 2, ll_pack(__float_as_uint(v.x), tag), ll_pack(__float_as_uint(v.y), tag));
           }
         }
       }
-      if (live) {
-        if (p.ab_flags & 64) {  // A/B: one row per thread, straight from the registers
-        if (top) {  // attention CTA b polls these slots directly
-          const uint32_t tag = (uint32_t)(s + 1);
-          u64* dst = p.h_ll + (size_t)b * p.Hs + u0;
-          ll_store2(dst, ll_pack(__float_as_uint(h[0]), tag), ll_pack(__float_as_uint(h[1]), tag));
-          ll_store2(dst + 2, ll_pack(__float_as_uint(h[2]), tag), ll_pack(__float_as_uint(h[3]), tag));
+      if (lane < 16) {
+        const int row = r0 + (lane >> 1), hf = lane & 1;
+        if (row < p.B) {
+          const float4 x0 = *reinterpret_cast<const float4*>(s_st + row * 20 + hf * 8), x1 = *reinterpret_cast<const float4*>(s_st + row * 20 + hf * 8 + 4);
+          const __nv_bfloat162 t0 = op2_from_f32(x0.x, x0.y, F16), t1 = op2_from_f32(x0.z, x0.w, F16);
+          const __nv_bfloat162 t2 = op2_from_f32(x1.x, x1.y, F16), t3 = op2_from_f32(x1.z, x1.w, F16);
+          *reinterpret_cast<uint4*>(p.hbuf[l][np] + (size_t)row * p.Hs + nb * DEC_UNITS + hf * 8) =
+              make_uint4(*reinterpret_cast<const uint32_t*>(&t0), *reinterpret_cast<const uint32_t*>(&t1),
+                         *reinterpret_cast<const uint32_t*>(&t2), *reinterpret_cast<const uint32_t*>(&t3));
         }
-        const __nv_bfloat162 t0 = op2_from_f32(h[0], h[1], F16), t1 = op2_from_f32(h[2], h[3], F16);
-        *reinterpret_cast<uint2*>(p.hbuf[l][np] + (size_t)b * p.Hs + u0) =
-            make_uint2(*reinterpret_cast<const uint32_t*>(&t0), *reinterpret_cast<const uint32_t*>(&t1));
+      }
+      if (live && s == S - 1) {
+        if (p.h_out) {
+#pragma unroll
+          for (int i = 0; i < 4; ++i) p.h_out[((size_t)l * p.Bfull + gb) * p.Hs + u0 + i] = h[i];
         }
-        if (s == S - 1) {
-          if (p.h_out) {
+        if (p.c_out) {
 #pragma unroll
-            for (int i = 0; i < 4; ++i) p.h_out[((size_t)l * p.Bfull + gb) * p.Hs + u0 + i] = h[i];
-          }
-          if (p.c_out) {
-#pragma unroll
-            for (int i = 0; i < 4; ++i) p.c_out[((size_t)l * p.c_out_rows + p.c_out_b0 + b) * p.Hs + u0 + i] = c[i];
-          }
+          for (int i = 0; i < 4; ++i) p.c_out[((size_t)l * p.c_out_rows + p.c_out_b0 + b) * p.Hs + u0 + i] = c[i];
         }
       }
       if (lead && trole >= 0) DEC_TRACE(trole, 4);
@@ -624,6 +593,7 @@ __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
       {
         const CUtensorMap* tm3 = first ? &p.tm_x3[par] : &p.tm_h3[l - 1][par ^ 1];
         if (ptx::elect_one()) {
+          // one instruction for the whole part: issuing eight 2-D copies took ~0.55 us (~68 ns each), all of it on the critical path
           if (trole == 0 && grp == 0) DEC_TRACE(4, 0);
           ptx::tma_load_3d(abuf, tm3, &full[0], 0, row0, 0);
           if (trole == 0 && grp == 0) DEC_TRACE(4, 2);
@@ -801,10 +771,9 @@ __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
       ptx::mbar_arrive(tmem_empty);
       const int np = (s + 1) & 1;
       // hand-off: the 64 x 16 block through shared memory ([batch row][20 floats]), then whole rows per warp (as in lstm_role)
-      // top layer: the {h, tag} slots the attention CTAs poll leave straight from the registers, before the staging barrier (-0.11 us/step;
-      // ab_flags bit 15 restores the staged whole-row stores)
-      const bool direct_ll = top && !(p.ab_flags & 32768);
-      if (direct_ll && warp_live) {
+      // top layer: the {h, tag} slots the attention CTAs poll leave straight from the registers, before the staging barrier
+      // (0.11 us/step faster than staged whole-row stores)
+      if (top && warp_live) {
         const uint32_t tag = (uint32_t)(s + 1);
 #pragma unroll
         for (int m = 0; m < 4; ++m)
@@ -816,17 +785,6 @@ __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
       }
       asm volatile("bar.sync 1, 256;" ::: "memory");
       const int r0 = (cs * 2 + q) * 8;  // this warp's 8 rows
-      if (top && !direct_ll && warp_live) {
-        const uint32_t tag = (uint32_t)(s + 1);
-#pragma unroll
-        for (int hf = 0; hf < 2; ++hf) {
-          const int rw = r0 + hf * 4 + (lane >> 3), piece = lane & 7;
-          if (rw < p.B) {
-            const float2 v = *reinterpret_cast<const float2*>(s_st + rw * 20 + piece * 2);
-            ll_store2(p.h_ll + (size_t)rw * p.Hs + nb * DEC_UNITS + piece * 2, ll_pack(__float_as_uint(v.x), tag), ll_pack(__float_as_uint(v.y), tag));
-          }
-        }
-      }
       if (lane < 16 && warp_live) {
         const int rw = r0 + (lane >> 1), hf = lane & 1;
         if (rw < p.B) {
@@ -953,8 +911,7 @@ __device__ void attention_role(const DecParams& p, uint8_t* smem, int b, int ran
   uint8_t* s_bop = reinterpret_cast<uint8_t*>(s_tm + 4);     // [2*nks core-K][2][8 rows][16 B]: row 0 = scores (bf16)
   const int nks = (U + 15) / 16;                              // UMMA K steps over the encoder axis
   const int CU = nks * 8;                                     // TMEM columns of one 128-feature tile of enc^T
-  // warps issuing the context UMMAs, one chain of nks instructions per feature tile (ab_flags bit 10: a single issuer)
-  const int niss = (ntm == 0) ? 0 : ((p.ab_flags & 1024) ? 1 : (ntm < 4 ? ntm : 4));
+  const int niss = ntm < 4 ? ntm : 4;  // warps issuing the context UMMAs, one chain of nks instructions per feature tile
 
   if (!p.wreg)
     for (int i = tid; i < D * Hs; i += DEC_THREADS) s_wphi[(size_t)(i / Hs) * WPS + (i % Hs)] = p.w_phi[i];
@@ -1044,24 +1001,17 @@ __device__ void attention_role(const DecParams& p, uint8_t* smem, int b, int ran
   ptx::tc_fence_after();
 
   const int hchunks = Hs >> 3, kchunks = KC >> 3;  // 16-byte chunks (8 bf16) of a W_phi row / W_cd row
-  // W_phi in registers: thread (d = tid / 8, part = tid % 8) keeps the chunks part, part + 8, ... of row d (32 registers)
-  // for all S steps, so the query GEMV reads only h from shared memory (the 64 KB of W_phi would otherwise be half of
-  // the step's shared-memory wavefronts).  Falls back to the shared-memory copy for D > 64 or Hs > 512.
+  // W_phi in registers (D <= 64, Hs <= 512; otherwise the shared-memory copy): the query GEMV reads only h from shared memory (the
+  // 64 KB of W_phi would otherwise be half of the step's shared-memory wavefronts).  Per-warp query partials: warp w owns
+  // h[32w, 32w+32) -- the values it polls itself -- and lane l the outputs d = l and l + 32 (32 registers of W_phi), so a warp starts
+  // its share of the GEMV the moment ITS OWN 32 values have arrived (the layer-1 CTAs finish up to ~0.5 us apart) instead of after a
+  // CTA-wide barrier; the 16 partial sums per output are added after one barrier.
   const bool wreg = p.wreg != 0;
-  // Per-warp query partials (default with W_phi in registers): warp w owns h[32w, 32w+32) -- the values it polls itself -- and lane
-  // l the outputs d = l and l + 32, so a warp starts its share of the GEMV the moment ITS OWN 32 values have arrived (the layer-1
-  // CTAs finish up to ~0.5 us apart) instead of after a CTA-wide barrier; the 16 partial sums per output are added after one barrier.
-  const bool qwarp = wreg && !(p.ab_flags & 32);
   uint4 wq[8];
 #pragma unroll
   for (int j = 0; j < 8; ++j) {
-    if (qwarp) {
-      const int d = lane + 32 * (j >> 2), k = 32 * warp + 8 * (j & 3);
-      wq[j] = (d < D && k < Hs) ? *reinterpret_cast<const uint4*>(p.w_phi + (size_t)d * Hs + k) : make_uint4(0, 0, 0, 0);
-    } else {
-      const int d = tid >> 3, c = (tid & 7) + 8 * j;
-      wq[j] = (wreg && d < D && c < hchunks) ? *reinterpret_cast<const uint4*>(p.w_phi + (size_t)d * Hs + 8 * c) : make_uint4(0, 0, 0, 0);
-    }
+    const int d = lane + 32 * (j >> 2), k = 32 * warp + 8 * (j & 3);
+    wq[j] = (wreg && d < D && k < Hs) ? *reinterpret_cast<const uint4*>(p.w_phi + (size_t)d * Hs + k) : make_uint4(0, 0, 0, 0);
   }
   const int Dp = (D + 3) & ~3, Vp = (V + 1) & ~1;
   const int nd4 = (D + 3) >> 2;                    // float4 chunks of a psi row
@@ -1070,7 +1020,7 @@ __device__ void attention_role(const DecParams& p, uint8_t* smem, int b, int ran
     const int np = (s + 1) & 1;
     const bool last = (s == p.steps - 1);
     // ---- A: this step's top-layer h, polled straight out of the LSTM epilogue's flag-in-data slots
-    if (qwarp) {
+    if (wreg) {
       float hv = 0.f;
       if (tid < Hs) {
         hv = __uint_as_float(ll_wait(p.h_ll + (size_t)b * Hs + tid, (uint32_t)(s + 1)));
@@ -1103,49 +1053,35 @@ __device__ void attention_role(const DecParams& p, uint8_t* smem, int b, int ran
         }
       }
     } else {
-    if (tid < Hs) s_h[xpos(tid)] = __uint_as_float(ll_wait(p.h_ll + (size_t)b * Hs + tid, (uint32_t)(s + 1)));
-    __syncthreads();
-    if (tid == 0) DEC_TRACE_ALL(0);
-    if (tid == 0 && b == 0) { DEC_TRACE(2, 0); DEC_TRACE(3, 0); if (p.trace && s < 32) p.trace[(2 * 32 + s) * 8 + 7] = clock64(); }
+      if (tid < Hs) s_h[xpos(tid)] = __uint_as_float(ll_wait(p.h_ll + (size_t)b * Hs + tid, (uint32_t)(s + 1)));
+      __syncthreads();
+      if (tid == 0) DEC_TRACE_ALL(0);
+      if (tid == 0 && b == 0) { DEC_TRACE(2, 0); DEC_TRACE(3, 0); if (p.trace && s < 32) p.trace[(2 * 32 + s) * 8 + 7] = clock64(); }
 
-    // ---- B: q = act(W_phi . h + b_phi)   (model/las_model.py:278): 8 lanes per output, interleaved 16-byte chunks
-    {
-      const int part = tid & 7;
-      for (int d = tid >> 3; d < Dp; d += DEC_THREADS / 8) {
-        float acc = 0.f;
-        if (wreg) {
-          float acc2 = 0.f;
-#pragma unroll
-          for (int j = 0; j < 8; j += 2) {
-            if (part + 8 * j < hchunks) {
-              const float4* xv = xchunk(s_h, part + 8 * j);
-              acc = dot8(wq[j], xv[0], xv[8], acc, F16);
-            }
-            if (part + 8 * (j + 1) < hchunks) {
-              const float4* xv = xchunk(s_h, part + 8 * (j + 1));
-              acc2 = dot8(wq[j + 1], xv[0], xv[8], acc2, F16);
-            }
-          }
-          acc += acc2;
-        } else if (d < D) {
-          const uint4* wr = reinterpret_cast<const uint4*>(s_wphi + (size_t)d * WPS);
+      // ---- B: q = act(W_phi . h + b_phi)   (model/las_model.py:278): 8 lanes per output, interleaved 16-byte chunks
+      {
+        const int part = tid & 7;
+        for (int d = tid >> 3; d < Dp; d += DEC_THREADS / 8) {
+          float acc = 0.f;
+          if (d < D) {
+            const uint4* wr = reinterpret_cast<const uint4*>(s_wphi + (size_t)d * WPS);
 #pragma unroll 4
-          for (int c = part; c < hchunks; c += 8) {
-            const float4* xv = xchunk(s_h, c);
-            acc = dot8(lds128(wr + c), xv[0], xv[8], acc, F16);
+            for (int c = part; c < hchunks; c += 8) {
+              const float4* xv = xchunk(s_h, c);
+              acc = dot8(lds128(wr + c), xv[0], xv[8], acc, F16);
+            }
           }
-        }
-        if (tid == 0 && b == 0) DEC_TRACE(3, 1);
-        acc += __shfl_xor_sync(0xffffffffu, acc, 1);
-        acc += __shfl_xor_sync(0xffffffffu, acc, 2);
-        acc += __shfl_xor_sync(0xffffffffu, acc, 4);
-        if (tid == 0 && b == 0) DEC_TRACE(3, 2);
-        if (part == 0 && d < D) {
-          acc += s_bphi[d];
-          s_q[d] = p.relu ? fmaxf(acc, 0.f) : acc;
+          if (tid == 0 && b == 0) DEC_TRACE(3, 1);
+          acc += __shfl_xor_sync(0xffffffffu, acc, 1);
+          acc += __shfl_xor_sync(0xffffffffu, acc, 2);
+          acc += __shfl_xor_sync(0xffffffffu, acc, 4);
+          if (tid == 0 && b == 0) DEC_TRACE(3, 2);
+          if (part == 0 && d < D) {
+            acc += s_bphi[d];
+            s_q[d] = p.relu ? fmaxf(acc, 0.f) : acc;
+          }
         }
       }
-    }
     }
     __syncthreads();
     if (tid == 0 && b == 0) { DEC_TRACE(2, 1); DEC_TRACE(3, 3); }
@@ -1227,8 +1163,7 @@ __device__ void attention_role(const DecParams& p, uint8_t* smem, int b, int ran
       inv = split ? 1.0f : 1.0f / sum_loc;  // split attention: the partial context stays unnormalised until the two halves are combined
     }
 
-    // ---- D: context[e] = sum_u score[u] * enc[b,u,e]  (:293-297); warps 1.. meanwhile evaluate the h half of the
-    //         character distribution, W_cd[:, :Hs] . h + b_cd  (16 lanes per output)
+    // ---- D: context[e] = sum_u score[u] * enc[b,u,e]  (:293-297)
     if (warp < niss) {
       // scores (bf16) are row 0 of a 16-row K-major operand in shared memory:
       // D_t[128 features, 16] = enc^T tile (TMEM) . scores^T ; column 0 of each accumulator is the context.
@@ -1239,63 +1174,28 @@ __device__ void attention_role(const DecParams& p, uint8_t* smem, int b, int ran
       if (ptx::elect_one()) {
         const UmmaLayout lb{0, 256, 128, 0};
         const uint32_t idesc = umma_idesc_bf16(128, 16, F16);
-        const uint32_t bop = ptx::smem_u32(s_bop);
-        if (p.ab_flags & 512) {  // A/B: descriptors rebuilt per instruction
-          for (int t = warp; t < ntm; t += niss)
-            for (int ks = 0; ks < nks; ++ks)
-              ptx::umma_bf16_ts(tmem + ntm * CU + t * 16, tmem + t * CU + ks * 8, umma_smem_desc(lb, bop, ks * 16), idesc, ks != 0);
-        } else {
-          // Consecutive K steps are 512 bytes apart in the score operand and 8 columns apart in tensor memory, so both operands
-          // advance by constants: 32 in the descriptor's 16-byte address field (which cannot carry out of its 14 bits: shared
-          // memory ends below 256 KB) and 8 in the tensor-memory address.
-          const uint64_t bd0 = umma_smem_desc(lb, bop, 0);
-          for (int t = warp; t < ntm; t += niss) {
-            uint64_t bd = bd0;
-            uint32_t a = tmem + t * CU;
-            const uint32_t dcol = tmem + ntm * CU + t * 16;
+        // Consecutive K steps are 512 bytes apart in the score operand and 8 columns apart in tensor memory, so both operands
+        // advance by constants: 32 in the descriptor's 16-byte address field (which cannot carry out of its 14 bits: shared
+        // memory ends below 256 KB) and 8 in the tensor-memory address.
+        const uint64_t bd0 = umma_smem_desc(lb, ptx::smem_u32(s_bop), 0);
+        for (int t = warp; t < ntm; t += niss) {
+          uint64_t bd = bd0;
+          uint32_t a = tmem + t * CU;
+          const uint32_t dcol = tmem + ntm * CU + t * 16;
 #pragma unroll 4
-            for (int ks = 0; ks < nks; ++ks) {
-              ptx::umma_bf16_ts(dcol, a, bd, idesc, ks != 0);
-              a += 8;
-              bd += 32;
-            }
+          for (int ks = 0; ks < nks; ++ks) {
+            ptx::umma_bf16_ts(dcol, a, bd, idesc, ks != 0);
+            a += 8;
+            bd += 32;
           }
         }
         ptx::umma_commit(ctx_bar);
       }
       __syncwarp();
     }
-    // The h half of the logits is evaluated together with the context half, AFTER the context has been published ("late"): the
-    // context UMMAs (four issuing warps) finish in ~0.9 us, sooner than a GEMV squeezed in next to them, and the publish must not
-    // wait for it.  ab_flags bit 12 (4096) selects the alternative for A/B runs: warps 0-3 -- the issuers, one per TMEM lane
-    // quadrant -- read the context out and publish it on their own named barrier while warps 4-15 evaluate the h half
-    // (measured 0.2 us/step slower: that GEMV is bound by the shared-memory pipe and delays the context half behind it).
-    const bool split_h = !split && !hybrid && ntm > 0 && (E >> 3) <= 128 && (p.ab_flags & 4096);
+    // The h half of the logits is evaluated together with the context half, AFTER the context has been published: the context UMMAs
+    // (four issuing warps) finish in ~0.9 us, sooner than a GEMV squeezed in next to them, and the publish must not wait for it.
     const bool owner = !split || rank == 0;  // of a split pair only the first CTA publishes the context and evaluates the logits / feedback
-    const bool late_h = !split_h;
-    // A/B hook (ab_flags bit 16 = 65536; measured neutral, 11.83 vs 11.80 us/step, so off): pure tensor-memory path, one CTA per
-    // utterance: publish the context straight from the read-out registers (bf16 pairs assembled by shuffles, 16-byte stores) instead
-    // of through s_ctx and a second barrier.
-    const bool direct_pub = !split && !hybrid && ntm > 0 && !split_h && (p.ab_flags & 65536);
-    if (split_h && warp >= 4) {
-      const int part = tid & 15;
-      for (int v = (tid - 128) >> 4; v < Vp; v += (DEC_THREADS - 128) / 16) {
-        float acc = 0.f;
-        if (v < V) {
-          const uint4* wr = reinterpret_cast<const uint4*>(s_wcd + (size_t)v * WCS);
-#pragma unroll 4
-          for (int c = part; c < hchunks; c += 16) {
-            const float4* xv = xchunk(s_h, c);
-            acc = dot8(lds128(wr + c), xv[0], xv[8], acc, F16);
-          }
-        }
-        acc += __shfl_xor_sync(0xffffffffu, acc, 1);
-        acc += __shfl_xor_sync(0xffffffffu, acc, 2);
-        acc += __shfl_xor_sync(0xffffffffu, acc, 4);
-        acc += __shfl_xor_sync(0xffffffffu, acc, 8);
-        if (part == 0 && v < V) s_logit[v] = acc + s_bcd[v];
-      }
-    }
     __nv_bfloat16* xr = p.xbuf[np] + (size_t)b * E;        // next LSTM input: context row
     __nv_bfloat16* wr_next = p.wbuf[np] + (size_t)b * DEC_VP;  // ... and dense word row (padded to 64)
     if (Ec > 0) {
@@ -1333,24 +1233,16 @@ __device__ void attention_role(const DecParams& p, uint8_t* smem, int b, int ran
         dst[1] = make_float4(acc[4], acc[5], acc[6], acc[7]);
       }
     }
-    if (ntm > 0 && (!split_h || warp < 4)) {
+    if (ntm > 0) {
       ptx::mbar_wait(ctx_bar, (uint32_t)(s & 1));
       ptx::tc_fence_after();
       if (tid == 0 && b == 0 && !hybrid) DEC_TRACE(2, 3);
       const int qd = warp & 3;
-      for (int t = split_h ? 0 : (warp >> 2); t < ntm; t += split_h ? 1 : NWARP / 4) {
+      for (int t = warp >> 2; t < ntm; t += NWARP / 4) {
         const uint32_t r = ptx::tmem_ld_32x32b_x1(tmem + ((uint32_t)(qd * 32) << 16) + ntm * CU + t * 16);
         ptx::tmem_ld_wait();
         const int e = t * 128 + qd * 32 + lane;
         const float cv = __uint_as_float(r) * inv;
-        if (direct_pub) {
-          // publish straight from the registers: lanes 8j..8j+7 hold 8 consecutive features -> lane 8j stores their 16 bytes
-          const uint32_t mine = (uint32_t)__bfloat16_as_ushort(op_from_f32(cv, F16));
-          const uint32_t nb1 = __shfl_down_sync(0xffffffffu, mine, 1);
-          const uint32_t pair = mine | (nb1 << 16);                        // valid in even lanes: features (e, e+1)
-          const uint32_t p1 = __shfl_down_sync(0xffffffffu, pair, 2), p2 = __shfl_down_sync(0xffffffffu, pair, 4), p3 = __shfl_down_sync(0xffffffffu, pair, 6);
-          if ((lane & 7) == 0) *reinterpret_cast<uint4*>(p.xbuf[np] + (size_t)b * E + e) = make_uint4(pair, p1, p2, p3);
-        }
         if (split) {  // partial context: own copy + the peer's receive buffer of this step's parity
           s_own[e] = cv;
           asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(ptx::mapa(ptx::smem_u32(s_recv + (size_t)(s & 1) * (E + 4) + e), peer)), "f"(cv) : "memory");
@@ -1400,18 +1292,7 @@ __device__ void attention_role(const DecParams& p, uint8_t* smem, int b, int ran
         if (last && p.ctx_out) p.ctx_out[(size_t)gb * E + e_cc + ee] = acc;
       }
     }
-    if (split_h) {
-      if (warp < 4) asm volatile("bar.sync 3, 128;" ::: "memory");  // s_ctx complete: written by warps 0-3 only
-    } else {
-      __syncthreads();
-    }
-    if (direct_pub) {  // the context row left from the registers above; the barrier made the release cumulative over all warps' stores
-      if (tid == 0) {
-        red_release_add(ctx_ctr, 1u);
-        DEC_TRACE_ALL(3);
-        if (b == 0) DEC_TRACE(2, 4);
-      }
-    } else
+    __syncthreads();
     // publish the context row (bf16) with 16-byte stores from the first E/8 threads -- few, sector-filling writes keep the
     // release short -- then release: layer 0 starts its context GEMM while the character distribution is evaluated here
     if (owner) {
@@ -1436,7 +1317,6 @@ __device__ void attention_role(const DecParams& p, uint8_t* smem, int b, int ran
       }
     }
 
-    if (split_h) __syncthreads();  // s_ctx (warps 0-3) and the h half of the logits (warps 4-15) are both in place
     if (p.attn && (tid & 1) == 0) {  // attention record (:292, returned to the caller): off the critical path, after the publish
 #pragma unroll
       for (int ps = 0; ps < ATT_MAXP; ++ps) {
@@ -1461,19 +1341,17 @@ __device__ void attention_role(const DecParams& p, uint8_t* smem, int b, int ran
             const float4* xv = xchunk(s_ctx, c);
             acc = dot8(lds128(wr + hchunks + c), xv[0], xv[8], acc, F16);
           }
-          if (late_h) {  // the h half was not evaluated during the context reduction
 #pragma unroll 4
-            for (int c = part; c < hchunks; c += 16) {
-              const float4* xv = xchunk(s_h, c);
-              acc = dot8(lds128(wr + c), xv[0], xv[8], acc, F16);
-            }
+          for (int c = part; c < hchunks; c += 16) {
+            const float4* xv = xchunk(s_h, c);
+            acc = dot8(lds128(wr + c), xv[0], xv[8], acc, F16);
           }
         }
         acc += __shfl_xor_sync(0xffffffffu, acc, 1);
         acc += __shfl_xor_sync(0xffffffffu, acc, 2);
         acc += __shfl_xor_sync(0xffffffffu, acc, 4);
         acc += __shfl_xor_sync(0xffffffffu, acc, 8);
-        if (part == 0 && v < V) s_logit[v] = late_h ? acc + s_bcd[v] : s_logit[v] + acc;
+        if (part == 0 && v < V) s_logit[v] = acc + s_bcd[v];
       }
       asm volatile("bar.sync 4, %0;" ::"n"(DEC_THREADS - 32) : "memory");   // logits complete (warps 1-15)
       asm volatile("bar.arrive 5, %0;" ::"n"(DEC_THREADS) : "memory");      // ... and s_h / s_ctx no longer read: warp 0 may move on
@@ -1630,8 +1508,8 @@ __global__ void dec_init_kernel(DecParams p, const float* enc_f32, const float* 
       p.hbuf[l][0][(size_t)b * p.Hs + i] = op_from_f32(h_in ? h_in[((size_t)l * p.Bfull + gb) * p.Hs + i] : 0.f, p.f16);
 }
 
-int g_dec_ctx_tmem = 1;  // las_debug_set_option(2, v)
-int g_dec_ab_flags = 0;  // las_debug_set_option(5, v)
+int g_dec_ctx_tmem = 1;   // las_debug_set_option(2, 0): the context on the CUDA cores only
+int g_dec_lstm_role = 0;  // las_debug_set_option(5, 1): lstm_role (shared-memory operands, per-atom 2-D copies) where lstm_role_ts would run
 
 struct Shape {
   int ncl, natoms[MAX_SL];
@@ -1671,7 +1549,7 @@ RingCfg ring_cfg(const las_speller_dims* d, int rows) {
   r.smem = fixed + (size_t)r.nstages * r.stage_bytes + (r.box_rows == 64 ? 0 : 0);
   return r;
 }
-bool att_wreg(const las_speller_dims* d) { return d->D <= DEC_THREADS / 8 && d->Hs <= 512 && !(g_dec_ab_flags & 1); }
+bool att_wreg(const las_speller_dims* d) { return d->D <= DEC_THREADS / 8 && d->Hs <= 512; }
 size_t att_smem(const las_speller_dims* d, bool k_in, bool hybrid = false, bool split = false) {
   return att_layout(d->Hs, d->E, split ? att_split_half(d->U) : d->U, d->D, d->V, k_in, att_wreg(d), hybrid, split).total + 64;
 }
@@ -1690,11 +1568,9 @@ int ctx_tiles_fit(int U, int E) {
 // a cluster of two CTAs attends each utterance (flash-decoding style partial softmax, combined through DSMEM) -- provided the LSTM
 // CTAs pair up (even count) and the chip has room for two attention CTAs per utterance.
 bool att_split_ok(const las_speller_dims* d) {
-  if (!g_dec_att_split || g_dec_ctx_tmem <= 0 || d->E % 128 != 0) return false;
+  if (!g_dec_att_split || !g_dec_ctx_tmem || d->E % 128 != 0) return false;
   const int NT = d->E / 128;
-  // one CTA is enough ... unless the split is forced (option 11 = 2) or the encoder is long enough that halving the energy /
-  // softmax pass and the context UMMA chains pays for the DSMEM exchange (U > 256: two passes of the 256-step energy loop)
-  if (ctx_tiles_fit(d->U, d->E) == NT && g_dec_att_split != 2 && !(g_dec_att_split == 3 && d->U > 256)) return false;
+  if (ctx_tiles_fit(d->U, d->E) == NT) return false;  // one CTA is enough
   const int n_lstm = d->sl * (d->Hs / DEC_UNITS);
   return ctx_tiles_fit(att_split_half(d->U), d->E) == NT && (n_lstm % 2 == 0) && n_lstm + 2 <= sm_count() &&
          att_smem(d, true, false, true) <= 220 * 1024;
@@ -1778,11 +1654,11 @@ bool fast_speller_fits(const las_speller_dims* d) {
   const bool ok = supported(d) == LAS_OK && d->sl * (d->Hs / DEC_UNITS) + 1 <= sm_count();
   return ok;
 }
-void fast_set_option_speller(int key, int value) {
-  if (key == 2) g_dec_ctx_tmem = value;
-  if (key == 5) g_dec_ab_flags = value;
-  if (key == 11) g_dec_att_split = value;
-  if (key == 19) g_dec_groups = value;
+bool fast_set_option_speller(int key, int value) {
+  int* opt = key == 2 ? &g_dec_ctx_tmem : key == 5 ? &g_dec_lstm_role : key == 11 ? &g_dec_att_split : key == 19 ? &g_dec_groups : nullptr;
+  if (!opt || (value != 0 && value != 1)) return false;
+  *opt = value;
+  return true;
 }
 
 size_t fast_speller_packed_bytes(const las_speller_dims* d) { return pack_layout(d, nullptr).bytes; }
@@ -1856,8 +1732,8 @@ int fast_speller_decode_segment(const las_decode_io* io, const void* packed_f32,
       const int NT = d->E / 128;
       // all feature tiles of enc[b]^T in tensor memory when they fit its 512 columns (U <= 224 at E = 512); otherwise as many
       // as fit, the rest on the CUDA cores (hybrid; needs the score operand in its own shared-memory region)
-      int ntm = g_dec_ctx_tmem > 0 ? ctx_tiles_fit(d->U, d->E) : 0;
-      if (ntm > 0 && ntm < NT && (g_dec_ctx_tmem == 2 || (512 % ((d->E - ntm * 128) / 8)) != 0)) ntm = 0;  // option 2: value 2 = no hybrid
+      int ntm = g_dec_ctx_tmem ? ctx_tiles_fit(d->U, d->E) : 0;
+      if (ntm > 0 && ntm < NT && (512 % ((d->E - ntm * 128) / 8)) != 0) ntm = 0;
       p.ctx_ntm = ntm;
       p.ctx_tmem = ntm > 0;
       const bool hyb = ntm > 0 && ntm < NT;
@@ -1865,10 +1741,9 @@ int fast_speller_decode_segment(const las_decode_io* io, const void* packed_f32,
       if (hyb && att_smem(d, p.k_in_smem != 0, true) > 220 * 1024) { p.ctx_ntm = 0; p.ctx_tmem = 0; p.k_in_smem = att_smem(d, true, false) <= 220 * 1024; }
     }
     RingCfg rc = ring_cfg(d, Bc);
-    // weights-stationary LSTM CTAs: whole 64-wide atoms, one 3-D copy per part, critical weights within 384 tensor-memory columns
-    // (ab_flags bit 14 = 16384 selects the round-1 operand roles for A/B runs)
-    p.tma3d = (d->Hs % 64 == 0 && d->E % 64 == 0 && !(g_dec_ab_flags & 4)) ? 1 : 0;
-    p.lstm_ts = (p.tma3d && d->Hs <= 768 && d->E <= 768 && !(g_dec_ab_flags & 16384)) ? 1 : 0;
+    // weights-stationary LSTM CTAs: whole 64-wide atoms (E == Hs), one 3-D copy per part, critical weights within 256 tensor-memory
+    // columns (Hs <= 512)
+    p.lstm_ts = (d->Hs % 64 == 0 && !g_dec_lstm_role) ? 1 : 0;
     // two utterance groups of 32 pipelined through the LSTM CTAs (lstm_role_ts) when the launch has more than 32 utterances
     p.groups = (p.lstm_ts && Bc > 32 && g_dec_groups != 0) ? 2 : 1;
     p.gsz = p.groups == 2 ? 32 : 64;
@@ -1890,7 +1765,7 @@ int fast_speller_decode_segment(const las_decode_io* io, const void* packed_f32,
       LAS_TRY(make_tmap_bf16_box(&p.tm_x[k], w.xbuf[k], Bc, d->E, d->E, rc.box_rows));
       LAS_TRY(make_tmap_bf16_box(&p.tm_w[k], w.wbuf[k], Bc, DEC_VP, DEC_VP, rc.box_rows));
     }
-    if (p.tma3d) {
+    if (p.lstm_ts) {
       for (int l = 0; l < d->sl; ++l)
         for (int k = 0; k < 2; ++k) LAS_TRY(make_tmap_bf16_atoms(&p.tm_h3[l][k], w.hbuf[l][k], Bc, d->Hs / 64, d->Hs, rc.box_rows, d->Hs / 64));
       for (int k = 0; k < 2; ++k)
@@ -1918,9 +1793,8 @@ int fast_speller_decode_segment(const las_decode_io* io, const void* packed_f32,
     p.sync = w.sync;
     p.h_ll = w.h_ll;
     p.tok_ll = w.tok_ll;
-    // the fed-back word is an index (greedy argmax / index teacher forcing) unless a dense vector is asked for
-    p.ab_flags = g_dec_ab_flags;
     p.f16 = op_f16();
+    // the fed-back word is an index (greedy argmax / index teacher forcing) unless a dense vector is asked for
     p.word_gather = io->gt_dense ? 0 : (io->gt_index ? 1 : (decode_mode != LAS_DECODE_RAW ? 1 : 0));
     p.sample_seed = io->sample_seed;
     p.trace = (fast_get_trace() && first_seg) ? fast_get_trace() + 512 : nullptr;  // needs 5 roles x 32 steps x 8 stamps behind the recurrence trace

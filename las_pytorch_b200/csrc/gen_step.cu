@@ -38,9 +38,7 @@ __device__ __forceinline__ void st_cluster_f32(uint32_t addr, float v) {
 // =========================================================================================================
 // gen_cell_step_kernel.  CTA c owns 64 / G consecutive cells and all G gate rows of each (LSTM: i,f,g,o; GRU: r,z,n_x,n_h; RNN: 1),
 // i.e. 64 rows of the packed [R, Kp] weights (kernels_f32.cu gen_pack_w_kernel; Kp is a multiple of 64).  The weights are the A
-// operand (M = 128 in the instruction; rows 64-127 of the tile are whatever follows in shared memory and land in tensor-memory lanes
-// nobody reads -- M = 128 costs the same and keeps the lane = row layout), the activations [B, Kp] the B operand (N = B rounded
-// up to 16, rows beyond B are TMA zero fill).
+// operand (M = 64), the activations [B, Kp] the B operand (N = B rounded up to 16, rows beyond B are TMA zero fill).
 //   warp 0 (one thread)  TMA producer.  One ring stage = GS_KBS 64-column K blocks, fetched by TWO copies: a 4-D box {64 k, 64/G
 //                        cells, G gates, GS_KBS blocks} of the weights and a 3-D box {64 k, N, GS_KBS} of the activations (per-copy cost
 //                        dominates small boxes: one 16-row box per gate and block ran at 0.42 us per block, 5x slower)
@@ -64,7 +62,6 @@ struct GenStepArgs {
   int B, H, G, cell, Kp, NB, stages, f16, st_first;
   int early;         // trigger the dependent launch at once (last layer: the attention kernel's prologue reads only constants)
   int region;        // activations in their own region (two copies per launch) instead of riding in the ring stages
-  int m64;           // M = 64 instruction shape: accumulator row i in tensor-memory lane (i / 16) * 32 + i % 16
   long long* trace;  // nullable (tools/gen_step_probe.py): clock64 stamps of CTA 0
 };
 
@@ -77,7 +74,7 @@ gen_cell_step_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_cons
   // ring stage: [w block 0][w block 1] and, unless the activations have their own region, [a block 0][a block 1]
   const int stage_bytes = p.region ? GS_KBS * GS_WBYTES : GS_KBS * (GS_WBYTES + a_bytes);
   const int k_blocks = p.Kp / 64, n_stages = (k_blocks + GS_KBS - 1) / GS_KBS;
-  uint8_t* const acts = ring + (size_t)p.stages * stage_bytes + GS_WBYTES;  // (+ slack for an M = 128 view of the last block)
+  uint8_t* const acts = ring + (size_t)p.stages * stage_bytes;
   uint64_t* const full = reinterpret_cast<uint64_t*>(acts + (p.region ? (size_t)n_stages * GS_KBS * a_bytes : 0));
   uint64_t* const empty = full + p.stages;
   uint64_t* const done = empty + p.stages;
@@ -212,7 +209,7 @@ gen_cell_step_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_cons
     }
   } else if (warp == 1) {
     const UmmaLayout lw{1, 0, 1024, 0};
-    const uint32_t idesc = umma_idesc_bf16(p.m64 ? 64 : 128, (uint32_t)p.NB, p.f16);
+    const uint32_t idesc = umma_idesc_bf16(64, (uint32_t)p.NB, p.f16);
     const uint64_t wdesc0 = umma_smem_desc(lw, ring_a, 0),
                    adesc0 = umma_smem_desc(lw, p.region ? ptx::smem_u32(acts) : ring_a + GS_KBS * GS_WBYTES, 0);
     const uint32_t a16 = (uint32_t)a_bytes >> 4, stage16 = stage_b >> 4, end16 = ((uint32_t)p.stages * stage_b) >> 4;
@@ -256,17 +253,17 @@ gen_cell_step_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_cons
   if (tr && tid == 64) tr[4] = clock64();
   griddep_wait();  // (already satisfied: the dependent stages were loaded after the producer's wait)
 
-  // accumulator rows 0-63 -> shared memory (the ring is dead: every copy has landed and every MMA has read its operands)
+  // accumulator rows 0-63 -> shared memory (the ring is dead: every copy has landed and every MMA has read its operands).  M = 64:
+  // row i sits in tensor-memory lane (i / 16) * 32 + i % 16, so warps 4-7 each read their lane quadrant and keep lanes 0-15.
   float* const pre = reinterpret_cast<float*>(ring);
   const int ldp = p.NB + 1;
-  if (warp >= 4 && (p.m64 || warp < 6)) {
-    const int row = p.m64 ? (warp - 4) * 16 + lane : (warp - 4) * 32 + lane;
-    const bool keep = !p.m64 || lane < 16;
+  if (warp >= 4) {
+    const int row = (warp - 4) * 16 + lane;
     for (int c0 = 0; c0 < p.NB; c0 += 16) {
       uint32_t v[16];
       ptx::tmem_ld_32x32b_x16(tmem + ((uint32_t)((warp - 4) * 32) << 16) + (uint32_t)c0, v);
       ptx::tmem_ld_wait();
-      if (keep) {
+      if (lane < 16) {
 #pragma unroll
         for (int j = 0; j < 16; ++j) pre[row * ldp + c0 + j] = __uint_as_float(v[j]);
       }
@@ -597,18 +594,14 @@ __global__ void __launch_bounds__(AC_THREADS, 1) attend_cluster_kernel(const Att
 
 int g_gen_fused = 1;    // las_debug_set_option(12, 0): the unfused generic step (GEMM + cell + operand kernels, one-CTA attention)
 int g_gen_cluster = 0;  // las_debug_set_option(13, C): force the attention cluster size (0 = by batch)
-int g_gen_m64 = 1;      // las_debug_set_option(15, 0): M = 128 instruction shape in the cell kernel (rows 64-127 unused; bit-identical)
-int g_gen_pdl = 1;      // las_debug_set_option(16, 0): plain stream order between the step's launches
-int g_gen_early = 1;    // las_debug_set_option(18, 0): the last layer triggers the attention kernel only after its own dependency
 
 }  // namespace
 
-void fast_set_option_gen(int key, int value) {
-  if (key == 12) g_gen_fused = value;
-  if (key == 13) g_gen_cluster = value;
-  if (key == 15) g_gen_m64 = value;
-  if (key == 16) g_gen_pdl = value;
-  if (key == 18) g_gen_early = value;
+bool fast_set_option_gen(int key, int value) {
+  if (key == 12 && (value == 0 || value == 1)) g_gen_fused = value;
+  else if (key == 13 && (value == 0 || value == 1 || value == 2 || value == 4 || value == 8)) g_gen_cluster = value;
+  else return false;
+  return true;
 }
 bool gen_step_fused(int B) { return g_gen_fused != 0 && B <= 256; }
 
@@ -657,13 +650,12 @@ int launch_gen_cell_step(const GenStepMaps& m, int parity, const float* bias, fl
   p.stages = (int)((200 * 1024 - region_bytes) / (GS_KBS * (GS_WBYTES + (p.region ? 0 : p.NB * 128))));  // ring + region <= 200 KB
   if (p.stages > 10) p.stages = 10;
   p.f16 = op_f16();
-  p.m64 = g_gen_m64;
-  p.early = (o2 == nullptr && g_gen_early) ? 1 : 0;
+  p.early = (o2 == nullptr) ? 1 : 0;
   const int n_stages = (Kp / 64 + GS_KBS - 1) / GS_KBS, first = (Kxp + 64 * GS_KBS - 1) / (64 * GS_KBS);
   p.st_first = first < n_stages ? first : n_stages;
   p.trace = fast_get_trace() ? fast_get_trace() + 16 * (1 + trace_slot) : nullptr;
   const int cells = GS_ROWS / p.G;
-  const size_t smem = 1024 + (size_t)p.stages * GS_KBS * (GS_WBYTES + (p.region ? 0 : p.NB * 128)) + GS_WBYTES + region_bytes + 8 * (2 * p.stages + 3) + 16;
+  const size_t smem = 1024 + (size_t)p.stages * GS_KBS * (GS_WBYTES + (p.region ? 0 : p.NB * 128)) + region_bytes + 8 * (2 * p.stages + 3) + 16;
   LAS_CUDA_OK(cudaFuncSetAttribute(gen_cell_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
@@ -675,7 +667,7 @@ int launch_gen_cell_step(const GenStepMaps& m, int parity, const float* bias, fl
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = at;
-  cfg.numAttrs = (pdl && g_gen_pdl) ? 1 : 0;
+  cfg.numAttrs = pdl ? 1 : 0;
   LAS_CUDA_OK(cudaLaunchKernelEx(&cfg, gen_cell_step_kernel, m.w, m.a[parity & 1], m.a_ind[parity & 1], m.a_dep[parity & 1], p));
   LAS_LAUNCH_OK("gen_cell_step_kernel");
   return LAS_OK;
@@ -712,7 +704,7 @@ int launch_attend_cluster(const AttendArgs& a, bool pdl, cudaStream_t st) {
     at[n].val.clusterDim.z = 1;
     ++n;
   }
-  if (pdl && g_gen_pdl) {
+  if (pdl) {
     at[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[n].val.programmaticStreamSerializationAllowed = 1;
     ++n;

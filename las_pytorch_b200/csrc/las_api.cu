@@ -881,7 +881,7 @@ int las_debug_gemm_bf16(const void* a, const void* w, const float* bias, float* 
                              static_cast<cudaStream_t>(stream));
 }
 int las_debug_set_option(int key, int value) {
-  fast_set_option(key, value);
+  LAS_REQUIRE(fast_set_option(key, value), "las_debug_set_option: key %d is not an option, or %d is not one of its values", key, value);
   return LAS_OK;
 }
 int las_debug_set_trace(void* dev_buf) {

@@ -3,6 +3,7 @@
 Tolerances (BASELINE.json north_star): pyramid reshape / masks / argmax bit-exact; log-probs <= 1e-4 max-abs in
 fp32 mode and <= 2e-2 in bf16 mode; greedy token sequences agree on >= 99% of characters.
 """
+import ctypes
 import glob
 import os
 
@@ -122,12 +123,10 @@ def test_matches_reference_golden(name, precision):
     assert np.abs(attn.sum(-1) - 1).max() < 1e-4
 
 
-@pytest.mark.parametrize("precision", precisions())
-def test_against_numpy_oracle_on_seeded_inputs(precision):
-    """Same seeded inputs/weights through the CUDA path and the fp64 numpy oracle (sizes the oracle does in seconds)."""
-    cfgname, B, T, S = "small", 6, 256, 40
-    c = tl.CONFIGS[cfgname]
-    las = tl.build_model(cfgname, max_label_len=S, seed=23, gain=3.0, precision=precision)
+def check_against_numpy_oracle(c, precision, B=6, T=256, S=40):
+    """Same seeded inputs/weights of config `c` through the CUDA path and the fp64 numpy oracle, teacher forced and free running
+    (sizes the oracle does in seconds).  Returns the model (on the GPU) and the inputs."""
+    las = tl.build_model(c, max_label_len=S, seed=23, gain=3.0, precision=precision)
     sd = tl.state_dict_numpy(las)
     x, labels = tl.make_inputs(B, T, c["F"], S, c["V"], seed=23, pad_tail=32)
     ref_tf = O.las_forward(x.numpy(), sd, c["L"], c["sl"], S, ground_truth=labels.numpy(), teacher_forced=True, dtype=np.float64)
@@ -156,6 +155,43 @@ def test_against_numpy_oracle_on_seeded_inputs(precision):
     if precision == "fp32":
         assert np.abs(logp_g - ref_gr["logp"]).max() <= tol["logp"]
         assert np.array_equal(las.speller.last_tokens.cpu().numpy(), logp_g.argmax(-1))
+    return las, x
+
+
+@pytest.mark.parametrize("precision", precisions())
+def test_against_numpy_oracle_on_seeded_inputs(precision):
+    check_against_numpy_oracle(tl.CONFIGS["small"], precision)
+
+
+@pytest.mark.parametrize("precision", [p for p in precisions() if p != "fp32"])
+@pytest.mark.parametrize("path", ["decoder_w_phi_in_shared_memory", "listener_layer0_gemm"])
+def test_shape_selected_tensor_core_paths_against_numpy_oracle(path, precision):
+    """Two paths of the tensor-core modes that only the model's shape selects, against the fp64 oracle: the persistent decoder with
+    W_phi in shared memory (attention dim D > 64; up to 64 the attention threads keep it in registers), and the cluster recurrence
+    with layer 0's input projection as a separate GEMM (2F not a multiple of 16; otherwise the recurrence multiplies x_t itself)."""
+    from las_pytorch_b200 import _cabi
+
+    lib = _cabi.load_library()
+    S = 40
+    c = dict(tl.CONFIGS["small"], **({"D": 128} if path.startswith("decoder") else {"F": 44}))
+    las, x = check_against_numpy_oracle(c, precision, S=S)
+    x = x.cuda()
+    if path.startswith("decoder"):
+        enc = las.listener(x)
+        torch.cuda.synchronize()
+        lib.las_launch_count(1)
+        las.speller(enc, None, 0.0)
+        torch.cuda.synchronize()
+        assert lib.las_launch_count(0) < S  # the persistent kernel ran: the generic path launches at least once per step
+    else:
+        buf = ctypes.create_string_buffer(1 << 16)
+        lib.las_prof_enable(1)
+        try:
+            las.listener(x)
+            _cabi.check(lib.las_prof_report(buf, len(buf)))
+        finally:
+            lib.las_prof_enable(0)
+        assert "listener.L0.input_gemm" in buf.value.decode()
 
 
 @pytest.mark.parametrize("precision", precisions())
@@ -324,9 +360,10 @@ def test_bf16_listener_overlap_is_bit_identical_to_sequential():
 
 
 def test_bf16_decoder_single_3d_copy_matches_per_atom_copies():
-    """The decoder's activation parts arrive as ONE 3-D TMA copy when Hs and E are multiples of 64, and as one 2-D copy per
-    64-column atom otherwise (las_debug_set_option(5, 4) forces the latter): same bytes in shared memory, so greedy tokens,
-    log-probs and attention must be bit-identical."""
+    """The decoder's LSTM CTAs take each activation part as ONE 3-D TMA copy in the weights-stationary form (lstm_role_ts, Hs a
+    multiple of 64), and as one 2-D copy per 64-column atom in the shared-memory-operand form (lstm_role: other Hs;
+    las_debug_set_option(5, 1) forces it): same bytes in shared memory, the same sums per output, so greedy tokens, log-probs and
+    attention must be bit-identical."""
     if "bf16" not in precisions():
         pytest.skip("bf16 path not built")
     from las_pytorch_b200 import _cabi
@@ -343,7 +380,7 @@ def test_bf16_decoder_single_3d_copy_matches_per_atom_copies():
         return torch.stack(pred).clone(), torch.stack([a[0] for a in att]).clone()
 
     try:
-        lib.las_debug_set_option(5, 4)
+        _cabi.check(lib.las_debug_set_option(5, 1))
         p2, a2 = run()
     finally:
         lib.las_debug_set_option(5, 0)

@@ -7,8 +7,8 @@ mkdir -p gpurun_out
 for rep in 1 2; do
   echo "== decoder, tree=new";   python tools/decoder_ab.py 0
   for o in $OTHERS; do echo "== decoder, tree=$o"; LAS_ROOT=$PWD/$o python tools/decoder_ab.py 0; done
-  echo "== listener, tree=new";   python tools/listener_ab.py 1=1
-  for o in $OTHERS; do echo "== listener, tree=$o"; LAS_ROOT=$PWD/$o python tools/listener_ab.py 1=1; done
+  echo "== listener, tree=new";   python tools/listener_ab.py
+  for o in $OTHERS; do echo "== listener, tree=$o"; LAS_ROOT=$PWD/$o python tools/listener_ab.py; done
 done
 } > gpurun_out/ab_$TAG.log 2>&1
 cat gpurun_out/ab_$TAG.log

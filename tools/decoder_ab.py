@@ -1,6 +1,6 @@
-"""A/B timing of decoder variants selected with las_debug_set_option(5, flags), interleaved on the same box.
+"""A/B timing of the decoder's LSTM CTA forms selected with las_debug_set_option(5, v), interleaved on the same box.
 
-    python tools/decoder_ab.py 0 1 [0 1 ...]      # flag values to compare
+    python tools/decoder_ab.py 0 1 [0 1 ...]      # 0 = weights-stationary form (default), 1 = shared-memory operands
 """
 import os
 import sys
@@ -24,8 +24,8 @@ def main():
     enc = las.listener(x.cuda())
     res = {f: [] for f in flags}
     outs = {}
-    for f in flags:  # same instructions in the same order per accumulator: every variant must be bit-identical to the first
-        lib.las_debug_set_option(5, f)
+    for f in flags:  # same sums in the same order per output: every variant must be bit-identical to the first
+        _cabi.check(lib.las_debug_set_option(5, f))
         pred, _ = las.speller(enc, None, 0.0)
         outs[f] = (torch.stack(pred).clone(), las.speller.last_tokens.clone())
     for f in flags[1:]:

@@ -31,10 +31,8 @@ def main():
     print(f"speller c3 bf16: {e0.elapsed_time(e1) / 3:.3f} ms  ({e0.elapsed_time(e1) / 3 / S * 1e3:.2f} us/step)")
     buf = torch.zeros(512 + 5 * 32 * 8 + 148 * 8, dtype=torch.int64, device="cuda")
     lib.las_debug_set_trace(_cabi.ptr(buf))
-    lib.las_debug_set_option(5, int(os.environ.get("LAS_AB_FLAGS", "0")))
     las.speller(enc, None, 0.0)
     torch.cuda.synchronize()
-    lib.las_debug_set_option(5, 0)
     lib.las_debug_set_trace(None)
     raw = buf.cpu().numpy()
     t = raw[512:512 + 5 * 32 * 8].reshape(5, 32, 8)

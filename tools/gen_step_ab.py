@@ -33,7 +33,7 @@ def run():
 
 
 base, t0 = run()
-lib.las_debug_set_option(key, val)
+_cabi.check(lib.las_debug_set_option(key, val))
 try:
     alt, t1 = run()
 finally:

@@ -16,7 +16,7 @@ U = int(sys.argv[3]) if len(sys.argv) > 3 else 200
 lib = _cabi.load_library()
 for kv in filter(None, os.environ.get("LAS_PROBE_OPTS", "").split(",")):
     k, v = kv.split("=")
-    lib.las_debug_set_option(int(k), int(v))
+    _cabi.check(lib.las_debug_set_option(int(k), int(v)))
 c = tl.CONFIGS["shipped"]
 las = tl.build_model("shipped", max_label_len=S, seed=17, gain=3.0, precision=os.environ.get("LAS_PROBE_PRECISION", "bf16")).cuda()
 g = torch.Generator().manual_seed(1)

@@ -22,7 +22,7 @@ def main():
     outs = []
     for v in variants:  # outputs of every variant against the first one
         for k, val in v.items():
-            lib.las_debug_set_option(k, val)
+            _cabi.check(lib.las_debug_set_option(k, val))
         outs.append(lis(x).clone())
     for v, o in zip(variants[1:], outs[1:]):
         print(f"{v} vs {variants[0]}: max-abs diff {float((o - outs[0]).abs().max()):.3e}  bit-identical={torch.equal(o, outs[0])}")

@@ -75,14 +75,9 @@ def trace():
     x, _ = tl.make_inputs(64, 1600, c["F"], 4, c["V"], seed=17)
     lis = tl.build_model("paper", max_label_len=4, seed=17, gain=3.0, precision="bf16").listener.cuda()
     x = x.cuda()
-    import sys as _s
-    opt = int(_s.argv[2]) if len(_s.argv) > 2 else 1
-    lib.las_debug_set_option(1, opt)
-    nacc = int(_s.argv[3]) if len(_s.argv) > 3 else 0
-    lib.las_debug_set_option(4, nacc)
-    if len(_s.argv) > 4:  # utterances per recurrence cluster (16 / 32 / 64): 64 is the form that runs under the decoder
-        lib.las_debug_set_option(9, int(_s.argv[4]))
-    print(f"recurrence A operand in TMEM: {opt}; accumulators: {nacc or 'default'}")
+    bc = int(sys.argv[2]) if len(sys.argv) > 2 else 0  # utterances per recurrence cluster (16 / 32 / 64): 64 is the form that runs under the decoder
+    _cabi.check(lib.las_debug_set_option(9, bc))
+    print(f"utterances per recurrence cluster: {bc or 'automatic'}")
     ref = tl.build_model("paper", max_label_len=4, seed=17, gain=3.0, precision="fp32").listener.cuda()(x)
     out = lis(x)
     print(f"bf16 vs fp32 listener max err {float((out - ref).abs().max()):.3e}")

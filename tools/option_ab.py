@@ -38,7 +38,7 @@ def run():
 
 
 base = run()
-lib.las_debug_set_option(key, val)
+_cabi.check(lib.las_debug_set_option(key, val))
 alt = run()
 same = all(bool(torch.equal(a, b)) for a, b in zip(base[:3], alt[:3]))
 print(f"{cfg} B={B} T={T} S={S}: option {key}={val}: {alt[3]:.3f} ms per decode = {1000 * alt[3] / S:.2f} us/step "

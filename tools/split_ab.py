@@ -1,5 +1,5 @@
 """A/B of the attention split (las_debug_set_option(11, v)): decoder us/step per workload shape.
-    python tools/split_ab.py c2|c3|c4 v1 v2 ..."""
+    python tools/split_ab.py c2|c3|c4 v1 v2 ...      # 1 = split long encoders over two CTAs (default), 0 = never"""
 import os
 import sys
 
@@ -23,7 +23,7 @@ res = {v: [] for v in vals}
 toks = {}
 for rep in range(3):
     for v in vals:
-        lib.las_debug_set_option(11, v)
+        _cabi.check(lib.las_debug_set_option(11, v))
         las.speller(enc, None, 0.0)
         toks[v] = las.speller.last_tokens.clone()
         torch.cuda.synchronize()
