@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define LAS_B200_ABI_VERSION 5
+#define LAS_B200_ABI_VERSION 6
 
 enum {
   LAS_OK = 0,
@@ -219,6 +219,38 @@ size_t las_speller_workspace_bytes(const las_speller_dims* d, int steps, int mod
 /* Runs `steps` decoder steps (Speller.forward loop, :209-236).  relu: attention activation flag. */
 int las_speller_decode(const las_decode_io* io, const void* packed, const las_speller_dims* d, int steps,
                        int decode_mode, int mode, int relu, void* workspace, size_t workspace_bytes, void* stream);
+
+/* --------------------------------------------------------------------------------------------------------
+ * Beam search (extension: the reference decodes greedily).  Every utterance keeps `beam` = K hypotheses as K decoder rows of the
+ * step-per-launch decoder (the fp32 mode's loop and the unfused generic tensor-core step); the K rows share the utterance's encoder
+ * features.  Semantics, with S = steps:
+ *   - start: K rows in the initial state (<sos>, context = enc[b,0], h = c = 0); row 0 scores 0, the others -inf;
+ *   - each step every row runs the decoder step.  A live row k offers (k, v, score[k] + logp[k,v]) for every v (one fp32 add), a
+ *     finished row exactly (k, eos_token, score[k]) with token log-prob 0, a -inf row nothing.  The K best candidates by
+ *     (score desc, parent asc, token asc) become the new rows (parent's h, c and context; fed-back word one_hot(token)); a row is
+ *     finished once its token is eos_token.  A slot left without a finite candidate scores -inf.  All S steps run;
+ *   - the K final rows are ranked by score / length^length_penalty (fp32 powf; ties to the lower slot), length = tokens up to and
+ *     including the first eos_token, or S.  The first `nbest` = N are returned: tokens [B,N,S] (eos_token after the end),
+ *     token_logp [B,N,S] (0 after the end), lengths [B,N], scores [B,N] = the raw sums of token_logp.  A -inf slot has length 0.
+ * Limits: 1 <= K <= 32, 1 <= N <= K, 0 <= eos_token < V, length_penalty finite and >= 0, steps >= 1.
+ * ------------------------------------------------------------------------------------------------------ */
+typedef struct las_beam_io {
+  const float* enc;            /* [B,U,E] listener features */
+  const int32_t* enc_lengths;  /* nullable [B] (per utterance, not per hypothesis): attention length mask */
+  int32_t beam, nbest, eos_token;
+  float length_penalty;
+  int32_t* tokens;             /* [B,N,S] */
+  float* token_logp;           /* nullable [B,N,S] */
+  int32_t* lengths;            /* [B,N] */
+  float* scores;               /* [B,N] */
+} las_beam_io;
+/* The beam pack: in LAS_MODE_BF16 / LAS_MODE_F16 always the fp32 block followed by the generic tensor-core layout (also for shapes the
+ * persistent decoder covers); in LAS_MODE_FP32 the ordinary pack.  The size queries return 0 for arguments the calls reject. */
+size_t las_speller_beam_packed_bytes(const las_speller_dims* d, int mode);
+int las_speller_beam_pack(const las_speller_weights* w, const las_speller_dims* d, int mode, void* packed, size_t bytes, void* stream);
+size_t las_speller_beam_workspace_bytes(const las_speller_dims* d, int steps, int beam, int mode);
+int las_speller_beam_search(const las_beam_io* io, const void* packed, const las_speller_dims* d, int steps, int mode, int relu,
+                            void* workspace, size_t workspace_bytes, void* stream);
 
 /* --------------------------------------------------------------------------------------------------------
  * Cross-batch serving pipeline.  One call stands for `las_speller_decode` of batch i AND `las_listener_forward[_masked]` of batch

@@ -5,11 +5,11 @@
 The arithmetic lives in `liblas_b200.so` (hand-written CUDA, C ABI in include/las_b200.h); build it with
 `python -m las_pytorch_b200.build`.  There is no CPU fallback.
 """
-from .las_model import LAS, Attention, Listener, Speller, pBLSTMLayer  # noqa: F401
+from .las_model import LAS, Attention, BeamSearchResult, Listener, Speller, pBLSTMLayer  # noqa: F401
 from .functions import CreateOnehotVariable, TimeDistributed  # noqa: F401
 from ._cabi import LasB200Error, load_library  # noqa: F401
 
 __all__ = [
-    "LAS", "Attention", "Listener", "Speller", "pBLSTMLayer",
+    "LAS", "Attention", "BeamSearchResult", "Listener", "Speller", "pBLSTMLayer",
     "CreateOnehotVariable", "TimeDistributed", "LasB200Error", "load_library",
 ]

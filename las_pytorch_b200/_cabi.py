@@ -12,7 +12,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "liblas_b200.so")
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 MODE_FP32 = 0
 MODE_BF16 = 1
 MODE_F16 = 2
@@ -60,6 +60,14 @@ class DecodeIO(C.Structure):
     ]
 
 
+class BeamIO(C.Structure):
+    _fields_ = [
+        ("enc", C.c_void_p), ("enc_lengths", C.c_void_p),
+        ("beam", C.c_int32), ("nbest", C.c_int32), ("eos_token", C.c_int32), ("length_penalty", C.c_float),
+        ("tokens", C.c_void_p), ("token_logp", C.c_void_p), ("lengths", C.c_void_p), ("scores", C.c_void_p),
+    ]
+
+
 class PipelineArgs(C.Structure):
     _fields_ = [
         ("dec_io", C.POINTER(DecodeIO)), ("speller_packed", C.c_void_p), ("speller_dims", C.POINTER(SpellerDims)),
@@ -90,6 +98,11 @@ PROTOTYPES = {
     "las_attention_forward": (C.c_int, [C.c_void_p] * 5 + [C.c_int] * 7 + [C.c_void_p] * 6),
     "las_speller_workspace_bytes": (C.c_size_t, [C.POINTER(SpellerDims), C.c_int, C.c_int]),
     "las_speller_decode": (C.c_int, [C.POINTER(DecodeIO), C.c_void_p, C.POINTER(SpellerDims), C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "las_speller_beam_packed_bytes": (C.c_size_t, [C.POINTER(SpellerDims), C.c_int]),
+    "las_speller_beam_pack": (C.c_int, [C.POINTER(SpellerWeights), C.POINTER(SpellerDims), C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "las_speller_beam_workspace_bytes": (C.c_size_t, [C.POINTER(SpellerDims), C.c_int, C.c_int, C.c_int]),
+    "las_speller_beam_search": (C.c_int, [C.POINTER(BeamIO), C.c_void_p, C.POINTER(SpellerDims), C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                          C.c_size_t, C.c_void_p]),
     "las_pipeline_step": (C.c_int, [C.POINTER(PipelineArgs), C.c_int, C.c_void_p]),
     "las_pipeline_overlaps": (C.c_int, [C.POINTER(ListenerDims), C.POINTER(SpellerDims), C.c_int, C.c_int]),
     "las_debug_gemm_bf16": (C.c_int, [C.c_void_p] * 4 + [C.c_int] * 3 + [C.c_void_p]),

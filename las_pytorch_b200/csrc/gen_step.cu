@@ -347,6 +347,8 @@ __device__ __noinline__ float warp_dot(const float* w, const float* x, int n, in
 }
 __device__ __forceinline__ bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
+// kShared: several decoder rows per utterance (a.rows_per_utt > 1, beam search); the one-row form keeps the division out of the prologue
+template <bool kShared>
 __global__ void __launch_bounds__(AC_THREADS, 1) attend_cluster_kernel(const AttendArgs a, const int C) {
   extern __shared__ __align__(16) float sm[];
   const int nown = AC_SLICES / C;
@@ -381,13 +383,14 @@ __global__ void __launch_bounds__(AC_THREADS, 1) attend_cluster_kernel(const Att
   }
   // (biases and the utterance's length do not depend on the launch in front of this one)
   const int u_begin = min(a.U, r * nown * us), u_end = min(a.U, (r + 1) * nown * us);
-  const float* psib = a.psi + (size_t)b * a.U * a.D;
-  const float* encb = a.enc + (size_t)b * a.U * a.E;
+  const int bu = kShared ? b / a.rows_per_utt : b;  // the utterance whose encoder features row b attends over
+  const float* psib = a.psi + (size_t)bu * a.U * a.D;
+  const float* encb = a.enc + (size_t)bu * a.U * a.E;
   {
     if (a.w_phi) for (int d = tid; d < a.D; d += AC_THREADS) s_bias[d] = a.b_phi[d];
     if (a.w_cd) for (int v = tid; v < a.V; v += AC_THREADS) s_bias[D4 + v] = a.b_cd[v];
   }
-  const int ulen = a.enc_lengths ? min(max(a.enc_lengths[b], 1), a.U) : a.U;
+  const int ulen = a.enc_lengths ? min(max(a.enc_lengths[bu], 1), a.U) : a.U;
   griddep_wait();
   griddep_launch();
   if (tr) { tr[1] = clock64(); tr[10] = gtime(); }
@@ -688,7 +691,9 @@ int launch_attend_cluster(const AttendArgs& a, bool pdl, cudaStream_t st) {
                   (size_t)AC_SLICES * (a.E + 4) + 4 /* barrier */ + (size_t)3 * a.E /* row-group sums */;
   const size_t smem = sizeof(float) * floats + 16;
   LAS_REQUIRE(smem <= 200 * 1024, "attention step needs %zu bytes of shared memory (U=%d E=%d)", smem, a.U, a.E);
-  LAS_CUDA_OK(cudaFuncSetAttribute(attend_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const bool shared = a.rows_per_utt > 1;
+  LAS_CUDA_OK(cudaFuncSetAttribute(shared ? attend_cluster_kernel<true> : attend_cluster_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   (int)smem));
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
   cfg.gridDim = dim3((unsigned)(a.B * C));
@@ -713,7 +718,7 @@ int launch_attend_cluster(const AttendArgs& a, bool pdl, cudaStream_t st) {
   cfg.numAttrs = n;
   AttendArgs at2 = a;
   at2.trace = fast_get_trace();
-  LAS_CUDA_OK(cudaLaunchKernelEx(&cfg, attend_cluster_kernel, at2, C));
+  LAS_CUDA_OK(cudaLaunchKernelEx(&cfg, shared ? attend_cluster_kernel<true> : attend_cluster_kernel<false>, at2, C));
   LAS_LAUNCH_OK("attend_cluster_kernel");
   return LAS_OK;
 }

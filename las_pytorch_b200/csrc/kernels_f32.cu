@@ -252,9 +252,10 @@ __global__ void __launch_bounds__(1024) attend_f32_kernel(AttendArgs a) {
   }
   __syncthreads();
 
-  const int ulen = a.enc_lengths ? min(max(a.enc_lengths[b], 1), a.U) : a.U;
-  const float* psib = a.psi + (size_t)b * a.U * a.D;
-  const float* encb = a.enc + (size_t)b * a.U * a.E;
+  const int bu = a.rows_per_utt > 1 ? b / a.rows_per_utt : b;  // the utterance whose encoder features row b attends over
+  const int ulen = a.enc_lengths ? min(max(a.enc_lengths[bu], 1), a.U) : a.U;
+  const float* psib = a.psi + (size_t)bu * a.U * a.D;
+  const float* encb = a.enc + (size_t)bu * a.U * a.E;
   for (int hd = 0; hd < NH; ++hd) {
     // energy[u] = <q_head, psi[b,u,:]>   (:289-291 / :299-305)
     const float* qh = s_q + hd * a.D;

@@ -2,6 +2,7 @@
 #include "las_kernels.cuh"
 #include "las_fast.cuh"
 
+#include <math.h>
 #include <string.h>
 
 namespace las {
@@ -366,6 +367,108 @@ static SpellerWsGen speller_ws_layout_gen(const las_speller_dims* d, void* base)
 // psi GEMM / cell GEMMs read bf16 rows through TMA: 16-byte aligned rows
 static bool gen_ok(const las_speller_dims* d) { return d->no_mlp || d->E % 8 == 0; }
 
+// psi = act(enc . W_psi^T + b_psi) of B utterances into `psi` (generic path: a bf16 copy of enc in `enc16` and a tcgen05 GEMM); without
+// the attention MLP the keys are the listener features themselves
+static const float* speller_psi(const las_speller_dims* d, int B, const SpellerPackF32& pk, const SpellerPackGen* gp, const float* enc, float* psi,
+                                __nv_bfloat16* enc16, int relu, cudaStream_t st, int* status) {
+  *status = LAS_OK;
+  if (d->no_mlp) return enc;  // use_mlp_in_attention=False (model/las_model.py:283-285)
+  const int U = d->U, E = d->E, D = d->D;
+  ProfScope ps("speller.psi", st);
+  if (gp) {
+    if ((*status = launch_f32_to_bf16(enc, enc16, (size_t)B * U * E, st)) != LAS_OK) return nullptr;
+    *status = launch_gemm_bf16_tc(enc16, E, gp->w_psi, E, pk.b_psi, psi, D, B * U, D, E, st, relu != 0);
+  } else {
+    *status = launch_sgemm_nt_bias(enc, E, pk.w_psi, E, pk.b_psi, psi, D, B * U, D, E, relu != 0, st);
+  }
+  return psi;
+}
+
+// One decoder step of the launch-per-step loop on `rows` decoder rows: the stacked cells (fused generic step, or per layer
+// lstm_cell_f32 / gen_build_a + GEMM + gen_cell), then the attention + character distribution with `t` (see speller_attend_args).
+struct StepPath {
+  const las_speller_dims* d;
+  int rows;
+  SpellerPackF32 pk;
+  const SpellerPackGen* gp;  // generic tensor-core path, else nullptr (fp32 mode)
+  GenGeom gg;
+  __nv_bfloat16* a;          // generic path: [rows, Kp_max] GEMM operand
+  float* pre;                // [rows, R] gate pre-activations
+  const float* zero;         // [256] zeros
+  float* xin;                // [rows, V+E] layer-0 input: fed-back word | context
+  float* c;                  // [sl, rows, Hs]
+  bool fused;                // fused generic step (gen_step.cu) with its operand rows in abuf
+  const GenStepMaps* maps;
+  __nv_bfloat16* (*abuf)[2];
+  bool cluster_att;          // attend_cluster_kernel instead of attend_f32_kernel
+};
+static AttendArgs speller_attend_args(const StepPath& p, const float* enc, const float* psi, const int32_t* enc_lengths, const float* hn, int relu) {
+  const las_speller_dims* d = p.d;
+  AttendArgs t;
+  memset(&t, 0, sizeof(t));
+  t.state = hn + (size_t)(d->sl - 1) * p.rows * d->Hs;
+  t.state_ld = d->Hs;
+  t.enc = enc;
+  t.psi = psi;
+  t.w_phi = d->no_mlp ? nullptr : p.pk.w_phi; t.b_phi = p.pk.b_phi; t.w_cd = p.pk.w_cd; t.b_cd = p.pk.b_cd;
+  t.enc_lengths = enc_lengths;
+  t.B = p.rows; t.U = d->U; t.E = d->E; t.Hs = d->Hs; t.V = d->V; t.D = att_dim(d);
+  t.relu = d->no_mlp ? 0 : relu;
+  t.heads = n_heads(d); t.w_dr = p.pk.w_dr; t.b_dr = p.pk.b_dr;
+  t.ctx_out = p.xin + d->V;
+  t.ctx_ld = d->V + d->E;
+  t.word_out = p.xin;
+  t.word_ld = d->V + d->E;
+  return t;
+}
+static int speller_step(const StepPath& p, int s, const float* hp, float* hn, const AttendArgs& t, cudaStream_t st) {
+  const las_speller_dims* d = p.d;
+  const int B = p.rows, Hs = d->Hs, sl = d->sl, xld = d->V + d->E;
+  const GenGeom& gg = p.gg;
+  for (int l = 0; l < sl; ++l) {
+    if (p.fused) {
+      const int q = s & 1;
+      LAS_TRY(launch_gen_cell_step(p.maps[l], q, p.gp->bias[l], p.c + (size_t)l * B * Hs, hp + (size_t)l * B * Hs, Hs, hn + (size_t)l * B * Hs, Hs,
+                                   p.abuf[l][q ^ 1] + gg.Kxp[l], gg.Kp[l], l + 1 < sl ? p.abuf[l + 1][q] : nullptr, l + 1 < sl ? gg.Kp[l + 1] : 0, B,
+                                   Hs, d->cell, gg.Kxp[l], gg.Kp[l], true, st, l));
+      continue;
+    }
+    if (p.gp) {
+      const float* xin_l = (l == 0) ? p.xin : hn + (size_t)(l - 1) * B * Hs;
+      const float* hp_l = hp + (size_t)l * B * Hs;
+      LAS_TRY(launch_gen_build_a(xin_l, (l == 0) ? xld : Hs, hp_l, Hs, p.a, B, Hs, gg.Kx[l], gg.Kxp[l], gg.Kp[l], st));
+      if (B <= 64) {
+        // Small batches: the GEMM's 128 x 256 tiles would leave it R/256 CTAs (16 at R = 4096), each streaming 1 MB of weights.  With
+        // the operands swapped -- "M" = the R weight rows, "N" = the batch -- R/128 CTAs stream half as much each; the result arrives
+        // transposed ([R, B]) and the cell kernel adds the bias.
+        LAS_TRY(launch_gemm_bf16_tc(p.gp->w[l], gg.Kp[l], p.a, gg.Kp[l], p.zero, p.pre, B, gg.R, B, gg.Kp[l], st));
+        LAS_TRY(launch_gen_cell(p.pre, 1, B, p.gp->bias[l], hp_l, Hs, p.c + (size_t)l * B * Hs, hn + (size_t)l * B * Hs, Hs, B, Hs, d->cell, st));
+      } else {
+        LAS_TRY(launch_gemm_bf16_tc(p.a, gg.Kp[l], p.gp->w[l], gg.Kp[l], p.gp->bias[l], p.pre, gg.R, B, gg.R, gg.Kp[l], st));
+        LAS_TRY(launch_gen_cell(p.pre, gg.R, 1, nullptr, hp_l, Hs, p.c + (size_t)l * B * Hs, hn + (size_t)l * B * Hs, Hs, B, Hs, d->cell, st));
+      }
+      continue;
+    }
+    CellArgs a;
+    memset(&a, 0, sizeof(a));
+    a.x = (l == 0) ? p.xin : hn + (size_t)(l - 1) * B * Hs;
+    a.x_ld = (l == 0) ? xld : Hs;
+    a.Kx = (l == 0) ? xld : Hs;
+    a.w_ih = p.pk.w_ih[l];
+    a.h_prev = hp + (size_t)l * B * Hs;
+    a.h_ld = Hs;
+    a.w_hh = p.pk.w_hh[l];
+    a.b_ih = p.pk.b_ih[l];
+    a.b_hh = p.pk.b_hh[l];
+    a.c = p.c + (size_t)l * B * Hs;
+    a.h_out = hn + (size_t)l * B * Hs;
+    a.hout_ld = Hs;
+    LAS_TRY(launch_lstm_cell_f32(&a, 1, B, Hs, st, d->cell));
+  }
+  if (p.cluster_att) return launch_attend_cluster(t, p.gp != nullptr, st);
+  return launch_attend_f32(t, st);
+}
+
 static int speller_decode_f32(const las_decode_io* io, const void* packed, const las_speller_dims* d, int steps,
                               int decode_mode, int relu, void* ws, cudaStream_t st, const void* packed_gen = nullptr, void* ws_gen = nullptr) {
   const SpellerPackF32 pk = speller_pack_layout_f32(d, const_cast<void*>(packed));
@@ -382,23 +485,16 @@ static int speller_decode_f32(const las_decode_io* io, const void* packed, const
     gw = speller_ws_layout_gen(d, ws_gen);
     LAS_CUDA_OK(cudaMemsetAsync(gw.zero, 0, sizeof(float) * 256, st));
   }
-  const int B = d->B, Hs = d->Hs, V = d->V, E = d->E, U = d->U, D = d->D, sl = d->sl;
+  const int B = d->B, Hs = d->Hs, V = d->V, E = d->E, U = d->U, sl = d->sl;
   const int xld = V + E;
   const size_t state_n = (size_t)sl * B * Hs;
 
   const int NH = n_heads(d);
   const float* psi = io->psi;
-  if (d->no_mlp) {
-    psi = io->enc;  // use_mlp_in_attention=False (model/las_model.py:283-285): the keys are the listener features themselves
-  } else if (!psi) {
-    ProfScope ps("speller.psi", st);
-    if (gen) {
-      LAS_TRY(launch_f32_to_bf16(io->enc, gw.enc, (size_t)B * U * E, st));
-      LAS_TRY(launch_gemm_bf16_tc(gw.enc, E, gp.w_psi, E, pk.b_psi, w.psi, D, B * U, D, E, st, relu != 0));
-    } else {
-      LAS_TRY(launch_sgemm_nt_bias(io->enc, E, pk.w_psi, E, pk.b_psi, w.psi, D, B * U, D, E, relu != 0, st));
-    }
-    psi = w.psi;
+  if (d->no_mlp || !psi) {
+    int status;
+    psi = speller_psi(d, B, pk, gen ? &gp : nullptr, io->enc, w.psi, gw.enc, relu, st, &status);
+    LAS_TRY(status);
   }
   if (io->word && io->context) {
     LAS_TRY(launch_copy2d(w.xin, xld, io->word, V, B, V, st));
@@ -432,68 +528,18 @@ static int speller_decode_f32(const las_decode_io* io, const void* packed, const
     }
   }
 
+  StepPath path;
+  path.d = d; path.rows = B; path.pk = pk; path.gp = gen ? &gp : nullptr; path.gg = gg;
+  path.a = gw.a; path.pre = gw.pre; path.zero = gw.zero; path.xin = w.xin; path.c = w.c;
+  path.fused = fused; path.maps = maps; path.abuf = abuf; path.cluster_att = cluster_att;
   ProfScope ps_steps("speller.steps", st);
   for (int s = 0; s < steps; ++s) {
     float* hp = w.h[s & 1];
     float* hn = w.h[(s & 1) ^ 1];
-    for (int l = 0; l < sl; ++l) {
-      if (fused) {
-        const int q = s & 1;
-        LAS_TRY(launch_gen_cell_step(maps[l], q, gp.bias[l], w.c + (size_t)l * B * Hs, hp + (size_t)l * B * Hs, Hs, hn + (size_t)l * B * Hs, Hs,
-                                     abuf[l][q ^ 1] + gg.Kxp[l], gg.Kp[l], l + 1 < sl ? abuf[l + 1][q] : nullptr, l + 1 < sl ? gg.Kp[l + 1] : 0, B,
-                                     Hs, d->cell, gg.Kxp[l], gg.Kp[l], true, st, l));
-        continue;
-      }
-      if (gen) {
-        const float* xin_l = (l == 0) ? w.xin : hn + (size_t)(l - 1) * B * Hs;
-        const float* hp_l = hp + (size_t)l * B * Hs;
-        LAS_TRY(launch_gen_build_a(xin_l, (l == 0) ? xld : Hs, hp_l, Hs, gw.a, B, Hs, gg.Kx[l], gg.Kxp[l], gg.Kp[l], st));
-        if (B <= 64) {
-          // Small batches: the GEMM's 128 x 256 tiles would leave it R/256 CTAs (16 at R = 4096), each streaming 1 MB of weights.  With
-          // the operands swapped -- "M" = the R weight rows, "N" = the batch -- R/128 CTAs stream half as much each; the result arrives
-          // transposed ([R, B]) and the cell kernel adds the bias.
-          LAS_TRY(launch_gemm_bf16_tc(gp.w[l], gg.Kp[l], gw.a, gg.Kp[l], gw.zero, gw.pre, B, gg.R, B, gg.Kp[l], st));
-          LAS_TRY(launch_gen_cell(gw.pre, 1, B, gp.bias[l], hp_l, Hs, w.c + (size_t)l * B * Hs, hn + (size_t)l * B * Hs, Hs, B, Hs, d->cell, st));
-        } else {
-          LAS_TRY(launch_gemm_bf16_tc(gw.a, gg.Kp[l], gp.w[l], gg.Kp[l], gp.bias[l], gw.pre, gg.R, B, gg.R, gg.Kp[l], st));
-          LAS_TRY(launch_gen_cell(gw.pre, gg.R, 1, nullptr, hp_l, Hs, w.c + (size_t)l * B * Hs, hn + (size_t)l * B * Hs, Hs, B, Hs, d->cell, st));
-        }
-        continue;
-      }
-      CellArgs a;
-      memset(&a, 0, sizeof(a));
-      a.x = (l == 0) ? w.xin : hn + (size_t)(l - 1) * B * Hs;
-      a.x_ld = (l == 0) ? xld : Hs;
-      a.Kx = (l == 0) ? xld : Hs;
-      a.w_ih = pk.w_ih[l];
-      a.h_prev = hp + (size_t)l * B * Hs;
-      a.h_ld = Hs;
-      a.w_hh = pk.w_hh[l];
-      a.b_ih = pk.b_ih[l];
-      a.b_hh = pk.b_hh[l];
-      a.c = w.c + (size_t)l * B * Hs;
-      a.h_out = hn + (size_t)l * B * Hs;
-      a.hout_ld = Hs;
-      LAS_TRY(launch_lstm_cell_f32(&a, 1, B, Hs, st, d->cell));
-    }
-    AttendArgs t;
-    memset(&t, 0, sizeof(t));
-    t.state = hn + (size_t)(sl - 1) * B * Hs;
-    t.state_ld = Hs;
-    t.enc = io->enc;
-    t.psi = psi;
-    t.w_phi = d->no_mlp ? nullptr : pk.w_phi; t.b_phi = pk.b_phi; t.w_cd = pk.w_cd; t.b_cd = pk.b_cd;
-    t.enc_lengths = io->enc_lengths;
-    t.B = B; t.U = U; t.E = E; t.Hs = Hs; t.V = V; t.D = att_dim(d);
-    t.relu = d->no_mlp ? 0 : relu;
-    t.heads = NH; t.w_dr = pk.w_dr; t.b_dr = pk.b_dr;
+    AttendArgs t = speller_attend_args(path, io->enc, psi, io->enc_lengths, hn, relu);
     t.score_out = io->attn ? io->attn + (size_t)s * NH * B * U : nullptr;
-    t.ctx_out = w.xin + V;
-    t.ctx_ld = xld;
     t.logp_out = io->logp + (size_t)s * B * V;
     t.token_out = io->tokens ? io->tokens + (size_t)s * B : nullptr;
-    t.word_out = w.xin;
-    t.word_ld = xld;
     if (io->gt_dense) {
       t.gt_dense_step = io->gt_dense + (size_t)s * V;
       t.gt_ld = (long long)io->gt_steps * V;
@@ -514,8 +560,7 @@ static int speller_decode_f32(const las_decode_io* io, const void* packed, const
       t.op_ld = gg.Kp[0];
       t.op_f16 = op_f16();
     }
-    if (cluster_att) LAS_TRY(launch_attend_cluster(t, gen, st));
-    else LAS_TRY(launch_attend_f32(t, st));
+    LAS_TRY(speller_step(path, s, hp, hn, t, st));
   }
   if (io->h_state && (io->c_state || d->cell != LAS_CELL_LSTM)) {
     LAS_CUDA_OK(cudaMemcpyAsync(io->h_state, w.h[steps & 1], sizeof(float) * state_n, cudaMemcpyDeviceToDevice, st));
@@ -540,6 +585,113 @@ static int speller_decode_f32(const las_decode_io* io, const void* packed, const
     }
   }
   return LAS_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// Beam search (include/las_b200.h las_beam_io) on the launch-per-step decoder: B*K decoder rows, row b*K + k = hypothesis k of
+// utterance b.  The whole recurrent state is xin / h / c in fp32, so beam_step_kernel reorders hypotheses with a row gather.
+// ---------------------------------------------------------------------------------------------------------
+static int beam_args_check(const las_speller_dims* d, int steps, int beam) {
+  LAS_TRY(speller_check(d));
+  LAS_REQUIRE(beam >= 1 && beam <= 32, "beam width must be in [1, 32] (beam=%d)", beam);
+  LAS_REQUIRE(steps >= 1, "beam search needs steps >= 1 (steps=%d)", steps);
+  return LAS_OK;
+}
+struct BeamWs {
+  float* psi;        // [B*U, D] (per utterance)
+  float* xin;        // [BK, V+E]
+  float* h[2];       // [sl, BK, Hs]
+  float* c;          // [sl, BK, Hs]
+  float* logp;       // [BK, V] one step's log-probabilities
+  float* score;      // [BK]
+  int32_t* fin;      // [BK]
+  int32_t* parent;   // [S, B, K] back-pointers
+  int32_t* token;    // [S, B, K]
+  float* token_logp; // [S, B, K]
+  // generic tensor-core path
+  __nv_bfloat16* a;  // [BK, Kp_max]
+  float* pre;        // [BK, R]
+  __nv_bfloat16* enc16;  // [B*U, E]
+  float* zero;       // [256]
+  size_t bytes;
+};
+static BeamWs beam_ws_layout(const las_speller_dims* d, int steps, int beam, bool gen, void* base) {
+  BeamWs w;
+  Carver cv(base);
+  const size_t B = d->B, BK = B * beam;
+  w.psi = cv.take<float>(B * d->U * (d->no_mlp ? 0 : d->D));
+  w.xin = cv.take<float>(BK * (d->V + d->E));
+  w.h[0] = cv.take<float>((size_t)d->sl * BK * d->Hs);
+  w.h[1] = cv.take<float>((size_t)d->sl * BK * d->Hs);
+  w.c = cv.take<float>((size_t)d->sl * BK * d->Hs);
+  w.logp = cv.take<float>(BK * d->V);
+  w.score = cv.take<float>(BK);
+  w.fin = cv.take<int32_t>(BK);
+  w.parent = cv.take<int32_t>((size_t)steps * BK);
+  w.token = cv.take<int32_t>((size_t)steps * BK);
+  w.token_logp = cv.take<float>((size_t)steps * BK);
+  const GenGeom g = gen_geom(d);
+  w.a = cv.take<__nv_bfloat16>(gen ? BK * g.Kp_max : 0);
+  w.pre = cv.take<float>(gen ? BK * g.R : 0);
+  w.enc16 = cv.take<__nv_bfloat16>(gen && !d->no_mlp ? B * d->U * d->E : 0);
+  w.zero = cv.take<float>(gen ? 256 : 0);
+  w.bytes = cv.total();
+  return w;
+}
+
+static int speller_beam_f32(const las_beam_io* io, const void* packed, const las_speller_dims* d, int steps, int relu, void* ws, cudaStream_t st,
+                            const void* packed_gen) {
+  const int B = d->B, K = io->beam, BK = B * K, V = d->V, E = d->E, Hs = d->Hs;
+  const bool gen = packed_gen != nullptr;
+  const SpellerPackF32 pk = speller_pack_layout_f32(d, const_cast<void*>(packed));
+  SpellerPackGen gp;
+  memset(&gp, 0, sizeof(gp));
+  if (gen) gp = speller_pack_layout_gen(d, const_cast<void*>(packed_gen));
+  const BeamWs w = beam_ws_layout(d, steps, K, gen, ws);
+  if (gen) LAS_CUDA_OK(cudaMemsetAsync(w.zero, 0, sizeof(float) * 256, st));
+  las_speller_dims dk = *d;  // the decoder sees B*K rows
+  dk.B = BK;
+
+  int status;
+  const float* psi = speller_psi(d, B, pk, gen ? &gp : nullptr, io->enc, w.psi, w.enc16, relu, st, &status);  // once per utterance
+  LAS_TRY(status);
+  LAS_TRY(launch_beam_init(w.xin, V + E, io->enc, w.score, w.fin, B, K, d->U, E, V, st));
+  const size_t state_n = (size_t)d->sl * BK * Hs;
+  LAS_CUDA_OK(cudaMemsetAsync(w.h[0], 0, sizeof(float) * state_n, st));
+  LAS_CUDA_OK(cudaMemsetAsync(w.c, 0, sizeof(float) * state_n, st));
+
+  StepPath path;
+  memset(&path, 0, sizeof(path));
+  path.d = &dk; path.rows = BK; path.pk = pk; path.gp = gen ? &gp : nullptr; path.gg = gen_geom(d);
+  path.a = w.a; path.pre = w.pre; path.zero = w.zero; path.xin = w.xin; path.c = w.c;
+  path.cluster_att = n_heads(d) == 1 && E % 4 == 0 && gen_step_fused(1);  // the greedy step's choice
+  BeamStepArgs ba;
+  memset(&ba, 0, sizeof(ba));
+  ba.logp = w.logp; ba.score = w.score; ba.fin = w.fin;
+  ba.c = d->cell == LAS_CELL_LSTM ? w.c : nullptr;
+  ba.xin = w.xin; ba.xld = V + E;
+  ba.B = B; ba.K = K; ba.V = V; ba.E = E; ba.Hs = Hs; ba.sl = d->sl; ba.eos = io->eos_token;
+  ProfScope ps_steps("speller.beam_steps", st);
+  for (int s = 0; s < steps; ++s) {
+    float* hp = w.h[s & 1];
+    float* hn = w.h[(s & 1) ^ 1];
+    AttendArgs t = speller_attend_args(path, io->enc, psi, io->enc_lengths, hn, relu);
+    t.rows_per_utt = K;
+    t.word_out = nullptr;  // beam_step_kernel writes the fed-back words
+    t.logp_out = w.logp;
+    LAS_TRY(speller_step(path, s, hp, hn, t, st));
+    ba.parent = w.parent + (size_t)s * BK;
+    ba.token = w.token + (size_t)s * BK;
+    ba.token_logp = w.token_logp + (size_t)s * BK;
+    ba.h = hn;
+    LAS_TRY(launch_beam_step(ba, st));
+  }
+  BeamFinalArgs fa;
+  memset(&fa, 0, sizeof(fa));
+  fa.score = w.score; fa.parent = w.parent; fa.token = w.token; fa.token_logp = w.token_logp;
+  fa.tokens_out = io->tokens; fa.token_logp_out = io->token_logp; fa.lengths_out = io->lengths; fa.scores_out = io->scores;
+  fa.B = B; fa.K = K; fa.N = io->nbest; fa.S = steps; fa.eos = io->eos_token; fa.alpha = io->length_penalty;
+  return launch_beam_finalize(fa, st);
 }
 
 }  // namespace las
@@ -680,8 +832,9 @@ size_t las_speller_packed_bytes(const las_speller_dims* d, int mode) {
   return f32;
 }
 
-int las_speller_pack(const las_speller_weights* w, const las_speller_dims* d, int mode, void* packed, size_t packed_bytes,
-                     void* stream) {
+// generic_layout: the tensor-core modes pack the generic step's layout even where the persistent decoder covers the shape (beam pack)
+static int speller_pack(const las_speller_weights* w, const las_speller_dims* d, int mode, void* packed, size_t packed_bytes, void* stream,
+                        bool generic_layout) {
   set_operand_mode(mode);
   LAS_TRY(speller_check(d));
   LAS_REQUIRE(w && packed && w->rnn_host, "null weights / packed buffer");
@@ -689,11 +842,12 @@ int las_speller_pack(const las_speller_weights* w, const las_speller_dims* d, in
   LAS_REQUIRE(w->w_cd && w->b_cd, "null output weight pointer");
   LAS_REQUIRE(d->no_mlp || (w->w_phi && w->b_phi && w->w_psi && w->b_psi), "null attention weight pointer");
   LAS_REQUIRE(n_heads(d) == 1 || (w->w_dr && w->b_dr), "multi_head > 1 needs attention.dim_reduce weights");
-  LAS_REQUIRE(!tc_mode(mode) || fast_speller_fits(d) || gen_ok(d),
+  const bool fast = tc_mode(mode) && fast_speller_fits(d) && !generic_layout;
+  LAS_REQUIRE(!tc_mode(mode) || fast || gen_ok(d),
               "LAS_MODE_BF16 needs E %% 8 == 0 for the psi GEMM's TMA rows (E=%d); use LAS_MODE_FP32", d->E);
   LAS_TRY(device_ok());
-  if (packed_bytes < las_speller_packed_bytes(d, mode))
-    return fail(LAS_ENOMEM, "packed buffer too small: %zu < %zu", packed_bytes, las_speller_packed_bytes(d, mode));
+  const size_t need = generic_layout ? las_speller_beam_packed_bytes(d, mode) : las_speller_packed_bytes(d, mode);
+  if (packed_bytes < need) return fail(LAS_ENOMEM, "packed buffer too small: %zu < %zu", packed_bytes, need);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const SpellerPackF32 pk = speller_pack_layout_f32(d, packed);
   const size_t G = (size_t)n_gates(d->cell) * d->Hs;
@@ -720,7 +874,7 @@ int las_speller_pack(const las_speller_weights* w, const las_speller_dims* d, in
     CP(pk.b_dr, w->b_dr, d->E);
   }
 #undef CP
-  if (tc_mode(mode) && fast_speller_fits(d)) return fast_speller_pack(w, d, static_cast<char*>(packed) + pk.bytes, st);
+  if (fast) return fast_speller_pack(w, d, static_cast<char*>(packed) + pk.bytes, st);
   if (tc_mode(mode)) {  // generic tensor-core path: [W_ih | W_hh] per layer as one bf16 matrix, psi weights in bf16
     const SpellerPackGen gp = speller_pack_layout_gen(d, static_cast<char*>(packed) + pk.bytes);
     const GenGeom g = gen_geom(d);
@@ -731,6 +885,11 @@ int las_speller_pack(const las_speller_weights* w, const las_speller_dims* d, in
     if (!d->no_mlp) LAS_TRY(launch_f32_to_bf16(w->w_psi, gp.w_psi, (size_t)d->D * d->E, st));
   }
   return LAS_OK;
+}
+
+int las_speller_pack(const las_speller_weights* w, const las_speller_dims* d, int mode, void* packed, size_t packed_bytes,
+                     void* stream) {
+  return speller_pack(w, d, mode, packed, packed_bytes, stream, false);
 }
 
 int las_psi_precompute(const float* enc, const float* w_psi, const float* b_psi, int B, int U, int E, int D, int relu,
@@ -805,6 +964,42 @@ int las_speller_decode(const las_decode_io* io, const void* packed, const las_sp
                                static_cast<char*>(workspace) + f32w, st);
   }
   return speller_decode_f32(io, packed, d, steps, decode_mode, relu, workspace, st);
+}
+
+// ---- beam search -----------------------------------------------------------------------------------------
+size_t las_speller_beam_packed_bytes(const las_speller_dims* d, int mode) {
+  if (speller_check(d) != LAS_OK) return 0;
+  if (mode != LAS_MODE_FP32 && !tc_mode(mode)) return 0;
+  const size_t f32 = speller_pack_layout_f32(d, nullptr).bytes;
+  return tc_mode(mode) ? f32 + speller_pack_layout_gen(d, nullptr).bytes : f32;
+}
+
+int las_speller_beam_pack(const las_speller_weights* w, const las_speller_dims* d, int mode, void* packed, size_t bytes, void* stream) {
+  return speller_pack(w, d, mode, packed, bytes, stream, true);
+}
+
+size_t las_speller_beam_workspace_bytes(const las_speller_dims* d, int steps, int beam, int mode) {
+  if (beam_args_check(d, steps, beam) != LAS_OK) return 0;
+  if (mode != LAS_MODE_FP32 && !tc_mode(mode)) return 0;
+  return beam_ws_layout(d, steps, beam, tc_mode(mode), nullptr).bytes;
+}
+
+int las_speller_beam_search(const las_beam_io* io, const void* packed, const las_speller_dims* d, int steps, int mode, int relu,
+                            void* workspace, size_t workspace_bytes, void* stream) {
+  set_operand_mode(mode);
+  LAS_REQUIRE(io && packed && workspace, "null pointer argument");
+  LAS_TRY(beam_args_check(d, steps, io->beam));
+  LAS_REQUIRE(io->enc && io->tokens && io->lengths && io->scores, "io->enc, io->tokens, io->lengths and io->scores are required");
+  LAS_REQUIRE(io->nbest >= 1 && io->nbest <= io->beam, "nbest must be in [1, beam] (nbest=%d beam=%d)", io->nbest, io->beam);
+  LAS_REQUIRE(io->eos_token >= 0 && io->eos_token < d->V, "eos_token %d is not in [0, V=%d)", io->eos_token, d->V);
+  LAS_REQUIRE(isfinite(io->length_penalty) && io->length_penalty >= 0.f, "length_penalty must be finite and >= 0 (%g)", (double)io->length_penalty);
+  LAS_REQUIRE(mode == LAS_MODE_FP32 || tc_mode(mode), "unknown mode %d", mode);
+  LAS_REQUIRE(!tc_mode(mode) || gen_ok(d), "LAS_MODE_BF16 beam search needs E %% 8 == 0 (E=%d); use LAS_MODE_FP32", d->E);
+  LAS_TRY(device_ok());
+  const size_t need = las_speller_beam_workspace_bytes(d, steps, io->beam, mode);
+  if (workspace_bytes < need) return fail(LAS_ENOMEM, "workspace too small: %zu < %zu", workspace_bytes, need);
+  const void* packed_gen = tc_mode(mode) ? static_cast<const char*>(packed) + speller_pack_layout_f32(d, nullptr).bytes : nullptr;
+  return speller_beam_f32(io, packed, d, steps, relu, workspace, static_cast<cudaStream_t>(stream), packed_gen);
 }
 
 int las_pipeline_step(const las_pipeline_args* a, int mode, void* stream) {

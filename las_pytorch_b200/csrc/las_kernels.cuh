@@ -44,6 +44,7 @@ struct AttendArgs {
   const float* b_cd;
   const int32_t* enc_lengths;  // nullable
   int B, U, E, Hs, V, D;
+  int rows_per_utt;     // 0 or 1: one decoder row per utterance; R > 1: rows b*R .. b*R+R-1 share enc / psi / enc_lengths of utterance b
   int relu;
   int heads;            // >= 1; phi has D*heads outputs, each head attends over the same psi
   const float* w_dr;    // [E, E*heads] (heads > 1)
@@ -95,6 +96,37 @@ int launch_gen_build_a(const float* x, long long x_ld, const float* h, long long
                        cudaStream_t st);
 int launch_gen_cell(const float* pre, long long ldb, long long ldr, const float* bias, const float* h_prev, long long h_ld, float* c, float* h_out,
                     long long hout_ld, int B, int H, int cell, cudaStream_t st);
+
+// beam search (beam_search.cu): B utterances of K rows each
+// xin[r, 0:V] = onehot(0), xin[r, V:V+E] = enc[r / K, 0, :]; score[r] = 0 for r % K == 0, else -inf; fin[r] = 0
+int launch_beam_init(float* xin, int xin_ld, const float* enc, float* score, int32_t* fin, int B, int K, int U, int E, int V, cudaStream_t st);
+struct BeamStepArgs {
+  const float* logp;       // [B*K, V] this step's log-probabilities
+  float* score;            // [B*K] in/out
+  int32_t* fin;            // [B*K] in/out: the row has emitted eos
+  int32_t* parent;         // [B, K] this step's back-pointers (slice of [S, B, K])
+  int32_t* token;          // [B, K]
+  float* token_logp;       // [B, K]
+  float* h;                // [sl, B*K, Hs] the state the next step reads; permuted in place
+  float* c;                // nullable [sl, B*K, Hs]
+  float* xin;              // [B*K, xld]: word [V] | context [E]; word written, context permuted
+  int xld;
+  int B, K, V, E, Hs, sl, eos;
+};
+int launch_beam_step(const BeamStepArgs& a, cudaStream_t st);
+struct BeamFinalArgs {
+  const float* score;      // [B*K]
+  const int32_t* parent;   // [S, B, K]
+  const int32_t* token;
+  const float* token_logp;
+  int32_t* tokens_out;     // [B, N, S]
+  float* token_logp_out;   // nullable [B, N, S]
+  int32_t* lengths_out;    // [B, N]
+  float* scores_out;       // [B, N]
+  int B, K, N, S, eos;
+  float alpha;
+};
+int launch_beam_finalize(const BeamFinalArgs& a, cudaStream_t st);
 
 // <eos> early exit bookkeeping (las_decode_io.early_exit): `state` = 66 int32 {stop, steps decoded, done[64]} per launch group
 int launch_eos_check(const int32_t* tokens, int Bfull, int b0, int Bc, int s_begin, int s_end, int eos, int32_t* state, cudaStream_t st);

@@ -18,7 +18,9 @@ reproducible under torch.manual_seed but not draw-for-draw equal to the referenc
 """
 from __future__ import annotations
 
+import collections
 import ctypes as C
+import math
 import os
 import threading
 
@@ -27,7 +29,7 @@ import torch
 import torch.nn as nn
 
 from . import _cabi
-from ._cabi import DecodeIO, ListenerDims, LstmWeights, SpellerDims, SpellerWeights, check, current_stream_ptr, ptr
+from ._cabi import BeamIO, DecodeIO, ListenerDims, LstmWeights, SpellerDims, SpellerWeights, check, current_stream_ptr, ptr
 from .params import LinearWeights, LSTMWeights
 
 _MODES = {"fp32": _cabi.MODE_FP32, "bf16": _cabi.MODE_BF16, "fp16": _cabi.MODE_F16}
@@ -237,6 +239,18 @@ class LAS(nn.Module):
                                                           enc_lengths=enc_lengths, nll_labels=nll_labels)
         return raw_pred_seq, attention_record
 
+    def beam_search(self, batch_data, beam_width=8, nbest=1, length_penalty=0.0, input_lengths=None):
+        """Beam-search decoding (extension; the reference decodes greedily): the listener (with the length mask when
+        `input_lengths` is given), then `Speller.beam_search` over `max_label_len` steps.  Returns a BeamSearchResult."""
+        _check_beam_args(beam_width, nbest, length_penalty, self.speller.max_label_len)
+        enc_lengths = None
+        if input_lengths is None:
+            listener_feature = self.listener(batch_data)
+        else:
+            listener_feature, enc_lengths = self.listener(batch_data, input_lengths=input_lengths)
+        return self.speller.beam_search(listener_feature, beam_width=beam_width, nbest=nbest, length_penalty=length_penalty,
+                                        enc_lengths=enc_lengths)
+
     # ---- large free-running batches: the serving pipeline applied INSIDE one forward call ------------------------------------
     CHUNK = 64  # utterances per persistent decoder launch group (one attention CTA each next to the 64 LSTM CTAs)
 
@@ -384,6 +398,25 @@ class ServingPipeline:
         sp = self.las.speller
         logp, attn, tokens = sp._decode(enc, sp.max_label_len, enc_lengths=enc_lens, want_attn=self.want_attention)
         return ServingResult(logp, attn[:, 0] if attn is not None and attn.size(1) == 1 else attn, tokens)
+
+
+BeamSearchResult = collections.namedtuple("BeamSearchResult", ["tokens", "lengths", "scores", "token_logp"])
+BeamSearchResult.__doc__ = """n-best hypotheses per utterance, best first (device tensors): tokens [B,N,S] int32 (<eos> after the end), lengths
+[B,N] int32 (tokens up to and including the first <eos>, or S), scores [B,N] fp32 (sum of token_logp), token_logp [B,N,S] fp32 (0 after
+the end)."""
+
+
+def _check_beam_args(beam_width, nbest, length_penalty, steps):
+    """The library's limits, checked on the host so that bad arguments fail before anything reaches the device."""
+    if isinstance(beam_width, bool) or not isinstance(beam_width, int) or not 1 <= beam_width <= 32:
+        raise ValueError(f"beam_width must be an int in [1, 32], got {beam_width!r}")
+    if isinstance(nbest, bool) or not isinstance(nbest, int) or not 1 <= nbest <= beam_width:
+        raise ValueError(f"nbest must be an int in [1, beam_width={beam_width}], got {nbest!r}")
+    if isinstance(length_penalty, bool) or not isinstance(length_penalty, (int, float)) or not math.isfinite(length_penalty) \
+            or length_penalty < 0:
+        raise ValueError(f"length_penalty must be a finite number >= 0, got {length_penalty!r}")
+    if isinstance(steps, bool) or not isinstance(steps, int) or steps < 1:
+        raise ValueError(f"the number of decoder steps must be an int >= 1, got {steps!r}")
 
 
 def _check_unit(rnn_unit, precision="fp32"):
@@ -562,14 +595,16 @@ class Speller(nn.Module):
                            at.preprocess_mlp_dim if at.mlp_preprocess_input else 0, at.multi_head, 0 if at.mlp_preprocess_input else 1,
                            _cabi.CELLS[self.cell])
 
-    def _packed(self, lib, dims, mode, device, st):
+    def _packed(self, lib, dims, mode, device, st, beam=False):
+        """Packed weights of the greedy decoder, or with `beam` those of beam search (las_speller_beam_pack), cached side by side."""
         tensors = _weight_tensors(self)
         for w in tensors:
             _require_cuda(w, "speller weight")
             if w.device != device:
                 raise RuntimeError(f"speller weights are on {w.device}, listener_feature on {device}")
-        key = _Cache.tensors_key(tensors, mode)
-        packed = self._cache.lookup(device, mode, key, getattr(self, "_is_replica", False))
+        slot = ("beam", mode) if beam else mode
+        key = _Cache.tensors_key(tensors, slot)
+        packed = self._cache.lookup(device, slot, key, getattr(self, "_is_replica", False))
         if packed is None:
             arr, keep = _lstm_weight_array(self.rnn_layer, self.num_layers, 1)
             at, cd = self.attention, self.character_distribution
@@ -585,10 +620,12 @@ class Speller(nn.Module):
                 td = [_f32c(t) for t in (at.dim_reduce.weight, at.dim_reduce.bias)]
                 w.w_dr, w.b_dr = (t.data_ptr() for t in td)
                 ts += td
-            nbytes = lib.las_speller_packed_bytes(C.byref(dims), mode)
+            size_fn, pack_fn = (lib.las_speller_beam_packed_bytes, lib.las_speller_beam_pack) if beam else \
+                (lib.las_speller_packed_bytes, lib.las_speller_pack)
+            nbytes = size_fn(C.byref(dims), mode)
             packed = torch.empty(max(nbytes, 256), dtype=torch.uint8, device=device)
-            check(lib.las_speller_pack(C.byref(w), C.byref(dims), mode, ptr(packed), packed.numel(), st))
-            self._cache.store(device, mode, key, packed)
+            check(pack_fn(C.byref(w), C.byref(dims), mode, ptr(packed), packed.numel(), st))
+            self._cache.store(device, slot, key, packed)
             del keep, ts
         return packed
 
@@ -675,6 +712,45 @@ class Speller(nn.Module):
             check(c.lib.las_speller_decode(C.byref(c.io), ptr(c.packed), C.byref(c.dims), steps, c.decode_mode, c.mode, c.relu, ptr(c.ws),
                                            c.ws.numel(), c.st))
         return c.logp, c.attn, c.tokens
+
+    def beam_search(self, listener_feature, beam_width=8, nbest=1, length_penalty=0.0, enc_lengths=None, max_steps=None):
+        """Beam-search decoding on the device (extension; include/las_b200.h las_speller_beam_search has the exact semantics).
+        Every utterance keeps `beam_width` hypotheses for `max_steps` (default max_label_len) steps; a hypothesis ends at <eos>
+        (`self.eos_token`, default 1).  The `nbest` best by score / length**length_penalty are returned, best first, as a
+        BeamSearchResult of device tensors.  Draws nothing from numpy's or torch's random generators."""
+        steps = self.max_label_len if max_steps is None else max_steps
+        _check_beam_args(beam_width, nbest, length_penalty, steps)
+        eos = getattr(self, "eos_token", 1)
+        if not 0 <= eos < self.label_dim:
+            raise ValueError(f"eos_token {eos} is not in [0, {self.label_dim})")
+        if listener_feature.dim() != 3 or listener_feature.size(2) != self.hidden_size:
+            raise ValueError(f"listener_feature has shape {tuple(listener_feature.shape)}; expected [B, U, {self.hidden_size}]")
+        b, u, e = listener_feature.shape
+        if enc_lengths is not None and enc_lengths.numel() != b:
+            raise ValueError(f"enc_lengths has {enc_lengths.numel()} entries for a batch of {b}")
+        _require_cuda(listener_feature, "listener_feature")
+        lib = _cabi.load_library()
+        dev = listener_feature.device
+        mode = _mode_of(self.precision)
+        with torch.cuda.device(dev), self._cache.enqueue_lock(dev):
+            enc = _f32c(listener_feature)
+            dims = self._dims(b, u, e)
+            st = current_stream_ptr(dev)
+            packed = self._packed(lib, dims, mode, dev, st, beam=True)
+            ws_bytes = lib.las_speller_beam_workspace_bytes(C.byref(dims), steps, beam_width, mode)
+            ws = self._cache.workspace(("beam", dev, mode, st.value), ws_bytes, dev)
+            lens = None if enc_lengths is None else enc_lengths.to(device=dev, dtype=torch.int32).contiguous()
+            out = BeamSearchResult(tokens=torch.empty(b, nbest, steps, dtype=torch.int32, device=dev),
+                                   lengths=torch.empty(b, nbest, dtype=torch.int32, device=dev),
+                                   scores=torch.empty(b, nbest, dtype=torch.float32, device=dev),
+                                   token_logp=torch.empty(b, nbest, steps, dtype=torch.float32, device=dev))
+            io = BeamIO()
+            io.enc, io.enc_lengths = enc.data_ptr(), (lens.data_ptr() if lens is not None else None)
+            io.beam, io.nbest, io.eos_token, io.length_penalty = beam_width, nbest, eos, float(length_penalty)
+            io.tokens, io.token_logp, io.lengths, io.scores = (t.data_ptr() for t in (out.tokens, out.token_logp, out.lengths, out.scores))
+            check(lib.las_speller_beam_search(C.byref(io), ptr(packed), C.byref(dims), steps, mode, self.attention.relu_flag, ptr(ws),
+                                              ws.numel(), st))
+        return out
 
     # ---- reference API ---------------------------------------------------------------------------------
     def forward_step(self, input_word, last_hidden_state, listener_feature):
