@@ -82,13 +82,13 @@ int fast_pipeline_bc(const las_listener_dims* ld, const las_speller_dims* sd, in
   return 0;
 }
 
-int fast_pipeline_step(const las_decode_io* io, const void* spl_packed_f32, const void* spl_packed_fast, const las_speller_dims* sd, int steps,
-                       int decode_mode, int relu, void* spl_ws_f32, void* spl_ws_fast, const float* x, const int32_t* x_lengths,
-                       const void* lis_packed, const las_listener_dims* ld, float* enc, int32_t* enc_lengths, void* lis_ws, cudaStream_t st) {
+int fast_pipeline_step(const las_decode_io* io, const SpellerF32Inputs& spl_f32, const void* spl_packed_fast, const las_speller_dims* sd,
+                       int steps, int decode_mode, int relu, void* spl_ws_fast, const float* x, const int32_t* x_lengths, const void* lis_packed,
+                       const las_listener_dims* ld, float* enc, int32_t* enc_lengths, void* lis_ws, cudaStream_t st) {
   const int bc = fast_pipeline_bc(ld, sd, steps);
   if (bc == 0 || io->early_exit) {
     // no room next to the decoder (or a decoder that may stop early): one after the other
-    LAS_TRY(fast_speller_decode(io, spl_packed_f32, spl_packed_fast, sd, steps, decode_mode, relu, spl_ws_f32, spl_ws_fast, st));
+    LAS_TRY(fast_speller_decode(io, spl_f32, spl_packed_fast, sd, steps, decode_mode, relu, spl_ws_fast, st));
     return fast_listener_forward(x, x_lengths, lis_packed, ld, enc, enc_lengths, lis_ws, st);
   }
   PipeEvents* pe = nullptr;
@@ -127,8 +127,8 @@ int fast_pipeline_step(const las_decode_io* io, const void* spl_packed_f32, cons
     // ... then the decoder's segment on the SMs it leaves free
     wait_resident_kernel<<<1, 1, 0, st>>>(pe->resident + l, rec_ctas);
     LAS_LAUNCH_OK("wait_resident_kernel");
-    LAS_TRY(fast_speller_decode_segment(io, spl_packed_f32, spl_packed_fast, sd, 0, Bc, sb, seg[l], sb == 0, l == L - 1, decode_mode, relu,
-                                        spl_ws_f32, spl_ws_fast, st));
+    LAS_TRY(fast_speller_decode_segment(io, spl_f32, spl_packed_fast, sd, 0, Bc, sb, seg[l], sb == 0, l == L - 1, decode_mode, relu, spl_ws_fast,
+                                        st));
     sb += seg[l];
     LAS_CUDA_OK(cudaStreamWaitEvent(st, pe->rec_done[l], 0));
     if (l + 1 < L) {

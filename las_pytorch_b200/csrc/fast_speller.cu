@@ -1530,14 +1530,13 @@ struct RingCfg {
   int box_rows, stage_bytes, nstages;
   size_t smem;
 };
-// ring geometry for a launch covering `rows` utterances: as many stages as shared memory allows (up to 12), so that a
-// whole step's critical input can be in flight at once
-RingCfg ring_cfg(const las_speller_dims* d, int rows) {
+// ring geometry of a launch (64-row boxes; a launch with two utterance groups narrows them to 32 rows): as many stages as shared
+// memory allows (up to 12), so that a whole step's critical input can be in flight at once
+RingCfg ring_cfg(const las_speller_dims* d) {
   const Shape s = shape_of(d);
   int mx = 0;
   for (int l = 0; l < d->sl; ++l) mx = s.natoms[l] > mx ? s.natoms[l] : mx;
   RingCfg r;
-  (void)rows;
   r.box_rows = 64;
   r.stage_bytes = r.box_rows * 128;
   const size_t fixed = (size_t)mx * WATOM_BYTES + DEC_NW * 4 + (DEC_MAX_STAGES + 4) * 8 + 64 + 64 * 20 * 4;  // + the epilogue's staging block
@@ -1546,7 +1545,7 @@ RingCfg ring_cfg(const las_speller_dims* d, int rows) {
   const int nc0 = (d->E + 63) / 64;
   if (nc0 > need) need = nc0;
   r.nstages = need + 1;
-  r.smem = fixed + (size_t)r.nstages * r.stage_bytes + (r.box_rows == 64 ? 0 : 0);
+  r.smem = fixed + (size_t)r.nstages * r.stage_bytes;
   return r;
 }
 bool att_wreg(const las_speller_dims* d) { return d->D <= DEC_THREADS / 8 && d->Hs <= 512; }
@@ -1581,7 +1580,7 @@ int supported(const las_speller_dims* d) {
   LAS_REQUIRE(d->V <= DEC_VP, "LAS_MODE_BF16 speller supports vocabularies up to %d (V=%d)", DEC_VP, d->V);
   LAS_REQUIRE(d->E % 8 == 0 && d->E / 8 <= DEC_THREADS, "LAS_MODE_BF16 speller needs E %% 8 == 0 and E <= 4096 (E=%d)", d->E);
   LAS_REQUIRE(d->U <= ATT_MAXP * 256, "LAS_MODE_BF16 speller supports at most %d encoder steps (U=%d)", ATT_MAXP * 256, d->U);
-  LAS_REQUIRE(att_smem(d, false) <= 220 * 1024 && ring_cfg(d, 64).smem <= 224 * 1024 && ring_cfg(d, 64).nstages <= DEC_MAX_STAGES,
+  LAS_REQUIRE(att_smem(d, false) <= 220 * 1024 && ring_cfg(d).smem <= 224 * 1024 && ring_cfg(d).nstages <= DEC_MAX_STAGES,
               "LAS_MODE_BF16 speller: model does not fit shared memory (U=%d, Hs=%d)", d->U, d->Hs);
   return LAS_OK;
 }
@@ -1646,9 +1645,8 @@ SpellerWsFast ws_layout(const las_speller_dims* d, void* base) {
 
 }  // namespace
 
-bool fast_available() { return true; }
-// Does the persistent decoder hold this model on chip?  (No error message is left behind: the caller falls back to the generic
-// tensor-core path, las_api.cu speller_decode_generic.)
+// Does the persistent decoder hold this model on chip?  (Otherwise las_api.cu runs the generic tensor-core path: speller_decode_f32 on
+// the generic layout.)
 bool fast_speller_fits(const las_speller_dims* d) {
   if (d->cell != LAS_CELL_LSTM || d->heads > 1 || d->no_mlp) return false;
   const bool ok = supported(d) == LAS_OK && d->sl * (d->Hs / DEC_UNITS) + 1 <= sm_count();
@@ -1662,7 +1660,7 @@ bool fast_set_option_speller(int key, int value) {
 }
 
 size_t fast_speller_packed_bytes(const las_speller_dims* d) { return pack_layout(d, nullptr).bytes; }
-size_t fast_speller_workspace_bytes(const las_speller_dims* d, int) { return ws_layout(d, nullptr).bytes; }
+size_t fast_speller_workspace_bytes(const las_speller_dims* d) { return ws_layout(d, nullptr).bytes; }
 
 int fast_speller_pack(const las_speller_weights* w, const las_speller_dims* d, void* packed_fast, cudaStream_t st) {
   LAS_TRY(supported(d));
@@ -1686,32 +1684,15 @@ int fast_speller_pack(const las_speller_weights* w, const las_speller_dims* d, v
 //   last_seg:  hand the recurrent state back to the caller (io->h_state / c_state / word / context);
 // between segments the state lives in the workspace: h / context / dense word in the parity-0 hand-off buffers (s_count is even
 // for every segment but the last), c and the fed-back token in the carry buffers.
-int fast_speller_decode_segment(const las_decode_io* io, const void* packed_f32, const void* packed_fast, const las_speller_dims* d,
+int fast_speller_decode_segment(const las_decode_io* io, const SpellerF32Inputs& f32, const void* packed_fast, const las_speller_dims* d,
                                 int b0, int Bc, int s_begin, int s_count, bool first_seg, bool last_seg, int decode_mode, int relu,
-                                void* ws_f32, void* ws_fast, cudaStream_t st) {
+                                void* ws_fast, cudaStream_t st) {
   const Shape s = shape_of(d);
   const int n_lstm = d->sl * s.ncl;
   LAS_REQUIRE(last_seg || (s_count % 2 == 0), "decoder segments must have an even number of steps (%d)", s_count);
   LAS_REQUIRE(s_begin % 2 == 0, "decoder segments must start at an even step (%d)", s_begin);
   const SpellerPackFast pk = pack_layout(d, const_cast<void*>(packed_fast));
-  // fp32 block of the pack (las_api.cu layout): psi / phi / cd weights and biases in the reference's own shapes
-  struct F32View { const float *w_psi, *b_psi, *b_phi, *b_cd; } fv;
-  {
-    Carver cv(const_cast<void*>(packed_f32));
-    const size_t G = 4 * (size_t)d->Hs;
-    for (int l = 0; l < d->sl; ++l) {
-      const size_t Kx = (l == 0) ? (size_t)d->V + d->E : (size_t)d->Hs;
-      cv.take<float>(G * Kx); cv.take<float>(G * d->Hs); cv.take<float>(G); cv.take<float>(G);
-    }
-    cv.take<float>((size_t)d->D * d->Hs);
-    fv.b_phi = cv.take<float>(d->D);
-    fv.w_psi = cv.take<float>((size_t)d->D * d->E);
-    fv.b_psi = cv.take<float>(d->D);
-    cv.take<float>((size_t)d->V * (d->Hs + d->E));
-    fv.b_cd = cv.take<float>(d->V);
-  }
-  float* psi_ws = static_cast<float*>(ws_f32);  // first buffer of the fp32 workspace layout: psi [B,U,D]
-  const float* psi = io->psi ? io->psi : psi_ws;
+  const float* psi = io->psi ? io->psi : f32.psi;
 
   {
     las_speller_dims dc = *d;
@@ -1740,7 +1721,7 @@ int fast_speller_decode_segment(const las_decode_io* io, const void* packed_f32,
       p.k_in_smem = att_smem(d, true, hyb) <= 220 * 1024;
       if (hyb && att_smem(d, p.k_in_smem != 0, true) > 220 * 1024) { p.ctx_ntm = 0; p.ctx_tmem = 0; p.k_in_smem = att_smem(d, true, false) <= 220 * 1024; }
     }
-    RingCfg rc = ring_cfg(d, Bc);
+    RingCfg rc = ring_cfg(d);
     // weights-stationary LSTM CTAs: whole 64-wide atoms (E == Hs), one 3-D copy per part, critical weights within 256 tensor-memory
     // columns (Hs <= 512)
     p.lstm_ts = (d->Hs % 64 == 0 && !g_dec_lstm_role) ? 1 : 0;
@@ -1783,7 +1764,7 @@ int fast_speller_decode_segment(const las_decode_io* io, const void* packed_f32,
     p.stop = (io->early_exit && !first_seg) ? w.stop : nullptr;
     p.enc = w.enc_bf16;
     p.psi = psi;
-    p.w_phi = pk.w_phi; p.b_phi = fv.b_phi; p.w_cd = pk.w_cd; p.b_cd = fv.b_cd;
+    p.w_phi = pk.w_phi; p.b_phi = f32.b_phi; p.w_cd = pk.w_cd; p.b_cd = f32.b_cd;
     p.gt_dense = io->gt_dense;
     p.gt_index = io->gt_index;
     p.enc_lengths = io->enc_lengths;
@@ -1812,7 +1793,7 @@ int fast_speller_decode_segment(const las_decode_io* io, const void* packed_f32,
       // psi(enc) once per utterance (model/las_model.py:279 recomputes it every step): the same tcgen05 GEMM as the
       // listener's input projection, bf16 operands (the enc copy made above), fp32 accumulate + bias + relu
       ProfScope pp("speller.psi", st);
-      LAS_TRY(launch_gemm_bf16_tc(w.enc_bf16, d->E, pk.w_psi, d->E, fv.b_psi, psi_ws + so * d->U * d->D, d->D, Bc * d->U, d->D, d->E, st,
+      LAS_TRY(launch_gemm_bf16_tc(w.enc_bf16, d->E, pk.w_psi, d->E, f32.b_psi, f32.psi + so * d->U * d->D, d->D, Bc * d->U, d->D, d->E, st,
                                   relu != 0));
     }
     ProfScope ps("speller.steps", st);
@@ -1855,36 +1836,14 @@ int fast_speller_max_group(const las_speller_dims* d) {
 
 int fast_speller_ctas(const las_speller_dims* d) { return d->sl * shape_of(d).ncl + (att_split_ok(d) ? 2 : 1) * d->B; }
 
-// <eos> bookkeeping of one launch group between / after its segments (io->early_exit)
-int fast_speller_eos_begin(const las_speller_dims* d, int Bc, void* ws_fast, cudaStream_t st) {
-  las_speller_dims dc = *d;
-  dc.B = Bc;
-  const SpellerWsFast w = ws_layout(&dc, ws_fast);
-  LAS_CUDA_OK(cudaMemsetAsync(w.stop, 0, sizeof(int32_t) * (2 + 64), st));  // stop, group_steps, done[64]
-  return LAS_OK;
-}
-int fast_speller_eos_check(const las_decode_io* io, const las_speller_dims* d, int b0, int Bc, int s_begin, int s_end, void* ws_fast,
-                           cudaStream_t st) {
-  las_speller_dims dc = *d;
-  dc.B = Bc;
-  const SpellerWsFast w = ws_layout(&dc, ws_fast);
-  return launch_eos_check(io->tokens, d->B, b0, Bc, s_begin, s_end, io->eos_token, w.stop, st);
-}
-int fast_speller_eos_fill(const las_decode_io* io, const las_speller_dims* d, int b0, int Bc, int steps, void* ws_fast, cudaStream_t st) {
-  las_speller_dims dc = *d;
-  dc.B = Bc;
-  const SpellerWsFast w = ws_layout(&dc, ws_fast);
-  return launch_eos_fill(w.stop, steps, d->B, b0, Bc, d->V, d->U, 1, io->eos_token, io->logp, io->attn, io->tokens, io->nll_terms, io->steps_done, st);
-}
-
 // Segment lengths: `seg` steps each (even), the remainder in the last one.  seg <= 0: one segment.
 static int next_segment(int s_begin, int steps, int seg) {
   if (seg <= 0 || s_begin + seg >= steps) return steps - s_begin;
   return seg;
 }
 
-int fast_speller_decode(const las_decode_io* io, const void* packed_f32, const void* packed_fast, const las_speller_dims* d, int steps,
-                        int decode_mode, int relu, void* ws_f32, void* ws_fast, cudaStream_t st) {
+int fast_speller_decode(const las_decode_io* io, const SpellerF32Inputs& f32, const void* packed_fast, const las_speller_dims* d, int steps,
+                        int decode_mode, int relu, void* ws_fast, cudaStream_t st) {
   LAS_TRY(supported(d));
   const Shape s = shape_of(d);
   const int n_lstm = d->sl * s.ncl;
@@ -1898,15 +1857,18 @@ int fast_speller_decode(const las_decode_io* io, const void* packed_f32, const v
   if (eos && io->steps_done) LAS_CUDA_OK(cudaMemsetAsync(io->steps_done, 0, sizeof(int32_t), st));
   for (int b0 = 0; b0 < d->B; b0 += max_b) {
     const int Bc = (d->B - b0) < max_b ? (d->B - b0) : max_b;
-    if (eos) LAS_TRY(fast_speller_eos_begin(d, Bc, ws_fast, st));
+    las_speller_dims dc = *d;
+    dc.B = Bc;
+    int32_t* const stop = ws_layout(&dc, ws_fast).stop;  // <eos> bookkeeping of the launch group: stop, group_steps, done[64]
+    if (eos) LAS_CUDA_OK(cudaMemsetAsync(stop, 0, sizeof(int32_t) * (2 + 64), st));
     for (int sb = 0; sb < steps;) {
       const int n = next_segment(sb, steps, seg);
-      LAS_TRY(fast_speller_decode_segment(io, packed_f32, packed_fast, d, b0, Bc, sb, n, sb == 0, sb + n == steps, decode_mode, relu, ws_f32,
-                                          ws_fast, st));
-      if (eos) LAS_TRY(fast_speller_eos_check(io, d, b0, Bc, sb, sb + n, ws_fast, st));
+      LAS_TRY(fast_speller_decode_segment(io, f32, packed_fast, d, b0, Bc, sb, n, sb == 0, sb + n == steps, decode_mode, relu, ws_fast, st));
+      if (eos) LAS_TRY(launch_eos_check(io->tokens, d->B, b0, Bc, sb, sb + n, io->eos_token, stop, st));
       sb += n;
     }
-    if (eos) LAS_TRY(fast_speller_eos_fill(io, d, b0, Bc, steps, ws_fast, st));
+    if (eos)
+      LAS_TRY(launch_eos_fill(stop, steps, d->B, b0, Bc, d->V, d->U, 1, io->eos_token, io->logp, io->attn, io->tokens, io->nll_terms, io->steps_done, st));
   }
   return LAS_OK;
 }

@@ -496,7 +496,7 @@ int launch_eos_fill(const int32_t* state, int S, int Bfull, int b0, int Bc, int 
 
 // =========================================================================================================
 // Generic tensor-core decoder step (LAS_MODE_BF16 for the shapes / variants the persistent decoder does not hold on chip:
-// 1024-wide cells, GRU / RNN cells; las_api.cu speller_decode_generic): per layer and step
+// 1024-wide cells, GRU / RNN cells; las_api.cu speller_step): per layer and step
 //     A = bf16([x | h_prev])  ->  tcgen05 GEMM with the packed [R, Kp] bf16 weights (+ bias)  ->  fp32 cell update.
 // Packed rows R: LSTM 4H (i,f,g,o), RNN H, GRU 4H = (r, z, n_x, n_h) -- the n gate's input and hidden parts are kept apart
 // (torch: n = tanh(W_in x + b_in + r * (W_hn h + b_hn))) by giving them separate rows with a zero block each.

@@ -158,18 +158,51 @@ static ListenerGen listener_ws_layout_gen(const las_listener_dims* d, void* base
   return p;
 }
 
-static int listener_forward_f32(const float* x, const int32_t* x_lengths, const void* packed, const las_listener_dims* d, float* enc,
-                                int32_t* enc_lengths, void* ws, cudaStream_t st, const void* packed_gen = nullptr, void* ws_gen = nullptr) {
-  const ListenerPackF32 pk = listener_pack_layout_f32(d, const_cast<void*>(packed));
-  const ListenerWsF32 w = listener_ws_layout_f32(d, ws);
-  const bool gen = packed_gen != nullptr;
-  ListenerGen gp, gw;
-  memset(&gp, 0, sizeof(gp));
-  memset(&gw, 0, sizeof(gw));
-  if (gen) {
-    gp = listener_pack_layout_gen(d, const_cast<void*>(packed_gen));
-    gw = listener_ws_layout_gen(d, ws_gen);
+// The kernels that run a model, and with them the layout of its pack and workspace
+enum class Path {
+  F32,   // fp32 kernels on the fp32 layouts
+  GEN,   // tensor-core modes, generic path: the fp32 layouts, and the generic (16-bit) layouts behind them
+  FAST,  // tensor-core modes: the persistent decoder / the cluster-resident recurrence (fast_*.cu), which own their blocks' layouts
+};
+static void* behind(const void* base, size_t offset) { return base ? static_cast<char*>(const_cast<void*>(base)) + offset : nullptr; }
+
+// The one place that decides the listener's path and knows where its blocks sit: the fp32 layouts at the start of the pack and
+// the workspace, the generic ones behind them; or the cluster-resident recurrence's own layouts, which then fill both buffers.
+// Null bases give the sizes alone.  `d` has passed listener_check.
+struct ListenerLayout {
+  Path path;
+  ListenerPackF32 pk;  // F32, GEN
+  ListenerWsF32 ws;
+  ListenerGen gp, gw;  // GEN
+  size_t pack_bytes, ws_bytes;
+};
+static ListenerLayout listener_layout(const las_listener_dims* d, int mode, const void* packed, void* ws) {
+  ListenerLayout L = {};
+  L.path = !tc_mode(mode) ? Path::F32 : fast_listener_fits(d) ? Path::FAST : Path::GEN;
+  if (L.path == Path::FAST) {
+    L.pack_bytes = fast_listener_packed_bytes(d);
+    L.ws_bytes = fast_listener_workspace_bytes(d);
+    return L;
   }
+  L.pk = listener_pack_layout_f32(d, const_cast<void*>(packed));
+  L.ws = listener_ws_layout_f32(d, ws);
+  L.pack_bytes = L.pk.bytes;
+  L.ws_bytes = L.ws.bytes;
+  if (L.path == Path::GEN) {
+    L.gp = listener_pack_layout_gen(d, behind(packed, L.pk.bytes));
+    L.gw = listener_ws_layout_gen(d, behind(ws, L.ws.bytes));
+    L.pack_bytes += L.gp.bytes;
+    L.ws_bytes += L.gw.bytes;
+  }
+  return L;
+}
+
+static int listener_forward_f32(const float* x, const int32_t* x_lengths, const las_listener_dims* d, const ListenerLayout& L, float* enc,
+                                int32_t* enc_lengths, cudaStream_t st) {
+  const ListenerPackF32& pk = L.pk;
+  const ListenerWsF32& w = L.ws;
+  const ListenerGen &gp = L.gp, &gw = L.gw;
+  const bool gen = L.path == Path::GEN;
   const int B = d->B, H = d->H;
   const int GH = n_gates(d->cell) * H;
   const bool lstm = d->cell == LAS_CELL_LSTM;
@@ -367,6 +400,42 @@ static SpellerWsGen speller_ws_layout_gen(const las_speller_dims* d, void* base)
 // psi GEMM / cell GEMMs read bf16 rows through TMA: 16-byte aligned rows
 static bool gen_ok(const las_speller_dims* d) { return d->no_mlp || d->E % 8 == 0; }
 
+// The one place that decides the speller's path and knows where its blocks sit: the fp32 layouts at the start of the pack and the
+// workspace (in the tensor-core modes too: the persistent decoder reads biases and psi there), then in the tensor-core modes the
+// generic layouts or the persistent decoder's blocks.  The beam pack holds the generic layout also where the persistent decoder covers
+// the model.  Null bases give the sizes alone.  `d` has passed speller_check.
+struct SpellerLayout {
+  Path path;
+  SpellerPackF32 pk;
+  SpellerWsF32 ws;
+  SpellerPackGen gp;  // GEN
+  SpellerWsGen gw;
+  void* pk_fast;      // FAST
+  void* ws_fast;
+  size_t pack_bytes, ws_bytes;
+};
+static SpellerLayout speller_layout(const las_speller_dims* d, int mode, bool beam_pack, const void* packed, void* ws) {
+  SpellerLayout L = {};
+  L.path = !tc_mode(mode) ? Path::F32 : (!beam_pack && fast_speller_fits(d)) ? Path::FAST : Path::GEN;
+  L.pk = speller_pack_layout_f32(d, const_cast<void*>(packed));
+  L.ws = speller_ws_layout_f32(d, ws);
+  L.pack_bytes = L.pk.bytes;
+  L.ws_bytes = L.ws.bytes;
+  if (L.path == Path::GEN) {
+    L.gp = speller_pack_layout_gen(d, behind(packed, L.pk.bytes));
+    L.gw = speller_ws_layout_gen(d, behind(ws, L.ws.bytes));
+    L.pack_bytes += L.gp.bytes;
+    L.ws_bytes += L.gw.bytes;
+  } else if (L.path == Path::FAST) {
+    L.pk_fast = behind(packed, L.pk.bytes);
+    L.ws_fast = behind(ws, L.ws.bytes);
+    L.pack_bytes += fast_speller_packed_bytes(d);
+    L.ws_bytes += fast_speller_workspace_bytes(d);
+  }
+  return L;
+}
+static SpellerF32Inputs fast_f32_inputs(const SpellerLayout& L) { return {L.pk.b_phi, L.pk.b_psi, L.pk.b_cd, L.ws.psi}; }
+
 // psi = act(enc . W_psi^T + b_psi) of B utterances into `psi` (generic path: a bf16 copy of enc in `enc16` and a tcgen05 GEMM); without
 // the attention MLP the keys are the listener features themselves
 static const float* speller_psi(const las_speller_dims* d, int B, const SpellerPackF32& pk, const SpellerPackGen* gp, const float* enc, float* psi,
@@ -469,22 +538,16 @@ static int speller_step(const StepPath& p, int s, const float* hp, float* hn, co
   return launch_attend_f32(t, st);
 }
 
-static int speller_decode_f32(const las_decode_io* io, const void* packed, const las_speller_dims* d, int steps,
-                              int decode_mode, int relu, void* ws, cudaStream_t st, const void* packed_gen = nullptr, void* ws_gen = nullptr) {
-  const SpellerPackF32 pk = speller_pack_layout_f32(d, const_cast<void*>(packed));
-  const SpellerWsF32 w = speller_ws_layout_f32(d, ws);
-  // packed_gen != nullptr: the generic tensor-core path of LAS_MODE_BF16 (see above); everything but the GEMMs is shared
-  const bool gen = packed_gen != nullptr;
+static int speller_decode_f32(const las_decode_io* io, const las_speller_dims* d, const SpellerLayout& L, int steps, int decode_mode, int relu,
+                              cudaStream_t st) {
+  const SpellerPackF32& pk = L.pk;
+  const SpellerWsF32& w = L.ws;
+  const SpellerPackGen& gp = L.gp;
+  const SpellerWsGen& gw = L.gw;
+  // the generic tensor-core path of LAS_MODE_BF16 (see above); everything but the GEMMs is shared
+  const bool gen = L.path == Path::GEN;
   const GenGeom gg = gen_geom(d);
-  SpellerPackGen gp;
-  SpellerWsGen gw;
-  memset(&gp, 0, sizeof(gp));
-  memset(&gw, 0, sizeof(gw));
-  if (gen) {
-    gp = speller_pack_layout_gen(d, const_cast<void*>(packed_gen));
-    gw = speller_ws_layout_gen(d, ws_gen);
-    LAS_CUDA_OK(cudaMemsetAsync(gw.zero, 0, sizeof(float) * 256, st));
-  }
+  if (gen) LAS_CUDA_OK(cudaMemsetAsync(gw.zero, 0, sizeof(float) * 256, st));
   const int B = d->B, Hs = d->Hs, V = d->V, E = d->E, U = d->U, sl = d->sl;
   const int xld = V + E;
   const size_t state_n = (size_t)sl * B * Hs;
@@ -639,14 +702,13 @@ static BeamWs beam_ws_layout(const las_speller_dims* d, int steps, int beam, boo
   return w;
 }
 
-static int speller_beam_f32(const las_beam_io* io, const void* packed, const las_speller_dims* d, int steps, int relu, void* ws, cudaStream_t st,
-                            const void* packed_gen) {
+// `L`: the beam pack's layout
+static int speller_beam_f32(const las_beam_io* io, const las_speller_dims* d, const SpellerLayout& L, int steps, int relu, void* ws,
+                            cudaStream_t st) {
   const int B = d->B, K = io->beam, BK = B * K, V = d->V, E = d->E, Hs = d->Hs;
-  const bool gen = packed_gen != nullptr;
-  const SpellerPackF32 pk = speller_pack_layout_f32(d, const_cast<void*>(packed));
-  SpellerPackGen gp;
-  memset(&gp, 0, sizeof(gp));
-  if (gen) gp = speller_pack_layout_gen(d, const_cast<void*>(packed_gen));
+  const bool gen = L.path == Path::GEN;
+  const SpellerPackF32& pk = L.pk;
+  const SpellerPackGen& gp = L.gp;
   const BeamWs w = beam_ws_layout(d, steps, K, gen, ws);
   if (gen) LAS_CUDA_OK(cudaMemsetAsync(w.zero, 0, sizeof(float) * 256, st));
   las_speller_dims dk = *d;  // the decoder sees B*K rows
@@ -694,6 +756,30 @@ static int speller_beam_f32(const las_beam_io* io, const void* packed, const las
   return launch_beam_finalize(fa, st);
 }
 
+// The las_decode_io checks of las_speller_decode, which las_pipeline_step's concurrent branch makes as well.  `d` has passed
+// speller_check.
+static int decode_args_check(const las_decode_io* io, const las_speller_dims* d, int steps, int decode_mode, int mode, size_t ws_bytes) {
+  LAS_REQUIRE(io->enc && io->logp, "io->enc and io->logp are required");
+  LAS_REQUIRE(steps >= 0, "steps must be >= 0");
+  LAS_REQUIRE(mode == LAS_MODE_FP32 || tc_mode(mode), "unknown mode %d", mode);
+  LAS_REQUIRE(decode_mode == LAS_DECODE_RAW || decode_mode == LAS_DECODE_GREEDY || decode_mode == LAS_DECODE_SAMPLE,
+              "decode_mode %d is not supported (0 = raw, 1 = greedy, 2 = sample)", decode_mode);
+  LAS_REQUIRE(!(io->gt_dense || io->gt_index) || io->gt_steps >= steps, "ground truth has %d steps, %d requested", io->gt_steps, steps);
+  LAS_REQUIRE(d->cell != LAS_CELL_LSTM || (io->h_state == nullptr) == (io->c_state == nullptr), "h_state and c_state must be given together");
+  LAS_REQUIRE((io->word == nullptr) == (io->context == nullptr), "word and context must be given together");
+  LAS_REQUIRE(!io->early_exit || io->tokens, "<eos> early exit needs io->tokens");
+  LAS_TRY(device_ok());
+  const size_t need = speller_layout(d, mode, false, nullptr, nullptr).ws_bytes;
+  if (ws_bytes < need) return fail(LAS_ENOMEM, "workspace too small: %zu < %zu", ws_bytes, need);
+  return LAS_OK;
+}
+
+// Can las_pipeline_step run the listener next to the persistent decoder (fast_pipeline.cu)?  Both models valid, both on their FAST paths.
+static bool pipeline_fast(const las_listener_dims* ld, const las_speller_dims* sd, int mode) {
+  return ld && sd && listener_check(ld) == LAS_OK && speller_check(sd) == LAS_OK && listener_layout(ld, mode, nullptr, nullptr).path == Path::FAST &&
+         speller_layout(sd, mode, false, nullptr, nullptr).path == Path::FAST;
+}
+
 }  // namespace las
 
 using namespace las;
@@ -703,7 +789,7 @@ extern "C" {
 int las_abi_version(void) { return LAS_B200_ABI_VERSION; }
 const char* las_last_error(void) { return err_buf(); }
 int las_device_check(void) { return device_ok(); }
-int las_mode_available(int mode) { return mode == LAS_MODE_FP32 || (tc_mode(mode) && fast_available()); }
+int las_mode_available(int mode) { return mode == LAS_MODE_FP32 || tc_mode(mode); }
 int las_prof_enable(int on) {
   for (int i = 0; i < g_prof_n; ++i) {
     cudaEventDestroy(g_prof[i].e0);
@@ -744,9 +830,7 @@ int64_t las_launch_count(int reset) {
 // ---- listener ------------------------------------------------------------------------------------------
 size_t las_listener_packed_bytes(const las_listener_dims* d, int mode) {
   if (listener_check(d) != LAS_OK) return 0;
-  if (tc_mode(mode) && fast_listener_fits(d)) return fast_listener_packed_bytes(d);
-  if (tc_mode(mode)) return listener_pack_layout_f32(d, nullptr).bytes + listener_pack_layout_gen(d, nullptr).bytes;
-  return listener_pack_layout_f32(d, nullptr).bytes;
+  return listener_layout(d, mode, nullptr, nullptr).pack_bytes;
 }
 
 int las_listener_pack(const las_lstm_weights* w, const las_listener_dims* d, int mode, void* packed, size_t packed_bytes,
@@ -756,13 +840,13 @@ int las_listener_pack(const las_lstm_weights* w, const las_listener_dims* d, int
   LAS_REQUIRE(w && packed, "null weights / packed buffer");
   LAS_REQUIRE(mode == LAS_MODE_FP32 || tc_mode(mode), "unknown mode %d", mode);
   LAS_TRY(device_ok());
-  if (packed_bytes < las_listener_packed_bytes(d, mode))
-    return fail(LAS_ENOMEM, "packed buffer too small: %zu < %zu", packed_bytes, las_listener_packed_bytes(d, mode));
+  const ListenerLayout L = listener_layout(d, mode, packed, nullptr);
+  if (packed_bytes < L.pack_bytes) return fail(LAS_ENOMEM, "packed buffer too small: %zu < %zu", packed_bytes, L.pack_bytes);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  LAS_REQUIRE(!tc_mode(mode) || fast_listener_fits(d) || listener_gen_ok(d),
+  LAS_REQUIRE(L.path != Path::GEN || listener_gen_ok(d),
               "LAS_MODE_BF16 needs 16-byte aligned bf16 rows for TMA: 2F (%d) and 4H (%d) must be multiples of 8; use LAS_MODE_FP32", 2 * d->F, 4 * d->H);
-  if (tc_mode(mode) && fast_listener_fits(d)) return fast_listener_pack(w, d, packed, st);
-  const ListenerPackF32 pk = listener_pack_layout_f32(d, packed);
+  if (L.path == Path::FAST) return fast_listener_pack(w, d, packed, st);
+  const ListenerPackF32& pk = L.pk;
   const size_t H = d->H, GH = (size_t)n_gates(d->cell) * H;
   for (int l = 0; l < d->L; ++l) {
     const size_t K = (l == 0) ? 2 * (size_t)d->F : 4 * H;
@@ -780,11 +864,10 @@ int las_listener_pack(const las_lstm_weights* w, const las_listener_dims* d, int
       }
     }
   }
-  if (tc_mode(mode)) {  // generic path: bf16 copies of [W_ih fwd ; W_ih reverse] behind the fp32 pack
-    const ListenerGen gp = listener_pack_layout_gen(d, static_cast<char*>(packed) + pk.bytes);
+  if (L.path == Path::GEN) {  // bf16 copies of [W_ih fwd ; W_ih reverse]
     for (int l = 0; l < d->L; ++l) {
       const size_t K = (l == 0) ? 2 * (size_t)d->F : 4 * H;
-      LAS_TRY(launch_f32_to_bf16(pk.wcat[l], gp.w[l], 2 * GH * K, st));
+      LAS_TRY(launch_f32_to_bf16(pk.wcat[l], L.gp.w[l], 2 * GH * K, st));
     }
   }
   return LAS_OK;
@@ -792,9 +875,7 @@ int las_listener_pack(const las_lstm_weights* w, const las_listener_dims* d, int
 
 size_t las_listener_workspace_bytes(const las_listener_dims* d, int mode) {
   if (listener_check(d) != LAS_OK) return 0;
-  if (tc_mode(mode) && fast_listener_fits(d)) return fast_listener_workspace_bytes(d);
-  if (tc_mode(mode)) return listener_ws_layout_f32(d, nullptr).bytes + listener_ws_layout_gen(d, nullptr).bytes;
-  return listener_ws_layout_f32(d, nullptr).bytes;
+  return listener_layout(d, mode, nullptr, nullptr).ws_bytes;
 }
 
 int las_listener_forward(const float* x, const void* packed, const las_listener_dims* d, int mode, float* enc,
@@ -810,31 +891,23 @@ int las_listener_forward_masked(const float* x, const int32_t* x_lengths, const 
   LAS_REQUIRE(x && packed && enc && workspace, "null pointer argument");
   LAS_REQUIRE(mode == LAS_MODE_FP32 || tc_mode(mode), "unknown mode %d", mode);
   LAS_TRY(device_ok());
-  if (workspace_bytes < las_listener_workspace_bytes(d, mode))
-    return fail(LAS_ENOMEM, "workspace too small: %zu < %zu", workspace_bytes, las_listener_workspace_bytes(d, mode));
+  const ListenerLayout L = listener_layout(d, mode, packed, workspace);
+  if (workspace_bytes < L.ws_bytes) return fail(LAS_ENOMEM, "workspace too small: %zu < %zu", workspace_bytes, L.ws_bytes);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (tc_mode(mode) && fast_listener_fits(d)) return fast_listener_forward(x, x_lengths, packed, d, enc, enc_lengths, workspace, st);
-  if (tc_mode(mode)) {
-    LAS_REQUIRE(listener_gen_ok(d), "LAS_MODE_BF16 needs 2F (%d) and 4H (%d) to be multiples of 8; use LAS_MODE_FP32", 2 * d->F, 4 * d->H);
-    return listener_forward_f32(x, x_lengths, packed, d, enc, enc_lengths, workspace, st,
-                                static_cast<const char*>(packed) + listener_pack_layout_f32(d, nullptr).bytes,
-                                static_cast<char*>(workspace) + listener_ws_layout_f32(d, nullptr).bytes);
-  }
-  return listener_forward_f32(x, x_lengths, packed, d, enc, enc_lengths, workspace, st);
+  if (L.path == Path::FAST) return fast_listener_forward(x, x_lengths, packed, d, enc, enc_lengths, workspace, st);
+  LAS_REQUIRE(L.path != Path::GEN || listener_gen_ok(d), "LAS_MODE_BF16 needs 2F (%d) and 4H (%d) to be multiples of 8; use LAS_MODE_FP32",
+              2 * d->F, 4 * d->H);
+  return listener_forward_f32(x, x_lengths, d, L, enc, enc_lengths, st);
 }
 
 // ---- speller -------------------------------------------------------------------------------------------
 size_t las_speller_packed_bytes(const las_speller_dims* d, int mode) {
   if (speller_check(d) != LAS_OK) return 0;
-  // the bf16 pack keeps the fp32 block first (phi/psi/cd and fallbacks read it), then its own layouts
-  const size_t f32 = speller_pack_layout_f32(d, nullptr).bytes;
-  if (tc_mode(mode)) return f32 + (fast_speller_fits(d) ? fast_speller_packed_bytes(d) : speller_pack_layout_gen(d, nullptr).bytes);
-  return f32;
+  return speller_layout(d, mode, false, nullptr, nullptr).pack_bytes;
 }
 
-// generic_layout: the tensor-core modes pack the generic step's layout even where the persistent decoder covers the shape (beam pack)
 static int speller_pack(const las_speller_weights* w, const las_speller_dims* d, int mode, void* packed, size_t packed_bytes, void* stream,
-                        bool generic_layout) {
+                        bool beam_pack) {
   set_operand_mode(mode);
   LAS_TRY(speller_check(d));
   LAS_REQUIRE(w && packed && w->rnn_host, "null weights / packed buffer");
@@ -842,14 +915,12 @@ static int speller_pack(const las_speller_weights* w, const las_speller_dims* d,
   LAS_REQUIRE(w->w_cd && w->b_cd, "null output weight pointer");
   LAS_REQUIRE(d->no_mlp || (w->w_phi && w->b_phi && w->w_psi && w->b_psi), "null attention weight pointer");
   LAS_REQUIRE(n_heads(d) == 1 || (w->w_dr && w->b_dr), "multi_head > 1 needs attention.dim_reduce weights");
-  const bool fast = tc_mode(mode) && fast_speller_fits(d) && !generic_layout;
-  LAS_REQUIRE(!tc_mode(mode) || fast || gen_ok(d),
-              "LAS_MODE_BF16 needs E %% 8 == 0 for the psi GEMM's TMA rows (E=%d); use LAS_MODE_FP32", d->E);
+  const SpellerLayout L = speller_layout(d, mode, beam_pack, packed, nullptr);
+  LAS_REQUIRE(L.path != Path::GEN || gen_ok(d), "LAS_MODE_BF16 needs E %% 8 == 0 for the psi GEMM's TMA rows (E=%d); use LAS_MODE_FP32", d->E);
   LAS_TRY(device_ok());
-  const size_t need = generic_layout ? las_speller_beam_packed_bytes(d, mode) : las_speller_packed_bytes(d, mode);
-  if (packed_bytes < need) return fail(LAS_ENOMEM, "packed buffer too small: %zu < %zu", packed_bytes, need);
+  if (packed_bytes < L.pack_bytes) return fail(LAS_ENOMEM, "packed buffer too small: %zu < %zu", packed_bytes, L.pack_bytes);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const SpellerPackF32 pk = speller_pack_layout_f32(d, packed);
+  const SpellerPackF32& pk = L.pk;
   const size_t G = (size_t)n_gates(d->cell) * d->Hs;
 #define CP(dst, src, n) LAS_CUDA_OK(cudaMemcpyAsync(dst, src, sizeof(float) * (n), cudaMemcpyDeviceToDevice, st))
   for (int l = 0; l < d->sl; ++l) {
@@ -874,9 +945,9 @@ static int speller_pack(const las_speller_weights* w, const las_speller_dims* d,
     CP(pk.b_dr, w->b_dr, d->E);
   }
 #undef CP
-  if (fast) return fast_speller_pack(w, d, static_cast<char*>(packed) + pk.bytes, st);
-  if (tc_mode(mode)) {  // generic tensor-core path: [W_ih | W_hh] per layer as one bf16 matrix, psi weights in bf16
-    const SpellerPackGen gp = speller_pack_layout_gen(d, static_cast<char*>(packed) + pk.bytes);
+  if (L.path == Path::FAST) return fast_speller_pack(w, d, L.pk_fast, st);
+  if (L.path == Path::GEN) {  // generic tensor-core path: [W_ih | W_hh] per layer as one bf16 matrix, psi weights in bf16
+    const SpellerPackGen& gp = L.gp;
     const GenGeom g = gen_geom(d);
     for (int l = 0; l < d->sl; ++l) {
       const las_lstm_weights& s = w->rnn_host[l];
@@ -926,9 +997,7 @@ int las_attention_forward(const float* state, const float* enc, const float* psi
 
 size_t las_speller_workspace_bytes(const las_speller_dims* d, int steps, int mode) {
   if (speller_check(d) != LAS_OK || steps < 0) return 0;
-  const size_t f32 = speller_ws_layout_f32(d, nullptr).bytes;
-  if (tc_mode(mode)) return f32 + (fast_speller_fits(d) ? fast_speller_workspace_bytes(d, steps) : speller_ws_layout_gen(d, nullptr).bytes);
-  return f32;
+  return speller_layout(d, mode, false, nullptr, nullptr).ws_bytes;
 }
 
 int las_speller_decode(const las_decode_io* io, const void* packed, const las_speller_dims* d, int steps, int decode_mode,
@@ -936,42 +1005,20 @@ int las_speller_decode(const las_decode_io* io, const void* packed, const las_sp
   set_operand_mode(mode);
   LAS_TRY(speller_check(d));
   LAS_REQUIRE(io && packed && workspace, "null pointer argument");
-  LAS_REQUIRE(io->enc && io->logp, "io->enc and io->logp are required");
-  LAS_REQUIRE(steps >= 0, "steps must be >= 0");
-  LAS_REQUIRE(mode == LAS_MODE_FP32 || tc_mode(mode), "unknown mode %d", mode);
-  LAS_REQUIRE(decode_mode == LAS_DECODE_RAW || decode_mode == LAS_DECODE_GREEDY || decode_mode == LAS_DECODE_SAMPLE,
-              "decode_mode %d is not supported (0 = raw, 1 = greedy, 2 = sample)", decode_mode);
-  LAS_REQUIRE(!(io->gt_dense || io->gt_index) || io->gt_steps >= steps, "ground truth has %d steps, %d requested", io->gt_steps, steps);
-  LAS_REQUIRE(d->cell != LAS_CELL_LSTM || (io->h_state == nullptr) == (io->c_state == nullptr), "h_state and c_state must be given together");
-  LAS_REQUIRE((io->word == nullptr) == (io->context == nullptr), "word and context must be given together");
-  LAS_REQUIRE(!io->early_exit || io->tokens, "<eos> early exit needs io->tokens");
-  LAS_TRY(device_ok());
-  if (workspace_bytes < las_speller_workspace_bytes(d, steps, mode))
-    return fail(LAS_ENOMEM, "workspace too small: %zu < %zu", workspace_bytes, las_speller_workspace_bytes(d, steps, mode));
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  LAS_TRY(decode_args_check(io, d, steps, decode_mode, mode, workspace_bytes));
   if (steps == 0) return LAS_OK;
-  if (tc_mode(mode) && !fast_speller_fits(d)) {
-    LAS_REQUIRE(gen_ok(d), "LAS_MODE_BF16 needs E %% 8 == 0 (E=%d); use LAS_MODE_FP32", d->E);
-    const size_t f32p = speller_pack_layout_f32(d, nullptr).bytes;
-    const size_t f32w = speller_ws_layout_f32(d, nullptr).bytes;
-    return speller_decode_f32(io, packed, d, steps, decode_mode, relu, workspace, st, static_cast<const char*>(packed) + f32p,
-                              static_cast<char*>(workspace) + f32w);
-  }
-  if (tc_mode(mode)) {
-    const size_t f32p = speller_pack_layout_f32(d, nullptr).bytes;
-    const size_t f32w = speller_ws_layout_f32(d, nullptr).bytes;
-    return fast_speller_decode(io, packed, static_cast<const char*>(packed) + f32p, d, steps, decode_mode, relu, workspace,
-                               static_cast<char*>(workspace) + f32w, st);
-  }
-  return speller_decode_f32(io, packed, d, steps, decode_mode, relu, workspace, st);
+  const SpellerLayout L = speller_layout(d, mode, false, packed, workspace);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (L.path == Path::FAST) return fast_speller_decode(io, fast_f32_inputs(L), L.pk_fast, d, steps, decode_mode, relu, L.ws_fast, st);
+  LAS_REQUIRE(L.path != Path::GEN || gen_ok(d), "LAS_MODE_BF16 needs E %% 8 == 0 (E=%d); use LAS_MODE_FP32", d->E);
+  return speller_decode_f32(io, d, L, steps, decode_mode, relu, st);
 }
 
 // ---- beam search -----------------------------------------------------------------------------------------
 size_t las_speller_beam_packed_bytes(const las_speller_dims* d, int mode) {
   if (speller_check(d) != LAS_OK) return 0;
   if (mode != LAS_MODE_FP32 && !tc_mode(mode)) return 0;
-  const size_t f32 = speller_pack_layout_f32(d, nullptr).bytes;
-  return tc_mode(mode) ? f32 + speller_pack_layout_gen(d, nullptr).bytes : f32;
+  return speller_layout(d, mode, true, nullptr, nullptr).pack_bytes;
 }
 
 int las_speller_beam_pack(const las_speller_weights* w, const las_speller_dims* d, int mode, void* packed, size_t bytes, void* stream) {
@@ -981,7 +1028,7 @@ int las_speller_beam_pack(const las_speller_weights* w, const las_speller_dims* 
 size_t las_speller_beam_workspace_bytes(const las_speller_dims* d, int steps, int beam, int mode) {
   if (beam_args_check(d, steps, beam) != LAS_OK) return 0;
   if (mode != LAS_MODE_FP32 && !tc_mode(mode)) return 0;
-  return beam_ws_layout(d, steps, beam, tc_mode(mode), nullptr).bytes;
+  return beam_ws_layout(d, steps, beam, speller_layout(d, mode, true, nullptr, nullptr).path == Path::GEN, nullptr).bytes;
 }
 
 int las_speller_beam_search(const las_beam_io* io, const void* packed, const las_speller_dims* d, int steps, int mode, int relu,
@@ -998,8 +1045,7 @@ int las_speller_beam_search(const las_beam_io* io, const void* packed, const las
   LAS_TRY(device_ok());
   const size_t need = las_speller_beam_workspace_bytes(d, steps, io->beam, mode);
   if (workspace_bytes < need) return fail(LAS_ENOMEM, "workspace too small: %zu < %zu", workspace_bytes, need);
-  const void* packed_gen = tc_mode(mode) ? static_cast<const char*>(packed) + speller_pack_layout_f32(d, nullptr).bytes : nullptr;
-  return speller_beam_f32(io, packed, d, steps, relu, workspace, static_cast<cudaStream_t>(stream), packed_gen);
+  return speller_beam_f32(io, d, speller_layout(d, mode, true, packed, nullptr), steps, relu, workspace, static_cast<cudaStream_t>(stream));
 }
 
 int las_pipeline_step(const las_pipeline_args* a, int mode, void* stream) {
@@ -1015,41 +1061,24 @@ int las_pipeline_step(const las_pipeline_args* a, int mode, void* stream) {
                               a->speller_ws_bytes, stream);
   const las_speller_dims* sd = a->speller_dims;
   const las_listener_dims* ld = a->listener_dims;
-  const bool fast = tc_mode(mode) && sd && ld && speller_check(sd) == LAS_OK && fast_speller_fits(sd) && listener_check(ld) == LAS_OK &&
-                    fast_listener_fits(ld) && a->steps > 0;
-  if (!fast) {  // fp32 mode / variants: the same results, one after the other
+  if (!pipeline_fast(ld, sd, mode) || a->steps <= 0) {  // fp32 mode / variants: the same results, one after the other
     LAS_TRY(las_speller_decode(a->dec_io, a->speller_packed, sd, a->steps, a->decode_mode, mode, a->relu, a->speller_ws, a->speller_ws_bytes, stream));
     return las_listener_forward_masked(a->x, a->x_lengths, a->listener_packed, ld, mode, a->enc, a->enc_lengths, a->listener_ws,
                                        a->listener_ws_bytes, stream);
   }
-  // argument checks of the two entry points this call stands for
-  LAS_TRY(speller_check(sd));
-  LAS_TRY(listener_check(ld));
+  // argument checks of the two entry points this call stands for (both dims have passed their checks)
   const las_decode_io* io = a->dec_io;
   LAS_REQUIRE(a->speller_packed && a->speller_ws && a->listener_packed && a->listener_ws && a->enc, "null pointer argument");
-  LAS_REQUIRE(io->enc && io->logp, "io->enc and io->logp are required");
-  LAS_REQUIRE(a->decode_mode == LAS_DECODE_RAW || a->decode_mode == LAS_DECODE_GREEDY || a->decode_mode == LAS_DECODE_SAMPLE,
-              "decode_mode %d is not supported (0 = raw, 1 = greedy, 2 = sample)", a->decode_mode);
-  LAS_REQUIRE(!(io->gt_dense || io->gt_index) || io->gt_steps >= a->steps, "ground truth has %d steps, %d requested", io->gt_steps, a->steps);
-  LAS_REQUIRE((io->h_state == nullptr) == (io->c_state == nullptr), "h_state and c_state must be given together");
-  LAS_REQUIRE((io->word == nullptr) == (io->context == nullptr), "word and context must be given together");
-  LAS_REQUIRE(!io->early_exit || io->tokens, "<eos> early exit needs io->tokens");
-  LAS_TRY(device_ok());
-  if (a->speller_ws_bytes < las_speller_workspace_bytes(sd, a->steps, mode))
-    return fail(LAS_ENOMEM, "speller workspace too small: %zu < %zu", a->speller_ws_bytes, las_speller_workspace_bytes(sd, a->steps, mode));
-  if (a->listener_ws_bytes < las_listener_workspace_bytes(ld, mode))
-    return fail(LAS_ENOMEM, "listener workspace too small: %zu < %zu", a->listener_ws_bytes, las_listener_workspace_bytes(ld, mode));
-  const size_t f32p = speller_pack_layout_f32(sd, nullptr).bytes;
-  const size_t f32w = speller_ws_layout_f32(sd, nullptr).bytes;
-  return fast_pipeline_step(io, a->speller_packed, static_cast<const char*>(a->speller_packed) + f32p, sd, a->steps, a->decode_mode, a->relu,
-                            a->speller_ws, static_cast<char*>(a->speller_ws) + f32w, a->x, a->x_lengths, a->listener_packed, ld, a->enc,
-                            a->enc_lengths, a->listener_ws, static_cast<cudaStream_t>(stream));
+  LAS_TRY(decode_args_check(io, sd, a->steps, a->decode_mode, mode, a->speller_ws_bytes));
+  const ListenerLayout LL = listener_layout(ld, mode, a->listener_packed, a->listener_ws);
+  if (a->listener_ws_bytes < LL.ws_bytes) return fail(LAS_ENOMEM, "listener workspace too small: %zu < %zu", a->listener_ws_bytes, LL.ws_bytes);
+  const SpellerLayout SL = speller_layout(sd, mode, false, a->speller_packed, a->speller_ws);
+  return fast_pipeline_step(io, fast_f32_inputs(SL), SL.pk_fast, sd, a->steps, a->decode_mode, a->relu, SL.ws_fast, a->x, a->x_lengths,
+                            a->listener_packed, ld, a->enc, a->enc_lengths, a->listener_ws, static_cast<cudaStream_t>(stream));
 }
 
 int las_pipeline_overlaps(const las_listener_dims* ld, const las_speller_dims* sd, int steps, int mode) {
-  if (!tc_mode(mode) || !ld || !sd || listener_check(ld) != LAS_OK || speller_check(sd) != LAS_OK) return 0;
-  if (!fast_speller_fits(sd) || !fast_listener_fits(ld)) return 0;
-  return fast_pipeline_bc(ld, sd, steps) > 0 ? 1 : 0;
+  return pipeline_fast(ld, sd, mode) && fast_pipeline_bc(ld, sd, steps) > 0 ? 1 : 0;
 }
 
 int las_nll_sums(const float* logp, const int32_t* labels, int S, int S_lab, int B, int V, int max_label_len, float* out2,

@@ -6,8 +6,6 @@
 
 namespace las {
 
-bool fast_available();
-
 bool fast_listener_fits(const las_listener_dims* d);
 size_t fast_listener_packed_bytes(const las_listener_dims* d);
 int fast_listener_pack(const las_lstm_weights* w_host, const las_listener_dims* d, void* packed, cudaStream_t st);
@@ -18,16 +16,20 @@ int fast_listener_forward(const float* x, const int32_t* x_lengths, const void* 
 bool fast_speller_fits(const las_speller_dims* d);
 size_t fast_speller_packed_bytes(const las_speller_dims* d);
 int fast_speller_pack(const las_speller_weights* w, const las_speller_dims* d, void* packed_fast, cudaStream_t st);
-size_t fast_speller_workspace_bytes(const las_speller_dims* d, int steps);
-int fast_speller_decode(const las_decode_io* io, const void* packed_f32, const void* packed_fast,
-                        const las_speller_dims* d, int steps, int decode_mode, int relu, void* ws_f32, void* ws_fast,
-                        cudaStream_t st);
+size_t fast_speller_workspace_bytes(const las_speller_dims* d);
+// What the persistent decoder reads from the fp32 block of the speller's pack and workspace (layout: las_api.cu speller_layout)
+struct SpellerF32Inputs {
+  const float *b_phi, *b_psi, *b_cd;
+  float* psi;  // [B, U, D] psi(enc), computed here when the caller passes no io->psi
+};
+int fast_speller_decode(const las_decode_io* io, const SpellerF32Inputs& f32, const void* packed_fast, const las_speller_dims* d, int steps,
+                        int decode_mode, int relu, void* ws_fast, cudaStream_t st);
 
 // segments / launch groups of the persistent decoder (fast_speller.cu), stages of the listener (fast_listener.cu), and the
 // serving pipeline that interleaves them (fast_pipeline.cu)
-int fast_speller_decode_segment(const las_decode_io* io, const void* packed_f32, const void* packed_fast, const las_speller_dims* d,
+int fast_speller_decode_segment(const las_decode_io* io, const SpellerF32Inputs& f32, const void* packed_fast, const las_speller_dims* d,
                                 int b0, int Bc, int s_begin, int s_count, bool first_seg, bool last_seg, int decode_mode, int relu,
-                                void* ws_f32, void* ws_fast, cudaStream_t st);
+                                void* ws_fast, cudaStream_t st);
 int fast_speller_max_group(const las_speller_dims* d);
 int fast_speller_ctas(const las_speller_dims* d);  // CTAs of one persistent launch covering d->B utterances
 int fast_listener_stage(const float* x, const int32_t* x_lengths, const void* packed, const las_listener_dims* d, float* enc,
@@ -35,9 +37,9 @@ int fast_listener_stage(const float* x, const int32_t* x_lengths, const void* pa
 int fast_listener_rec_ctas(const las_listener_dims* d, int bc);
 int fast_side_stream(cudaStream_t* s);
 int fast_pipeline_bc(const las_listener_dims* ld, const las_speller_dims* sd, int steps);
-int fast_pipeline_step(const las_decode_io* io, const void* spl_packed_f32, const void* spl_packed_fast, const las_speller_dims* sd, int steps,
-                       int decode_mode, int relu, void* spl_ws_f32, void* spl_ws_fast, const float* x, const int32_t* x_lengths,
-                       const void* lis_packed, const las_listener_dims* ld, float* enc, int32_t* enc_lengths, void* lis_ws, cudaStream_t st);
+int fast_pipeline_step(const las_decode_io* io, const SpellerF32Inputs& spl_f32, const void* spl_packed_fast, const las_speller_dims* sd,
+                       int steps, int decode_mode, int relu, void* spl_ws_fast, const float* x, const int32_t* x_lengths, const void* lis_packed,
+                       const las_listener_dims* ld, float* enc, int32_t* enc_lengths, void* lis_ws, cudaStream_t st);
 bool fast_set_option_pipeline(int key, int value);
 
 // las_debug_set_option: each module's setter applies a key it owns and returns true, or returns false for another key or a value
