@@ -312,8 +312,6 @@ int las_debug_set_trace(void* dev_buf);
  * here or a value outside the key's set.
  *   key 2:  decoder context through tensor memory (1, default: all feature tiles when they fit, otherwise as many as fit + the rest
  *           on the CUDA cores) or on the CUDA cores only (0);
- *   key 5:  persistent decoder LSTM CTAs in the weights-stationary form with one 3-D TMA copy per activation part (0, default where
- *           Hs is a multiple of 64) or with shared-memory operands and one 2-D copy per 64-column atom (1);
  *   key 6:  listener input-projection GEMM concurrent with the recurrence (1, default) or in front of it (0);
  *   key 8:  tcgen05 GEMM epilogue with row-per-thread global stores (1) instead of shared-memory staging + TMA stores (0, default);
  *   key 9:  batch chunk per recurrence cluster (16 / 32 / 64; 0 = automatic);

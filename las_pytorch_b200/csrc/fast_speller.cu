@@ -3,15 +3,17 @@
 //
 // CTA roles (one CTA per SM, all co-resident; cudaLaunchAttributeCooperative guarantees it):
 //   * LSTM CTAs: layer l, block nb owns 16 hidden units (64 gate columns, unit-major / gate-minor).  Its slice of
-//     [W_hh | W_word | W_in] (bf16, 128-byte-swizzled K-major atoms) stays in shared memory for all S steps as the B
-//     operand; the A operand is the activation matrix [batch (M = 128 TMEM lanes), K] streamed per step by TMA:
+//     [W_hh | W_word | W_in] (bf16, 128-byte-swizzled K-major atoms) stays on chip for all S steps as the A operand
+//     (the critical input's part in tensor memory, the rest in shared memory); the B operand is the activation matrix
+//     [batch (N), K] streamed per step by TMA:
 //       part 0   the layer's own h_{s-1}            (ready long before it is needed; accumulator 0)
 //       part 1a  the critical input: the context of step s-1 (layer 0) / the lower layer's fresh h (accumulator 1)
 //       part 1b  layer 0 only, and only when the fed-back word is a dense vector (decode_mode 0, dense teacher
 //                forcing, the first step): the word atom.  For greedy decoding / index teacher forcing the word is
 //                an index, and the epilogue adds the matching column of W_word straight from the resident atom.
-//     tcgen05.mma accumulates in TMEM; the epilogue thread of batch row b holds that row's cell state c in registers
-//     (fp32) and writes h (bf16 operand copy for the TMA consumers; fp32 flag-in-data copy for the attention CTAs).
+//     tcgen05.mma accumulates in TMEM; the epilogue thread of a gate row holds the cell state c of four (unit, batch)
+//     cells in registers (fp32) and writes h (bf16 operand copy for the TMA consumers; fp32 flag-in-data copy for the
+//     attention CTAs).
 //   * attention CTAs: one per utterance.  W_phi, W_cd (bf16) and psi(enc)[b] (fp32) are resident in shared memory,
 //     enc[b]^T in tensor memory; per step: q = relu(W_phi h + b), energies, length-masked softmax, context (UMMA with
 //     the scores as the B operand), publish the context, then character distribution, log-softmax, argmax / teacher
@@ -49,10 +51,10 @@ constexpr int ATT_MAXP = 3;       // encoder steps per attention CTA <= ATT_MAXP
 typedef unsigned long long u64;
 
 struct DecParams {
-  CUtensorMap tm_h[MAX_SL][2];  // hbuf[l][parity]  bf16 [B, Hs]
+  CUtensorMap tm_h[MAX_SL][2];  // hbuf[l][parity]  bf16 [B, Hs]   one 64-column atom per copy (set where Hs % 64 != 0)
   CUtensorMap tm_x[2];          // xbuf[parity]     bf16 [B, E]   the context fed to layer 0 (same pitch as an h buffer)
   CUtensorMap tm_w[2];          // wbuf[parity]     bf16 [B, VP]  the dense word fed to layer 0 (one atom)
-  CUtensorMap tm_h3[MAX_SL][2]; // the same buffers as {64 k, B, atoms}: one copy brings a whole activation part (lstm_role_ts)
+  CUtensorMap tm_h3[MAX_SL][2]; // the same buffers as {64 k, B, atoms}: one copy brings a whole activation part (set where Hs % 64 == 0)
   CUtensorMap tm_x3[2];
   const uint8_t* w_img[MAX_SL]; // [ncl][atoms_l] swizzled 64x64 bf16 atoms: h part, (layer 0: word atom), input part
   const float* bias[MAX_SL];    // [ncl*64] b_ih + b_hh in CTA column order
@@ -97,13 +99,12 @@ struct DecParams {
   unsigned long long sample_seed;  // LAS_DECODE_SAMPLE
   int word_gather;  // 1: the fed-back word is an index (greedy argmax / gt_index); 0: a dense vector (part 1b)
   int f16;          // GEMM operand format: 0 = bf16 (LAS_MODE_BF16), 1 = IEEE fp16 (LAS_MODE_F16)
-  int lstm_ts;      // 1: LSTM CTAs use the weights-stationary operand roles and one 3-D copy per part (lstm_role_ts); 0: lstm_role
   int att_split;    // 2: every utterance is attended by a CLUSTER of two CTAs, each holding half of the encoder steps (long encoders:
                     // all of enc[b]^T stays in tensor memory; partial softmax / context combined through DSMEM); 1: one CTA
   int ctx_tmem;     // > 0: enc[b]^T is resident in the attention CTA's tensor memory and the context is a UMMA
   int ctx_ntm;      // 128-feature tiles of enc[b]^T held in tensor memory: E/128 = all of them; fewer (long encoders, e.g. U = 375:
                     // 2 of 4) = hybrid, the remaining features are reduced on the CUDA cores from the L2-resident bf16 copy
-  int groups, gsz;  // utterance groups pipelined through the LSTM CTAs (1, or 2 groups of gsz = 32 rows: lstm_role_ts) -- see lstm_role_ts
+  int groups, gsz;  // utterance groups pipelined through the LSTM CTAs (1, or 2 groups of gsz = 32 rows) -- see lstm_role_ts
   int nstages, stage_bytes;  // activation slots: [64 batch rows x 64 bf16], 128-byte swizzled; last slot = word atom
   long long* trace;  // nullable test hook: [3 roles][32 steps][8] globaltimer stamps (layer-0 CTA 0, top-layer CTA 0, attention CTA 0)
 };
@@ -155,9 +156,6 @@ __device__ __forceinline__ u64 ll_load(const u64* p) {
   return v;
 }
 __device__ __forceinline__ void ll_store(u64* p, u64 v) { asm volatile("st.relaxed.gpu.global.b64 [%0], %1;" ::"l"(p), "l"(v) : "memory"); }
-__device__ __forceinline__ void ll_store2(u64* p, u64 a, u64 b) {
-  asm volatile("st.relaxed.gpu.global.v2.b64 [%0], {%1, %2};" ::"l"(p), "l"(a), "l"(b) : "memory");
-}
 __device__ __forceinline__ uint32_t ll_wait(const u64* p, uint32_t tag) {
 #if LAS_GUARD_LL
   ptx::SpinGuard g;
@@ -195,290 +193,15 @@ __device__ __forceinline__ float dot8(const uint4& w, const float4& x0, const fl
 }
 
 // ------------------------------------------------------------------------------------------------------------
-// LSTM role
-// ------------------------------------------------------------------------------------------------------------
-template <int F16>
-__device__ void lstm_role(const DecParams& p, uint8_t* smem, int l, int nb) {
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const bool first = (l == 0), top = (l == p.sl - 1);
-  const int nh = (p.Hs + 63) / 64;                                 // atoms of the layer's own h
-  const int nc = first ? (p.E + 63) / 64 : (p.Hs + 63) / 64;      // atoms of the critical input
-  const int nwd = first ? 1 : 0;                                   // word atom
-  const int natoms = nh + nwd + nc;
-  const int NBUF = p.nstages, STAGE_BYTES = p.stage_bytes;         // NBUF = max(nh, nc) + 1; the last slot holds the word atom
-  const int wslot = NBUF - 1;
-  // Activation buffer first, weights right behind it: with 64-row slots the UMMA (M = 128) also reads the 8 KB that
-  // follow a slot (the next slot or the first weight atom); those rows only feed accumulator lanes >= 64, never read.
-  uint8_t* abuf = smem;                                  // NBUF x STAGE_BYTES
-  uint8_t* wsm = abuf + (size_t)NBUF * STAGE_BYTES;      // natoms x 8 KB
-  float* bias_s = reinterpret_cast<float*>(wsm + (size_t)natoms * WATOM_BYTES);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(bias_s + DEC_NW);
-  uint64_t* full = bars;                         // [NBUF] one per slot: TMA bytes landed
-  uint64_t* part_empty = bars + DEC_MAX_STAGES;  // all MMAs issued so far have read their slots
-  uint64_t* tmem_full = part_empty + 1;
-  uint64_t* tmem_empty = tmem_full + 1;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_empty + 1);
-  float* s_st = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(tmem_slot + 2) + 15) & ~uintptr_t(15));  // [64 rows][20] epilogue staging
-  // Warp roles.  A launch covers at most 64 utterances, so only TMEM lane quadrants 0 and 1 (batch rows 0..63) carry
-  // data; the eight warps that can read them (warp % 4 < 2) form the epilogue, four per quadrant with four hidden
-  // units each.  The producer and the MMA issuer sit on the two idle quadrants.
-  constexpr int EPI_WARPS = 8, EPI_THREADS = EPI_WARPS * 32, PROD_WARP = 2, MMA_WARP = 3;
-
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < NBUF; ++i) ptx::mbar_init(&full[i], 1);
-    ptx::mbar_init(part_empty, 1);
-    ptx::mbar_init(tmem_full, 1);
-    ptx::mbar_init(tmem_empty, EPI_THREADS);
-    ptx::fence_mbar_init();
-  }
-  if (warp == MMA_WARP) ptx::tmem_alloc(tmem_slot, 128);
-  {  // resident weight slice + bias
-    const uint4* src = reinterpret_cast<const uint4*>(p.w_img[l] + (size_t)nb * natoms * WATOM_BYTES);
-    uint4* dst = reinterpret_cast<uint4*>(wsm);
-    for (int i = threadIdx.x; i < natoms * WATOM_BYTES / 16; i += DEC_THREADS) dst[i] = src[i];
-    if (threadIdx.x < DEC_NW) bias_s[threadIdx.x] = p.bias[l][nb * DEC_NW + threadIdx.x];
-  }
-  ptx::fence_proxy_async();
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  const uint32_t tmem = *tmem_slot;
-  const int S = p.steps;
-  uint32_t* my_ready = counter(p, l);
-  const int trole = (nb == 0 && l == 0) ? 0 : ((nb == 0 && top) ? 1 : -1);
-
-  if (warp == PROD_WARP) {
-    // ============================ TMA producer ============================
-    const uint32_t* own_ctr = counter(p, l);
-    const uint32_t* in_ctr = first ? counter(p, CTR_CTX) : counter(p, l - 1);
-    const uint32_t* word_ctr = counter(p, CTR_WORD);
-    int n = 0;  // commits on part_empty waited for so far
-    for (int s = 0; s < S; ++s) {
-      const int par = s & 1;
-      // ---- part 0: own h_{s-1}, complete once every CTA of this layer finished step s-1
-      if (n > 0) ptx::mbar_wait(part_empty, (uint32_t)((n - 1) & 1));
-      ++n;
-      if (lane == 0) wait_counter(own_ctr, (uint32_t)s * p.ncl);
-      __syncwarp();
-      fence_proxy_async_global();  // other SMs' generic-proxy stores (acquired above) -> this warp's TMA reads
-      if (ptx::elect_one()) {
-        for (int i = 0; i < nh; ++i) {
-          ptx::mbar_arrive_expect_tx(&full[i], STAGE_BYTES);
-          ptx::tma_load_2d(abuf + (size_t)i * STAGE_BYTES, &p.tm_h[l][par], &full[i], i * 64, 0);
-        }
-      }
-      __syncwarp();
-      // ---- part 1a: context of step s-1 (layer 0) / the lower layer's h of THIS step
-      ptx::mbar_wait(part_empty, (uint32_t)((n - 1) & 1));
-      ++n;
-      if (ptx::elect_one())  // slots are free: arm their barriers now, so that only the copies are left to issue once the input is there
-        for (int i = 0; i < nc; ++i) ptx::mbar_arrive_expect_tx(&full[i], STAGE_BYTES);
-      __syncwarp();
-      if (lane == 0) {
-        wait_counter(in_ctr, first ? (uint32_t)s * p.B : (uint32_t)(s + 1) * p.ncl);
-        if (trole >= 0) DEC_TRACE(trole, 0);
-        DEC_TRACE_ALL(0);
-      }
-      __syncwarp();
-      fence_proxy_async_global();
-      if (lane == 0 && trole >= 0) DEC_TRACE(4, 6 + trole);
-      {
-        const CUtensorMap* tm = first ? &p.tm_x[par] : &p.tm_h[l - 1][par ^ 1];
-        if (ptx::elect_one())
-          for (int i = 0; i < nc; ++i) ptx::tma_load_2d(abuf + (size_t)i * STAGE_BYTES, tm, &full[i], i * 64, 0);
-        __syncwarp();
-      }
-      if (lane == 0 && trole >= 0) DEC_TRACE(trole, 1);
-      // ---- part 1b: dense word vector of step s-1
-      if (first && (p.s0 + s == 0 || !p.word_gather)) {
-        if (lane == 0) wait_counter(word_ctr, (uint32_t)s * p.B);
-        __syncwarp();
-        fence_proxy_async_global();
-        if (ptx::elect_one()) {
-          ptx::mbar_arrive_expect_tx(&full[wslot], STAGE_BYTES);
-          ptx::tma_load_2d(abuf + (size_t)wslot * STAGE_BYTES, &p.tm_w[par], &full[wslot], 0, 0);
-        }
-        __syncwarp();
-      }
-    }
-  } else if (warp == MMA_WARP) {
-    // ============================ MMA issuer ============================
-    const UmmaLayout la{1, 0, 1024, (uint32_t)STAGE_BYTES}, lb{1, 0, 1024, WATOM_BYTES};
-    const uint32_t idesc = umma_idesc_bf16(128, DEC_NW, F16);
-    const uint32_t a0 = ptx::smem_u32(abuf), w_addr = ptx::smem_u32(wsm);
-    uint32_t phase_bits = 0;  // per-slot phase parity
-    for (int s = 0; s < S; ++s) {
-      const bool wd = first && (p.s0 + s == 0 || !p.word_gather);
-      ptx::mbar_wait(tmem_empty, (uint32_t)((s & 1) ^ 1));
-      ptx::tc_fence_after();
-      for (int part = 0; part < 2; ++part) {
-        const int na = part == 0 ? nh : nc;
-        const uint32_t d = tmem + (part == 0 ? 0u : (uint32_t)DEC_NW);  // separate accumulators for the two parts
-        // All boxes of the part landed, then one elected thread issues the part's MMAs back to back (~57 cycles apart, the
-        // rate the tensor pipe accepts).  Issuing box by box as they land is slower: MMAs issued while later boxes are
-        // still being written into shared memory slow both down (measured per group size 1 / 2 / 4 / all boxes:
-        // 15.3 / 14.8 / 14.3 / 14.2 us per step, profiles/r01_decoder_issue_groups.log).
-        for (int i = 0; i < na; ++i) ptx::mbar_wait(&full[i], (phase_bits >> i) & 1u);
-        phase_bits ^= (1u << na) - 1u;
-        ptx::tc_fence_after();
-        if (part == 1 && lane == 0 && trole >= 0) DEC_TRACE(4, 3 + 2 * trole);  // critical part landed
-        if (ptx::elect_one()) {
-          for (int i = 0; i < na; ++i) {
-            const uint32_t a_addr = a0 + i * STAGE_BYTES, b_addr = w_addr + (part == 0 ? i : nh + nwd + i) * WATOM_BYTES;
-#pragma unroll
-            for (int k = 0; k < 4; ++k)
-              ptx::umma_bf16(d, umma_smem_desc(la, a_addr, k * 16), umma_smem_desc(lb, b_addr, k * 16), idesc, !(i == 0 && k == 0));
-          }
-          if (part == 0 || !wd) {
-            ptx::umma_commit(part_empty);
-            if (part == 1) ptx::umma_commit(tmem_full);
-          }
-        }
-        __syncwarp();
-        if (part == 0 && lane == 0 && trole >= 0) DEC_TRACE(trole, 6);
-      }
-      if (wd) {
-        ptx::mbar_wait(&full[wslot], (phase_bits >> wslot) & 1u);
-        phase_bits ^= 1u << wslot;
-        ptx::tc_fence_after();
-        if (ptx::elect_one()) {
-          const uint32_t a_addr = a0 + wslot * STAGE_BYTES, b_addr = w_addr + nh * WATOM_BYTES;
-#pragma unroll
-          for (int k = 0; k < 4; ++k)
-            ptx::umma_bf16(tmem + (uint32_t)DEC_NW, umma_smem_desc(la, a_addr, k * 16), umma_smem_desc(lb, b_addr, k * 16), idesc, 1u);
-          ptx::umma_commit(part_empty);
-          ptx::umma_commit(tmem_full);
-        }
-        __syncwarp();
-      }
-      if (lane == 0 && trole >= 0) DEC_TRACE(trole, 2);
-    }
-  } else if ((warp & 3) < 2) {
-    // ============================ epilogue: gates, cell state, h ============================
-    const int q = warp & 3, cs = warp >> 2;            // TMEM lane quadrant (batch rows), column slice (4 units = 16 columns)
-    const int b = q * 32 + lane;                       // batch row = TMEM lane
-    const int u0 = nb * DEC_UNITS + cs * 4;            // first hidden unit of this thread
-    const int c0 = cs * 16;                            // first accumulator column
-    const bool live = b < p.B;
-    const bool warp_live = q * 32 < p.B;
-    const bool lead = (warp == 0 && lane == 0);
-    const int gb = p.b0 + b;
-    float c[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) c[i] = (live && p.c_init) ? p.c_init[((size_t)l * p.c_init_rows + p.c_init_b0 + b) * p.Hs + u0 + i] : 0.f;
-    float bias_r[16];
-#pragma unroll
-    for (int i = 0; i < 16; ++i) bias_r[i] = bias_s[c0 + i];
-    const uint8_t* watom = wsm + (size_t)nh * WATOM_BYTES;  // layer 0: resident word atom [64 gate columns x 64 vocabulary entries]
-    for (int s = 0; s < S; ++s) {
-      // Word contribution first: for an index word (greedy / index teacher forcing) the token is known about a microsecond
-      // before the context GEMM finishes, so its column of W_word is added to the bias while the MMAs are still running.
-      float pb[16];
-#pragma unroll
-      for (int i = 0; i < 16; ++i) pb[i] = bias_r[i];
-      if (first && p.s0 + s > 0 && p.word_gather && live) {
-        int tok = p.gt_index ? p.gt_index[(size_t)gb * p.gt_steps + (p.s0 + s - 1)]
-                             : (s > 0 ? (int)ll_wait(p.tok_ll + (size_t)nb * p.B + b, (uint32_t)s) : p.tok_init[b]);
-        if (tok >= 0 && tok < p.V) {
-          const uint32_t tok_off = (uint32_t)(tok & 7) * 2u, tok_chunk = (uint32_t)(tok >> 3);
-#pragma unroll
-          for (int i = 0; i < 16; ++i) {  // + W_word[c0 + i, tok]: the one-hot word times the word atom, without the GEMM
-            const uint32_t rr = (uint32_t)(c0 + i);
-            const uint32_t off = (rr >> 3) * 1024u + (rr & 7u) * 128u + (((tok_chunk ^ (rr & 7u)) & 7u) << 4) + tok_off;
-            pb[i] += op_to_f32(*reinterpret_cast<const __nv_bfloat16*>(watom + off), F16);
-          }
-        }
-      }
-      if (lead && trole == 0) DEC_TRACE(4, 1);
-      ptx::mbar_wait(tmem_full, (uint32_t)(s & 1));
-      if (lead && trole >= 0) DEC_TRACE(trole, 3);
-      if (lead) DEC_TRACE_ALL(1);
-      ptx::tc_fence_after();
-      float h[4];
-      if (warp_live) {
-        uint32_t a0[16], a1[16];
-        ptx::tmem_ld_32x32b_x16(tmem + ((uint32_t)(q * 32) << 16) + c0, a0);
-        ptx::tmem_ld_32x32b_x16(tmem + ((uint32_t)(q * 32) << 16) + DEC_NW + c0, a1);
-        ptx::tmem_ld_wait();
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          const float pi = __uint_as_float(a0[u * 4 + 0]) + __uint_as_float(a1[u * 4 + 0]) + pb[u * 4 + 0];
-          const float pf = __uint_as_float(a0[u * 4 + 1]) + __uint_as_float(a1[u * 4 + 1]) + pb[u * 4 + 1];
-          const float pg = __uint_as_float(a0[u * 4 + 2]) + __uint_as_float(a1[u * 4 + 2]) + pb[u * 4 + 2];
-          const float po = __uint_as_float(a0[u * 4 + 3]) + __uint_as_float(a1[u * 4 + 3]) + pb[u * 4 + 3];
-          const float cn = sigmoid_fast(pf) * c[u] + sigmoid_fast(pi) * tanh_fast(pg);
-          c[u] = cn;
-          h[u] = sigmoid_fast(po) * tanh_fast(cn);
-        }
-      }
-      ptx::tc_fence_before();
-      ptx::mbar_arrive(tmem_empty);
-      const int np = (s + 1) & 1;
-      // Coalesced hand-off stores.  A thread owns one batch row, so a warp-wide store of its values touches 32 different
-      // rows of the row-major hand-off buffers (32 partial sectors per instruction; the top layer's flag-in-data slots took
-      // up to ~1.4 us to become visible).  The 64 x 16 block goes through shared memory instead (rows padded to 20 floats:
-      // conflict-free 16-byte writes) and every warp writes 8 whole rows: full 128-byte lines of {h, tag} slots for the
-      // attention CTAs, full 32-byte sectors of the bf16 operand copy.
-      if (warp_live) *reinterpret_cast<float4*>(s_st + b * 20 + cs * 4) = make_float4(h[0], h[1], h[2], h[3]);
-      asm volatile("bar.sync 1, 256;" ::: "memory");
-      const int r0 = (cs * 2 + q) * 8;  // this warp's 8 rows
-      if (top) {
-        const uint32_t tag = (uint32_t)(s + 1);
-#pragma unroll
-        for (int hf = 0; hf < 2; ++hf) {
-          const int row = r0 + hf * 4 + (lane >> 3), piece = lane & 7;
-          if (row < p.B) {
-            const float2 v = *reinterpret_cast<const float2*>(s_st + row * 20 + piece * 2);
-            ll_store2(p.h_ll + (size_t)row * p.Hs + nb * DEC_UNITS + piece * 2, ll_pack(__float_as_uint(v.x), tag), ll_pack(__float_as_uint(v.y), tag));
-          }
-        }
-      }
-      if (lane < 16) {
-        const int row = r0 + (lane >> 1), hf = lane & 1;
-        if (row < p.B) {
-          const float4 x0 = *reinterpret_cast<const float4*>(s_st + row * 20 + hf * 8), x1 = *reinterpret_cast<const float4*>(s_st + row * 20 + hf * 8 + 4);
-          const __nv_bfloat162 t0 = op2_from_f32(x0.x, x0.y, F16), t1 = op2_from_f32(x0.z, x0.w, F16);
-          const __nv_bfloat162 t2 = op2_from_f32(x1.x, x1.y, F16), t3 = op2_from_f32(x1.z, x1.w, F16);
-          *reinterpret_cast<uint4*>(p.hbuf[l][np] + (size_t)row * p.Hs + nb * DEC_UNITS + hf * 8) =
-              make_uint4(*reinterpret_cast<const uint32_t*>(&t0), *reinterpret_cast<const uint32_t*>(&t1),
-                         *reinterpret_cast<const uint32_t*>(&t2), *reinterpret_cast<const uint32_t*>(&t3));
-        }
-      }
-      if (live && s == S - 1) {
-        if (p.h_out) {
-#pragma unroll
-          for (int i = 0; i < 4; ++i) p.h_out[((size_t)l * p.Bfull + gb) * p.Hs + u0 + i] = h[i];
-        }
-        if (p.c_out) {
-#pragma unroll
-          for (int i = 0; i < 4; ++i) p.c_out[((size_t)l * p.c_out_rows + p.c_out_b0 + b) * p.Hs + u0 + i] = c[i];
-        }
-      }
-      if (lead && trole >= 0) DEC_TRACE(trole, 4);
-      if (lead) DEC_TRACE_ALL(2);
-      asm volatile("bar.sync 1, 256;" ::: "memory");  // all rows stored; the release below is cumulative over the barrier
-      if (lead) {
-        red_release_add(my_ready, 1u);
-        if (trole >= 0) DEC_TRACE(trole, 5);
-        DEC_TRACE_ALL(3);
-      }
-    }
-  }
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (warp == MMA_WARP) ptx::tmem_dealloc(tmem, 128);
-}
-
-// ------------------------------------------------------------------------------------------------------------
 // LSTM role, weights-stationary operand roles ("TS form")
 // ------------------------------------------------------------------------------------------------------------
-// Same CTA, same data flow and hand-offs as lstm_role, but the two GEMM operands trade places on the critical part:
+// The weights are the A operand and the activations (one part at a time, see the file header) the B operand:
 //     D[gate row (64 of the 128 TMEM lanes), batch (N = 64)] = W_slice[64(128), K] . act[batch, K]^T
 // so that the layer's critical input weights (context / lower-layer h part, K = 512 -> 256 tensor-memory columns) are the A operand
 // IN TENSOR MEMORY: a tcgen05.mma with A in TMEM issues at its ~32-cycle math floor (N = 64), against ~57 cycles when both
-// operands come from shared memory (tools/microbench.cu: the shared-memory A read is exposed).  The part's 32 instructions were
-// ~1.05 us of each layer's critical path; here ~0.55 us.  The own-h part (ready long before it is needed) stays in the
-// shared-memory form with the same operand roles, so both parts land in accumulators of the same orientation.
+// operands come from shared memory (tools/microbench.cu: the shared-memory A read is exposed).  The part's 32 instructions take
+// ~0.55 us of each layer's critical path instead of ~1.05 us.  The own-h part (ready long before it is needed) takes both operands
+// from shared memory, in the same roles, so both parts land in accumulators of the same orientation.
 // M = 128 although a CTA owns only 64 gate rows: lanes 64..127 hold zeros / read the atom behind (the instruction costs the same
 // for M = 64 and 128), which keeps the plain lane = row layout.
 // Epilogue: thread = gate row (lane; unit-major / gate-minor, so the four gates of a unit sit in four adjacent lanes), 16 batch
@@ -559,7 +282,17 @@ __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
   const int trole = (nb == 0 && l == 0) ? 0 : ((nb == 0 && top) ? 1 : -1);
 
   if (warp == PROD_WARP) {
-    // ============================ TMA producer (as in lstm_role) ============================
+    // ============================ TMA producer ============================
+    // A part lands as consecutive [GSZ batch rows x 64 k] atoms in slots 0, 1, ... and completes on full[0].  Where Hs (= E) is a
+    // multiple of 64 it is ONE 3-D copy over the {64 k, batch, atoms} view of the hand-off buffer: issuing eight 2-D copies took
+    // ~0.55 us (~68 ns each), all of it on the critical path.  That view cannot describe a row of any other length; there every
+    // atom is a 2-D copy, and TMA fills the columns past Hs with zeros (the weights' columns there are zeros too).
+    const bool whole_atoms = p.Hs % 64 == 0;
+    auto load_part = [&](const CUtensorMap* tm3, const CUtensorMap* tm2, int na, int row0) {
+      if (whole_atoms) ptx::tma_load_3d(abuf, tm3, &full[0], 0, row0, 0);
+      else
+        for (int i = 0; i < na; ++i) ptx::tma_load_2d(abuf + (size_t)i * STAGE_BYTES, tm2, &full[0], i * 64, row0);
+    };
     int n = 0;
     for (int it = 0; it < S * G; ++it) {
       const int s = it / G, grp = it - s * G, row0 = grp * GSZ;
@@ -575,7 +308,7 @@ __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
       fence_proxy_async_global();
       if (ptx::elect_one()) {
         ptx::mbar_arrive_expect_tx(&full[0], nh * STAGE_BYTES);
-        ptx::tma_load_3d(abuf, &p.tm_h3[l][par], &full[0], 0, row0, 0);
+        load_part(&p.tm_h3[l][par], &p.tm_h[l][par], nh, row0);
       }
       __syncwarp();
       ptx::mbar_wait(part_empty, (uint32_t)((n - 1) & 1));
@@ -592,10 +325,10 @@ __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
       if (lane == 0 && trole >= 0 && grp == 0) DEC_TRACE(4, 6 + trole);
       {
         const CUtensorMap* tm3 = first ? &p.tm_x3[par] : &p.tm_h3[l - 1][par ^ 1];
+        const CUtensorMap* tm2 = first ? &p.tm_x[par] : &p.tm_h[l - 1][par ^ 1];
         if (ptx::elect_one()) {
-          // one instruction for the whole part: issuing eight 2-D copies took ~0.55 us (~68 ns each), all of it on the critical path
           if (trole == 0 && grp == 0) DEC_TRACE(4, 0);
-          ptx::tma_load_3d(abuf, tm3, &full[0], 0, row0, 0);
+          load_part(tm3, tm2, nc, row0);
           if (trole == 0 && grp == 0) DEC_TRACE(4, 2);
         }
         __syncwarp();
@@ -770,7 +503,8 @@ __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
       ptx::tc_fence_before();
       ptx::mbar_arrive(tmem_empty);
       const int np = (s + 1) & 1;
-      // hand-off: the 64 x 16 block through shared memory ([batch row][20 floats]), then whole rows per warp (as in lstm_role)
+      // hand-off: the 64 x 16 block through shared memory ([batch row][20 floats], conflict-free 16-byte reads), then every warp
+      // writes 8 whole rows of the bf16 operand copy (full 32-byte sectors instead of one partial sector per batch row)
       // top layer: the {h, tag} slots the attention CTAs poll leave straight from the registers, before the staging barrier
       // (0.11 us/step faster than staged whole-row stores)
       if (top && warp_live) {
@@ -1445,10 +1179,7 @@ __global__ void __launch_bounds__(DEC_THREADS, 1) speller_decode_persistent_kern
   uint8_t* smem = smem_raw + ((1024u - (ptx::smem_u32(smem_raw) & 1023u)) & 1023u);
   const int n_lstm = p.sl * p.ncl;
   if (p.stop && *reinterpret_cast<const volatile int32_t*>(p.stop) != 0) return;  // written before this launch: every CTA sees the same value
-  if ((int)blockIdx.x < n_lstm) {
-    if (p.lstm_ts) lstm_role_ts<F16>(p, smem, blockIdx.x / p.ncl, blockIdx.x % p.ncl);
-    else lstm_role<F16>(p, smem, blockIdx.x / p.ncl, blockIdx.x % p.ncl);
-  }
+  if ((int)blockIdx.x < n_lstm) lstm_role_ts<F16>(p, smem, blockIdx.x / p.ncl, blockIdx.x % p.ncl);
   else if (p.att_split == 2) attention_role<F16>(p, smem, (blockIdx.x - n_lstm) >> 1, (blockIdx.x - n_lstm) & 1);
   else attention_role<F16>(p, smem, blockIdx.x - n_lstm, 0);
 }
@@ -1509,7 +1240,6 @@ __global__ void dec_init_kernel(DecParams p, const float* enc_f32, const float* 
 }
 
 int g_dec_ctx_tmem = 1;   // las_debug_set_option(2, 0): the context on the CUDA cores only
-int g_dec_lstm_role = 0;  // las_debug_set_option(5, 1): lstm_role (shared-memory operands, per-atom 2-D copies) where lstm_role_ts would run
 
 struct Shape {
   int ncl, natoms[MAX_SL];
@@ -1653,7 +1383,7 @@ bool fast_speller_fits(const las_speller_dims* d) {
   return ok;
 }
 bool fast_set_option_speller(int key, int value) {
-  int* opt = key == 2 ? &g_dec_ctx_tmem : key == 5 ? &g_dec_lstm_role : key == 11 ? &g_dec_att_split : key == 19 ? &g_dec_groups : nullptr;
+  int* opt = key == 2 ? &g_dec_ctx_tmem : key == 11 ? &g_dec_att_split : key == 19 ? &g_dec_groups : nullptr;
   if (!opt || (value != 0 && value != 1)) return false;
   *opt = value;
   return true;
@@ -1722,35 +1452,30 @@ int fast_speller_decode_segment(const las_decode_io* io, const SpellerF32Inputs&
       if (hyb && att_smem(d, p.k_in_smem != 0, true) > 220 * 1024) { p.ctx_ntm = 0; p.ctx_tmem = 0; p.k_in_smem = att_smem(d, true, false) <= 220 * 1024; }
     }
     RingCfg rc = ring_cfg(d);
-    // weights-stationary LSTM CTAs: whole 64-wide atoms (E == Hs), one 3-D copy per part, critical weights within 256 tensor-memory
-    // columns (Hs <= 512)
-    p.lstm_ts = (d->Hs % 64 == 0 && !g_dec_lstm_role) ? 1 : 0;
-    // two utterance groups of 32 pipelined through the LSTM CTAs (lstm_role_ts) when the launch has more than 32 utterances
-    p.groups = (p.lstm_ts && Bc > 32 && g_dec_groups != 0) ? 2 : 1;
+    // two utterance groups of 32 pipelined through the LSTM CTAs when the launch has more than 32 utterances
+    p.groups = (Bc > 32 && g_dec_groups != 0) ? 2 : 1;
     p.gsz = p.groups == 2 ? 32 : 64;
     rc.box_rows = p.gsz;
     rc.stage_bytes = rc.box_rows * 128;
     p.nstages = rc.nstages;
     p.stage_bytes = rc.stage_bytes;
+    // the LSTM CTAs fetch an activation part as one 3-D copy where its rows are whole 64-column atoms (E == Hs), else atom by atom
+    const bool whole_atoms = d->Hs % 64 == 0;
     for (int l = 0; l < d->sl; ++l) {
       p.w_img[l] = pk.w_img[l];
       p.bias[l] = pk.bias[l];
       for (int k = 0; k < 2; ++k) {
         p.hbuf[l][k] = w.hbuf[l][k];
-        LAS_TRY(make_tmap_bf16_box(&p.tm_h[l][k], w.hbuf[l][k], Bc, d->Hs, d->Hs, rc.box_rows));
+        if (whole_atoms) LAS_TRY(make_tmap_bf16_atoms(&p.tm_h3[l][k], w.hbuf[l][k], Bc, d->Hs / 64, d->Hs, rc.box_rows, d->Hs / 64));
+        else LAS_TRY(make_tmap_bf16_box(&p.tm_h[l][k], w.hbuf[l][k], Bc, d->Hs, d->Hs, rc.box_rows));
       }
     }
     for (int k = 0; k < 2; ++k) {
       p.xbuf[k] = w.xbuf[k];
       p.wbuf[k] = w.wbuf[k];
-      LAS_TRY(make_tmap_bf16_box(&p.tm_x[k], w.xbuf[k], Bc, d->E, d->E, rc.box_rows));
+      if (whole_atoms) LAS_TRY(make_tmap_bf16_atoms(&p.tm_x3[k], w.xbuf[k], Bc, d->E / 64, d->E, rc.box_rows, d->E / 64));
+      else LAS_TRY(make_tmap_bf16_box(&p.tm_x[k], w.xbuf[k], Bc, d->E, d->E, rc.box_rows));
       LAS_TRY(make_tmap_bf16_box(&p.tm_w[k], w.wbuf[k], Bc, DEC_VP, DEC_VP, rc.box_rows));
-    }
-    if (p.lstm_ts) {
-      for (int l = 0; l < d->sl; ++l)
-        for (int k = 0; k < 2; ++k) LAS_TRY(make_tmap_bf16_atoms(&p.tm_h3[l][k], w.hbuf[l][k], Bc, d->Hs / 64, d->Hs, rc.box_rows, d->Hs / 64));
-      for (int k = 0; k < 2; ++k)
-        LAS_TRY(make_tmap_bf16_atoms(&p.tm_x3[k], w.xbuf[k], Bc, d->E / 64, d->E, rc.box_rows, d->E / 64));
     }
     const size_t so = (size_t)b0;  // batch offset into caller tensors
     p.Bfull = d->B;

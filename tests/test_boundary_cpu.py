@@ -50,8 +50,8 @@ def test_debug_options_take_documented_values_and_reject_the_rest():
     timing the default kernel twice."""
     lib = _cabi.load_library()
     overlap = 0 if os.environ.get("LAS_B200_NO_OVERLAP", "") not in ("", "0") else 1  # as _cabi.load_library leaves key 6
-    defaults = {2: 1, 5: 0, 6: overlap, 8: 0, 9: 0, 11: 1, 12: 1, 13: 0, 19: 1, **{20 + l: 0 for l in range(8)}}
-    values = {2: [0, 1], 5: [0, 1], 6: [0, 1], 8: [0, 1], 9: [0, 16, 32, 64], 11: [0, 1], 12: [0, 1], 13: [0, 1, 2, 4, 8], 19: [0, 1],
+    defaults = {2: 1, 6: overlap, 8: 0, 9: 0, 11: 1, 12: 1, 13: 0, 19: 1, **{20 + l: 0 for l in range(8)}}
+    values = {2: [0, 1], 6: [0, 1], 8: [0, 1], 9: [0, 16, 32, 64], 11: [0, 1], 12: [0, 1], 13: [0, 1, 2, 4, 8], 19: [0, 1],
               **{20 + l: [0, 1, 160] for l in range(8)}}
     try:
         for key, vals in values.items():
@@ -61,7 +61,7 @@ def test_debug_options_take_documented_values_and_reject_the_rest():
         for key, v in defaults.items():
             assert lib.las_debug_set_option(key, v) == 0, (key, v)
     rejected = [(k, 1) for k in (1, 4, 7, 10, 15, 16, 18)] + [(k, 0) for k in (0, 3, 14, 17, 28, 99, -1)]
-    rejected += [(5, 4), (5, 16384), (2, 2), (11, 2), (11, 3), (19, 2), (13, 3), (13, 16), (9, 8), (6, 2), (8, -1), (12, 2), (20, -1)]
+    rejected += [(5, 0), (5, 1), (5, 4), (5, 16384), (2, 2), (11, 2), (11, 3), (19, 2), (13, 3), (13, 16), (9, 8), (6, 2), (8, -1), (12, 2), (20, -1)]
     for key, v in rejected:
         assert lib.las_debug_set_option(key, v) == -1, (key, v)  # LAS_EINVAL
         assert f"key {key} ".encode() in lib.las_last_error(), (key, v)

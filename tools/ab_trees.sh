@@ -5,8 +5,8 @@ TAG=${1:-x}; shift; OTHERS=${@:-.ab_head}
 mkdir -p gpurun_out
 {
 for rep in 1 2; do
-  echo "== decoder, tree=new";   python tools/decoder_ab.py 0
-  for o in $OTHERS; do echo "== decoder, tree=$o"; LAS_ROOT=$PWD/$o python tools/decoder_ab.py 0; done
+  echo "== decoder, tree=new";   python tools/decoder_ab.py
+  for o in $OTHERS; do echo "== decoder, tree=$o"; LAS_ROOT=$PWD/$o python tools/decoder_ab.py; done
   echo "== listener, tree=new";   python tools/listener_ab.py
   for o in $OTHERS; do echo "== listener, tree=$o"; LAS_ROOT=$PWD/$o python tools/listener_ab.py; done
 done
