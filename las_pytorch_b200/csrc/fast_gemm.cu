@@ -368,7 +368,7 @@ int make_tmap_x_core(CUtensorMap* tm, const void* x_bf16, int B, int Tl, int Kx,
 }
 
 int launch_gemm_bf16_tc(const __nv_bfloat16* A, long long lda, const __nv_bfloat16* W, long long ldw, const float* bias, float* C,
-                        long long ldc, int M, int N, int K, cudaStream_t st, bool relu) {
+                        long long ldc, int M, int N, int K, bool f16, cudaStream_t st, bool relu) {
   LAS_REQUIRE(M > 0 && N > 0 && K > 0, "bad GEMM shape %dx%dx%d", M, N, K);
   CUtensorMap tm_a, tm_b;
   LAS_TRY(make_tmap_bf16(&tm_a, A, M, K, lda, BM));
@@ -382,7 +382,7 @@ int launch_gemm_bf16_tc(const __nv_bfloat16* A, long long lda, const __nv_bfloat
   const size_t smem = sizeof(GemmSmem) + 1024;
   // per launch, not cached: the attribute belongs to the current device's context and a host thread may serve several devices
   LAS_CUDA_OK(cudaFuncSetAttribute(gemm_bf16_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  gemm_bf16_tc_kernel<<<grid, GEMM_THREADS, smem, st>>>(tm_a, tm_b, tm_c, bias, C, ldc, M, N, K, relu ? 1 : 0, ts ? 1 : 0, GemmSched{0, 0, 0, op_f16(), nullptr});
+  gemm_bf16_tc_kernel<<<grid, GEMM_THREADS, smem, st>>>(tm_a, tm_b, tm_c, bias, C, ldc, M, N, K, relu ? 1 : 0, ts ? 1 : 0, GemmSched{0, 0, 0, f16, nullptr});
   LAS_LAUNCH_OK("gemm_bf16_tc_kernel");
   return LAS_OK;
 }
@@ -395,7 +395,7 @@ int listener_padded_batch(int B) {
 }
 
 int launch_gemm_listener(const __nv_bfloat16* A, int B, int Tl, int K, const __nv_bfloat16* W, const float* bias, float* C, int N,
-                         uint32_t* flags, int max_ctas, cudaStream_t st) {
+                         uint32_t* flags, int max_ctas, bool f16, cudaStream_t st) {
   LAS_REQUIRE(B > 0 && Tl > 0 && N > 0 && K > 0, "bad listener GEMM shape B=%d Tl=%d N=%d K=%d", B, Tl, N, K);
   const int Bp = listener_padded_batch(B);
   const int M = Tl * Bp;
@@ -430,7 +430,7 @@ int launch_gemm_listener(const __nv_bfloat16* A, int B, int Tl, int K, const __n
   // forward-direction columns are the first half of N; when the halves do not fall on tile boundaries every column tile
   // serves both directions and the natural (front-first) order is kept
   const int nfwd = ((N / 2) % BN == 0) ? (N / 2) / BN : n_tiles;
-  gemm_bf16_tc_kernel<<<grid, GEMM_THREADS, smem, st>>>(tm_a, tm_b, tm_c, bias, C, (long long)N, M, N, K, 0, ts ? 1 : 0, GemmSched{1, Bp, nfwd, op_f16(), flags});
+  gemm_bf16_tc_kernel<<<grid, GEMM_THREADS, smem, st>>>(tm_a, tm_b, tm_c, bias, C, (long long)N, M, N, K, 0, ts ? 1 : 0, GemmSched{1, Bp, nfwd, f16, flags});
   LAS_LAUNCH_OK("gemm_bf16_tc_kernel");
   return LAS_OK;
 }
@@ -549,11 +549,11 @@ __global__ void f32_to_bf16_kernel(const float* __restrict__ src, __nv_bfloat16*
     }
   }
 }
-int launch_f32_to_bf16(const float* src, __nv_bfloat16* dst, size_t n, cudaStream_t st) {
+int launch_f32_to_bf16(const float* src, __nv_bfloat16* dst, size_t n, bool f16, cudaStream_t st) {
   if (n == 0) return LAS_OK;
   LAS_REQUIRE((reinterpret_cast<uintptr_t>(src) & 15) == 0 && (reinterpret_cast<uintptr_t>(dst) & 7) == 0, "unaligned cast buffers");
   const size_t blocks = (n / 4 + 255) / 256;
-  f32_to_bf16_kernel<<<(unsigned)(blocks < 2368 ? (blocks ? blocks : 1) : 2368), 256, 0, st>>>(src, dst, n, op_f16());
+  f32_to_bf16_kernel<<<(unsigned)(blocks < 2368 ? (blocks ? blocks : 1) : 2368), 256, 0, st>>>(src, dst, n, f16);
   LAS_LAUNCH_OK("f32_to_bf16_kernel");
   return LAS_OK;
 }

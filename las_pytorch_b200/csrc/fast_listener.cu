@@ -614,7 +614,7 @@ bool fast_listener_fits(const las_listener_dims* d) {
 size_t fast_listener_packed_bytes(const las_listener_dims* d) { return pack_layout(d, nullptr).bytes; }
 size_t fast_listener_workspace_bytes(const las_listener_dims* d) { return ws_layout(d, nullptr).bytes; }
 
-int fast_listener_pack(const las_lstm_weights* w, const las_listener_dims* d, void* packed, cudaStream_t st) {
+int fast_listener_pack(const las_lstm_weights* w, const las_listener_dims* d, void* packed, bool f16, cudaStream_t st) {
   LAS_TRY(shape_ok(d));
   const Geo g = geometry(d->H);
   const ListenerPackFast pk = pack_layout(d, packed);
@@ -622,11 +622,11 @@ int fast_listener_pack(const las_lstm_weights* w, const las_listener_dims* d, vo
     const int K = (l == 0) ? 2 * d->F : 4 * d->H;
     const las_lstm_weights &f = w[2 * l], &r = w[2 * l + 1];
     LAS_REQUIRE(f.w_ih && f.w_hh && f.b_ih && f.b_hh && r.w_ih && r.w_hh && r.b_ih && r.b_hh, "null weight pointer in layer %d", l);
-    pack_wih_kernel<<<592, 256, 0, st>>>(f.w_ih, r.w_ih, pk.wih[l], d->H, g.Hp, K, op_f16());
+    pack_wih_kernel<<<592, 256, 0, st>>>(f.w_ih, r.w_ih, pk.wih[l], d->H, g.Hp, K, f16);
     LAS_LAUNCH_OK("pack_wih_kernel");
     pack_bias_kernel<<<(8 * g.Hp + 255) / 256, 256, 0, st>>>(f.b_ih, f.b_hh, r.b_ih, r.b_hh, pk.bias[l], d->H, g.Hp);
     LAS_LAUNCH_OK("pack_bias_kernel");
-    pack_whh_kernel<<<592, 256, 0, st>>>(f.w_hh, r.w_hh, pk.whh[l], d->H, g.Hp, g.CS, op_f16());
+    pack_whh_kernel<<<592, 256, 0, st>>>(f.w_hh, r.w_hh, pk.whh[l], d->H, g.Hp, g.CS, f16);
     LAS_LAUNCH_OK("pack_whh_kernel");
   }
   return LAS_OK;
@@ -648,7 +648,7 @@ static LayerGeom layer_geom(const las_listener_dims* d, const Geo& g, const List
   return q;
 }
 static RecParams rec_params(const las_listener_dims* d, const Geo& g, const ListenerPackFast& pk, const ListenerWsFast& w, int l, float* enc,
-                            const int32_t* len_l, int bc) {
+                            const int32_t* len_l, int bc, bool f16) {
   const LayerGeom q = layer_geom(d, g, w, l);
   const bool last = (l == d->L - 1);
   RecParams rp;
@@ -664,7 +664,7 @@ static RecParams rec_params(const las_listener_dims* d, const Geo& g, const List
   rp.trace = (l == 0) ? g_rec_trace : nullptr;
   rp.nchunks = (d->B + bc - 1) / bc;
   rp.resident = nullptr;
-  rp.f16 = op_f16();
+  rp.f16 = f16;
   rp.Kx = 0;
   rp.wih_img = nullptr;
   rp.bias = nullptr;
@@ -700,7 +700,7 @@ int fast_listener_rec_ctas(const las_listener_dims* d, int bc) {
 }
 
 int fast_listener_stage(const float* x, const int32_t* x_lengths, const void* packed, const las_listener_dims* d, float* enc,
-                        int32_t* enc_lengths, void* ws, int stage, int bc, int* resident, cudaStream_t st) {
+                        int32_t* enc_lengths, void* ws, int stage, int bc, int* resident, bool f16, cudaStream_t st) {
   LAS_TRY(shape_ok(d));
   const Geo g = geometry(d->H);
   const ListenerPackFast pk = pack_layout(d, const_cast<void*>(packed));
@@ -708,7 +708,7 @@ int fast_listener_stage(const float* x, const int32_t* x_lengths, const void* pa
   char nm[48];
   if (stage == 0) {
     ProfScope ps("listener.cast_bf16", st);
-    return launch_f32_to_bf16(x, w.xb, (size_t)d->B * d->T * d->F, st);
+    return launch_f32_to_bf16(x, w.xb, (size_t)d->B * d->T * d->F, f16, st);
   }
   const int l = (stage - 1) / 2;
   const LayerGeom q = layer_geom(d, g, w, l);
@@ -717,9 +717,9 @@ int fast_listener_stage(const float* x, const int32_t* x_lengths, const void* pa
     if (fuse_x(d, l)) return LAS_OK;  // the recurrence does the projection itself
     snprintf(nm, sizeof(nm), "listener.L%d.input_gemm", l);
     ProfScope ps(nm, st);
-    return launch_gemm_listener(q.in, d->B, q.Tl, q.K, pk.wih[l], pk.bias[l], w.P, q.NP, nullptr, 0, st);
+    return launch_gemm_listener(q.in, d->B, q.Tl, q.K, pk.wih[l], pk.bias[l], w.P, q.NP, nullptr, 0, f16, st);
   }
-  RecParams rp = rec_params(d, g, pk, w, l, enc, x_lengths ? w.len + (size_t)l * d->B : nullptr, bc);
+  RecParams rp = rec_params(d, g, pk, w, l, enc, x_lengths ? w.len + (size_t)l * d->B : nullptr, bc, f16);
   rp.resident = resident;
   if (fuse_x(d, l)) LAS_TRY(rec_fuse(rp, d, pk, w, bc));
   snprintf(nm, sizeof(nm), "listener.L%d.recurrence", l);
@@ -741,13 +741,13 @@ int fast_side_stream(cudaStream_t* s) {
 }
 
 int fast_listener_forward(const float* x, const int32_t* x_lengths, const void* packed, const las_listener_dims* d, float* enc,
-                          int32_t* enc_lengths, void* ws, cudaStream_t st) {
+                          int32_t* enc_lengths, void* ws, bool f16, cudaStream_t st) {
   LAS_TRY(shape_ok(d));
   const Geo g = geometry(d->H);
   const ListenerPackFast pk = pack_layout(d, const_cast<void*>(packed));
   const ListenerWsFast w = ws_layout(d, ws);
   const int B = d->B;
-  LAS_TRY(fast_listener_stage(x, x_lengths, packed, d, enc, enc_lengths, ws, 0, 0, nullptr, st));
+  LAS_TRY(fast_listener_stage(x, x_lengths, packed, d, enc, enc_lengths, ws, 0, 0, nullptr, f16, st));
   for (int l = 0; l < d->L; ++l) {
     const LayerGeom q = layer_geom(d, g, w, l);
     const int32_t* len_l = nullptr;
@@ -756,7 +756,7 @@ int fast_listener_forward(const float* x, const int32_t* x_lengths, const void* 
       len_l = w.len + (size_t)l * B;
     }
     const int bc = g_rec_force_bc ? g_rec_force_bc : pick_bc(B, g.CS);
-    RecParams rp = rec_params(d, g, pk, w, l, enc, len_l, bc);
+    RecParams rp = rec_params(d, g, pk, w, l, enc, len_l, bc, f16);
     // The GEMM emits its tiles in the recurrence's consumption order and flags each one, so it can run next to the recurrence
     // (which occupies 2 * nchunks * CS SMs) on the remaining SMs instead of in front of it.  Needs the two directions' columns
     // to fall on separate column tiles and enough free SMs to be worth it.
@@ -787,7 +787,7 @@ int fast_listener_forward(const float* x, const int32_t* x_lengths, const void* 
       }
       snprintf(nm, sizeof(nm), overlap ? "listener.L%d.input_gemm.overlapped" : "listener.L%d.input_gemm", l);
       ProfScope ps(nm, gs);
-      LAS_TRY(launch_gemm_listener(q.in, B, q.Tl, q.K, pk.wih[l], pk.bias[l], w.P, q.NP, overlap ? w.flags : nullptr, overlap ? gemm_ctas : 0, gs));
+      LAS_TRY(launch_gemm_listener(q.in, B, q.Tl, q.K, pk.wih[l], pk.bias[l], w.P, q.NP, overlap ? w.flags : nullptr, overlap ? gemm_ctas : 0, f16, gs));
     }
     {
       snprintf(nm, sizeof(nm), "listener.L%d.recurrence", l);

@@ -84,12 +84,12 @@ int fast_pipeline_bc(const las_listener_dims* ld, const las_speller_dims* sd, in
 
 int fast_pipeline_step(const las_decode_io* io, const SpellerF32Inputs& spl_f32, const void* spl_packed_fast, const las_speller_dims* sd,
                        int steps, int decode_mode, int relu, void* spl_ws_fast, const float* x, const int32_t* x_lengths, const void* lis_packed,
-                       const las_listener_dims* ld, float* enc, int32_t* enc_lengths, void* lis_ws, cudaStream_t st) {
+                       const las_listener_dims* ld, float* enc, int32_t* enc_lengths, void* lis_ws, bool f16, cudaStream_t st) {
   const int bc = fast_pipeline_bc(ld, sd, steps);
   if (bc == 0 || io->early_exit) {
     // no room next to the decoder (or a decoder that may stop early): one after the other
-    LAS_TRY(fast_speller_decode(io, spl_f32, spl_packed_fast, sd, steps, decode_mode, relu, spl_ws_fast, st));
-    return fast_listener_forward(x, x_lengths, lis_packed, ld, enc, enc_lengths, lis_ws, st);
+    LAS_TRY(fast_speller_decode(io, spl_f32, spl_packed_fast, sd, steps, decode_mode, relu, spl_ws_fast, f16, st));
+    return fast_listener_forward(x, x_lengths, lis_packed, ld, enc, enc_lengths, lis_ws, f16, st);
   }
   PipeEvents* pe = nullptr;
   LAS_TRY(pipe_events(&pe));
@@ -115,24 +115,24 @@ int fast_pipeline_step(const las_decode_io* io, const SpellerF32Inputs& spl_f32,
   const int rec_ctas = fast_listener_rec_ctas(ld, bc);
   const int Bc = sd->B;
   LAS_CUDA_OK(cudaMemsetAsync(pe->resident, 0, sizeof(int) * 8, st));
-  LAS_TRY(fast_listener_stage(x, x_lengths, lis_packed, ld, enc, enc_lengths, lis_ws, 0, bc, nullptr, st));
-  LAS_TRY(fast_listener_stage(x, x_lengths, lis_packed, ld, enc, enc_lengths, lis_ws, 1, bc, nullptr, st));
+  LAS_TRY(fast_listener_stage(x, x_lengths, lis_packed, ld, enc, enc_lengths, lis_ws, 0, bc, nullptr, f16, st));
+  LAS_TRY(fast_listener_stage(x, x_lengths, lis_packed, ld, enc, enc_lengths, lis_ws, 1, bc, nullptr, f16, st));
   LAS_CUDA_OK(cudaEventRecord(pe->gemm_done[0], st));
   int sb = 0;
   for (int l = 0; l < L; ++l) {
     // recurrence of layer l on the side stream, placed first ...
     LAS_CUDA_OK(cudaStreamWaitEvent(side, pe->gemm_done[l], 0));
-    LAS_TRY(fast_listener_stage(x, x_lengths, lis_packed, ld, enc, enc_lengths, lis_ws, 2 + 2 * l, bc, pe->resident + l, side));
+    LAS_TRY(fast_listener_stage(x, x_lengths, lis_packed, ld, enc, enc_lengths, lis_ws, 2 + 2 * l, bc, pe->resident + l, f16, side));
     LAS_CUDA_OK(cudaEventRecord(pe->rec_done[l], side));
     // ... then the decoder's segment on the SMs it leaves free
     wait_resident_kernel<<<1, 1, 0, st>>>(pe->resident + l, rec_ctas);
     LAS_LAUNCH_OK("wait_resident_kernel");
     LAS_TRY(fast_speller_decode_segment(io, spl_f32, spl_packed_fast, sd, 0, Bc, sb, seg[l], sb == 0, l == L - 1, decode_mode, relu, spl_ws_fast,
-                                        st));
+                                        f16, st));
     sb += seg[l];
     LAS_CUDA_OK(cudaStreamWaitEvent(st, pe->rec_done[l], 0));
     if (l + 1 < L) {
-      LAS_TRY(fast_listener_stage(x, x_lengths, lis_packed, ld, enc, enc_lengths, lis_ws, 3 + 2 * l, bc, nullptr, st));
+      LAS_TRY(fast_listener_stage(x, x_lengths, lis_packed, ld, enc, enc_lengths, lis_ws, 3 + 2 * l, bc, nullptr, f16, st));
       LAS_CUDA_OK(cudaEventRecord(pe->gemm_done[l + 1], st));
     }
   }

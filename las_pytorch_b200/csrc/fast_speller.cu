@@ -1392,20 +1392,20 @@ bool fast_set_option_speller(int key, int value) {
 size_t fast_speller_packed_bytes(const las_speller_dims* d) { return pack_layout(d, nullptr).bytes; }
 size_t fast_speller_workspace_bytes(const las_speller_dims* d) { return ws_layout(d, nullptr).bytes; }
 
-int fast_speller_pack(const las_speller_weights* w, const las_speller_dims* d, void* packed_fast, cudaStream_t st) {
+int fast_speller_pack(const las_speller_weights* w, const las_speller_dims* d, void* packed_fast, bool f16, cudaStream_t st) {
   LAS_TRY(supported(d));
   const SpellerPackFast pk = pack_layout(d, packed_fast);
   const Shape s = shape_of(d);
   for (int l = 0; l < d->sl; ++l) {
     const las_lstm_weights& lw = w->rnn_host[l];
-    pack_dec_w_kernel<<<592, 256, 0, st>>>(lw.w_ih, lw.w_hh, pk.w_img[l], l, d->Hs, d->E, d->V, s.ncl, op_f16());
+    pack_dec_w_kernel<<<592, 256, 0, st>>>(lw.w_ih, lw.w_hh, pk.w_img[l], l, d->Hs, d->E, d->V, s.ncl, f16);
     LAS_LAUNCH_OK("pack_dec_w_kernel");
     pack_dec_bias_kernel<<<(4 * d->Hs + 255) / 256, 256, 0, st>>>(lw.b_ih, lw.b_hh, pk.bias[l], d->Hs);
     LAS_LAUNCH_OK("pack_dec_bias_kernel");
   }
-  LAS_TRY(launch_f32_to_bf16(w->w_phi, pk.w_phi, (size_t)d->D * d->Hs, st));
-  LAS_TRY(launch_f32_to_bf16(w->w_cd, pk.w_cd, (size_t)d->V * (d->Hs + d->E), st));
-  LAS_TRY(launch_f32_to_bf16(w->w_psi, pk.w_psi, (size_t)d->D * d->E, st));
+  LAS_TRY(launch_f32_to_bf16(w->w_phi, pk.w_phi, (size_t)d->D * d->Hs, f16, st));
+  LAS_TRY(launch_f32_to_bf16(w->w_cd, pk.w_cd, (size_t)d->V * (d->Hs + d->E), f16, st));
+  LAS_TRY(launch_f32_to_bf16(w->w_psi, pk.w_psi, (size_t)d->D * d->E, f16, st));
   return LAS_OK;
 }
 
@@ -1416,7 +1416,7 @@ int fast_speller_pack(const las_speller_weights* w, const las_speller_dims* d, v
 // for every segment but the last), c and the fed-back token in the carry buffers.
 int fast_speller_decode_segment(const las_decode_io* io, const SpellerF32Inputs& f32, const void* packed_fast, const las_speller_dims* d,
                                 int b0, int Bc, int s_begin, int s_count, bool first_seg, bool last_seg, int decode_mode, int relu,
-                                void* ws_fast, cudaStream_t st) {
+                                void* ws_fast, bool f16, cudaStream_t st) {
   const Shape s = shape_of(d);
   const int n_lstm = d->sl * s.ncl;
   LAS_REQUIRE(last_seg || (s_count % 2 == 0), "decoder segments must have an even number of steps (%d)", s_count);
@@ -1499,7 +1499,7 @@ int fast_speller_decode_segment(const las_decode_io* io, const SpellerF32Inputs&
     p.sync = w.sync;
     p.h_ll = w.h_ll;
     p.tok_ll = w.tok_ll;
-    p.f16 = op_f16();
+    p.f16 = f16;
     // the fed-back word is an index (greedy argmax / index teacher forcing) unless a dense vector is asked for
     p.word_gather = io->gt_dense ? 0 : (io->gt_index ? 1 : (decode_mode != LAS_DECODE_RAW ? 1 : 0));
     p.sample_seed = io->sample_seed;
@@ -1507,7 +1507,7 @@ int fast_speller_decode_segment(const las_decode_io* io, const SpellerF32Inputs&
 
     {
       ProfScope ps("speller.prepare", st);
-      if (first_seg) LAS_TRY(launch_f32_to_bf16(io->enc + so * d->U * d->E, w.enc_bf16, (size_t)Bc * d->U * d->E, st));
+      if (first_seg) LAS_TRY(launch_f32_to_bf16(io->enc + so * d->U * d->E, w.enc_bf16, (size_t)Bc * d->U * d->E, f16, st));
       LAS_CUDA_OK(cudaMemsetAsync(w.flags, 0, w.flag_bytes, st));
       if (first_seg) {
         dec_init_kernel<<<Bc, 256, 0, st>>>(p, io->enc, io->word, io->context, io->h_state);
@@ -1518,8 +1518,8 @@ int fast_speller_decode_segment(const las_decode_io* io, const SpellerF32Inputs&
       // psi(enc) once per utterance (model/las_model.py:279 recomputes it every step): the same tcgen05 GEMM as the
       // listener's input projection, bf16 operands (the enc copy made above), fp32 accumulate + bias + relu
       ProfScope pp("speller.psi", st);
-      LAS_TRY(launch_gemm_bf16_tc(w.enc_bf16, d->E, pk.w_psi, d->E, f32.b_psi, f32.psi + so * d->U * d->D, d->D, Bc * d->U, d->D, d->E, st,
-                                  relu != 0));
+      LAS_TRY(launch_gemm_bf16_tc(w.enc_bf16, d->E, pk.w_psi, d->E, f32.b_psi, f32.psi + so * d->U * d->D, d->D, Bc * d->U, d->D, d->E, f16,
+                                  st, relu != 0));
     }
     ProfScope ps("speller.steps", st);
     const size_t smem_l = rc.smem, smem_a = att_smem(d, p.k_in_smem != 0, p.ctx_ntm > 0 && p.ctx_ntm < d->E / 128, p.att_split == 2);
@@ -1568,7 +1568,7 @@ static int next_segment(int s_begin, int steps, int seg) {
 }
 
 int fast_speller_decode(const las_decode_io* io, const SpellerF32Inputs& f32, const void* packed_fast, const las_speller_dims* d, int steps,
-                        int decode_mode, int relu, void* ws_fast, cudaStream_t st) {
+                        int decode_mode, int relu, void* ws_fast, bool f16, cudaStream_t st) {
   LAS_TRY(supported(d));
   const Shape s = shape_of(d);
   const int n_lstm = d->sl * s.ncl;
@@ -1588,7 +1588,7 @@ int fast_speller_decode(const las_decode_io* io, const SpellerF32Inputs& f32, co
     if (eos) LAS_CUDA_OK(cudaMemsetAsync(stop, 0, sizeof(int32_t) * (2 + 64), st));
     for (int sb = 0; sb < steps;) {
       const int n = next_segment(sb, steps, seg);
-      LAS_TRY(fast_speller_decode_segment(io, f32, packed_fast, d, b0, Bc, sb, n, sb == 0, sb + n == steps, decode_mode, relu, ws_fast, st));
+      LAS_TRY(fast_speller_decode_segment(io, f32, packed_fast, d, b0, Bc, sb, n, sb == 0, sb + n == steps, decode_mode, relu, ws_fast, f16, st));
       if (eos) LAS_TRY(launch_eos_check(io->tokens, d->B, b0, Bc, sb, sb + n, io->eos_token, stop, st));
       sb += n;
     }

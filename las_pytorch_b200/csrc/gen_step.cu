@@ -641,7 +641,7 @@ int gen_step_make_maps(GenStepMaps* m, const __nv_bfloat16* w, const __nv_bfloat
 
 int launch_gen_cell_step(const GenStepMaps& m, int parity, const float* bias, float* c, const float* h_prev, long long h_ld, float* h_out,
                          long long hout_ld, __nv_bfloat16* o1, long long o1_ld, __nv_bfloat16* o2, long long o2_ld, int B, int H, int cell,
-                         int Kxp, int Kp, bool pdl, cudaStream_t st, int trace_slot) {
+                         int Kxp, int Kp, bool pdl, bool f16, cudaStream_t st, int trace_slot) {
   GenStepArgs p;
   memset(&p, 0, sizeof(p));
   p.bias = bias; p.c = c; p.h_prev = h_prev; p.h_ld = h_ld; p.h_out = h_out; p.hout_ld = hout_ld;
@@ -652,7 +652,7 @@ int launch_gen_cell_step(const GenStepMaps& m, int parity, const float* bias, fl
   const size_t region_bytes = p.region ? (size_t)((Kp / 64 + GS_KBS - 1) / GS_KBS) * GS_KBS * p.NB * 128 : 0;
   p.stages = (int)((200 * 1024 - region_bytes) / (GS_KBS * (GS_WBYTES + (p.region ? 0 : p.NB * 128))));  // ring + region <= 200 KB
   if (p.stages > 10) p.stages = 10;
-  p.f16 = op_f16();
+  p.f16 = f16;
   p.early = (o2 == nullptr) ? 1 : 0;
   const int n_stages = (Kp / 64 + GS_KBS - 1) / GS_KBS, first = (Kxp + 64 * GS_KBS - 1) / (64 * GS_KBS);
   p.st_first = first < n_stages ? first : n_stages;

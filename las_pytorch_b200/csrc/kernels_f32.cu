@@ -524,8 +524,8 @@ __global__ void gen_pack_w_kernel(const float* w_ih, const float* w_hh, const fl
   }
 }
 int launch_gen_pack_w(const float* w_ih, const float* w_hh, const float* b_ih, const float* b_hh, __nv_bfloat16* dst, float* bias, int cell,
-                      int H, int Kx, int Kxp, int Kp, cudaStream_t st) {
-  gen_pack_w_kernel<<<592, 256, 0, st>>>(w_ih, w_hh, b_ih, b_hh, dst, bias, cell, H, Kx, Kxp, Kp, op_f16());
+                      int H, int Kx, int Kxp, int Kp, bool f16, cudaStream_t st) {
+  gen_pack_w_kernel<<<592, 256, 0, st>>>(w_ih, w_hh, b_ih, b_hh, dst, bias, cell, H, Kx, Kxp, Kp, f16);
   LAS_LAUNCH_OK("gen_pack_w_kernel");
   return LAS_OK;
 }
@@ -542,9 +542,9 @@ __global__ void gen_build_a_kernel(const float* x, long long x_ld, const float* 
   }
 }
 int launch_gen_build_a(const float* x, long long x_ld, const float* h, long long h_ld, __nv_bfloat16* A, int B, int H, int Kx, int Kxp, int Kp,
-                       cudaStream_t st) {
+                       bool f16, cudaStream_t st) {
   const size_t n = (size_t)B * Kp;
-  gen_build_a_kernel<<<(unsigned)((n + 255) / 256 < 592 ? (n + 255) / 256 : 592), 256, 0, st>>>(x, x_ld, h, h_ld, A, B, H, Kx, Kxp, Kp, op_f16());
+  gen_build_a_kernel<<<(unsigned)((n + 255) / 256 < 592 ? (n + 255) / 256 : 592), 256, 0, st>>>(x, x_ld, h, h_ld, A, B, H, Kx, Kxp, Kp, f16);
   LAS_LAUNCH_OK("gen_build_a_kernel");
   return LAS_OK;
 }

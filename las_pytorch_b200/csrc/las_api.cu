@@ -20,11 +20,8 @@ int fail(int code, const char* fmt, ...) {
 }
 void count_launch(int n) { g_launches += n; }
 
-// tensor-core modes (same kernels; they differ in the 16-bit operand format) and the calling thread's current one
+// tensor-core modes (same kernels; they differ in the 16-bit operand format)
 static inline bool tc_mode(int mode) { return mode == LAS_MODE_BF16 || mode == LAS_MODE_F16; }
-static thread_local int g_op_f16 = 0;
-void set_operand_mode(int mode) { g_op_f16 = (mode == LAS_MODE_F16) ? 1 : 0; }
-int op_f16() { return g_op_f16; }
 
 // ---- profiling registry (thread-local) ------------------------------------------------------------------
 struct ProfRec {
@@ -166,11 +163,12 @@ enum class Path {
 };
 static void* behind(const void* base, size_t offset) { return base ? static_cast<char*>(const_cast<void*>(base)) + offset : nullptr; }
 
-// The one place that decides the listener's path and knows where its blocks sit: the fp32 layouts at the start of the pack and
-// the workspace, the generic ones behind them; or the cluster-resident recurrence's own layouts, which then fill both buffers.
-// Null bases give the sizes alone.  `d` has passed listener_check.
+// The one place that decides the listener's path and its 16-bit operand format, and knows where its blocks sit: the fp32 layouts at
+// the start of the pack and the workspace, the generic ones behind them; or the cluster-resident recurrence's own layouts, which then
+// fill both buffers.  Null bases give the sizes alone.  `d` has passed listener_check.
 struct ListenerLayout {
   Path path;
+  bool f16;            // GEN, FAST: IEEE fp16 operands (LAS_MODE_F16), else bf16
   ListenerPackF32 pk;  // F32, GEN
   ListenerWsF32 ws;
   ListenerGen gp, gw;  // GEN
@@ -179,6 +177,7 @@ struct ListenerLayout {
 static ListenerLayout listener_layout(const las_listener_dims* d, int mode, const void* packed, void* ws) {
   ListenerLayout L = {};
   L.path = !tc_mode(mode) ? Path::F32 : fast_listener_fits(d) ? Path::FAST : Path::GEN;
+  L.f16 = mode == LAS_MODE_F16;
   if (L.path == Path::FAST) {
     L.pack_bytes = fast_listener_packed_bytes(d);
     L.ws_bytes = fast_listener_workspace_bytes(d);
@@ -221,8 +220,8 @@ static int listener_forward_f32(const float* x, const int32_t* x_lengths, const 
       snprintf(nm, sizeof(nm), "listener.L%d.input_gemm", l);
       ProfScope ps(nm, st);
       if (gen) {
-        LAS_TRY(launch_f32_to_bf16(cur, gw.w[0], (size_t)M * K, st));
-        LAS_TRY(launch_gemm_bf16_tc(gw.w[0], K, gp.w[l], K, pk.bias[l], w.P, 2 * GH, M, 2 * GH, K, st));
+        LAS_TRY(launch_f32_to_bf16(cur, gw.w[0], (size_t)M * K, L.f16, st));
+        LAS_TRY(launch_gemm_bf16_tc(gw.w[0], K, gp.w[l], K, pk.bias[l], w.P, 2 * GH, M, 2 * GH, K, L.f16, st));
       } else {
         LAS_TRY(launch_sgemm_nt_bias(cur, K, pk.wcat[l], K, pk.bias[l], w.P, 2 * GH, M, 2 * GH, K, false, st));
       }
@@ -400,12 +399,13 @@ static SpellerWsGen speller_ws_layout_gen(const las_speller_dims* d, void* base)
 // psi GEMM / cell GEMMs read bf16 rows through TMA: 16-byte aligned rows
 static bool gen_ok(const las_speller_dims* d) { return d->no_mlp || d->E % 8 == 0; }
 
-// The one place that decides the speller's path and knows where its blocks sit: the fp32 layouts at the start of the pack and the
-// workspace (in the tensor-core modes too: the persistent decoder reads biases and psi there), then in the tensor-core modes the
-// generic layouts or the persistent decoder's blocks.  The beam pack holds the generic layout also where the persistent decoder covers
-// the model.  Null bases give the sizes alone.  `d` has passed speller_check.
+// The one place that decides the speller's path and its 16-bit operand format, and knows where its blocks sit: the fp32 layouts at
+// the start of the pack and the workspace (in the tensor-core modes too: the persistent decoder reads biases and psi there), then in
+// the tensor-core modes the generic layouts or the persistent decoder's blocks.  The beam pack holds the generic layout also where the
+// persistent decoder covers the model.  Null bases give the sizes alone.  `d` has passed speller_check.
 struct SpellerLayout {
   Path path;
+  bool f16;           // GEN, FAST: IEEE fp16 operands (LAS_MODE_F16), else bf16
   SpellerPackF32 pk;
   SpellerWsF32 ws;
   SpellerPackGen gp;  // GEN
@@ -417,6 +417,7 @@ struct SpellerLayout {
 static SpellerLayout speller_layout(const las_speller_dims* d, int mode, bool beam_pack, const void* packed, void* ws) {
   SpellerLayout L = {};
   L.path = !tc_mode(mode) ? Path::F32 : (!beam_pack && fast_speller_fits(d)) ? Path::FAST : Path::GEN;
+  L.f16 = mode == LAS_MODE_F16;
   L.pk = speller_pack_layout_f32(d, const_cast<void*>(packed));
   L.ws = speller_ws_layout_f32(d, ws);
   L.pack_bytes = L.pk.bytes;
@@ -439,14 +440,14 @@ static SpellerF32Inputs fast_f32_inputs(const SpellerLayout& L) { return {L.pk.b
 // psi = act(enc . W_psi^T + b_psi) of B utterances into `psi` (generic path: a bf16 copy of enc in `enc16` and a tcgen05 GEMM); without
 // the attention MLP the keys are the listener features themselves
 static const float* speller_psi(const las_speller_dims* d, int B, const SpellerPackF32& pk, const SpellerPackGen* gp, const float* enc, float* psi,
-                                __nv_bfloat16* enc16, int relu, cudaStream_t st, int* status) {
+                                __nv_bfloat16* enc16, int relu, bool f16, cudaStream_t st, int* status) {
   *status = LAS_OK;
   if (d->no_mlp) return enc;  // use_mlp_in_attention=False (model/las_model.py:283-285)
   const int U = d->U, E = d->E, D = d->D;
   ProfScope ps("speller.psi", st);
   if (gp) {
-    if ((*status = launch_f32_to_bf16(enc, enc16, (size_t)B * U * E, st)) != LAS_OK) return nullptr;
-    *status = launch_gemm_bf16_tc(enc16, E, gp->w_psi, E, pk.b_psi, psi, D, B * U, D, E, st, relu != 0);
+    if ((*status = launch_f32_to_bf16(enc, enc16, (size_t)B * U * E, f16, st)) != LAS_OK) return nullptr;
+    *status = launch_gemm_bf16_tc(enc16, E, gp->w_psi, E, pk.b_psi, psi, D, B * U, D, E, f16, st, relu != 0);
   } else {
     *status = launch_sgemm_nt_bias(enc, E, pk.w_psi, E, pk.b_psi, psi, D, B * U, D, E, relu != 0, st);
   }
@@ -460,6 +461,7 @@ struct StepPath {
   int rows;
   SpellerPackF32 pk;
   const SpellerPackGen* gp;  // generic tensor-core path, else nullptr (fp32 mode)
+  bool f16;                  // generic path: the 16-bit operand format (SpellerLayout::f16)
   GenGeom gg;
   __nv_bfloat16* a;          // generic path: [rows, Kp_max] GEMM operand
   float* pre;                // [rows, R] gate pre-activations
@@ -499,21 +501,21 @@ static int speller_step(const StepPath& p, int s, const float* hp, float* hn, co
       const int q = s & 1;
       LAS_TRY(launch_gen_cell_step(p.maps[l], q, p.gp->bias[l], p.c + (size_t)l * B * Hs, hp + (size_t)l * B * Hs, Hs, hn + (size_t)l * B * Hs, Hs,
                                    p.abuf[l][q ^ 1] + gg.Kxp[l], gg.Kp[l], l + 1 < sl ? p.abuf[l + 1][q] : nullptr, l + 1 < sl ? gg.Kp[l + 1] : 0, B,
-                                   Hs, d->cell, gg.Kxp[l], gg.Kp[l], true, st, l));
+                                   Hs, d->cell, gg.Kxp[l], gg.Kp[l], true, p.f16, st, l));
       continue;
     }
     if (p.gp) {
       const float* xin_l = (l == 0) ? p.xin : hn + (size_t)(l - 1) * B * Hs;
       const float* hp_l = hp + (size_t)l * B * Hs;
-      LAS_TRY(launch_gen_build_a(xin_l, (l == 0) ? xld : Hs, hp_l, Hs, p.a, B, Hs, gg.Kx[l], gg.Kxp[l], gg.Kp[l], st));
+      LAS_TRY(launch_gen_build_a(xin_l, (l == 0) ? xld : Hs, hp_l, Hs, p.a, B, Hs, gg.Kx[l], gg.Kxp[l], gg.Kp[l], p.f16, st));
       if (B <= 64) {
         // Small batches: the GEMM's 128 x 256 tiles would leave it R/256 CTAs (16 at R = 4096), each streaming 1 MB of weights.  With
         // the operands swapped -- "M" = the R weight rows, "N" = the batch -- R/128 CTAs stream half as much each; the result arrives
         // transposed ([R, B]) and the cell kernel adds the bias.
-        LAS_TRY(launch_gemm_bf16_tc(p.gp->w[l], gg.Kp[l], p.a, gg.Kp[l], p.zero, p.pre, B, gg.R, B, gg.Kp[l], st));
+        LAS_TRY(launch_gemm_bf16_tc(p.gp->w[l], gg.Kp[l], p.a, gg.Kp[l], p.zero, p.pre, B, gg.R, B, gg.Kp[l], p.f16, st));
         LAS_TRY(launch_gen_cell(p.pre, 1, B, p.gp->bias[l], hp_l, Hs, p.c + (size_t)l * B * Hs, hn + (size_t)l * B * Hs, Hs, B, Hs, d->cell, st));
       } else {
-        LAS_TRY(launch_gemm_bf16_tc(p.a, gg.Kp[l], p.gp->w[l], gg.Kp[l], p.gp->bias[l], p.pre, gg.R, B, gg.R, gg.Kp[l], st));
+        LAS_TRY(launch_gemm_bf16_tc(p.a, gg.Kp[l], p.gp->w[l], gg.Kp[l], p.gp->bias[l], p.pre, gg.R, B, gg.R, gg.Kp[l], p.f16, st));
         LAS_TRY(launch_gen_cell(p.pre, gg.R, 1, nullptr, hp_l, Hs, p.c + (size_t)l * B * Hs, hn + (size_t)l * B * Hs, Hs, B, Hs, d->cell, st));
       }
       continue;
@@ -556,7 +558,7 @@ static int speller_decode_f32(const las_decode_io* io, const las_speller_dims* d
   const float* psi = io->psi;
   if (d->no_mlp || !psi) {
     int status;
-    psi = speller_psi(d, B, pk, gen ? &gp : nullptr, io->enc, w.psi, gw.enc, relu, st, &status);
+    psi = speller_psi(d, B, pk, gen ? &gp : nullptr, io->enc, w.psi, gw.enc, relu, L.f16, st, &status);
     LAS_TRY(status);
   }
   if (io->word && io->context) {
@@ -587,12 +589,12 @@ static int speller_decode_f32(const las_decode_io* io, const las_speller_dims* d
       for (int q = 0; q < 2; ++q) abuf[l][q] = gw.a2 + (size_t)(l * 2 + q) * B * gg.Kp_max;
       LAS_TRY(gen_step_make_maps(&maps[l], gp.w[l], abuf[l][0], abuf[l][1], Hs, d->cell == LAS_CELL_RNN ? 1 : 4, B, gg.Kxp[l], gg.Kp[l]));
       LAS_TRY(launch_gen_build_a(l == 0 ? w.xin : w.h[0], l == 0 ? xld : Hs, w.h[0] + (size_t)l * B * Hs, Hs, abuf[l][0], B, Hs, gg.Kx[l],
-                                 gg.Kxp[l], gg.Kp[l], st));
+                                 gg.Kxp[l], gg.Kp[l], L.f16, st));
     }
   }
 
   StepPath path;
-  path.d = d; path.rows = B; path.pk = pk; path.gp = gen ? &gp : nullptr; path.gg = gg;
+  path.d = d; path.rows = B; path.pk = pk; path.gp = gen ? &gp : nullptr; path.f16 = L.f16; path.gg = gg;
   path.a = gw.a; path.pre = gw.pre; path.zero = gw.zero; path.xin = w.xin; path.c = w.c;
   path.fused = fused; path.maps = maps; path.abuf = abuf; path.cluster_att = cluster_att;
   ProfScope ps_steps("speller.steps", st);
@@ -621,7 +623,7 @@ static int speller_decode_f32(const las_decode_io* io, const las_speller_dims* d
     if (fused) {
       t.op_out = abuf[0][(s & 1) ^ 1];
       t.op_ld = gg.Kp[0];
-      t.op_f16 = op_f16();
+      t.op_f16 = L.f16;
     }
     LAS_TRY(speller_step(path, s, hp, hn, t, st));
   }
@@ -715,7 +717,7 @@ static int speller_beam_f32(const las_beam_io* io, const las_speller_dims* d, co
   dk.B = BK;
 
   int status;
-  const float* psi = speller_psi(d, B, pk, gen ? &gp : nullptr, io->enc, w.psi, w.enc16, relu, st, &status);  // once per utterance
+  const float* psi = speller_psi(d, B, pk, gen ? &gp : nullptr, io->enc, w.psi, w.enc16, relu, L.f16, st, &status);  // once per utterance
   LAS_TRY(status);
   LAS_TRY(launch_beam_init(w.xin, V + E, io->enc, w.score, w.fin, B, K, d->U, E, V, st));
   const size_t state_n = (size_t)d->sl * BK * Hs;
@@ -724,7 +726,7 @@ static int speller_beam_f32(const las_beam_io* io, const las_speller_dims* d, co
 
   StepPath path;
   memset(&path, 0, sizeof(path));
-  path.d = &dk; path.rows = BK; path.pk = pk; path.gp = gen ? &gp : nullptr; path.gg = gen_geom(d);
+  path.d = &dk; path.rows = BK; path.pk = pk; path.gp = gen ? &gp : nullptr; path.f16 = L.f16; path.gg = gen_geom(d);
   path.a = w.a; path.pre = w.pre; path.zero = w.zero; path.xin = w.xin; path.c = w.c;
   path.cluster_att = n_heads(d) == 1 && E % 4 == 0 && gen_step_fused(1);  // the greedy step's choice
   BeamStepArgs ba;
@@ -835,7 +837,6 @@ size_t las_listener_packed_bytes(const las_listener_dims* d, int mode) {
 
 int las_listener_pack(const las_lstm_weights* w, const las_listener_dims* d, int mode, void* packed, size_t packed_bytes,
                       void* stream) {
-  set_operand_mode(mode);
   LAS_TRY(listener_check(d));
   LAS_REQUIRE(w && packed, "null weights / packed buffer");
   LAS_REQUIRE(mode == LAS_MODE_FP32 || tc_mode(mode), "unknown mode %d", mode);
@@ -845,7 +846,7 @@ int las_listener_pack(const las_lstm_weights* w, const las_listener_dims* d, int
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   LAS_REQUIRE(L.path != Path::GEN || listener_gen_ok(d),
               "LAS_MODE_BF16 needs 16-byte aligned bf16 rows for TMA: 2F (%d) and 4H (%d) must be multiples of 8; use LAS_MODE_FP32", 2 * d->F, 4 * d->H);
-  if (L.path == Path::FAST) return fast_listener_pack(w, d, packed, st);
+  if (L.path == Path::FAST) return fast_listener_pack(w, d, packed, L.f16, st);
   const ListenerPackF32& pk = L.pk;
   const size_t H = d->H, GH = (size_t)n_gates(d->cell) * H;
   for (int l = 0; l < d->L; ++l) {
@@ -867,7 +868,7 @@ int las_listener_pack(const las_lstm_weights* w, const las_listener_dims* d, int
   if (L.path == Path::GEN) {  // bf16 copies of [W_ih fwd ; W_ih reverse]
     for (int l = 0; l < d->L; ++l) {
       const size_t K = (l == 0) ? 2 * (size_t)d->F : 4 * H;
-      LAS_TRY(launch_f32_to_bf16(pk.wcat[l], L.gp.w[l], 2 * GH * K, st));
+      LAS_TRY(launch_f32_to_bf16(pk.wcat[l], L.gp.w[l], 2 * GH * K, L.f16, st));
     }
   }
   return LAS_OK;
@@ -886,7 +887,6 @@ int las_listener_forward(const float* x, const void* packed, const las_listener_
 int las_listener_forward_masked(const float* x, const int32_t* x_lengths, const void* packed, const las_listener_dims* d,
                                 int mode, float* enc, int32_t* enc_lengths, void* workspace, size_t workspace_bytes,
                                 void* stream) {
-  set_operand_mode(mode);
   LAS_TRY(listener_check(d));
   LAS_REQUIRE(x && packed && enc && workspace, "null pointer argument");
   LAS_REQUIRE(mode == LAS_MODE_FP32 || tc_mode(mode), "unknown mode %d", mode);
@@ -894,7 +894,7 @@ int las_listener_forward_masked(const float* x, const int32_t* x_lengths, const 
   const ListenerLayout L = listener_layout(d, mode, packed, workspace);
   if (workspace_bytes < L.ws_bytes) return fail(LAS_ENOMEM, "workspace too small: %zu < %zu", workspace_bytes, L.ws_bytes);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (L.path == Path::FAST) return fast_listener_forward(x, x_lengths, packed, d, enc, enc_lengths, workspace, st);
+  if (L.path == Path::FAST) return fast_listener_forward(x, x_lengths, packed, d, enc, enc_lengths, workspace, L.f16, st);
   LAS_REQUIRE(L.path != Path::GEN || listener_gen_ok(d), "LAS_MODE_BF16 needs 2F (%d) and 4H (%d) to be multiples of 8; use LAS_MODE_FP32",
               2 * d->F, 4 * d->H);
   return listener_forward_f32(x, x_lengths, d, L, enc, enc_lengths, st);
@@ -908,7 +908,6 @@ size_t las_speller_packed_bytes(const las_speller_dims* d, int mode) {
 
 static int speller_pack(const las_speller_weights* w, const las_speller_dims* d, int mode, void* packed, size_t packed_bytes, void* stream,
                         bool beam_pack) {
-  set_operand_mode(mode);
   LAS_TRY(speller_check(d));
   LAS_REQUIRE(w && packed && w->rnn_host, "null weights / packed buffer");
   LAS_REQUIRE(mode == LAS_MODE_FP32 || tc_mode(mode), "unknown mode %d", mode);
@@ -945,15 +944,15 @@ static int speller_pack(const las_speller_weights* w, const las_speller_dims* d,
     CP(pk.b_dr, w->b_dr, d->E);
   }
 #undef CP
-  if (L.path == Path::FAST) return fast_speller_pack(w, d, L.pk_fast, st);
+  if (L.path == Path::FAST) return fast_speller_pack(w, d, L.pk_fast, L.f16, st);
   if (L.path == Path::GEN) {  // generic tensor-core path: [W_ih | W_hh] per layer as one bf16 matrix, psi weights in bf16
     const SpellerPackGen& gp = L.gp;
     const GenGeom g = gen_geom(d);
     for (int l = 0; l < d->sl; ++l) {
       const las_lstm_weights& s = w->rnn_host[l];
-      LAS_TRY(launch_gen_pack_w(s.w_ih, s.w_hh, s.b_ih, s.b_hh, gp.w[l], gp.bias[l], d->cell, d->Hs, g.Kx[l], g.Kxp[l], g.Kp[l], st));
+      LAS_TRY(launch_gen_pack_w(s.w_ih, s.w_hh, s.b_ih, s.b_hh, gp.w[l], gp.bias[l], d->cell, d->Hs, g.Kx[l], g.Kxp[l], g.Kp[l], L.f16, st));
     }
-    if (!d->no_mlp) LAS_TRY(launch_f32_to_bf16(w->w_psi, gp.w_psi, (size_t)d->D * d->E, st));
+    if (!d->no_mlp) LAS_TRY(launch_f32_to_bf16(w->w_psi, gp.w_psi, (size_t)d->D * d->E, L.f16, st));
   }
   return LAS_OK;
 }
@@ -965,7 +964,6 @@ int las_speller_pack(const las_speller_weights* w, const las_speller_dims* d, in
 
 int las_psi_precompute(const float* enc, const float* w_psi, const float* b_psi, int B, int U, int E, int D, int relu,
                        float* psi, void* stream) {
-  set_operand_mode(LAS_MODE_BF16);
   LAS_REQUIRE(enc && w_psi && b_psi && psi, "null pointer argument");
   LAS_REQUIRE(B > 0 && U > 0 && E > 0 && D > 0, "bad dims (B=%d U=%d E=%d D=%d)", B, U, E, D);
   LAS_TRY(device_ok());
@@ -1002,14 +1000,13 @@ size_t las_speller_workspace_bytes(const las_speller_dims* d, int steps, int mod
 
 int las_speller_decode(const las_decode_io* io, const void* packed, const las_speller_dims* d, int steps, int decode_mode,
                        int mode, int relu, void* workspace, size_t workspace_bytes, void* stream) {
-  set_operand_mode(mode);
   LAS_TRY(speller_check(d));
   LAS_REQUIRE(io && packed && workspace, "null pointer argument");
   LAS_TRY(decode_args_check(io, d, steps, decode_mode, mode, workspace_bytes));
   if (steps == 0) return LAS_OK;
   const SpellerLayout L = speller_layout(d, mode, false, packed, workspace);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (L.path == Path::FAST) return fast_speller_decode(io, fast_f32_inputs(L), L.pk_fast, d, steps, decode_mode, relu, L.ws_fast, st);
+  if (L.path == Path::FAST) return fast_speller_decode(io, fast_f32_inputs(L), L.pk_fast, d, steps, decode_mode, relu, L.ws_fast, L.f16, st);
   LAS_REQUIRE(L.path != Path::GEN || gen_ok(d), "LAS_MODE_BF16 needs E %% 8 == 0 (E=%d); use LAS_MODE_FP32", d->E);
   return speller_decode_f32(io, d, L, steps, decode_mode, relu, st);
 }
@@ -1033,7 +1030,6 @@ size_t las_speller_beam_workspace_bytes(const las_speller_dims* d, int steps, in
 
 int las_speller_beam_search(const las_beam_io* io, const void* packed, const las_speller_dims* d, int steps, int mode, int relu,
                             void* workspace, size_t workspace_bytes, void* stream) {
-  set_operand_mode(mode);
   LAS_REQUIRE(io && packed && workspace, "null pointer argument");
   LAS_TRY(beam_args_check(d, steps, io->beam));
   LAS_REQUIRE(io->enc && io->tokens && io->lengths && io->scores, "io->enc, io->tokens, io->lengths and io->scores are required");
@@ -1049,7 +1045,6 @@ int las_speller_beam_search(const las_beam_io* io, const void* packed, const las
 }
 
 int las_pipeline_step(const las_pipeline_args* a, int mode, void* stream) {
-  set_operand_mode(mode);
   LAS_REQUIRE(a, "null pointer argument");
   const bool dec = a->dec_io != nullptr, lis = a->x != nullptr;
   LAS_REQUIRE(dec || lis, "nothing to do: neither a batch to decode nor a batch to encode");
@@ -1074,7 +1069,7 @@ int las_pipeline_step(const las_pipeline_args* a, int mode, void* stream) {
   if (a->listener_ws_bytes < LL.ws_bytes) return fail(LAS_ENOMEM, "listener workspace too small: %zu < %zu", a->listener_ws_bytes, LL.ws_bytes);
   const SpellerLayout SL = speller_layout(sd, mode, false, a->speller_packed, a->speller_ws);
   return fast_pipeline_step(io, fast_f32_inputs(SL), SL.pk_fast, sd, a->steps, a->decode_mode, a->relu, SL.ws_fast, a->x, a->x_lengths,
-                            a->listener_packed, ld, a->enc, a->enc_lengths, a->listener_ws, static_cast<cudaStream_t>(stream));
+                            a->listener_packed, ld, a->enc, a->enc_lengths, a->listener_ws, SL.f16, static_cast<cudaStream_t>(stream));
 }
 
 int las_pipeline_overlaps(const las_listener_dims* ld, const las_speller_dims* sd, int steps, int mode) {
@@ -1098,10 +1093,9 @@ int las_label_smoothing_terms(const float* logp, const int32_t* labels, int S, i
 }
 
 int las_debug_gemm_bf16(const void* a, const void* w, const float* bias, float* c, int M, int N, int K, void* stream) {
-  set_operand_mode(LAS_MODE_BF16);
   LAS_REQUIRE(a && w && bias && c, "null pointer argument");
   LAS_TRY(device_ok());
-  return launch_gemm_bf16_tc(static_cast<const __nv_bfloat16*>(a), K, static_cast<const __nv_bfloat16*>(w), K, bias, c, N, M, N, K,
+  return launch_gemm_bf16_tc(static_cast<const __nv_bfloat16*>(a), K, static_cast<const __nv_bfloat16*>(w), K, bias, c, N, M, N, K, false,
                              static_cast<cudaStream_t>(stream));
 }
 int las_debug_set_option(int key, int value) {
@@ -1113,7 +1107,6 @@ int las_debug_set_trace(void* dev_buf) {
   return LAS_OK;
 }
 int las_debug_umma_probe(const void* a, const void* b, float* d, int N, int K, int a_sw128, int b_sw128, int variant, void* stream) {
-  set_operand_mode(LAS_MODE_BF16);
   LAS_REQUIRE(a && b && d, "null pointer argument");
   LAS_TRY(device_ok());
   return launch_umma_probe(a, b, d, N, K, a_sw128, b_sw128, variant, static_cast<cudaStream_t>(stream));

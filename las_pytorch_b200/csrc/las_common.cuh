@@ -64,10 +64,8 @@ int sm_count();  // cached per device
 
 // 16-bit GEMM operand format of the tensor-core modes: bf16 (LAS_MODE_BF16) or IEEE fp16 (LAS_MODE_F16: same kernels, same speed, 10
 // mantissa bits instead of 7; the model's operands -- weights, activations in [-1,1], filterbank features -- sit far inside fp16's
-// range).  The C-ABI entry points record the mode of the call on the calling thread; the launchers read it when they fill kernel
-// parameters.  Operand buffers are typed __nv_bfloat16 throughout (16-bit containers); `f16` says how the bits are produced / read.
-void set_operand_mode(int mode);
-int op_f16();
+// range).  las_api.cu's layout resolvers set `f16` from the mode of the call, and every launcher of 16-bit operands takes it as an
+// argument.  Operand buffers are typed __nv_bfloat16 throughout (16-bit containers); `f16` says how the bits are produced / read.
 #ifdef __CUDACC__
 __device__ __forceinline__ __nv_bfloat16 op_from_f32(float x, int f16) {
   if (f16) {

@@ -91,9 +91,9 @@ int launch_nll_sums(const float* logp, const int32_t* labels, int S, int S_lab, 
 
 // generic tensor-core decoder step (LAS_MODE_BF16 beyond the persistent decoder's shapes; kernels_f32.cu)
 int launch_gen_pack_w(const float* w_ih, const float* w_hh, const float* b_ih, const float* b_hh, __nv_bfloat16* dst, float* bias, int cell,
-                      int H, int Kx, int Kxp, int Kp, cudaStream_t st);
+                      int H, int Kx, int Kxp, int Kp, bool f16, cudaStream_t st);
 int launch_gen_build_a(const float* x, long long x_ld, const float* h, long long h_ld, __nv_bfloat16* A, int B, int H, int Kx, int Kxp, int Kp,
-                       cudaStream_t st);
+                       bool f16, cudaStream_t st);
 int launch_gen_cell(const float* pre, long long ldb, long long ldr, const float* bias, const float* h_prev, long long h_ld, float* c, float* h_out,
                     long long hout_ld, int B, int H, int cell, cudaStream_t st);
 
