@@ -306,10 +306,12 @@ int las_debug_gemm_bf16(const void* a_bf16, const void* w_bf16, const float* bia
 int las_debug_umma_probe(const void* a_bf16, const void* b_bf16, float* d, int N, int K, int a_sw128, int b_sw128, int variant,
                          void* stream);
 
-/* Device buffer of 64*8 int64 that the layer-0 recurrence kernel fills with clock64 stamps (NULL disables). */
+/* Device buffer that the layer-0 recurrence, the generic decoder step and the persistent decoder fill with clock64 / globaltimer
+ * stamps (NULL disables).  Its size in int64: 512 + 5*32*8 + 8 * (SM count) wherever a persistent decoder can run, 64*8 otherwise
+ * (layout: TRACE_* in las_pytorch_b200/csrc/las_common.cuh). */
 int las_debug_set_trace(void* dev_buf);
 /* Process-wide switches for tests and measurements.  Returns LAS_EINVAL (las_last_error names the key) for a key not listed
- * here or a value outside the key's set.
+ * here or a value outside the key's set.  The table in las_debug_set_option (las_pytorch_b200/csrc/las_api.cu) is the one implementation of this list.
  *   key 2:  decoder context through tensor memory (1, default: all feature tiles when they fit, otherwise as many as fit + the rest
  *           on the CUDA cores) or on the CUDA cores only (0);
  *   key 6:  listener input-projection GEMM concurrent with the recurrence (1, default) or in front of it (0);

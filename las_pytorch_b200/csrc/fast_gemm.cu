@@ -44,8 +44,6 @@ struct __align__(1024) GemmSmem {
 //   (m = i / n_tiles,               n = i % n_tiles)   for the forward direction's column tiles  (n <  nfwd)
 //   (m = m_tiles - 1 - i / n_tiles, n = i % n_tiles)   for the backward direction's             (n >= nfwd)
 // i.e. the recurrence's consumption order: early time steps for the forward LSTM, late ones for the backward LSTM.
-int g_gemm_direct_store = 0;  // las_debug_set_option(8, 1): row-per-thread global stores instead of the TMA-store epilogue (A/B, tests)
-
 struct GemmSched {
   int mode, Bp, nfwd;
   int f16;          // operand format of A and W: 0 = bf16, 1 = IEEE fp16
@@ -292,16 +290,10 @@ int make_tmap_f32_store(CUtensorMap* tm, const void* base, long long rows, long 
 // TMA can address the output when the base and the row pitch are 16-byte aligned; otherwise the kernel stores rows directly.
 // Narrow outputs (psi: N = 64, two blocks per tile) are a little faster with direct stores (14.3 vs 16.4 us), so they keep them.
 bool tma_store_ok(const float* C, long long ldc, int N, const uint32_t* flags) {
-  return (reinterpret_cast<uintptr_t>(C) & 15) == 0 && (ldc * 4) % 16 == 0 && N >= 128 && !flags && !g_gemm_direct_store;
+  return (reinterpret_cast<uintptr_t>(C) & 15) == 0 && (ldc * 4) % 16 == 0 && N >= 128 && !flags && !debug_options().gemm_direct_store;
 }
 
 }  // namespace
-
-bool fast_set_option_gemm(int key, int value) {
-  if (key != 8 || (value != 0 && value != 1)) return false;
-  g_gemm_direct_store = value;
-  return true;
-}
 
 int make_tmap_bf16_box(CUtensorMap* tm, const void* base, long long rows, long long cols, long long ld, int box_rows) {
   return make_tmap_bf16(tm, base, rows, cols, ld, box_rows);

@@ -459,9 +459,6 @@ __global__ void pack_whh_kernel(const float* w_fwd, const float* w_rev, uint8_t*
   }
 }
 
-long long* g_rec_trace = nullptr;  // set through las_debug_set_trace (test hook)
-int g_rec_overlap = 1;             // las_debug_set_option(6, v): run each layer's input-projection GEMM concurrently with its recurrence
-
 // Side stream on which a layer's input-projection GEMM runs while the recurrence consumes its tiles on the caller's
 // stream.  One per host thread and device, created on first use and kept (entry points stay re-entrant: nothing here is
 // shared between threads).
@@ -489,7 +486,6 @@ int side_stream(SideStream** out) {
   *out = &g_side;
   return LAS_OK;
 }
-int g_rec_force_bc = 0;            // las_debug_set_option(9, v): batch chunk per recurrence cluster (0 = pick_bc)
 
 struct Geo {
   int Hp, CS;
@@ -591,20 +587,6 @@ int launch_rec(const RecParams& p, cudaStream_t st, bool exclusive_sm) {
 
 }  // namespace
 
-
-
-void fast_set_trace(long long* p) { g_rec_trace = p; }
-long long* fast_get_trace() { return g_rec_trace; }
-bool fast_set_option_speller(int key, int value);
-bool fast_set_option_gemm(int key, int value);  // fast_gemm.cu: 8 = direct-store epilogue
-bool fast_set_option(int key, int value) {
-  if (key == 6 && (value == 0 || value == 1)) g_rec_overlap = value;
-  else if (key == 9 && (value == 0 || value == 16 || value == 32 || value == 64)) g_rec_force_bc = value;
-  else return fast_set_option_speller(key, value) || fast_set_option_gemm(key, value) || fast_set_option_pipeline(key, value) ||
-              fast_set_option_gen(key, value);
-  return true;
-}
-
 // Does the cluster-resident recurrence cover this model?  (Otherwise las_api.cu runs the generic path: tensor-core input projection,
 // fp32 recurrent kernel.)
 bool fast_listener_fits(const las_listener_dims* d) {
@@ -661,7 +643,7 @@ static RecParams rec_params(const las_listener_dims* d, const Geo& g, const List
   rp.out_bf16 = last ? nullptr : w.act[l & 1];
   rp.lengths = len_l;
   rp.B = d->B; rp.Tl = q.Tl; rp.H = d->H; rp.Hp = g.Hp; rp.CS = g.CS;
-  rp.trace = (l == 0) ? g_rec_trace : nullptr;
+  rp.trace = (l == 0) ? debug_options().trace_at(TRACE_REC) : nullptr;
   rp.nchunks = (d->B + bc - 1) / bc;
   rp.resident = nullptr;
   rp.f16 = f16;
@@ -755,7 +737,7 @@ int fast_listener_forward(const float* x, const int32_t* x_lengths, const void* 
       LAS_TRY(launch_pyramid_lengths(l == 0 ? x_lengths : w.len + (size_t)(l - 1) * B, w.len + (size_t)l * B, B, q.Tl, st));
       len_l = w.len + (size_t)l * B;
     }
-    const int bc = g_rec_force_bc ? g_rec_force_bc : pick_bc(B, g.CS);
+    const int bc = debug_options().rec_force_bc ? debug_options().rec_force_bc : pick_bc(B, g.CS);
     RecParams rp = rec_params(d, g, pk, w, l, enc, len_l, bc, f16);
     // The GEMM emits its tiles in the recurrence's consumption order and flags each one, so it can run next to the recurrence
     // (which occupies 2 * nchunks * CS SMs) on the remaining SMs instead of in front of it.  Needs the two directions' columns
@@ -770,7 +752,7 @@ int fast_listener_forward(const float* x, const int32_t* x_lengths, const void* 
     }
     const int rec_ctas = 2 * rp.nchunks * g.CS;
     const int gemm_ctas = sm_count() - rec_ctas - 4;
-    const bool overlap = g_rec_overlap && ((q.NP / 2) % 256 == 0) && gemm_ctas >= 32;
+    const bool overlap = debug_options().rec_overlap && ((q.NP / 2) % 256 == 0) && gemm_ctas >= 32;
     SideStream* side = nullptr;
     if (overlap) LAS_TRY(side_stream(&side));
     if (overlap) rp.gemm_flags = w.flags;

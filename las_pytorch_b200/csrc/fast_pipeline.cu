@@ -61,15 +61,7 @@ int pipe_events(PipeEvents** out) {
   return LAS_OK;
 }
 
-int g_pipe_split[8] = {0};  // las_debug_set_option(20 + l, steps): decoder steps of segment l (0 = proportional to the layer's time steps)
-
 }  // namespace
-
-bool fast_set_option_pipeline(int key, int value) {
-  if (key < 20 || key >= 28 || value < 0) return false;
-  g_pipe_split[key - 20] = value;
-  return true;
-}
 
 // Can the listener of `ld` run next to the decoder of `sd`?  Returns the recurrence's batch chunk (16 / 32 / 64) or 0.
 int fast_pipeline_bc(const las_listener_dims* ld, const las_speller_dims* sd, int steps) {
@@ -101,10 +93,11 @@ int fast_pipeline_step(const las_decode_io* io, const SpellerF32Inputs& spl_f32,
   int seg[8], used = 0;
   {
     auto weight = [&](int l) { return (double)(ld->T >> (l + 1)) * (l == 0 ? 0.88 : 1.0); };
+    const int* split = debug_options().pipe_split;
     double tot = 0;
     for (int l = 0; l < L; ++l) tot += weight(l);
     for (int l = 0; l < L; ++l) {
-      int n = g_pipe_split[l] > 0 ? g_pipe_split[l] : (int)(steps * weight(l) / tot);
+      int n = split[l] > 0 ? split[l] : (int)(steps * weight(l) / tot);
       n &= ~1;
       if (n < 2) n = 2;
       if (l == L - 1 || used + n > steps - 2 * (L - 1 - l)) n = (l == L - 1) ? steps - used : ((steps - used - 2 * (L - 1 - l)) & ~1);

@@ -106,7 +106,7 @@ struct DecParams {
                     // 2 of 4) = hybrid, the remaining features are reduced on the CUDA cores from the L2-resident bf16 copy
   int groups, gsz;  // utterance groups pipelined through the LSTM CTAs (1, or 2 groups of gsz = 32 rows) -- see lstm_role_ts
   int nstages, stage_bytes;  // activation slots: [64 batch rows x 64 bf16], 128-byte swizzled; last slot = word atom
-  long long* trace;  // nullable test hook: [3 roles][32 steps][8] globaltimer stamps (layer-0 CTA 0, top-layer CTA 0, attention CTA 0)
+  long long* trace;  // nullable test hook (TRACE_DEC): [5 roles][32 steps][8] globaltimer stamps (layer-0 CTA 0, top-layer CTA 0, attention CTA 0, ...)
 };
 
 __device__ __forceinline__ long long gtimer() {
@@ -114,8 +114,8 @@ __device__ __forceinline__ long long gtimer() {
   asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
   return t;
 }
-// per-CTA stamps of step 8 (spread across CTAs): behind the 5 x 32 x 8 role trace, [gridDim][8]
-#define DEC_TRACE_ALL(slot) do { if (p.trace && s == 8) p.trace[5 * 32 * 8 + blockIdx.x * 8 + (slot)] = gtimer(); } while (0)
+// per-CTA stamps of step 8 (spread across CTAs): behind the role trace, [gridDim][8] (las_common.cuh TRACE_DEC_CTA)
+#define DEC_TRACE_ALL(slot) do { if (p.trace && s == 8) p.trace[TRACE_DEC_CTA - TRACE_DEC + blockIdx.x * 8 + (slot)] = gtimer(); } while (0)
 #define DEC_TRACE(role, slot) do { if (p.trace && s < 32) p.trace[((role) * 32 + s) * 8 + (slot)] = gtimer(); } while (0)
 
 __device__ __forceinline__ float tanh_fast(float x) {
@@ -1239,8 +1239,6 @@ __global__ void dec_init_kernel(DecParams p, const float* enc_f32, const float* 
       p.hbuf[l][0][(size_t)b * p.Hs + i] = op_from_f32(h_in ? h_in[((size_t)l * p.Bfull + gb) * p.Hs + i] : 0.f, p.f16);
 }
 
-int g_dec_ctx_tmem = 1;   // las_debug_set_option(2, 0): the context on the CUDA cores only
-
 struct Shape {
   int ncl, natoms[MAX_SL];
   size_t w_bytes[MAX_SL];
@@ -1282,8 +1280,6 @@ bool att_wreg(const las_speller_dims* d) { return d->D <= DEC_THREADS / 8 && d->
 size_t att_smem(const las_speller_dims* d, bool k_in, bool hybrid = false, bool split = false) {
   return att_layout(d->Hs, d->E, split ? att_split_half(d->U) : d->U, d->D, d->V, k_in, att_wreg(d), hybrid, split).total + 64;
 }
-int g_dec_groups = 1;     // las_debug_set_option(19, v): 1 = two utterance groups pipelined through the LSTM CTAs (default), 0 = lockstep
-int g_dec_att_split = 1;  // las_debug_set_option(11, v): 1 = split long encoders over a 2-CTA cluster (default), 0 = never
 // Tensor-memory geometry of the context path for `U` encoder steps per CTA: feature tiles of enc^T that fit the 512 columns
 int ctx_tiles_fit(int U, int E) {
   if (E % 128 != 0) return 0;
@@ -1297,7 +1293,7 @@ int ctx_tiles_fit(int U, int E) {
 // a cluster of two CTAs attends each utterance (flash-decoding style partial softmax, combined through DSMEM) -- provided the LSTM
 // CTAs pair up (even count) and the chip has room for two attention CTAs per utterance.
 bool att_split_ok(const las_speller_dims* d) {
-  if (!g_dec_att_split || !g_dec_ctx_tmem || d->E % 128 != 0) return false;
+  if (!debug_options().att_split || !debug_options().ctx_tmem || d->E % 128 != 0) return false;
   const int NT = d->E / 128;
   if (ctx_tiles_fit(d->U, d->E) == NT) return false;  // one CTA is enough
   const int n_lstm = d->sl * (d->Hs / DEC_UNITS);
@@ -1382,12 +1378,6 @@ bool fast_speller_fits(const las_speller_dims* d) {
   const bool ok = supported(d) == LAS_OK && d->sl * (d->Hs / DEC_UNITS) + 1 <= sm_count();
   return ok;
 }
-bool fast_set_option_speller(int key, int value) {
-  int* opt = key == 2 ? &g_dec_ctx_tmem : key == 11 ? &g_dec_att_split : key == 19 ? &g_dec_groups : nullptr;
-  if (!opt || (value != 0 && value != 1)) return false;
-  *opt = value;
-  return true;
-}
 
 size_t fast_speller_packed_bytes(const las_speller_dims* d) { return pack_layout(d, nullptr).bytes; }
 size_t fast_speller_workspace_bytes(const las_speller_dims* d) { return ws_layout(d, nullptr).bytes; }
@@ -1443,7 +1433,7 @@ int fast_speller_decode_segment(const las_decode_io* io, const SpellerF32Inputs&
       const int NT = d->E / 128;
       // all feature tiles of enc[b]^T in tensor memory when they fit its 512 columns (U <= 224 at E = 512); otherwise as many
       // as fit, the rest on the CUDA cores (hybrid; needs the score operand in its own shared-memory region)
-      int ntm = g_dec_ctx_tmem ? ctx_tiles_fit(d->U, d->E) : 0;
+      int ntm = debug_options().ctx_tmem ? ctx_tiles_fit(d->U, d->E) : 0;
       if (ntm > 0 && ntm < NT && (512 % ((d->E - ntm * 128) / 8)) != 0) ntm = 0;
       p.ctx_ntm = ntm;
       p.ctx_tmem = ntm > 0;
@@ -1453,7 +1443,7 @@ int fast_speller_decode_segment(const las_decode_io* io, const SpellerF32Inputs&
     }
     RingCfg rc = ring_cfg(d);
     // two utterance groups of 32 pipelined through the LSTM CTAs when the launch has more than 32 utterances
-    p.groups = (Bc > 32 && g_dec_groups != 0) ? 2 : 1;
+    p.groups = (Bc > 32 && debug_options().dec_groups != 0) ? 2 : 1;
     p.gsz = p.groups == 2 ? 32 : 64;
     rc.box_rows = p.gsz;
     rc.stage_bytes = rc.box_rows * 128;
@@ -1503,7 +1493,7 @@ int fast_speller_decode_segment(const las_decode_io* io, const SpellerF32Inputs&
     // the fed-back word is an index (greedy argmax / index teacher forcing) unless a dense vector is asked for
     p.word_gather = io->gt_dense ? 0 : (io->gt_index ? 1 : (decode_mode != LAS_DECODE_RAW ? 1 : 0));
     p.sample_seed = io->sample_seed;
-    p.trace = (fast_get_trace() && first_seg) ? fast_get_trace() + 512 : nullptr;  // needs 5 roles x 32 steps x 8 stamps behind the recurrence trace
+    p.trace = first_seg ? debug_options().trace_at(TRACE_DEC) : nullptr;
 
     {
       ProfScope ps("speller.prepare", st);

@@ -595,18 +595,7 @@ __global__ void __launch_bounds__(AC_THREADS, 1) attend_cluster_kernel(const Att
   if (tr) { tr[9] = clock64(); tr[11] = gtime(); }
 }
 
-int g_gen_fused = 1;    // las_debug_set_option(12, 0): the unfused generic step (GEMM + cell + operand kernels, one-CTA attention)
-int g_gen_cluster = 0;  // las_debug_set_option(13, C): force the attention cluster size (0 = by batch)
-
 }  // namespace
-
-bool fast_set_option_gen(int key, int value) {
-  if (key == 12 && (value == 0 || value == 1)) g_gen_fused = value;
-  else if (key == 13 && (value == 0 || value == 1 || value == 2 || value == 4 || value == 8)) g_gen_cluster = value;
-  else return false;
-  return true;
-}
-bool gen_step_fused(int B) { return g_gen_fused != 0 && B <= 256; }
 
 // Activations in their own shared-memory region (one copy per part and launch) while all K blocks of them fit 72 KB
 static bool gen_region(int nb, int Kp) { return (size_t)((Kp / 64 + GS_KBS - 1) / GS_KBS) * GS_KBS * nb * 128 <= 72 * 1024; }
@@ -656,7 +645,7 @@ int launch_gen_cell_step(const GenStepMaps& m, int parity, const float* bias, fl
   p.early = (o2 == nullptr) ? 1 : 0;
   const int n_stages = (Kp / 64 + GS_KBS - 1) / GS_KBS, first = (Kxp + 64 * GS_KBS - 1) / (64 * GS_KBS);
   p.st_first = first < n_stages ? first : n_stages;
-  p.trace = fast_get_trace() ? fast_get_trace() + 16 * (1 + trace_slot) : nullptr;
+  p.trace = debug_options().trace_at(TRACE_GEN + TRACE_GEN_SLOT * (1 + trace_slot));
   const int cells = GS_ROWS / p.G;
   const size_t smem = 1024 + (size_t)p.stages * GS_KBS * (GS_WBYTES + (p.region ? 0 : p.NB * 128)) + region_bytes + 8 * (2 * p.stages + 3) + 16;
   LAS_CUDA_OK(cudaFuncSetAttribute(gen_cell_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -679,7 +668,7 @@ int launch_gen_cell_step(const GenStepMaps& m, int parity, const float* bias, fl
 int launch_attend_cluster(const AttendArgs& a, bool pdl, cudaStream_t st) {
   LAS_REQUIRE(a.heads == 1 && a.E % 4 == 0, "attend_cluster_kernel is the single-head form with E %% 4 == 0 (heads=%d E=%d)", a.heads, a.E);
   if ((reinterpret_cast<uintptr_t>(a.enc) & 15) != 0 || a.E > 4 * AC_THREADS) return launch_attend_f32(a, st);  // (vector loads of the encoder rows; four features per thread)
-  int C = g_gen_cluster;
+  int C = debug_options().gen_cluster;
   if (C != 1 && C != 2 && C != 4 && C != 8) {
     // The step's kernels overlap pairwise (programmatic dependent launch) and each wants an SM to itself: keep this one to half the
     // chip so that the next step's first cell kernel (<= 64 CTAs) starts on the other half while it runs.
@@ -717,7 +706,7 @@ int launch_attend_cluster(const AttendArgs& a, bool pdl, cudaStream_t st) {
   cfg.attrs = at;
   cfg.numAttrs = n;
   AttendArgs at2 = a;
-  at2.trace = fast_get_trace();
+  at2.trace = debug_options().trace_at(TRACE_GEN);
   LAS_CUDA_OK(cudaLaunchKernelEx(&cfg, shared ? attend_cluster_kernel<true> : attend_cluster_kernel<false>, at2, C));
   LAS_LAUNCH_OK("attend_cluster_kernel");
   return LAS_OK;

@@ -20,6 +20,9 @@ int fail(int code, const char* fmt, ...) {
 }
 void count_launch(int n) { g_launches += n; }
 
+static DebugOptions g_debug;  // written by las_debug_set_option / las_debug_set_trace only
+const DebugOptions& debug_options() { return g_debug; }
+
 // tensor-core modes (same kernels; they differ in the 16-bit operand format)
 static inline bool tc_mode(int mode) { return mode == LAS_MODE_BF16 || mode == LAS_MODE_F16; }
 
@@ -539,6 +542,9 @@ static int speller_step(const StepPath& p, int s, const float* hp, float* hn, co
   if (p.cluster_att) return launch_attend_cluster(t, p.gp != nullptr, st);
   return launch_attend_f32(t, st);
 }
+// The attention kernel of greedy decoding and of beam search: the cluster kernel is plain fp32 arithmetic, so the fp32 mode uses it
+// as well; multi-head attention keeps the one-CTA kernel.
+static bool cluster_attention(const las_speller_dims* d) { return n_heads(d) == 1 && d->E % 4 == 0 && debug_options().gen_fused; }
 
 static int speller_decode_f32(const las_decode_io* io, const las_speller_dims* d, const SpellerLayout& L, int steps, int decode_mode, int relu,
                               cudaStream_t st) {
@@ -578,9 +584,7 @@ static int speller_decode_f32(const las_decode_io* io, const las_speller_dims* d
 
   // Fused generic step (gen_step.cu): per layer the 16-bit operand rows [x | h_prev] of even / odd steps live in abuf[l][parity]; the
   // kernels that produce x and h write them there directly.  Step 0's rows are built from the initial state here.
-  const bool fused = gen && gen_step_fused(B);
-  // (the cluster kernel is plain fp32 arithmetic: the fp32 mode uses it as well; multi-head attention keeps the one-CTA kernel)
-  const bool cluster_att = NH == 1 && E % 4 == 0 && gen_step_fused(1);
+  const bool fused = gen && debug_options().gen_fused && B <= 256;
   GenStepMaps maps[8];
   __nv_bfloat16* abuf[8][2];
   if (fused) {
@@ -596,7 +600,7 @@ static int speller_decode_f32(const las_decode_io* io, const las_speller_dims* d
   StepPath path;
   path.d = d; path.rows = B; path.pk = pk; path.gp = gen ? &gp : nullptr; path.f16 = L.f16; path.gg = gg;
   path.a = gw.a; path.pre = gw.pre; path.zero = gw.zero; path.xin = w.xin; path.c = w.c;
-  path.fused = fused; path.maps = maps; path.abuf = abuf; path.cluster_att = cluster_att;
+  path.fused = fused; path.maps = maps; path.abuf = abuf; path.cluster_att = cluster_attention(d);
   ProfScope ps_steps("speller.steps", st);
   for (int s = 0; s < steps; ++s) {
     float* hp = w.h[s & 1];
@@ -728,7 +732,7 @@ static int speller_beam_f32(const las_beam_io* io, const las_speller_dims* d, co
   memset(&path, 0, sizeof(path));
   path.d = &dk; path.rows = BK; path.pk = pk; path.gp = gen ? &gp : nullptr; path.f16 = L.f16; path.gg = gen_geom(d);
   path.a = w.a; path.pre = w.pre; path.zero = w.zero; path.xin = w.xin; path.c = w.c;
-  path.cluster_att = n_heads(d) == 1 && E % 4 == 0 && gen_step_fused(1);  // the greedy step's choice
+  path.cluster_att = cluster_attention(d);
   BeamStepArgs ba;
   memset(&ba, 0, sizeof(ba));
   ba.logp = w.logp; ba.score = w.score; ba.fin = w.fin;
@@ -1099,11 +1103,33 @@ int las_debug_gemm_bf16(const void* a, const void* w, const float* bias, float* 
                              static_cast<cudaStream_t>(stream));
 }
 int las_debug_set_option(int key, int value) {
-  LAS_REQUIRE(fast_set_option(key, value), "las_debug_set_option: key %d is not an option, or %d is not one of its values", key, value);
+  // The one implementation of the key list in include/las_b200.h: keys [key, key + n) set field[0, n) to a value `ok` accepts.
+  struct Key { int key, n; int* field; bool (*ok)(int); };
+  auto on_off = [](int v) { return v == 0 || v == 1; };
+  auto chunk = [](int v) { return v == 0 || v == 16 || v == 32 || v == 64; };
+  auto cluster = [](int v) { return v == 0 || v == 1 || v == 2 || v == 4 || v == 8; };
+  auto steps = [](int v) { return v >= 0; };
+  DebugOptions& o = g_debug;
+  const Key keys[] = {
+      {2, 1, &o.ctx_tmem, on_off},
+      {6, 1, &o.rec_overlap, on_off},
+      {8, 1, &o.gemm_direct_store, on_off},
+      {9, 1, &o.rec_force_bc, chunk},
+      {11, 1, &o.att_split, on_off},
+      {12, 1, &o.gen_fused, on_off},
+      {13, 1, &o.gen_cluster, cluster},
+      {19, 1, &o.dec_groups, on_off},
+      {20, 8, o.pipe_split, steps},
+  };
+  const Key* k = nullptr;
+  for (const Key& c : keys)
+    if (key >= c.key && key < c.key + c.n) k = &c;
+  LAS_REQUIRE(k && k->ok(value), "las_debug_set_option: key %d is not an option, or %d is not one of its values", key, value);
+  k->field[key - k->key] = value;
   return LAS_OK;
 }
 int las_debug_set_trace(void* dev_buf) {
-  fast_set_trace(static_cast<long long*>(dev_buf));
+  g_debug.trace = static_cast<long long*>(dev_buf);
   return LAS_OK;
 }
 int las_debug_umma_probe(const void* a, const void* b, float* d, int N, int K, int a_sw128, int b_sw128, int variant, void* stream) {

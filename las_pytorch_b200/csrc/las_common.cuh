@@ -62,6 +62,33 @@ struct Carver {
 
 int sm_count();  // cached per device
 
+// ---- las_debug_set_option switches and the las_debug_set_trace buffer -----------------------------------
+// Process-wide, written only by those two entry points (las_api.cu: its table maps each key of include/las_b200.h to a field
+// here and to the values it takes), read by the launchers at their decision points through debug_options().  Defaults are the
+// paths every call takes unless a test or a measurement asks for another.
+struct DebugOptions {
+  int ctx_tmem = 1;           // persistent decoder: context through tensor memory (0: CUDA cores only)
+  int rec_overlap = 1;        // listener: input-projection GEMM concurrent with the recurrence (0: in front of it)
+  int gemm_direct_store = 0;  // tcgen05 GEMM: row-per-thread global stores instead of the TMA-store epilogue
+  int rec_force_bc = 0;       // listener: batch chunk per recurrence cluster (0: pick_bc)
+  int att_split = 1;          // persistent decoder: long encoders split over a 2-CTA cluster (0: never)
+  int gen_fused = 1;          // fused generic decoder step and the cluster attention kernel (0: unfused step, one-CTA attention)
+  int gen_cluster = 0;        // CTAs per utterance of that attention cluster (0: by batch)
+  int dec_groups = 1;         // persistent decoder: two utterance groups through the LSTM CTAs (0: lockstep)
+  int pipe_split[8] = {};     // serving pipeline: decoder steps of segment l (0: proportional to the layer's time steps)
+  long long* trace = nullptr;  // device buffer of clock64 / globaltimer stamps, laid out as below (nullable)
+  long long* trace_at(int offset) const { return trace ? trace + offset : nullptr; }
+};
+const DebugOptions& debug_options();
+
+// Layout of the trace buffer, in int64 elements.  A caller provides TRACE_DEC_CTA + 8 * sm_count() of them wherever a persistent
+// decoder can run (include/las_b200.h).
+constexpr int TRACE_REC = 0;        // [64 steps][8]: the layer-0 recurrence, CTA 0 (fast_listener.cu)
+constexpr int TRACE_GEN = 0;        // generic decoder step, CTA 0 of each kernel (gen_step.cu): the attention at TRACE_GEN, layer l's
+constexpr int TRACE_GEN_SLOT = 16;  // cell step at TRACE_GEN + TRACE_GEN_SLOT * (1 + l); shares the front with the recurrence's block
+constexpr int TRACE_DEC = 512;      // [5 roles][32 steps][8]: the persistent decoder's role CTAs (fast_speller.cu)
+constexpr int TRACE_DEC_CTA = TRACE_DEC + 5 * 32 * 8;  // [CTA][8]: every CTA of the persistent decoder at step 8
+
 // 16-bit GEMM operand format of the tensor-core modes: bf16 (LAS_MODE_BF16) or IEEE fp16 (LAS_MODE_F16: same kernels, same speed, 10
 // mantissa bits instead of 7; the model's operands -- weights, activations in [-1,1], filterbank features -- sit far inside fp16's
 // range).  las_api.cu's layout resolvers set `f16` from the mode of the call, and every launcher of 16-bit operands takes it as an

@@ -40,13 +40,6 @@ int fast_pipeline_bc(const las_listener_dims* ld, const las_speller_dims* sd, in
 int fast_pipeline_step(const las_decode_io* io, const SpellerF32Inputs& spl_f32, const void* spl_packed_fast, const las_speller_dims* sd,
                        int steps, int decode_mode, int relu, void* spl_ws_fast, const float* x, const int32_t* x_lengths, const void* lis_packed,
                        const las_listener_dims* ld, float* enc, int32_t* enc_lengths, void* lis_ws, bool f16, cudaStream_t st);
-bool fast_set_option_pipeline(int key, int value);
-
-// las_debug_set_option: each module's setter applies a key it owns and returns true, or returns false for another key or a value
-// outside the key's documented set (include/las_b200.h)
-bool fast_set_option(int key, int value);
-void fast_set_trace(long long* dev_buf);
-long long* fast_get_trace();  // test hook: recurrence kernel timeline (64 steps x 8 clock64 stamps)
 
 // fast_gemm.cu
 int launch_gemm_bf16_tc(const __nv_bfloat16* A, long long lda, const __nv_bfloat16* W, long long ldw, const float* bias, float* C,
@@ -70,12 +63,10 @@ struct GenStepMaps {
   CUtensorMap w, a[2];  // packed weights [R, Kp]; the layer's operand rows [B, Kp] of even / odd steps (per-stage box)
   CUtensorMap a_ind[2], a_dep[2];  // the same rows, one box for all independent / all dependent K blocks
 };
-bool gen_step_fused(int B);
 int gen_step_make_maps(GenStepMaps* m, const __nv_bfloat16* w, const __nv_bfloat16* act0, const __nv_bfloat16* act1, int H, int G, int B, int Kxp,
                        int Kp);
 int launch_gen_cell_step(const GenStepMaps& m, int parity, const float* bias, float* c, const float* h_prev, long long h_ld, float* h_out,
                          long long hout_ld, __nv_bfloat16* o1, long long o1_ld, __nv_bfloat16* o2, long long o2_ld, int B, int H, int cell,
                          int Kxp, int Kp, bool pdl, bool f16, cudaStream_t st, int trace_slot = 0);
-bool fast_set_option_gen(int key, int value);
 
 }  // namespace las

@@ -29,14 +29,15 @@ def main():
     e1.record()
     torch.cuda.synchronize()
     print(f"speller c3 bf16: {e0.elapsed_time(e1) / 3:.3f} ms  ({e0.elapsed_time(e1) / 3 / S * 1e3:.2f} us/step)")
-    buf = torch.zeros(512 + 5 * 32 * 8 + 148 * 8, dtype=torch.int64, device="cuda")
+    n_sm = torch.cuda.get_device_properties(0).multi_processor_count
+    buf = torch.zeros(512 + 5 * 32 * 8 + 8 * n_sm, dtype=torch.int64, device="cuda")  # include/las_b200.h las_debug_set_trace
     lib.las_debug_set_trace(_cabi.ptr(buf))
     las.speller(enc, None, 0.0)
     torch.cuda.synchronize()
     lib.las_debug_set_trace(None)
     raw = buf.cpu().numpy()
     t = raw[512:512 + 5 * 32 * 8].reshape(5, 32, 8)
-    allc = raw[512 + 5 * 32 * 8:].reshape(148, 8)
+    allc = raw[512 + 5 * 32 * 8:].reshape(n_sm, 8)
     names = [["in ready", "tma issued", "mma issued", "tmem_full", "stored", "signalled", "h-part mma", "-"],
              ["in ready", "tma issued", "mma issued", "tmem_full", "stored", "signalled", "h-part mma", "-"],
              ["h arrived", "q", "softmax", "ctx mma", "ctx published", "logits", "word published", "-"]]

@@ -34,7 +34,8 @@ torch.cuda.synchronize()
 ms = e0.elapsed_time(e1) / reps
 print(f"B={B} S={S} U={U}: {ms:.3f} ms per decode, {1000 * ms / S:.2f} us per step (includes the per-call psi GEMM and prologue)")
 if os.environ.get("LAS_PROBE_TRACE"):
-    buf = torch.zeros(4096, dtype=torch.int64, device="cuda")
+    n_sm = torch.cuda.get_device_properties(0).multi_processor_count
+    buf = torch.zeros(512 + 5 * 32 * 8 + 8 * n_sm, dtype=torch.int64, device="cuda")  # include/las_b200.h las_debug_set_trace
     lib.las_debug_set_trace(_cabi.ptr(buf))
     las.speller(enc, None, 0.0)
     torch.cuda.synchronize()
