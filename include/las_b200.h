@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define LAS_B200_ABI_VERSION 6
+#define LAS_B200_ABI_VERSION 7
 
 enum {
   LAS_OK = 0,
@@ -228,11 +228,21 @@ int las_speller_decode(const las_decode_io* io, const void* packed, const las_sp
  *   - each step every row runs the decoder step.  A live row k offers (k, v, score[k] + logp[k,v]) for every v (one fp32 add), a
  *     finished row exactly (k, eos_token, score[k]) with token log-prob 0, a -inf row nothing.  The K best candidates by
  *     (score desc, parent asc, token asc) become the new rows (parent's h, c and context; fed-back word one_hot(token)); a row is
- *     finished once its token is eos_token.  A slot left without a finite candidate scores -inf.  All S steps run;
+ *     finished once its token is eos_token.  A slot left without a finite candidate scores -inf.  All S steps run (see early exit);
  *   - the K final rows are ranked by score / length^length_penalty (fp32 powf; ties to the lower slot), length = tokens up to and
  *     including the first eos_token, or S.  The first `nbest` = N are returned: tokens [B,N,S] (eos_token after the end),
- *     token_logp [B,N,S] (0 after the end), lengths [B,N], scores [B,N] = the raw sums of token_logp.  A -inf slot has length 0.
- * Limits: 1 <= K <= 32, 1 <= N <= K, 0 <= eos_token < V, length_penalty finite and >= 0, steps >= 1.
+ *     token_logp [B,N,S] (0 after the end), lengths [B,N], scores [B,N] = the raw sums of token_logp.  A -inf slot has length 0;
+ *   - attention (attn != NULL): attn[b,n,t] ([heads,U]) is the attention weight vector the decoder computed at step t for the row whose
+ *     candidate became token t of hypothesis n, i.e. the PARENT row at step t, before the step's reorder (token_logp follows the same
+ *     rule).  0 for t >= lengths[b,n] and for a -inf slot, as greedy early exit leaves undecoded steps; masked encoder steps hold what
+ *     greedy decoding's attention record holds;
+ *   - early exit (early_exit != 0): every `segment_steps` steps (0 = 32; any count >= 1) the library checks on the device whether all
+ *     B*K rows have ended (a -inf slot counts as ended) and, if so, issues no further steps.  The outputs are bit-identical to
+ *     early_exit = 0: once every row has ended, every later step keeps each row in place with eos at log-prob 0.  *steps_done receives
+ *     the number of steps run.  The loop is driven from the host, so this is the one exception to "nothing synchronises": at each
+ *     check the library copies the device flag back and waits on `stream`.  A call with early_exit on a stream that is being captured
+ *     returns LAS_EINVAL before anything is enqueued.
+ * Limits: 1 <= K <= 32, 1 <= N <= K, 0 <= eos_token < V, length_penalty finite and >= 0, steps >= 1, segment_steps >= 0.
  * ------------------------------------------------------------------------------------------------------ */
 typedef struct las_beam_io {
   const float* enc;            /* [B,U,E] listener features */
@@ -243,6 +253,12 @@ typedef struct las_beam_io {
   float* token_logp;           /* nullable [B,N,S] */
   int32_t* lengths;            /* [B,N] */
   float* scores;               /* [B,N] */
+  float* attn;                 /* nullable [B,N,S,heads,U] per-hypothesis attention (heads = max(d->heads, 1)) */
+  float* attn_work;            /* caller-owned scratch, required with attn: 4 * S * (heads*B*K*U + B*N) bytes, 4-byte aligned --
+                                  [S,heads,B*K,U] fp32 attention of every row and step, then [B,N,S] int32 source rows */
+  int32_t early_exit;          /* 0: run all S steps; else stop once every hypothesis has ended (see above) */
+  int32_t segment_steps;       /* steps between the early-exit checks (0 = 32) */
+  int32_t* steps_done;         /* device int32[1], required with early_exit: steps run */
 } las_beam_io;
 /* The beam pack: in LAS_MODE_BF16 / LAS_MODE_F16 always the fp32 block followed by the generic tensor-core layout (also for shapes the
  * persistent decoder covers); in LAS_MODE_FP32 the ordinary pack.  The size queries return 0 for arguments the calls reject. */

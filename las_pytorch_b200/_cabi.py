@@ -12,7 +12,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "liblas_b200.so")
 
-ABI_VERSION = 6
+ABI_VERSION = 7
 MODE_FP32 = 0
 MODE_BF16 = 1
 MODE_F16 = 2
@@ -65,6 +65,8 @@ class BeamIO(C.Structure):
         ("enc", C.c_void_p), ("enc_lengths", C.c_void_p),
         ("beam", C.c_int32), ("nbest", C.c_int32), ("eos_token", C.c_int32), ("length_penalty", C.c_float),
         ("tokens", C.c_void_p), ("token_logp", C.c_void_p), ("lengths", C.c_void_p), ("scores", C.c_void_p),
+        ("attn", C.c_void_p), ("attn_work", C.c_void_p),
+        ("early_exit", C.c_int32), ("segment_steps", C.c_int32), ("steps_done", C.c_void_p),
     ]
 
 

@@ -149,9 +149,11 @@ __global__ void __launch_bounds__(1024) beam_step_kernel(const BeamStepArgs a) {
   }
 }
 
-// One warp per utterance: lane k traces slot k back through the back-pointers.
+// One warp per utterance: lane k traces slot k back through the back-pointers of the S_run steps that were run; outputs have S_out
+// steps, the tail padded as a full run would have left it (every row had ended, so eos at log-prob 0).  src_rows records, along the
+// same path, the decoder row (b*K + parent) whose attention produced each token, -1 from the length on.
 __global__ void __launch_bounds__(32) beam_finalize_kernel(const BeamFinalArgs a) {
-  const int b = blockIdx.x, k = threadIdx.x, K = a.K, S = a.S;
+  const int b = blockIdx.x, k = threadIdx.x, K = a.K, S = a.S_run;
   const size_t bk = (size_t)a.B * K;
   float sc = -INFINITY, key = -INFINITY;
   int len = 0;
@@ -175,9 +177,14 @@ __global__ void __launch_bounds__(32) beam_finalize_kernel(const BeamFinalArgs a
     if (kq > key || (kq == key && q < k)) ++rank;
   }
   if (k >= K || rank >= a.N) return;
-  const size_t out = ((size_t)b * a.N + rank) * S;
+  const size_t out = ((size_t)b * a.N + rank) * a.S_out;
   a.lengths_out[(size_t)b * a.N + rank] = len;
   a.scores_out[(size_t)b * a.N + rank] = sc;
+  for (int t = S; t < a.S_out; ++t) {
+    a.tokens_out[out + t] = a.eos;
+    if (a.token_logp_out) a.token_logp_out[out + t] = 0.f;
+    if (a.src_rows) a.src_rows[out + t] = -1;
+  }
   int j = k;
   for (int t = S - 1; t >= 0; --t) {
     const size_t o = t * bk + (size_t)b * K + j;
@@ -185,7 +192,30 @@ __global__ void __launch_bounds__(32) beam_finalize_kernel(const BeamFinalArgs a
     a.tokens_out[out + t] = live ? a.token[o] : a.eos;
     if (a.token_logp_out) a.token_logp_out[out + t] = live ? a.token_logp[o] : 0.f;
     j = a.parent[o];
+    if (a.src_rows) a.src_rows[out + t] = live ? b * K + j : -1;
   }
+}
+
+// attn[b, n, t, h, :] = work[t, h, src_rows[b, n, t], :], zeros where src_rows is -1 (t >= length).  Block (b*N + n, chunk of t).
+constexpr int BT_STEPS = 8;  // steps per CTA
+__global__ void __launch_bounds__(256) beam_attention_trace_kernel(const float* work, const int32_t* src_rows, float* attn, int BK, int S,
+                                                                   int heads, int U) {
+  const int bn = blockIdx.x, t0 = blockIdx.y * BT_STEPS, hu = heads * U;
+  for (int t = t0; t < min(S, t0 + BT_STEPS); ++t) {
+    const int row = src_rows[(size_t)bn * S + t];
+    float* dst = attn + ((size_t)bn * S + t) * hu;
+    for (int i = threadIdx.x; i < hu; i += blockDim.x) {
+      const int h = i / U, u = i - h * U;
+      dst[i] = row >= 0 ? work[(((size_t)t * heads + h) * BK + row) * U + u] : 0.f;
+    }
+  }
+}
+
+// *steps_done = step when every one of the n rows has ended (fin != 0; a -inf slot counts as ended), else left as it is.
+__global__ void __launch_bounds__(256) beam_all_ended_kernel(const int32_t* fin, int n, int step, int32_t* steps_done) {
+  int all = 1;
+  for (int i = threadIdx.x; i < n; i += blockDim.x) all &= fin[i] != 0;
+  if (__syncthreads_and(all) && threadIdx.x == 0) *steps_done = step;
 }
 
 }  // namespace
@@ -206,8 +236,22 @@ int launch_beam_step(const BeamStepArgs& a, cudaStream_t st) {
 
 int launch_beam_finalize(const BeamFinalArgs& a, cudaStream_t st) {
   LAS_REQUIRE(a.K >= 1 && a.K <= BS_MAX_K && a.N >= 1 && a.N <= a.K, "beam width %d / n-best %d out of range", a.K, a.N);
+  LAS_REQUIRE(a.S_run >= 1 && a.S_run <= a.S_out, "steps run %d is not in [1, %d]", a.S_run, a.S_out);
   beam_finalize_kernel<<<a.B, 32, 0, st>>>(a);
   LAS_LAUNCH_OK("beam_finalize_kernel");
+  return LAS_OK;
+}
+
+int launch_beam_attention_trace(const float* work, const int32_t* src_rows, float* attn, int B, int K, int N, int S, int heads, int U,
+                                cudaStream_t st) {
+  beam_attention_trace_kernel<<<dim3(B * N, (S + BT_STEPS - 1) / BT_STEPS), 256, 0, st>>>(work, src_rows, attn, B * K, S, heads, U);
+  LAS_LAUNCH_OK("beam_attention_trace_kernel");
+  return LAS_OK;
+}
+
+int launch_beam_all_ended(const int32_t* fin, int n, int step, int32_t* steps_done, cudaStream_t st) {
+  beam_all_ended_kernel<<<1, 256, 0, st>>>(fin, n, step, steps_done);
+  LAS_LAUNCH_OK("beam_all_ended_kernel");
   return LAS_OK;
 }
 

@@ -739,6 +739,19 @@ static int speller_beam_f32(const las_beam_io* io, const las_speller_dims* d, co
   ba.c = d->cell == LAS_CELL_LSTM ? w.c : nullptr;
   ba.xin = w.xin; ba.xld = V + E;
   ba.B = B; ba.K = K; ba.V = V; ba.E = E; ba.Hs = Hs; ba.sl = d->sl; ba.eos = io->eos_token;
+  // attention scratch (las_beam_io.attn_work): every row's attention of every step, then the source rows of the n-best paths
+  const int NH = n_heads(d), U = d->U;
+  float* attn_work = io->attn ? io->attn_work : nullptr;
+  int32_t* src_rows = io->attn ? reinterpret_cast<int32_t*>(io->attn_work + (size_t)steps * NH * BK * U) : nullptr;
+  // Early exit.  Once every row has ended (a -inf slot counts as ended), each row's only candidate is itself: eos at log-prob 0, score
+  // unchanged.  Every merge fills the slots by rank, so the rows are already in (score desc, slot asc) order, which is the merge key
+  // of those candidates: every later step keeps every row in its slot and records parent = slot, eos, 0.  Stopping there and padding
+  // the tail with eos / 0 (finalize) and zero attention (the trace: its source rows are -1 past every length) therefore gives exactly
+  // the outputs of the full run.  The host has to learn the flag to stop issuing steps: one 4-byte copy and a stream synchronisation
+  // per check.
+  const int seg = io->segment_steps > 0 ? io->segment_steps : 32;
+  int steps_run = steps;
+  if (io->early_exit) LAS_CUDA_OK(cudaMemsetAsync(io->steps_done, 0, sizeof(int32_t), st));
   ProfScope ps_steps("speller.beam_steps", st);
   for (int s = 0; s < steps; ++s) {
     float* hp = w.h[s & 1];
@@ -747,19 +760,34 @@ static int speller_beam_f32(const las_beam_io* io, const las_speller_dims* d, co
     t.rows_per_utt = K;
     t.word_out = nullptr;  // beam_step_kernel writes the fed-back words
     t.logp_out = w.logp;
+    t.score_out = attn_work ? attn_work + (size_t)s * NH * BK * U : nullptr;  // [heads, B*K, U]: indexed by decoder row
     LAS_TRY(speller_step(path, s, hp, hn, t, st));
     ba.parent = w.parent + (size_t)s * BK;
     ba.token = w.token + (size_t)s * BK;
     ba.token_logp = w.token_logp + (size_t)s * BK;
     ba.h = hn;
     LAS_TRY(launch_beam_step(ba, st));
+    if (io->early_exit && (s + 1) % seg == 0 && s + 1 < steps) {
+      LAS_TRY(launch_beam_all_ended(w.fin, BK, s + 1, io->steps_done, st));
+      int32_t ended = 0;
+      LAS_CUDA_OK(cudaMemcpyAsync(&ended, io->steps_done, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+      LAS_CUDA_OK(cudaStreamSynchronize(st));
+      if (ended) {
+        steps_run = s + 1;
+        break;
+      }
+    }
   }
+  if (io->early_exit && steps_run == steps) LAS_CUDA_OK(cudaMemcpyAsync(io->steps_done, &steps, sizeof(int32_t), cudaMemcpyHostToDevice, st));
   BeamFinalArgs fa;
   memset(&fa, 0, sizeof(fa));
   fa.score = w.score; fa.parent = w.parent; fa.token = w.token; fa.token_logp = w.token_logp;
   fa.tokens_out = io->tokens; fa.token_logp_out = io->token_logp; fa.lengths_out = io->lengths; fa.scores_out = io->scores;
-  fa.B = B; fa.K = K; fa.N = io->nbest; fa.S = steps; fa.eos = io->eos_token; fa.alpha = io->length_penalty;
-  return launch_beam_finalize(fa, st);
+  fa.src_rows = src_rows;
+  fa.B = B; fa.K = K; fa.N = io->nbest; fa.S_run = steps_run; fa.S_out = steps; fa.eos = io->eos_token; fa.alpha = io->length_penalty;
+  LAS_TRY(launch_beam_finalize(fa, st));
+  if (io->attn) LAS_TRY(launch_beam_attention_trace(attn_work, src_rows, io->attn, B, K, io->nbest, steps, NH, U, st));
+  return LAS_OK;
 }
 
 // The las_decode_io checks of las_speller_decode, which las_pipeline_step's concurrent branch makes as well.  `d` has passed
@@ -1042,7 +1070,16 @@ int las_speller_beam_search(const las_beam_io* io, const void* packed, const las
   LAS_REQUIRE(isfinite(io->length_penalty) && io->length_penalty >= 0.f, "length_penalty must be finite and >= 0 (%g)", (double)io->length_penalty);
   LAS_REQUIRE(mode == LAS_MODE_FP32 || tc_mode(mode), "unknown mode %d", mode);
   LAS_REQUIRE(!tc_mode(mode) || gen_ok(d), "LAS_MODE_BF16 beam search needs E %% 8 == 0 (E=%d); use LAS_MODE_FP32", d->E);
+  LAS_REQUIRE(!io->attn || io->attn_work, "io->attn needs io->attn_work");
+  LAS_REQUIRE(!io->early_exit || io->steps_done, "io->early_exit needs io->steps_done");
+  LAS_REQUIRE(io->segment_steps >= 0, "segment_steps must be >= 0 (%d)", io->segment_steps);
   LAS_TRY(device_ok());
+  if (io->early_exit) {
+    // early exit waits on the stream for its flag, which a stream being captured into a graph cannot do
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    LAS_CUDA_OK(cudaStreamIsCapturing(static_cast<cudaStream_t>(stream), &cs));
+    LAS_REQUIRE(cs == cudaStreamCaptureStatusNone, "io->early_exit synchronises with the host and cannot run on a capturing stream");
+  }
   const size_t need = las_speller_beam_workspace_bytes(d, steps, io->beam, mode);
   if (workspace_bytes < need) return fail(LAS_ENOMEM, "workspace too small: %zu < %zu", workspace_bytes, need);
   return speller_beam_f32(io, d, speller_layout(d, mode, true, packed, nullptr), steps, relu, workspace, static_cast<cudaStream_t>(stream));

@@ -123,10 +123,18 @@ struct BeamFinalArgs {
   float* token_logp_out;   // nullable [B, N, S]
   int32_t* lengths_out;    // [B, N]
   float* scores_out;       // [B, N]
-  int B, K, N, S, eos;
+  int32_t* src_rows;       // nullable [B, N, S_out]: decoder row (b*K + parent) of each token's step, -1 from the length on
+  int B, K, N, eos;
+  int S_run;               // steps run: the back-pointers hold S_run steps (every row has ended if S_run < S_out)
+  int S_out;               // steps of the outputs; [S_run, S_out) is padded with eos / 0
   float alpha;
 };
 int launch_beam_finalize(const BeamFinalArgs& a, cudaStream_t st);
+// attn [B, N, S, heads, U] from the per-step attention of every decoder row, work [S, heads, B*K, U], along src_rows [B, N, S]
+int launch_beam_attention_trace(const float* work, const int32_t* src_rows, float* attn, int B, int K, int N, int S, int heads, int U,
+                                cudaStream_t st);
+// *steps_done = step if every fin[0 .. n) is set; otherwise *steps_done is left unchanged
+int launch_beam_all_ended(const int32_t* fin, int n, int step, int32_t* steps_done, cudaStream_t st);
 
 // <eos> early exit bookkeeping (las_decode_io.early_exit): `state` = 66 int32 {stop, steps decoded, done[64]} per launch group
 int launch_eos_check(const int32_t* tokens, int Bfull, int b0, int Bc, int s_begin, int s_end, int eos, int32_t* state, cudaStream_t st);

@@ -239,17 +239,19 @@ class LAS(nn.Module):
                                                           enc_lengths=enc_lengths, nll_labels=nll_labels)
         return raw_pred_seq, attention_record
 
-    def beam_search(self, batch_data, beam_width=8, nbest=1, length_penalty=0.0, input_lengths=None):
+    def beam_search(self, batch_data, beam_width=8, nbest=1, length_penalty=0.0, input_lengths=None, return_attention=False,
+                    early_exit=False):
         """Beam-search decoding (extension; the reference decodes greedily): the listener (with the length mask when
-        `input_lengths` is given), then `Speller.beam_search` over `max_label_len` steps.  Returns a BeamSearchResult."""
-        _check_beam_args(beam_width, nbest, length_penalty, self.speller.max_label_len)
+        `input_lengths` is given), then `Speller.beam_search` over `max_label_len` steps.  Returns a BeamSearchResult, or with
+        `return_attention` a BeamSearchAlignedResult; `early_exit` as in Speller.beam_search."""
+        _check_beam_args(beam_width, nbest, length_penalty, self.speller.max_label_len, return_attention, early_exit)
         enc_lengths = None
         if input_lengths is None:
             listener_feature = self.listener(batch_data)
         else:
             listener_feature, enc_lengths = self.listener(batch_data, input_lengths=input_lengths)
         return self.speller.beam_search(listener_feature, beam_width=beam_width, nbest=nbest, length_penalty=length_penalty,
-                                        enc_lengths=enc_lengths)
+                                        enc_lengths=enc_lengths, return_attention=return_attention, early_exit=early_exit)
 
     # ---- large free-running batches: the serving pipeline applied INSIDE one forward call ------------------------------------
     CHUNK = 64  # utterances per persistent decoder launch group (one attention CTA each next to the 64 LSTM CTAs)
@@ -406,8 +408,16 @@ BeamSearchResult.__doc__ = """n-best hypotheses per utterance, best first (devic
 the end)."""
 
 
-def _check_beam_args(beam_width, nbest, length_penalty, steps):
+BeamSearchAlignedResult = collections.namedtuple("BeamSearchAlignedResult", BeamSearchResult._fields + ("attention",))
+BeamSearchAlignedResult.__doc__ = """BeamSearchResult's fields plus attention [B,N,S,U] fp32 ([B,N,S,heads,U] with multi_head > 1): the attention
+weights the decoder computed at step t for the hypothesis row that token t was chosen from, 0 from lengths[b,n] on."""
+
+
+def _check_beam_args(beam_width, nbest, length_penalty, steps, return_attention=False, early_exit=False):
     """The library's limits, checked on the host so that bad arguments fail before anything reaches the device."""
+    for name, flag in (("return_attention", return_attention), ("early_exit", early_exit)):
+        if not isinstance(flag, bool):
+            raise ValueError(f"{name} must be a bool, got {flag!r}")
     if isinstance(beam_width, bool) or not isinstance(beam_width, int) or not 1 <= beam_width <= 32:
         raise ValueError(f"beam_width must be an int in [1, 32], got {beam_width!r}")
     if isinstance(nbest, bool) or not isinstance(nbest, int) or not 1 <= nbest <= beam_width:
@@ -713,13 +723,20 @@ class Speller(nn.Module):
                                            c.ws.numel(), c.st))
         return c.logp, c.attn, c.tokens
 
-    def beam_search(self, listener_feature, beam_width=8, nbest=1, length_penalty=0.0, enc_lengths=None, max_steps=None):
+    def beam_search(self, listener_feature, beam_width=8, nbest=1, length_penalty=0.0, enc_lengths=None, max_steps=None,
+                    return_attention=False, early_exit=False):
         """Beam-search decoding on the device (extension; include/las_b200.h las_speller_beam_search has the exact semantics).
         Every utterance keeps `beam_width` hypotheses for `max_steps` (default max_label_len) steps; a hypothesis ends at <eos>
         (`self.eos_token`, default 1).  The `nbest` best by score / length**length_penalty are returned, best first, as a
-        BeamSearchResult of device tensors.  Draws nothing from numpy's or torch's random generators."""
+        BeamSearchResult of device tensors.  Draws nothing from numpy's or torch's random generators.
+
+        `return_attention=True` returns a BeamSearchAlignedResult: the same fields plus each hypothesis's attention record.
+        `early_exit=True` stops issuing decoder steps once every hypothesis has ended, checked every `self.early_exit_every` (default
+        32) steps; the outputs are bit-identical to a full run.  Each check waits on the stream for a 4-byte flag, so it cannot be
+        captured into a CUDA graph.  The steps run are left in `self.last_steps_done` (device int32[1], overwritten by the next
+        early-exit beam search).  It is independent of `self.early_exit`, which only governs greedy decoding."""
         steps = self.max_label_len if max_steps is None else max_steps
-        _check_beam_args(beam_width, nbest, length_penalty, steps)
+        _check_beam_args(beam_width, nbest, length_penalty, steps, return_attention, early_exit)
         eos = getattr(self, "eos_token", 1)
         if not 0 <= eos < self.label_dim:
             raise ValueError(f"eos_token {eos} is not in [0, {self.label_dim})")
@@ -729,6 +746,9 @@ class Speller(nn.Module):
         if enc_lengths is not None and enc_lengths.numel() != b:
             raise ValueError(f"enc_lengths has {enc_lengths.numel()} entries for a batch of {b}")
         _require_cuda(listener_feature, "listener_feature")
+        if early_exit and torch.cuda.is_current_stream_capturing():
+            # (the library refuses it as well; raising here also keeps a first call's weight packing out of the graph)
+            raise RuntimeError("beam search with early_exit waits on the stream for its stop flag and cannot be captured into a CUDA graph")
         lib = _cabi.load_library()
         dev = listener_feature.device
         mode = _mode_of(self.precision)
@@ -748,8 +768,20 @@ class Speller(nn.Module):
             io.enc, io.enc_lengths = enc.data_ptr(), (lens.data_ptr() if lens is not None else None)
             io.beam, io.nbest, io.eos_token, io.length_penalty = beam_width, nbest, eos, float(length_penalty)
             io.tokens, io.token_logp, io.lengths, io.scores = (t.data_ptr() for t in (out.tokens, out.token_logp, out.lengths, out.scores))
+            if return_attention:
+                nh = self.attention.multi_head
+                attn = torch.empty((b, nbest, steps, u) if nh == 1 else (b, nbest, steps, nh, u), dtype=torch.float32, device=dev)
+                # las_beam_io.attn_work: [S, heads, B*K, U] fp32, then [B, N, S] int32
+                work = self._cache.workspace(("beam_attn", dev, st.value), 4 * steps * (nh * b * beam_width * u + b * nbest), dev)
+                io.attn, io.attn_work = attn.data_ptr(), work.data_ptr()
+                out = BeamSearchAlignedResult(*out, attention=attn)
+            if early_exit:
+                steps_done = self._cache.workspace(("beam_steps_done", dev, st.value), 4, dev)[:4].view(torch.int32)
+                io.early_exit, io.segment_steps, io.steps_done = 1, int(getattr(self, "early_exit_every", 32)), steps_done.data_ptr()
             check(lib.las_speller_beam_search(C.byref(io), ptr(packed), C.byref(dims), steps, mode, self.attention.relu_flag, ptr(ws),
                                               ws.numel(), st))
+            if early_exit:
+                self.last_steps_done = steps_done
         return out
 
     # ---- reference API ---------------------------------------------------------------------------------
