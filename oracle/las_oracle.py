@@ -201,6 +201,7 @@ def speller_forward(
     dtype=np.float32,
     prefix="speller",
     enc_lengths=None,
+    activate=True,
 ):
     """Speller step loop -- model/las_model.py:186-238 with forward_step :178-184.
 
@@ -209,6 +210,7 @@ def speller_forward(
                  (teacher forcing: next input is ground_truth[:, step], NOT shifted -- :216-217)
     steps        number of decode steps (max_label_len free-running, ground_truth.shape[1] teacher-forced)
     decode_mode  0: feed log-probs back (:220-221); 1: one-hot(argmax) (:223-227)
+    activate     relu on phi(state) and psi(enc) (mlp_activate_in_attention="relu"); False: both used raw ("None")
     returns dict(logp [S,B,V], attn [S,B,U], tokens [S,B] argmax of logp, context [S,B,E])
     """
     enc = np.asarray(enc, dtype=dtype)
@@ -223,7 +225,7 @@ def speller_forward(
             gt = np.eye(v, dtype=dtype)[gt]
         gt = gt.astype(dtype)
 
-    psi = psi_project(enc, sd, dtype, prefix) if f"{prefix}.attention.psi.weight" in sd else enc
+    psi = psi_project(enc, sd, dtype, prefix, activate) if f"{prefix}.attention.psi.weight" in sd else enc
     h = [np.zeros((b, hs), dtype=dtype) for _ in range(num_layers)]  # hidden_state=None -> zeros
     c = [np.zeros((b, hs), dtype=dtype) for _ in range(num_layers)]
     word = np.zeros((b, v), dtype=dtype)
@@ -238,7 +240,7 @@ def speller_forward(
             ph = h[l] @ _w(sd, f"{prefix}.rnn_layer.weight_hh_l{l}", dtype).T + _w(sd, f"{prefix}.rnn_layer.bias_hh_l{l}", dtype)
             h[l], c[l] = rnn_cell_step(px, ph, h[l], c[l])
             inp = h[l]
-        score, ctx = attention(h[-1], enc, psi, sd, dtype, prefix, enc_lengths=enc_lengths)  # (:180)
+        score, ctx = attention(h[-1], enc, psi, sd, dtype, prefix, activate, enc_lengths)  # (:180)
         logp = log_softmax(np.concatenate([h[-1], ctx], axis=-1) @ w_cd.T + b_cd)  # (:181-182)
         tok = logp.argmax(axis=-1)
         logps.append(logp.astype(dtype))
@@ -269,15 +271,16 @@ def las_forward(
     teacher_forced=False,
     decode_mode=1,
     dtype=np.float32,
+    activate=True,
 ):
     """LAS.forward -- model/las_model.py:30-40.  The teacher-forcing coin flip (:189) is resolved by the
     caller (`teacher_forced`), which also fixes the step count (:205-208)."""
     enc = listener_forward(x, sd, listener_layers, dtype)
     if teacher_forced and ground_truth is not None:
         steps = np.asarray(ground_truth).shape[1]
-        out = speller_forward(enc, sd, speller_layers, steps, ground_truth, decode_mode, dtype)
+        out = speller_forward(enc, sd, speller_layers, steps, ground_truth, decode_mode, dtype, activate=activate)
     else:
-        out = speller_forward(enc, sd, speller_layers, max_label_len, None, decode_mode, dtype)
+        out = speller_forward(enc, sd, speller_layers, max_label_len, None, decode_mode, dtype, activate=activate)
     out["enc"] = enc
     return out
 

@@ -64,7 +64,8 @@ CONFIGS = {
 
 def build_model(cfg, max_label_len, decode_mode=1, seed=17, gain=1.0, precision="fp32", module=None):
     """Construct (listener, speller, las) under torch.manual_seed(seed), then scale every 2-D parameter by `gain`
-    (the "gain-3" ladder of SURVEY.md A.6).  `module` = the module providing Listener/Speller/LAS (ours by default)."""
+    (the "gain-3" ladder of SURVEY.md A.6).  `module` = the module providing Listener/Speller/LAS (ours by default).
+    The optional config key `activate` is the attention MLP's activation ("relu", the default, or "None")."""
     if module is None:
         import las_pytorch_b200 as module
     c = CONFIGS[cfg] if isinstance(cfg, str) else cfg
@@ -75,7 +76,7 @@ def build_model(cfg, max_label_len, decode_mode=1, seed=17, gain=1.0, precision=
                                use_gpu=False, **extra)
     speller = module.Speller(vocab_size=c["V"], hidden_size=2 * c["H"], rnn_unit=unit, num_layers=c["sl"],
                              max_label_len=max_label_len, use_mlp_in_attention=c.get("use_mlp", True), mlp_dim_in_attention=c["D"],
-                             mlp_activate_in_attention="relu", listener_hidden_size=c["H"], multi_head=c.get("heads", 1),
+                             mlp_activate_in_attention=c.get("activate", "relu"), listener_hidden_size=c["H"], multi_head=c.get("heads", 1),
                              decode_mode=decode_mode, use_gpu=False, **extra)
     las = module.LAS(listener, speller)
     if gain != 1.0:
