@@ -1289,16 +1289,28 @@ int ctx_tiles_fit(int U, int E) {
   if (ntm == NT && att_bop_bytes(U) > 4096 * 4) ntm = 0;
   return ntm;
 }
-// Long encoders: when one CTA cannot hold all of enc[b]^T in tensor memory but half of the encoder steps fit (U <= 448 at E = 512),
-// a cluster of two CTAs attends each utterance (flash-decoding style partial softmax, combined through DSMEM) -- provided the LSTM
-// CTAs pair up (even count) and the chip has room for two attention CTAs per utterance.
-bool att_split_ok(const las_speller_dims* d) {
-  if (!debug_options().att_split || !debug_options().ctx_tmem || d->E % 128 != 0) return false;
-  const int NT = d->E / 128;
-  if (ctx_tiles_fit(d->U, d->E) == NT) return false;  // one CTA is enough
-  const int n_lstm = d->sl * (d->Hs / DEC_UNITS);
-  return ctx_tiles_fit(att_split_half(d->U), d->E) == NT && (n_lstm % 2 == 0) && n_lstm + 2 <= sm_count() &&
-         att_smem(d, true, false, true) <= 220 * 1024;
+// The form of the persistent decoder's attention CTAs, decided here alone; the one reader of debug keys 2 and 11
+struct AttPlan {
+  int split, ntm;                // CTAs per utterance; 128-feature tiles of enc[b]^T in tensor memory (hybrid: 0 < ntm < E/128)
+  bool hybrid, k_in_smem, wreg;
+  size_t smem;                   // the attention CTA's dynamic shared memory
+};
+AttPlan att_plan(const las_speller_dims* d) {
+  const DebugOptions& o = debug_options();
+  const int NT = d->E / 128, n_lstm = d->sl * (d->Hs / DEC_UNITS);
+  // Long encoders: when one CTA cannot hold all of enc[b]^T in tensor memory but half of the encoder steps fit (U <= 448 at E = 512),
+  // a cluster of two CTAs attends each utterance (flash-decoding style partial softmax, combined through DSMEM) -- provided the LSTM
+  // CTAs pair up (even count) and the chip has room for two attention CTAs per utterance.
+  if (o.att_split && o.ctx_tmem && d->E % 128 == 0 && ctx_tiles_fit(d->U, d->E) != NT && ctx_tiles_fit(att_split_half(d->U), d->E) == NT &&
+      n_lstm % 2 == 0 && n_lstm + 2 <= sm_count() && att_smem(d, true, false, true) <= 220 * 1024)
+    return {2, NT, false, true, att_wreg(d), att_smem(d, true, false, true)};
+  // all feature tiles of enc[b]^T in tensor memory when they fit its 512 columns (U <= 224 at E = 512); otherwise as many as fit,
+  // the rest on the CUDA cores (hybrid; needs the score operand in its own shared-memory region), or none where that does not fit
+  int ntm = o.ctx_tmem ? ctx_tiles_fit(d->U, d->E) : 0;
+  if (ntm > 0 && ntm < NT && (512 % ((d->E - ntm * 128) / 8)) != 0) ntm = 0;
+  bool hybrid = ntm > 0 && ntm < NT, k_in_smem = att_smem(d, true, hybrid) <= 220 * 1024;
+  if (hybrid && att_smem(d, k_in_smem, true) > 220 * 1024) { ntm = 0; hybrid = false; k_in_smem = att_smem(d, true) <= 220 * 1024; }
+  return {1, ntm, hybrid, k_in_smem, att_wreg(d), att_smem(d, k_in_smem, hybrid)};
 }
 int supported(const las_speller_dims* d) {
   LAS_REQUIRE(d->sl <= MAX_SL, "LAS_MODE_BF16 speller supports at most %d layers (sl=%d)", MAX_SL, d->sl);
@@ -1422,25 +1434,8 @@ int fast_speller_decode_segment(const las_decode_io* io, const SpellerF32Inputs&
     memset(&p, 0, sizeof(p));
     p.B = Bc; p.U = d->U; p.E = d->E; p.Hs = d->Hs; p.sl = d->sl; p.V = d->V; p.D = d->D;
     p.steps = s_count; p.s0 = s_begin; p.decode_mode = decode_mode; p.relu = relu; p.gt_steps = io->gt_steps; p.ncl = s.ncl;
-    p.wreg = att_wreg(d) ? 1 : 0;
-    p.k_in_smem = att_smem(d, true) <= 220 * 1024;
-    p.att_split = att_split_ok(d) ? 2 : 1;
-    if (p.att_split == 2) {
-      p.ctx_ntm = d->E / 128;
-      p.ctx_tmem = 1;
-      p.k_in_smem = 1;
-    } else {
-      const int NT = d->E / 128;
-      // all feature tiles of enc[b]^T in tensor memory when they fit its 512 columns (U <= 224 at E = 512); otherwise as many
-      // as fit, the rest on the CUDA cores (hybrid; needs the score operand in its own shared-memory region)
-      int ntm = debug_options().ctx_tmem ? ctx_tiles_fit(d->U, d->E) : 0;
-      if (ntm > 0 && ntm < NT && (512 % ((d->E - ntm * 128) / 8)) != 0) ntm = 0;
-      p.ctx_ntm = ntm;
-      p.ctx_tmem = ntm > 0;
-      const bool hyb = ntm > 0 && ntm < NT;
-      p.k_in_smem = att_smem(d, true, hyb) <= 220 * 1024;
-      if (hyb && att_smem(d, p.k_in_smem != 0, true) > 220 * 1024) { p.ctx_ntm = 0; p.ctx_tmem = 0; p.k_in_smem = att_smem(d, true, false) <= 220 * 1024; }
-    }
+    const AttPlan ap = att_plan(d);
+    p.att_split = ap.split; p.ctx_ntm = ap.ntm; p.ctx_tmem = ap.ntm > 0; p.k_in_smem = ap.k_in_smem; p.wreg = ap.wreg;
     RingCfg rc = ring_cfg(d);
     // two utterance groups of 32 pipelined through the LSTM CTAs when the launch has more than 32 utterances
     p.groups = (Bc > 32 && debug_options().dec_groups != 0) ? 2 : 1;
@@ -1512,8 +1507,7 @@ int fast_speller_decode_segment(const las_decode_io* io, const SpellerF32Inputs&
                                   st, relu != 0));
     }
     ProfScope ps("speller.steps", st);
-    const size_t smem_l = rc.smem, smem_a = att_smem(d, p.k_in_smem != 0, p.ctx_ntm > 0 && p.ctx_ntm < d->E / 128, p.att_split == 2);
-    const size_t smem = (smem_l > smem_a ? smem_l : smem_a) + 1024;
+    const size_t smem = (rc.smem > ap.smem ? rc.smem : ap.smem) + 1024;
     // the operand format is a template parameter: the conversions sit in the GEMV inner loops (a run-time branch there cost 20 %)
     auto kern = p.f16 ? speller_decode_persistent_kernel<1> : speller_decode_persistent_kernel<0>;
     LAS_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1541,15 +1535,13 @@ int fast_speller_decode_segment(const las_decode_io* io, const SpellerF32Inputs&
 }
 
 int fast_speller_max_group(const las_speller_dims* d) {
-  const Shape s = shape_of(d);
-  const int n_lstm = d->sl * s.ncl, nsm = sm_count();
   // utterances per persistent launch: one attention CTA each (two for split attention), and at most 64 (activation slots hold
   // 64 batch rows)
-  const int per = att_split_ok(d) ? 2 : 1;
-  return (nsm - n_lstm) / per < 64 ? (nsm - n_lstm) / per : 64;
+  const int n = (sm_count() - d->sl * shape_of(d).ncl) / att_plan(d).split;
+  return n < 64 ? n : 64;
 }
 
-int fast_speller_ctas(const las_speller_dims* d) { return d->sl * shape_of(d).ncl + (att_split_ok(d) ? 2 : 1) * d->B; }
+int fast_speller_ctas(const las_speller_dims* d) { return d->sl * shape_of(d).ncl + att_plan(d).split * d->B; }
 
 // Segment lengths: `seg` steps each (even), the remainder in the last one.  seg <= 0: one segment.
 static int next_segment(int s_begin, int steps, int seg) {

@@ -314,7 +314,7 @@ gen_cell_step_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_cons
 //   rank 0   log-softmax, NLL term, token, fed-back word (attend_tail)
 // Dot products read 16-byte vectors with four of them in flight per lane where the row is aligned for it.
 // =========================================================================================================
-constexpr int AC_SLICES = 8, AC_THREADS = 512, AC_SEGS = 4;
+constexpr int AC_SLICES = 8, AC_SEGS = 4;
 
 // lanes of one warp: sum_k w[k] * x[k] over [0, n), x in shared memory; vec: n % 4 == 0 and both 16-byte aligned
 // (One out-of-line copy each: the kernel runs once per launch, so its code size is paid in instruction fetches every decoder step.
@@ -665,16 +665,9 @@ int launch_gen_cell_step(const GenStepMaps& m, int parity, const float* bias, fl
   return LAS_OK;
 }
 
-int launch_attend_cluster(const AttendArgs& a, bool pdl, cudaStream_t st) {
-  LAS_REQUIRE(a.heads == 1 && a.E % 4 == 0, "attend_cluster_kernel is the single-head form with E %% 4 == 0 (heads=%d E=%d)", a.heads, a.E);
-  if ((reinterpret_cast<uintptr_t>(a.enc) & 15) != 0 || a.E > 4 * AC_THREADS) return launch_attend_f32(a, st);  // (vector loads of the encoder rows; four features per thread)
-  int C = debug_options().gen_cluster;
-  if (C != 1 && C != 2 && C != 4 && C != 8) {
-    // The step's kernels overlap pairwise (programmatic dependent launch) and each wants an SM to itself: keep this one to half the
-    // chip so that the next step's first cell kernel (<= 64 CTAs) starts on the other half while it runs.
-    const int half = sm_count() / 2;
-    C = a.B * 8 <= half ? 8 : (a.B * 4 <= half ? 4 : (a.B * 2 <= half ? 2 : 1));
-  }
+int launch_attend_cluster(const AttendArgs& a, int C, bool pdl, cudaStream_t st) {
+  LAS_REQUIRE(a.heads == 1 && a.E % 4 == 0 && a.E <= 4 * AC_THREADS && (reinterpret_cast<uintptr_t>(a.enc) & 15) == 0 && (C == 1 || C == 2 || C == 4 || C == 8),
+              "attend_cluster_kernel: heads == 1, E %% 4 == 0, E <= %d, aligned enc, C = 1 / 2 / 4 / 8 (heads=%d E=%d C=%d)", 4 * AC_THREADS, a.heads, a.E, C);
   auto r4 = [](size_t n) { return (n + 3) & ~(size_t)3; };
   size_t floats = r4(a.Hs) + a.E + r4(a.D) + r4(a.U) + 12 + r4(a.V) + r4((size_t)((a.V + C - 1) / C) * AC_SEGS) + 32 + r4(a.D) + r4(a.V) +
                   (size_t)AC_SLICES * (a.E + 4) + 4 /* barrier */ + (size_t)3 * a.E /* row-group sums */;

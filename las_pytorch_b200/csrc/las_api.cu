@@ -457,11 +457,32 @@ static const float* speller_psi(const las_speller_dims* d, int B, const SpellerP
   return psi;
 }
 
-// One decoder step of the launch-per-step loop on `rows` decoder rows: the stacked cells (fused generic step, or per layer
-// lstm_cell_f32 / gen_build_a + GEMM + gen_cell), then the attention + character distribution with `t` (see speller_attend_args).
+// Which kernels a launch-per-step decoder step runs on `rows` rows (greedy: B, beam: B*K), decided here alone; the one reader of debug keys 12 and 13
+struct StepPlan {
+  enum Cell { F32, SWAPPED, PLAIN, FUSED } cell;  // lstm_cell_f32 | gen_build_a + GEMM (operands swapped or not) + gen_cell | fused step
+  bool cluster_att; int C;                        // attend_cluster_kernel with C CTAs per row, else attend_f32_kernel
+};
+static StepPlan step_plan(const las_speller_dims* d, int rows, const SpellerLayout& L, bool beam, const float* enc) {
+  const DebugOptions& o = debug_options();
+  // beam search keeps to the unfused step (DESIGN §4f); small batches swap the GEMM's operands (speller_step)
+  const StepPlan::Cell cell = L.path != Path::GEN ? StepPlan::F32 : (!beam && o.gen_fused && rows <= 256) ? StepPlan::FUSED
+                              : rows <= 64 ? StepPlan::SWAPPED : StepPlan::PLAIN;
+  // The cluster kernel is plain fp32 arithmetic, so the fp32 mode uses it as well.  Multi-head attention keeps the one-CTA kernel, and
+  // so do encoders the cluster kernel cannot read (16-byte vector loads of the encoder rows, four features per thread).
+  const bool cluster_att = n_heads(d) == 1 && d->E % 4 == 0 && o.gen_fused && (reinterpret_cast<uintptr_t>(enc) & 15) == 0 && d->E <= 4 * AC_THREADS;
+  // The step's kernels overlap pairwise (programmatic dependent launch) and each wants an SM to itself: by default the attention keeps
+  // to half the chip so that the next step's first cell kernel (<= 64 CTAs) starts on the other half while it runs.
+  const int half = sm_count() / 2;
+  int C = o.gen_cluster;
+  if (C != 1 && C != 2 && C != 4 && C != 8) C = rows * 8 <= half ? 8 : (rows * 4 <= half ? 4 : (rows * 2 <= half ? 2 : 1));
+  return {cell, cluster_att, C};
+}
+
+// One decoder step of the launch-per-step loop on `rows` decoder rows, with the kernels of `plan` and the attention arguments `t`
 struct StepPath {
   const las_speller_dims* d;
   int rows;
+  StepPlan plan;
   SpellerPackF32 pk;
   const SpellerPackGen* gp;  // generic tensor-core path, else nullptr (fp32 mode)
   bool f16;                  // generic path: the 16-bit operand format (SpellerLayout::f16)
@@ -471,10 +492,8 @@ struct StepPath {
   const float* zero;         // [256] zeros
   float* xin;                // [rows, V+E] layer-0 input: fed-back word | context
   float* c;                  // [sl, rows, Hs]
-  bool fused;                // fused generic step (gen_step.cu) with its operand rows in abuf
-  const GenStepMaps* maps;
+  const GenStepMaps* maps;   // fused step
   __nv_bfloat16* (*abuf)[2];
-  bool cluster_att;          // attend_cluster_kernel instead of attend_f32_kernel
 };
 static AttendArgs speller_attend_args(const StepPath& p, const float* enc, const float* psi, const int32_t* enc_lengths, const float* hn, int relu) {
   const las_speller_dims* d = p.d;
@@ -500,18 +519,18 @@ static int speller_step(const StepPath& p, int s, const float* hp, float* hn, co
   const int B = p.rows, Hs = d->Hs, sl = d->sl, xld = d->V + d->E;
   const GenGeom& gg = p.gg;
   for (int l = 0; l < sl; ++l) {
-    if (p.fused) {
+    if (p.plan.cell == StepPlan::FUSED) {
       const int q = s & 1;
       LAS_TRY(launch_gen_cell_step(p.maps[l], q, p.gp->bias[l], p.c + (size_t)l * B * Hs, hp + (size_t)l * B * Hs, Hs, hn + (size_t)l * B * Hs, Hs,
                                    p.abuf[l][q ^ 1] + gg.Kxp[l], gg.Kp[l], l + 1 < sl ? p.abuf[l + 1][q] : nullptr, l + 1 < sl ? gg.Kp[l + 1] : 0, B,
                                    Hs, d->cell, gg.Kxp[l], gg.Kp[l], true, p.f16, st, l));
       continue;
     }
-    if (p.gp) {
+    if (p.plan.cell != StepPlan::F32) {
       const float* xin_l = (l == 0) ? p.xin : hn + (size_t)(l - 1) * B * Hs;
       const float* hp_l = hp + (size_t)l * B * Hs;
       LAS_TRY(launch_gen_build_a(xin_l, (l == 0) ? xld : Hs, hp_l, Hs, p.a, B, Hs, gg.Kx[l], gg.Kxp[l], gg.Kp[l], p.f16, st));
-      if (B <= 64) {
+      if (p.plan.cell == StepPlan::SWAPPED) {
         // Small batches: the GEMM's 128 x 256 tiles would leave it R/256 CTAs (16 at R = 4096), each streaming 1 MB of weights.  With
         // the operands swapped -- "M" = the R weight rows, "N" = the batch -- R/128 CTAs stream half as much each; the result arrives
         // transposed ([R, B]) and the cell kernel adds the bias.
@@ -539,12 +558,9 @@ static int speller_step(const StepPath& p, int s, const float* hp, float* hn, co
     a.hout_ld = Hs;
     LAS_TRY(launch_lstm_cell_f32(&a, 1, B, Hs, st, d->cell));
   }
-  if (p.cluster_att) return launch_attend_cluster(t, p.gp != nullptr, st);
+  if (p.plan.cluster_att) return launch_attend_cluster(t, p.plan.C, p.gp != nullptr, st);
   return launch_attend_f32(t, st);
 }
-// The attention kernel of greedy decoding and of beam search: the cluster kernel is plain fp32 arithmetic, so the fp32 mode uses it
-// as well; multi-head attention keeps the one-CTA kernel.
-static bool cluster_attention(const las_speller_dims* d) { return n_heads(d) == 1 && d->E % 4 == 0 && debug_options().gen_fused; }
 
 static int speller_decode_f32(const las_decode_io* io, const las_speller_dims* d, const SpellerLayout& L, int steps, int decode_mode, int relu,
                               cudaStream_t st) {
@@ -584,10 +600,10 @@ static int speller_decode_f32(const las_decode_io* io, const las_speller_dims* d
 
   // Fused generic step (gen_step.cu): per layer the 16-bit operand rows [x | h_prev] of even / odd steps live in abuf[l][parity]; the
   // kernels that produce x and h write them there directly.  Step 0's rows are built from the initial state here.
-  const bool fused = gen && debug_options().gen_fused && B <= 256;
+  const StepPlan plan = step_plan(d, B, L, false, io->enc);
   GenStepMaps maps[8];
   __nv_bfloat16* abuf[8][2];
-  if (fused) {
+  if (plan.cell == StepPlan::FUSED) {
     LAS_CUDA_OK(cudaMemsetAsync(gw.a2, 0, sizeof(__nv_bfloat16) * (size_t)sl * 2 * B * gg.Kp_max, st));
     for (int l = 0; l < sl; ++l) {
       for (int q = 0; q < 2; ++q) abuf[l][q] = gw.a2 + (size_t)(l * 2 + q) * B * gg.Kp_max;
@@ -598,9 +614,9 @@ static int speller_decode_f32(const las_decode_io* io, const las_speller_dims* d
   }
 
   StepPath path;
-  path.d = d; path.rows = B; path.pk = pk; path.gp = gen ? &gp : nullptr; path.f16 = L.f16; path.gg = gg;
+  path.d = d; path.rows = B; path.plan = plan; path.pk = pk; path.gp = gen ? &gp : nullptr; path.f16 = L.f16; path.gg = gg;
   path.a = gw.a; path.pre = gw.pre; path.zero = gw.zero; path.xin = w.xin; path.c = w.c;
-  path.fused = fused; path.maps = maps; path.abuf = abuf; path.cluster_att = cluster_attention(d);
+  path.maps = maps; path.abuf = abuf;
   ProfScope ps_steps("speller.steps", st);
   for (int s = 0; s < steps; ++s) {
     float* hp = w.h[s & 1];
@@ -624,7 +640,7 @@ static int speller_decode_f32(const las_decode_io* io, const las_speller_dims* d
       t.nll_label_step = (io->nll_labels && s < io->nll_steps) ? io->nll_labels + s : nullptr;
       t.nll_label_ld = io->nll_steps;
     }
-    if (fused) {
+    if (plan.cell == StepPlan::FUSED) {
       t.op_out = abuf[0][(s & 1) ^ 1];
       t.op_ld = gg.Kp[0];
       t.op_f16 = L.f16;
@@ -717,8 +733,6 @@ static int speller_beam_f32(const las_beam_io* io, const las_speller_dims* d, co
   const SpellerPackGen& gp = L.gp;
   const BeamWs w = beam_ws_layout(d, steps, K, gen, ws);
   if (gen) LAS_CUDA_OK(cudaMemsetAsync(w.zero, 0, sizeof(float) * 256, st));
-  las_speller_dims dk = *d;  // the decoder sees B*K rows
-  dk.B = BK;
 
   int status;
   const float* psi = speller_psi(d, B, pk, gen ? &gp : nullptr, io->enc, w.psi, w.enc16, relu, L.f16, st, &status);  // once per utterance
@@ -728,11 +742,10 @@ static int speller_beam_f32(const las_beam_io* io, const las_speller_dims* d, co
   LAS_CUDA_OK(cudaMemsetAsync(w.h[0], 0, sizeof(float) * state_n, st));
   LAS_CUDA_OK(cudaMemsetAsync(w.c, 0, sizeof(float) * state_n, st));
 
-  StepPath path;
-  memset(&path, 0, sizeof(path));
-  path.d = &dk; path.rows = BK; path.pk = pk; path.gp = gen ? &gp : nullptr; path.f16 = L.f16; path.gg = gen_geom(d);
+  StepPath path = {};
+  path.d = d; path.rows = BK; path.plan = step_plan(d, BK, L, true, io->enc); path.pk = pk; path.gp = gen ? &gp : nullptr;
+  path.f16 = L.f16; path.gg = gen_geom(d);
   path.a = w.a; path.pre = w.pre; path.zero = w.zero; path.xin = w.xin; path.c = w.c;
-  path.cluster_att = cluster_attention(d);
   BeamStepArgs ba;
   memset(&ba, 0, sizeof(ba));
   ba.logp = w.logp; ba.score = w.score; ba.fin = w.fin;

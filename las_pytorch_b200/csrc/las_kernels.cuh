@@ -75,8 +75,9 @@ struct AttendArgs {
   long long* trace;               // nullable test hook (attend_cluster_kernel): clock64 stamps of CTA 0
 };
 int launch_attend_f32(const AttendArgs& a, cudaStream_t st);
-// same step, heads == 1: a cluster of up to 8 CTAs per utterance (gen_step.cu); pdl = programmatic dependent launch
-int launch_attend_cluster(const AttendArgs& a, bool pdl, cudaStream_t st);
+// same step, heads == 1: a cluster of C = 1 / 2 / 4 / 8 CTAs per utterance (gen_step.cu); pdl = programmatic dependent launch
+constexpr int AC_THREADS = 512;  // its threads read 16-byte aligned encoder rows four features each: E <= 4 * AC_THREADS
+int launch_attend_cluster(const AttendArgs& a, int C, bool pdl, cudaStream_t st);
 
 // xin[b, 0:V] = onehot(0), xin[b, V:V+E] = enc[b, 0, :]   (model/las_model.py:193-198)
 int launch_speller_init(float* xin, int xin_ld, const float* enc, int B, int U, int E, int V, cudaStream_t st);
