@@ -272,8 +272,9 @@ int las_speller_beam_search(const las_beam_io* io, const void* packed, const las
  * Cross-batch serving pipeline.  One call stands for `las_speller_decode` of batch i AND `las_listener_forward[_masked]` of batch
  * i+1 (the two calls LAS.forward makes, model/las_model.py:31-39, for two consecutive batches) and produces exactly their
  * results.  In LAS_MODE_BF16, when the listener's recurrence fits on the SMs the persistent decoder leaves free, the two run
- * CONCURRENTLY: the decoder's step loop is cut into L segments, each layer's recurrence of the next batch runs next to one segment
- * and its input-projection GEMM alone on the chip between two segments (csrc/fast_pipeline.cu).  Otherwise (fp32 mode, variants,
+ * CONCURRENTLY: where those SMs also leave room for the input-projection GEMMs, the whole listener of the next batch runs beside ONE
+ * decoder launch; otherwise the decoder's step loop is cut into L segments, each layer's recurrence runs next to one segment and its
+ * GEMM alone on the chip between two segments (csrc/fast_pipeline.cu; debug key 31 forces the latter).  Otherwise (fp32 mode, variants,
  * no free SMs, early_exit) the two are simply enqueued one after the other.  dec_io == NULL: encode only; x == NULL: decode only.
  * `las_pipeline_overlaps` tells whether the concurrent schedule applies to a pair of shapes.
  * ------------------------------------------------------------------------------------------------------ */
@@ -339,7 +340,12 @@ int las_debug_set_trace(void* dev_buf);
  *           for the attention) or as separate GEMM / cell / operand kernels with one attention CTA per utterance (0);
  *   key 13: CTAs per utterance of that attention cluster (1 / 2 / 4 / 8; 0 = by batch size);
  *   key 19: two utterance groups pipelined through the persistent decoder's LSTM CTAs (1, default) or the whole batch in lockstep (0);
- *   keys 20 + l (l < 8): decoder steps of the serving pipeline's segment l (>= 0; 0 = proportional to the layer's time steps). */
+ *   keys 20 + l (l < 8): decoder steps of the serving pipeline's segment l (>= 0; 0 = proportional to the layer's time steps);
+ *   key 30: hidden units per LSTM CTA of the persistent decoder (0, default: 32 for the decoder launch the serving pipeline runs beside
+ *           the next batch's listener, 16 otherwise; 16; 32 -- a launch of more than 32
+ *           utterances in lockstep, key 19 = 0, then returns LAS_EINVAL);
+ *   key 31: serving pipeline schedule (1, default: the listener beside one decoder launch where the chip has room for it, segmented
+ *           otherwise; 0: always segmented). */
 int las_debug_set_option(int key, int value);
 
 #ifdef __cplusplus

@@ -682,7 +682,7 @@ int fast_listener_rec_ctas(const las_listener_dims* d, int bc) {
 }
 
 int fast_listener_stage(const float* x, const int32_t* x_lengths, const void* packed, const las_listener_dims* d, float* enc,
-                        int32_t* enc_lengths, void* ws, int stage, int bc, int* resident, bool f16, cudaStream_t st) {
+                        int32_t* enc_lengths, void* ws, int stage, int bc, int* resident, int max_ctas, bool f16, cudaStream_t st) {
   LAS_TRY(shape_ok(d));
   const Geo g = geometry(d->H);
   const ListenerPackFast pk = pack_layout(d, const_cast<void*>(packed));
@@ -699,7 +699,7 @@ int fast_listener_stage(const float* x, const int32_t* x_lengths, const void* pa
     if (fuse_x(d, l)) return LAS_OK;  // the recurrence does the projection itself
     snprintf(nm, sizeof(nm), "listener.L%d.input_gemm", l);
     ProfScope ps(nm, st);
-    return launch_gemm_listener(q.in, d->B, q.Tl, q.K, pk.wih[l], pk.bias[l], w.P, q.NP, nullptr, 0, f16, st);
+    return launch_gemm_listener(q.in, d->B, q.Tl, q.K, pk.wih[l], pk.bias[l], w.P, q.NP, nullptr, max_ctas, f16, st);
   }
   RecParams rp = rec_params(d, g, pk, w, l, enc, x_lengths ? w.len + (size_t)l * d->B : nullptr, bc, f16);
   rp.resident = resident;
@@ -729,7 +729,7 @@ int fast_listener_forward(const float* x, const int32_t* x_lengths, const void* 
   const ListenerPackFast pk = pack_layout(d, const_cast<void*>(packed));
   const ListenerWsFast w = ws_layout(d, ws);
   const int B = d->B;
-  LAS_TRY(fast_listener_stage(x, x_lengths, packed, d, enc, enc_lengths, ws, 0, 0, nullptr, f16, st));
+  LAS_TRY(fast_listener_stage(x, x_lengths, packed, d, enc, enc_lengths, ws, 0, 0, nullptr, 0, f16, st));
   for (int l = 0; l < d->L; ++l) {
     const LayerGeom q = layer_geom(d, g, w, l);
     const int32_t* len_l = nullptr;

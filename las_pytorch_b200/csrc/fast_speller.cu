@@ -39,7 +39,7 @@ int make_tmap_bf16_atoms(CUtensorMap* tm, const void* base, long long rows, int 
 
 namespace {
 
-constexpr int DEC_NW = 64;        // gate columns per LSTM CTA (16 hidden units x 4 gates)
+constexpr int DEC_NW = 64;        // gate columns per block of the packed image (16 hidden units x 4 gates)
 constexpr int DEC_UNITS = DEC_NW / 4;
 constexpr int DEC_MAX_STAGES = 16;
 constexpr int DEC_THREADS = 512;
@@ -56,8 +56,8 @@ struct DecParams {
   CUtensorMap tm_w[2];          // wbuf[parity]     bf16 [B, VP]  the dense word fed to layer 0 (one atom)
   CUtensorMap tm_h3[MAX_SL][2]; // the same buffers as {64 k, B, atoms}: one copy brings a whole activation part (set where Hs % 64 == 0)
   CUtensorMap tm_x3[2];
-  const uint8_t* w_img[MAX_SL]; // [ncl][atoms_l] swizzled 64x64 bf16 atoms: h part, (layer 0: word atom), input part
-  const float* bias[MAX_SL];    // [ncl*64] b_ih + b_hh in CTA column order
+  const uint8_t* w_img[MAX_SL]; // [Hs/16][atoms_l] swizzled 64x64 bf16 atoms: h part, (layer 0: word atom), input part
+  const float* bias[MAX_SL];    // [4*Hs] b_ih + b_hh in unit-major / gate-minor order
   __nv_bfloat16* hbuf[MAX_SL][2];
   __nv_bfloat16* xbuf[2];
   __nv_bfloat16* wbuf[2];
@@ -105,6 +105,7 @@ struct DecParams {
   int ctx_ntm;      // 128-feature tiles of enc[b]^T held in tensor memory: E/128 = all of them; fewer (long encoders, e.g. U = 375:
                     // 2 of 4) = hybrid, the remaining features are reduced on the CUDA cores from the L2-resident bf16 copy
   int groups, gsz;  // utterance groups pipelined through the LSTM CTAs (1, or 2 groups of gsz = 32 rows) -- see lstm_role_ts
+  int units;        // hidden units per LSTM CTA (16 or 32; lstm_plan); ncl = ceil(Hs / units)
   int nstages, stage_bytes;  // activation slots: [64 batch rows x 64 bf16], 128-byte swizzled; last slot = word atom
   long long* trace;  // nullable test hook (TRACE_DEC): [5 roles][32 steps][8] globaltimer stamps (layer-0 CTA 0, top-layer CTA 0, attention CTA 0, ...)
 };
@@ -202,11 +203,14 @@ __device__ __forceinline__ float dot8(const uint4& w, const float4& x0, const fl
 // operands come from shared memory (tools/microbench.cu: the shared-memory A read is exposed).  The part's 32 instructions take
 // ~0.55 us of each layer's critical path instead of ~1.05 us.  The own-h part (ready long before it is needed) takes both operands
 // from shared memory, in the same roles, so both parts land in accumulators of the same orientation.
-// M = 128 although a CTA owns only 64 gate rows: lanes 64..127 hold zeros / read the atom behind (the instruction costs the same
-// for M = 64 and 128), which keeps the plain lane = row layout.
+// M = 128 always.  A CTA owns 16 units (64 gate rows; lanes 64..127 hold zeros, the instruction costs the same for M = 64 and 128)
+// or 32 units (128 gate rows, every lane used: half as many CTAs for the same MMAs per step).  A 32-unit CTA n is built from the
+// 16-unit packed image: rows 0..63 of each [128 rows x 64 k] atom are that atom of image block 2n, rows 64..127 that of block 2n+1
+// (zeros past Hs) -- in the 128-byte-swizzled layout simply the two 8 KB halves of a 16 KB atom.
 // Epilogue: thread = gate row (lane; unit-major / gate-minor, so the four gates of a unit sit in four adjacent lanes), 16 batch
 // columns per warp; a 4x4 transpose inside each 4-lane group (two shuffle stages, as in the listener's recurrence) leaves every
-// lane with (i, f, g, o) of one (unit, batch) cell -- 4 cells per thread, cell state in registers.
+// lane with (i, f, g, o) of one (unit, batch) cell -- 4 cells per thread and iteration, cell state in registers.  Eight epilogue
+// warps cover the TMEM lane quadrants the CTA's rows occupy (2 or 4) x the 16-column slices (4 or 2).
 template <int F16>
 __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -214,22 +218,29 @@ __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
   const int nh = (p.Hs + 63) / 64;
   const int nc = first ? (p.E + 63) / 64 : (p.Hs + 63) / 64;
   const int nwd = first ? 1 : 0;
-  const int natoms = nh + nwd + nc;
+  const int natoms = nh + nwd + nc;                      // atoms of one image block
+  const int UNITS = p.units, ROWS = 4 * UNITS, HALVES = UNITS / DEC_UNITS, nblk = p.Hs / DEC_UNITS;
+  const int ST_PITCH = UNITS + 4;                        // staging row pitch (floats): 16-byte aligned, conflict-free reads
   const int NBUF = p.nstages, STAGE_BYTES = p.stage_bytes;
   const int wslot = NBUF - 1;
-  uint8_t* abuf = smem;                                  // NBUF x STAGE_BYTES activation slots ([64 batch rows x 64 k], SW128)
-  uint8_t* wsm = abuf + (size_t)NBUF * STAGE_BYTES;      // natoms x 8 KB weight atoms ([64 gate rows x 64 k], SW128)
-  float* bias_s = reinterpret_cast<float*>(wsm + (size_t)natoms * WATOM_BYTES);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(bias_s + DEC_NW);
+  // shared-memory weight atom: [ROWS gate rows x 64 k], SW128.  The M = 128 MMAs of a 16-unit CTA read 128 rows: lanes 64..127 take
+  // the 8 KB behind each atom (the next atom, or a zero pad behind the last one) and are never read back.
+  const int SATOM = ROWS * 128, WPAD = HALVES == 1 ? WATOM_BYTES : 0;
+  uint8_t* abuf = smem;                                  // NBUF x STAGE_BYTES activation slots ([gsz batch rows x 64 k], SW128)
+  uint8_t* wsm = abuf + (size_t)NBUF * STAGE_BYTES;      // (nh + nwd) weight atoms: own-h part, (layer 0) word atom; + WPAD
+  float* bias_s = reinterpret_cast<float*>(wsm + (size_t)(nh + nwd) * SATOM + WPAD);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(bias_s + ROWS);
   uint64_t* full = bars;
   uint64_t* part_empty = bars + DEC_MAX_STAGES;
   uint64_t* tmem_full = part_empty + 1;
   uint64_t* tmem_empty = tmem_full + 1;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_empty + 1);
-  float* s_st = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(tmem_slot + 2) + 15) & ~uintptr_t(15));  // [64 batch rows][20]
+  float* s_st = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(tmem_slot + 2) + 15) & ~uintptr_t(15));  // [64 batch rows][ST_PITCH]
   constexpr int EPI_WARPS = 8, EPI_THREADS = EPI_WARPS * 32, PROD_WARP = 2, MMA_WARP = 3;
   // tensor-memory map: critical weights [0, nc*32), accumulator of the own-h part, accumulator of the critical part (64 columns each)
   const uint32_t a_cols = (uint32_t)nc * 32u, acc0 = a_cols, acc1 = a_cols + 64u;
+  // image block of the CTA's row half hf (rows [64 hf, 64 hf + 64)), or -1: no such half / past Hs (zeros)
+  auto src_block = [&](int hf) { const int b = nb * HALVES + hf; return (hf < HALVES && b < nblk) ? b : -1; };
 
   if (threadIdx.x == 0) {
     for (int i = 0; i < NBUF; ++i) ptx::mbar_init(&full[i], 1);
@@ -239,11 +250,14 @@ __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
     ptx::fence_mbar_init();
   }
   if (warp == MMA_WARP) ptx::tmem_alloc(tmem_slot, 512);
-  {  // weight slice + bias -> shared memory
-    const uint4* src = reinterpret_cast<const uint4*>(p.w_img[l] + (size_t)nb * natoms * WATOM_BYTES);
-    uint4* dst = reinterpret_cast<uint4*>(wsm);
-    for (int i = threadIdx.x; i < natoms * WATOM_BYTES / 16; i += DEC_THREADS) dst[i] = src[i];
-    if (threadIdx.x < DEC_NW) bias_s[threadIdx.x] = p.bias[l][nb * DEC_NW + threadIdx.x];
+  {  // own-h (+ word) atoms + bias -> shared memory, each atom from HALVES 8 KB image atoms (a 32-unit CTA: two), then the pad
+    const uint4 z = make_uint4(0, 0, 0, 0);
+    for (int i = threadIdx.x; i < ((nh + nwd) * SATOM + WPAD) / 16; i += DEC_THREADS) {
+      const int a = i / (SATOM / 16), hf = (i / (WATOM_BYTES / 16)) % HALVES, o = i % (WATOM_BYTES / 16);
+      const int b = a < nh + nwd ? src_block(hf) : -1;
+      reinterpret_cast<uint4*>(wsm)[i] = b >= 0 ? reinterpret_cast<const uint4*>(p.w_img[l] + ((size_t)b * natoms + a) * WATOM_BYTES)[o] : z;
+    }
+    if (threadIdx.x < ROWS) bias_s[threadIdx.x] = nb * ROWS + threadIdx.x < 4 * p.Hs ? p.bias[l][nb * ROWS + threadIdx.x] : 0.f;
   }
   ptx::fence_proxy_async();
   ptx::tc_fence_before();
@@ -251,15 +265,15 @@ __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
   ptx::tc_fence_after();
   const uint32_t tmem = *tmem_slot;
   if (warp < 4) {
-    // critical-part weights: shared-memory atoms (128-byte swizzle undone) -> tensor memory, lane = gate row, two bf16 per column
-    const int row = warp * 32 + lane;
-    const uint8_t* wc = wsm + (size_t)(nh + nwd) * WATOM_BYTES;
+    // critical-part weights: global image atoms (128-byte swizzle undone) -> registers -> tensor memory, lane = gate row, two bf16 per
+    // column.  Not staged in shared memory: a 32-unit CTA's 8 atoms of 16 KB would not fit next to the own-h part.
+    const int row = warp * 32 + lane, r64 = row & 63, b = src_block(row >> 6);
     for (int i = 0; i < nc; ++i) {
-      const uint8_t* rb = wc + (size_t)i * WATOM_BYTES + (row >> 3) * 1024 + (row & 7) * 128;
+      const uint8_t* rb = p.w_img[l] + ((size_t)(b < 0 ? 0 : b) * natoms + nh + nwd + i) * WATOM_BYTES + (r64 >> 3) * 1024 + (r64 & 7) * 128;
 #pragma unroll
       for (int kk = 0; kk < 4; ++kk) {
         uint4 q0 = make_uint4(0, 0, 0, 0), q1 = q0;
-        if (row < DEC_NW) {
+        if (b >= 0) {
           q0 = *reinterpret_cast<const uint4*>(rb + (((2 * kk) ^ (row & 7)) << 4));
           q1 = *reinterpret_cast<const uint4*>(rb + (((2 * kk + 1) ^ (row & 7)) << 4));
         }
@@ -277,7 +291,7 @@ __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
   // attention -> layer 0) and with the whole batch in lockstep every stage idles two thirds of the time.  The LSTM CTAs therefore serve
   // the groups alternately -- iteration it = s * groups + grp -- with per-group counters, 32-row activation boxes and N = 32 MMAs, while
   // the attention CTAs (one per utterance anyway) simply follow their group's counters.  Every buffer is indexed by utterance row, a
-  // thread's cells all belong to one group, and an output column's sum does not depend on N: bit-identical to groups = 1.
+  // cell's state stays with one thread, and an output column's sum does not depend on N: bit-identical to groups = 1.
   const int G = p.groups, GSZ = p.gsz;
   const int trole = (nb == 0 && l == 0) ? 0 : ((nb == 0 && top) ? 1 : -1);
 
@@ -347,8 +361,8 @@ __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
     }
   } else if (warp == MMA_WARP) {
     // ============================ MMA issuer ============================
-    const UmmaLayout lact{1, 0, 1024, (uint32_t)STAGE_BYTES}, lw{1, 0, 1024, WATOM_BYTES};
-    const uint32_t idesc = umma_idesc_bf16(128, (uint32_t)GSZ, F16);  // M = 128 gate-row lanes (64 used), N = the group's batch columns
+    const UmmaLayout lact{1, 0, 1024, (uint32_t)STAGE_BYTES}, lw{1, 0, 1024, (uint32_t)SATOM};
+    const uint32_t idesc = umma_idesc_bf16(128, (uint32_t)GSZ, F16);  // M = 128 gate-row lanes (ROWS used), N = the group's batch columns
     const uint32_t a0 = ptx::smem_u32(abuf), w_addr = ptx::smem_u32(wsm);
     uint32_t phase0 = 0, phasew = 0;
     for (int it = 0; it < S * G; ++it) {
@@ -364,7 +378,7 @@ __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
         for (int i = 0; i < nh; ++i) {
 #pragma unroll
           for (int k = 0; k < 4; ++k)
-            ptx::umma_bf16(tmem + acc0, umma_smem_desc(lw, w_addr + i * WATOM_BYTES, k * 16), umma_smem_desc(lact, a0 + i * STAGE_BYTES, k * 16),
+            ptx::umma_bf16(tmem + acc0, umma_smem_desc(lw, w_addr + i * SATOM, k * 16), umma_smem_desc(lact, a0 + i * STAGE_BYTES, k * 16),
                            idesc, !(i == 0 && k == 0));
         }
         ptx::umma_commit(part_empty);
@@ -404,7 +418,7 @@ __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
         if (ptx::elect_one()) {
 #pragma unroll
           for (int k = 0; k < 4; ++k)
-            ptx::umma_bf16(tmem + acc1, umma_smem_desc(lw, w_addr + nh * WATOM_BYTES, k * 16), umma_smem_desc(lact, a0 + wslot * STAGE_BYTES, k * 16),
+            ptx::umma_bf16(tmem + acc1, umma_smem_desc(lw, w_addr + nh * SATOM, k * 16), umma_smem_desc(lact, a0 + wslot * STAGE_BYTES, k * 16),
                            idesc, 1u);
           ptx::umma_commit(part_empty);
           ptx::umma_commit(tmem_full);
@@ -413,29 +427,42 @@ __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
       }
       if (lane == 0 && trole >= 0 && grp == 0) DEC_TRACE(trole, 2);
     }
-  } else if ((warp & 3) < 2) {
+  } else if (UNITS == DEC_UNITS ? (warp & 3) < 2 : (warp >= 4 && warp < 4 + EPI_WARPS)) {
     // ============================ epilogue: gates, cell state, h ============================
-    const int q = warp & 3, cs = warp >> 2;        // TMEM lane quadrant (gate rows 32q..32q+31), batch slice [16cs, 16cs+16)
+    // 16 units: warps with quadrant 0 / 1 (rows 0..63) x 4 slices = 64 columns (the whole batch, or both groups side by side);
+    // 32 units: warps 4..11, two per quadrant (the producer and MMA warps sit in quadrants 2 and 3) x 2 slices = the 32 columns of
+    // the group being served, so every thread keeps the cells of both groups
+    const int NQ = ROWS / 32, NS = EPI_WARPS / NQ;  // TMEM lane quadrants, 16-column slices
+    const int q = warp & 3, cs = UNITS == DEC_UNITS ? warp >> 2 : (warp >> 2) - 1;  // gate rows 32q..32q+31, slice cs
     const int row = q * 32 + lane;                 // gate row of this CTA = 4 * unit + gate
     const int jj = row >> 2, g = row & 3;
     const bool bit0 = (g & 1) != 0, bit1 = (g & 2) != 0;
-    const int u = nb * DEC_UNITS + jj;             // hidden unit
-    const bool lead = (warp == 0 && lane == 0);
-    const bool warp_has_rows = cs * 16 < p.B;
-    const int my_grp = (cs * 16) / GSZ;           // the group this thread's cells belong to
-    const uint32_t acc_col = (uint32_t)(cs * 16 - my_grp * GSZ);
-    float c[4];
-    int bm[4];
+    const int u = nb * UNITS + jj;                 // hidden unit
+    const bool unit_ok = u < p.Hs;                 // (the upper half of the last 32-unit CTA where Hs % 32 == 16)
+    const bool lead = (warp == (UNITS == DEC_UNITS ? 0 : 4) && lane == 0);
+    const int spg = GSZ / 16, per = NS / spg;      // slices per group; groups the slices serve side by side (1 or 2)
+    const int sg = cs / spg, cw = cs % spg;        // the slice serves groups grp with grp % per == sg, columns [16cw, 16cw+16) of them
+    const uint32_t acc_col = (uint32_t)(cw * 16);
+    const int CPR = UNITS / 8, RPW = 16 / CPR;     // hand-off: 16-byte chunks per row, rows per warp
+    float c[2][4];                                 // cell state, slot k = grp / per
 #pragma unroll
-    for (int m = 0; m < 4; ++m) {
-      bm[m] = cs * 16 + 4 * m + g;                 // this thread's cell m: (unit u, batch bm[m])
-      c[m] = (bm[m] < p.B && p.c_init) ? p.c_init[((size_t)l * p.c_init_rows + p.c_init_b0 + bm[m]) * p.Hs + u] : 0.f;
+    for (int k = 0; k < 2; ++k) {
+      const int grp = k * per + sg;
+#pragma unroll
+      for (int m = 0; m < 4; ++m) {
+        const int b = grp * GSZ + cw * 16 + 4 * m + g;
+        c[k][m] = (grp < G && b < p.B && unit_ok && p.c_init) ? p.c_init[((size_t)l * p.c_init_rows + p.c_init_b0 + b) * p.Hs + u] : 0.f;
+      }
     }
     const float4 bias4 = *reinterpret_cast<const float4*>(bias_s + 4 * jj);
-    const uint8_t* watom = wsm + (size_t)nh * WATOM_BYTES;  // layer 0: word atom [64 gate rows x 64 vocabulary entries]
+    const uint8_t* watom = wsm + (size_t)nh * SATOM;  // layer 0: word atom [ROWS gate rows x 64 vocabulary entries]
     for (int it = 0; it < S * G; ++it) {
-      const int s = it / G, grp = it - s * G;
-      const bool warp_live = warp_has_rows && grp == my_grp;
+      const int s = it / G, grp = it - s * G, k = grp / per;
+      const int bw = grp * GSZ + cw * 16;          // first batch row of this warp's slice
+      const bool warp_live = grp % per == sg && bw < p.B;
+      int bm[4];
+#pragma unroll
+      for (int m = 0; m < 4; ++m) bm[m] = bw + 4 * m + g;  // this thread's cell m: (unit u, batch bm[m])
       uint32_t* my_ready = counter(p, l, grp);
       // bias + (index word) the token's column of W_word for this unit's four gate rows, per cell -- before the accumulators are ready.
       // The warp's 16 batches are polled by 16 lanes (ONE L2 round trip; four dependent polls per thread cost ~2.4 us and made the
@@ -444,7 +471,7 @@ __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
       int tokl = -1;
       const bool gather = first && p.s0 + s > 0 && p.word_gather && warp_live;
       if (gather) {
-        const int bb = cs * 16 + (lane & 15);
+        const int bb = bw + (lane & 15);
         if (bb < p.B)
           tokl = p.gt_index ? p.gt_index[(size_t)(p.b0 + bb) * p.gt_steps + (p.s0 + s - 1)]
                             : (s > 0 ? (int)ll_wait(p.tok_ll + (size_t)nb * p.B + bb, (uint32_t)s) : p.tok_init[bb]);
@@ -470,7 +497,7 @@ __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
       if (lead && trole >= 0 && grp == 0) DEC_TRACE(trole, 3);
       if (lead && grp == 0) DEC_TRACE_ALL(1);
       ptx::tc_fence_after();
-      float h[4] = {0.f, 0.f, 0.f, 0.f};
+      float h[4] = {0.f, 0.f, 0.f, 0.f}, cc[4];
       if (warp_live) {
         uint32_t x0[16], x1[16];
         ptx::tmem_ld_32x32b_x16(tmem + ((uint32_t)(q * 32) << 16) + acc0 + acc_col, x0);
@@ -495,19 +522,21 @@ __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
             v1 = bit1 ? r13 : v1; v3 = bit1 ? v3 : r13;
           }
           const float pi = v0 + pb[m].x, pf = v1 + pb[m].y, pg = v2 + pb[m].z, po = v3 + pb[m].w;
-          const float cn = sigmoid_fast(pf) * c[m] + sigmoid_fast(pi) * tanh_fast(pg);
-          c[m] = cn;
+          const float cn = sigmoid_fast(pf) * (k ? c[1][m] : c[0][m]) + sigmoid_fast(pi) * tanh_fast(pg);
+          if (k) c[1][m] = cn;
+          else c[0][m] = cn;
+          cc[m] = cn;
           h[m] = sigmoid_fast(po) * tanh_fast(cn);
         }
       }
       ptx::tc_fence_before();
       ptx::mbar_arrive(tmem_empty);
       const int np = (s + 1) & 1;
-      // hand-off: the 64 x 16 block through shared memory ([batch row][20 floats], conflict-free 16-byte reads), then every warp
-      // writes 8 whole rows of the bf16 operand copy (full 32-byte sectors instead of one partial sector per batch row)
+      // hand-off: the block through shared memory ([batch row][UNITS + 4 floats], conflict-free 16-byte reads), then every warp
+      // writes RPW whole rows of the bf16 operand copy (full 32-byte sectors instead of one partial sector per batch row)
       // top layer: the {h, tag} slots the attention CTAs poll leave straight from the registers, before the staging barrier
       // (0.11 us/step faster than staged whole-row stores)
-      if (top && warp_live) {
+      if (top && warp_live && unit_ok) {
         const uint32_t tag = (uint32_t)(s + 1);
 #pragma unroll
         for (int m = 0; m < 4; ++m)
@@ -515,27 +544,28 @@ __device__ void lstm_role_ts(const DecParams& p, uint8_t* smem, int l, int nb) {
       }
       if (warp_live) {
 #pragma unroll
-        for (int m = 0; m < 4; ++m) s_st[bm[m] * 20 + jj] = h[m];
+        for (int m = 0; m < 4; ++m) s_st[bm[m] * ST_PITCH + jj] = h[m];
       }
       asm volatile("bar.sync 1, 256;" ::: "memory");
-      const int r0 = (cs * 2 + q) * 8;  // this warp's 8 rows
+      const int r0 = grp * GSZ + (cw * NQ + q) * RPW;  // this warp's rows
       if (lane < 16 && warp_live) {
-        const int rw = r0 + (lane >> 1), hf = lane & 1;
-        if (rw < p.B) {
-          const float4 y0 = *reinterpret_cast<const float4*>(s_st + rw * 20 + hf * 8), y1 = *reinterpret_cast<const float4*>(s_st + rw * 20 + hf * 8 + 4);
+        const int rw = r0 + lane / CPR, ch = lane % CPR, u0 = nb * UNITS + ch * 8;
+        if (rw < p.B && u0 < p.Hs) {
+          const float* y = s_st + rw * ST_PITCH + ch * 8;
+          const float4 y0 = *reinterpret_cast<const float4*>(y), y1 = *reinterpret_cast<const float4*>(y + 4);
           const __nv_bfloat162 t0 = op2_from_f32(y0.x, y0.y, F16), t1 = op2_from_f32(y0.z, y0.w, F16);
           const __nv_bfloat162 t2 = op2_from_f32(y1.x, y1.y, F16), t3 = op2_from_f32(y1.z, y1.w, F16);
-          *reinterpret_cast<uint4*>(p.hbuf[l][np] + (size_t)rw * p.Hs + nb * DEC_UNITS + hf * 8) =
+          *reinterpret_cast<uint4*>(p.hbuf[l][np] + (size_t)rw * p.Hs + u0) =
               make_uint4(*reinterpret_cast<const uint32_t*>(&t0), *reinterpret_cast<const uint32_t*>(&t1),
                          *reinterpret_cast<const uint32_t*>(&t2), *reinterpret_cast<const uint32_t*>(&t3));
         }
       }
-      if (s == S - 1 && warp_live) {
+      if (s == S - 1 && warp_live && unit_ok) {
 #pragma unroll
         for (int m = 0; m < 4; ++m) {
           if (bm[m] < p.B) {
             if (p.h_out) p.h_out[((size_t)l * p.Bfull + p.b0 + bm[m]) * p.Hs + u] = h[m];
-            if (p.c_out) p.c_out[((size_t)l * p.c_out_rows + p.c_out_b0 + bm[m]) * p.Hs + u] = c[m];
+            if (p.c_out) p.c_out[((size_t)l * p.c_out_rows + p.c_out_b0 + bm[m]) * p.Hs + u] = cc[m];
           }
         }
       }
@@ -1239,18 +1269,19 @@ __global__ void dec_init_kernel(DecParams p, const float* enc_f32, const float* 
       p.hbuf[l][0][(size_t)b * p.Hs + i] = op_from_f32(h_in ? h_in[((size_t)l * p.Bfull + gb) * p.Hs + i] : 0.f, p.f16);
 }
 
+// The packed image: Hs / 16 blocks of 16 units (a 32-unit LSTM CTA reads two of them)
 struct Shape {
-  int ncl, natoms[MAX_SL];
+  int nblk, natoms[MAX_SL];
   size_t w_bytes[MAX_SL];
 };
 Shape shape_of(const las_speller_dims* d) {
   Shape s;
-  s.ncl = d->Hs / DEC_UNITS;
+  s.nblk = d->Hs / DEC_UNITS;
   for (int l = 0; l < d->sl && l < MAX_SL; ++l) {
     const int nh = (d->Hs + 63) / 64;
     const int nx = (l == 0) ? (DEC_VP + d->E + 63) / 64 : (d->Hs + 63) / 64;
     s.natoms[l] = nh + nx;
-    s.w_bytes[l] = (size_t)s.ncl * s.natoms[l] * WATOM_BYTES;
+    s.w_bytes[l] = (size_t)s.nblk * s.natoms[l] * WATOM_BYTES;
   }
   return s;
 }
@@ -1258,24 +1289,41 @@ struct RingCfg {
   int box_rows, stage_bytes, nstages;
   size_t smem;
 };
-// ring geometry of a launch (64-row boxes; a launch with two utterance groups narrows them to 32 rows): as many stages as shared
-// memory allows (up to 12), so that a whole step's critical input can be in flight at once
-RingCfg ring_cfg(const las_speller_dims* d) {
-  const Shape s = shape_of(d);
-  int mx = 0;
-  for (int l = 0; l < d->sl; ++l) mx = s.natoms[l] > mx ? s.natoms[l] : mx;
+// shared memory of an LSTM CTA with `units` hidden units whose activation boxes have `rows` batch rows: the own-h (+ word) atoms of
+// 4 * units gate rows (+ the 8 KB pad of the 16-unit form), the bias, the barriers, the epilogue's staging block [64 rows][units + 4] and one ring slot per atom of the larger
+// streamed part (own h: ceil(Hs/64); context / lower h: ceil(E/64)) + the word slot, so that a whole step's critical input can be in
+// flight at once
+RingCfg ring_cfg(const las_speller_dims* d, int units, int rows) {
+  const int nh = (d->Hs + 63) / 64, nc0 = (d->E + 63) / 64;
   RingCfg r;
-  r.box_rows = 64;
-  r.stage_bytes = r.box_rows * 128;
-  const size_t fixed = (size_t)mx * WATOM_BYTES + DEC_NW * 4 + (DEC_MAX_STAGES + 4) * 8 + 64 + 64 * 20 * 4;  // + the epilogue's staging block
-  // one slot per atom of the larger shared part (own h: ceil(Hs/64); context / lower h: ceil(E/64)) + the word slot
-  int need = (d->Hs + 63) / 64;
-  const int nc0 = (d->E + 63) / 64;
-  if (nc0 > need) need = nc0;
-  r.nstages = need + 1;
+  r.box_rows = rows;
+  r.stage_bytes = rows * 128;
+  r.nstages = (nh > nc0 ? nh : nc0) + 1;
+  const size_t fixed = (size_t)(nh + 1) * units * 4 * 128 + (units == DEC_UNITS ? WATOM_BYTES : 0) + 4 * units * 4 + (DEC_MAX_STAGES + 4) * 8 + 64 + 64 * (units + 4) * 4;
   r.smem = fixed + (size_t)r.nstages * r.stage_bytes;
   return r;
 }
+// The form of the persistent decoder's LSTM CTAs for a launch of Bc utterances, decided here alone; the one reader of debug keys
+// 19 and 30.  More than 32 utterances go through as two utterance groups of 32 rows (key 19 = 0: in lockstep, 64-row boxes).  A CTA
+// can take 32 hidden units (128 gate rows: all lanes of its M = 128 MMAs) wherever one iteration serves at most 32 rows, so that the
+// epilogue's eight warps still cover one group with four cells per thread -- half the LSTM CTAs of the 16-unit form.  It does so only
+// for a launch that shares the chip with the next batch's listener (`beside`, fast_pipeline.cu), where the SMs it frees are what the
+// listener runs on.  A decoder alone keeps 16 units: there the 32-unit form measured slower at Hs = 512 (DESIGN.md 4a).
+struct LstmPlan {
+  int groups, gsz, units, ncl;
+};
+LstmPlan lstm_plan(const las_speller_dims* d, int Bc, bool beside) {
+  const DebugOptions& o = debug_options();
+  LstmPlan lp;
+  lp.groups = (Bc > 32 && o.dec_groups != 0) ? 2 : 1;
+  lp.gsz = (lp.groups == 2 || Bc <= 32) ? 32 : 64;
+  const bool wide = beside && lp.gsz <= 32 && ring_cfg(d, 32, lp.gsz).smem <= 224 * 1024;
+  lp.units = o.dec_units ? o.dec_units : (wide ? 32 : 16);
+  lp.ncl = (d->Hs + lp.units - 1) / lp.units;
+  return lp;
+}
+// the launch group size the plan is made for when the batch is split into several launches (fast_speller_max_group)
+int plan_rows(const las_speller_dims* d) { return d->B < 64 ? d->B : 64; }
 bool att_wreg(const las_speller_dims* d) { return d->D <= DEC_THREADS / 8 && d->Hs <= 512; }
 size_t att_smem(const las_speller_dims* d, bool k_in, bool hybrid = false, bool split = false) {
   return att_layout(d->Hs, d->E, split ? att_split_half(d->U) : d->U, d->D, d->V, k_in, att_wreg(d), hybrid, split).total + 64;
@@ -1295,9 +1343,9 @@ struct AttPlan {
   bool hybrid, k_in_smem, wreg;
   size_t smem;                   // the attention CTA's dynamic shared memory
 };
-AttPlan att_plan(const las_speller_dims* d) {
+AttPlan att_plan(const las_speller_dims* d, int n_lstm) {
   const DebugOptions& o = debug_options();
-  const int NT = d->E / 128, n_lstm = d->sl * (d->Hs / DEC_UNITS);
+  const int NT = d->E / 128;
   // Long encoders: when one CTA cannot hold all of enc[b]^T in tensor memory but half of the encoder steps fit (U <= 448 at E = 512),
   // a cluster of two CTAs attends each utterance (flash-decoding style partial softmax, combined through DSMEM) -- provided the LSTM
   // CTAs pair up (even count) and the chip has room for two attention CTAs per utterance.
@@ -1318,7 +1366,7 @@ int supported(const las_speller_dims* d) {
   LAS_REQUIRE(d->V <= DEC_VP, "LAS_MODE_BF16 speller supports vocabularies up to %d (V=%d)", DEC_VP, d->V);
   LAS_REQUIRE(d->E % 8 == 0 && d->E / 8 <= DEC_THREADS, "LAS_MODE_BF16 speller needs E %% 8 == 0 and E <= 4096 (E=%d)", d->E);
   LAS_REQUIRE(d->U <= ATT_MAXP * 256, "LAS_MODE_BF16 speller supports at most %d encoder steps (U=%d)", ATT_MAXP * 256, d->U);
-  LAS_REQUIRE(att_smem(d, false) <= 220 * 1024 && ring_cfg(d).smem <= 224 * 1024 && ring_cfg(d).nstages <= DEC_MAX_STAGES,
+  LAS_REQUIRE(att_smem(d, false) <= 220 * 1024 && ring_cfg(d, 16, 64).smem <= 224 * 1024 && ring_cfg(d, 16, 64).nstages <= DEC_MAX_STAGES,
               "LAS_MODE_BF16 speller: model does not fit shared memory (U=%d, Hs=%d)", d->U, d->Hs);
   return LAS_OK;
 }
@@ -1387,7 +1435,7 @@ SpellerWsFast ws_layout(const las_speller_dims* d, void* base) {
 // the generic layout.)
 bool fast_speller_fits(const las_speller_dims* d) {
   if (d->cell != LAS_CELL_LSTM || d->heads > 1 || d->no_mlp) return false;
-  const bool ok = supported(d) == LAS_OK && d->sl * (d->Hs / DEC_UNITS) + 1 <= sm_count();
+  const bool ok = supported(d) == LAS_OK && d->sl * lstm_plan(d, plan_rows(d), false).ncl + 1 <= sm_count();
   return ok;
 }
 
@@ -1400,7 +1448,7 @@ int fast_speller_pack(const las_speller_weights* w, const las_speller_dims* d, v
   const Shape s = shape_of(d);
   for (int l = 0; l < d->sl; ++l) {
     const las_lstm_weights& lw = w->rnn_host[l];
-    pack_dec_w_kernel<<<592, 256, 0, st>>>(lw.w_ih, lw.w_hh, pk.w_img[l], l, d->Hs, d->E, d->V, s.ncl, f16);
+    pack_dec_w_kernel<<<592, 256, 0, st>>>(lw.w_ih, lw.w_hh, pk.w_img[l], l, d->Hs, d->E, d->V, s.nblk, f16);
     LAS_LAUNCH_OK("pack_dec_w_kernel");
     pack_dec_bias_kernel<<<(4 * d->Hs + 255) / 256, 256, 0, st>>>(lw.b_ih, lw.b_hh, pk.bias[l], d->Hs);
     LAS_LAUNCH_OK("pack_dec_bias_kernel");
@@ -1418,9 +1466,10 @@ int fast_speller_pack(const las_speller_weights* w, const las_speller_dims* d, v
 // for every segment but the last), c and the fed-back token in the carry buffers.
 int fast_speller_decode_segment(const las_decode_io* io, const SpellerF32Inputs& f32, const void* packed_fast, const las_speller_dims* d,
                                 int b0, int Bc, int s_begin, int s_count, bool first_seg, bool last_seg, int decode_mode, int relu,
-                                void* ws_fast, bool f16, cudaStream_t st) {
-  const Shape s = shape_of(d);
-  const int n_lstm = d->sl * s.ncl;
+                                void* ws_fast, bool f16, bool beside, cudaStream_t st) {
+  const LstmPlan lp = lstm_plan(d, Bc, beside);
+  const int n_lstm = d->sl * lp.ncl;
+  LAS_REQUIRE(lp.units == 16 || lp.gsz <= 32, "32 hidden units per LSTM CTA need at most 32 rows per iteration (%d utterances in lockstep)", Bc);
   LAS_REQUIRE(last_seg || (s_count % 2 == 0), "decoder segments must have an even number of steps (%d)", s_count);
   LAS_REQUIRE(s_begin % 2 == 0, "decoder segments must start at an even step (%d)", s_begin);
   const SpellerPackFast pk = pack_layout(d, const_cast<void*>(packed_fast));
@@ -1433,15 +1482,14 @@ int fast_speller_decode_segment(const las_decode_io* io, const SpellerF32Inputs&
     DecParams p;
     memset(&p, 0, sizeof(p));
     p.B = Bc; p.U = d->U; p.E = d->E; p.Hs = d->Hs; p.sl = d->sl; p.V = d->V; p.D = d->D;
-    p.steps = s_count; p.s0 = s_begin; p.decode_mode = decode_mode; p.relu = relu; p.gt_steps = io->gt_steps; p.ncl = s.ncl;
-    const AttPlan ap = att_plan(d);
+    p.steps = s_count; p.s0 = s_begin; p.decode_mode = decode_mode; p.relu = relu; p.gt_steps = io->gt_steps; p.ncl = lp.ncl;
+    const AttPlan ap = att_plan(d, n_lstm);
     p.att_split = ap.split; p.ctx_ntm = ap.ntm; p.ctx_tmem = ap.ntm > 0; p.k_in_smem = ap.k_in_smem; p.wreg = ap.wreg;
-    RingCfg rc = ring_cfg(d);
-    // two utterance groups of 32 pipelined through the LSTM CTAs when the launch has more than 32 utterances
-    p.groups = (Bc > 32 && debug_options().dec_groups != 0) ? 2 : 1;
-    p.gsz = p.groups == 2 ? 32 : 64;
-    rc.box_rows = p.gsz;
-    rc.stage_bytes = rc.box_rows * 128;
+    const RingCfg rc = ring_cfg(d, lp.units, lp.gsz);
+    LAS_REQUIRE(rc.smem <= 224 * 1024, "LAS_MODE_BF16 speller: %d-unit LSTM CTAs do not fit shared memory (Hs=%d)", lp.units, d->Hs);
+    p.groups = lp.groups;
+    p.gsz = lp.gsz;
+    p.units = lp.units;
     p.nstages = rc.nstages;
     p.stage_bytes = rc.stage_bytes;
     // the LSTM CTAs fetch an activation part as one 3-D copy where its rows are whole 64-column atoms (E == Hs), else atom by atom
@@ -1537,11 +1585,15 @@ int fast_speller_decode_segment(const las_decode_io* io, const SpellerF32Inputs&
 int fast_speller_max_group(const las_speller_dims* d) {
   // utterances per persistent launch: one attention CTA each (two for split attention), and at most 64 (activation slots hold
   // 64 batch rows)
-  const int n = (sm_count() - d->sl * shape_of(d).ncl) / att_plan(d).split;
+  const int n_lstm = d->sl * lstm_plan(d, plan_rows(d), false).ncl;
+  const int n = (sm_count() - n_lstm) / att_plan(d, n_lstm).split;
   return n < 64 ? n : 64;
 }
 
-int fast_speller_ctas(const las_speller_dims* d) { return d->sl * shape_of(d).ncl + att_plan(d).split * d->B; }
+int fast_speller_ctas(const las_speller_dims* d, bool beside) {
+  const int n_lstm = d->sl * lstm_plan(d, d->B, beside).ncl;
+  return n_lstm + att_plan(d, n_lstm).split * d->B;
+}
 
 // Segment lengths: `seg` steps each (even), the remainder in the last one.  seg <= 0: one segment.
 static int next_segment(int s_begin, int steps, int seg) {
@@ -1552,8 +1604,7 @@ static int next_segment(int s_begin, int steps, int seg) {
 int fast_speller_decode(const las_decode_io* io, const SpellerF32Inputs& f32, const void* packed_fast, const las_speller_dims* d, int steps,
                         int decode_mode, int relu, void* ws_fast, bool f16, cudaStream_t st) {
   LAS_TRY(supported(d));
-  const Shape s = shape_of(d);
-  const int n_lstm = d->sl * s.ncl;
+  const int n_lstm = d->sl * lstm_plan(d, plan_rows(d), false).ncl;
   const int nsm = sm_count();
   LAS_REQUIRE(n_lstm + 1 <= nsm, "LAS_MODE_BF16 speller: %d LSTM CTAs do not fit %d SMs", n_lstm, nsm);
   const int max_b = fast_speller_max_group(d);
@@ -1570,7 +1621,7 @@ int fast_speller_decode(const las_decode_io* io, const SpellerF32Inputs& f32, co
     if (eos) LAS_CUDA_OK(cudaMemsetAsync(stop, 0, sizeof(int32_t) * (2 + 64), st));
     for (int sb = 0; sb < steps;) {
       const int n = next_segment(sb, steps, seg);
-      LAS_TRY(fast_speller_decode_segment(io, f32, packed_fast, d, b0, Bc, sb, n, sb == 0, sb + n == steps, decode_mode, relu, ws_fast, f16, st));
+      LAS_TRY(fast_speller_decode_segment(io, f32, packed_fast, d, b0, Bc, sb, n, sb == 0, sb + n == steps, decode_mode, relu, ws_fast, f16, false, st));
       if (eos) LAS_TRY(launch_eos_check(io->tokens, d->B, b0, Bc, sb, sb + n, io->eos_token, stop, st));
       sb += n;
     }

@@ -1127,7 +1127,7 @@ int las_pipeline_step(const las_pipeline_args* a, int mode, void* stream) {
 }
 
 int las_pipeline_overlaps(const las_listener_dims* ld, const las_speller_dims* sd, int steps, int mode) {
-  return pipeline_fast(ld, sd, mode) && fast_pipeline_bc(ld, sd, steps) > 0 ? 1 : 0;
+  return pipeline_fast(ld, sd, mode) && fast_pipeline_plan(ld, sd, steps).bc > 0 ? 1 : 0;
 }
 
 int las_nll_sums(const float* logp, const int32_t* labels, int S, int S_lab, int B, int V, int max_label_len, float* out2,
@@ -1159,6 +1159,7 @@ int las_debug_set_option(int key, int value) {
   auto chunk = [](int v) { return v == 0 || v == 16 || v == 32 || v == 64; };
   auto cluster = [](int v) { return v == 0 || v == 1 || v == 2 || v == 4 || v == 8; };
   auto steps = [](int v) { return v >= 0; };
+  auto units = [](int v) { return v == 0 || v == 16 || v == 32; };
   DebugOptions& o = g_debug;
   const Key keys[] = {
       {2, 1, &o.ctx_tmem, on_off},
@@ -1170,6 +1171,8 @@ int las_debug_set_option(int key, int value) {
       {13, 1, &o.gen_cluster, cluster},
       {19, 1, &o.dec_groups, on_off},
       {20, 8, o.pipe_split, steps},
+      {30, 1, &o.dec_units, units},
+      {31, 1, &o.pipe_beside, on_off},
   };
   const Key* k = nullptr;
   for (const Key& c : keys)

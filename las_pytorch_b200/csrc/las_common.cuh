@@ -75,6 +75,8 @@ struct DebugOptions {
   int gen_fused = 1;          // fused generic decoder step and the cluster attention kernel (0: unfused step, one-CTA attention)
   int gen_cluster = 0;        // CTAs per utterance of that attention cluster (0: by batch)
   int dec_groups = 1;         // persistent decoder: two utterance groups through the LSTM CTAs (0: lockstep)
+  int dec_units = 0;          // persistent decoder: hidden units per LSTM CTA (16 / 32; 0: lstm_plan)
+  int pipe_beside = 1;        // serving pipeline: the beside schedule where the chip has room for it (0: always segmented)
   int pipe_split[8] = {};     // serving pipeline: decoder steps of segment l (0: proportional to the layer's time steps)
   long long* trace = nullptr;  // device buffer of clock64 / globaltimer stamps, laid out as below (nullable)
   long long* trace_at(int offset) const { return trace ? trace + offset : nullptr; }

@@ -29,14 +29,18 @@ int fast_speller_decode(const las_decode_io* io, const SpellerF32Inputs& f32, co
 // serving pipeline that interleaves them (fast_pipeline.cu)
 int fast_speller_decode_segment(const las_decode_io* io, const SpellerF32Inputs& f32, const void* packed_fast, const las_speller_dims* d,
                                 int b0, int Bc, int s_begin, int s_count, bool first_seg, bool last_seg, int decode_mode, int relu,
-                                void* ws_fast, bool f16, cudaStream_t st);
+                                void* ws_fast, bool f16, bool beside, cudaStream_t st);  // beside: shares the chip with the listener
 int fast_speller_max_group(const las_speller_dims* d);
-int fast_speller_ctas(const las_speller_dims* d);  // CTAs of one persistent launch covering d->B utterances
+int fast_speller_ctas(const las_speller_dims* d, bool beside);  // CTAs of one persistent launch covering d->B utterances
 int fast_listener_stage(const float* x, const int32_t* x_lengths, const void* packed, const las_listener_dims* d, float* enc,
-                        int32_t* enc_lengths, void* ws, int stage, int bc, int* resident, bool f16, cudaStream_t st);
+                        int32_t* enc_lengths, void* ws, int stage, int bc, int* resident, int max_ctas, bool f16, cudaStream_t st);
 int fast_listener_rec_ctas(const las_listener_dims* d, int bc);
 int fast_side_stream(cudaStream_t* s);
-int fast_pipeline_bc(const las_listener_dims* ld, const las_speller_dims* sd, int steps);
+struct PipePlan {
+  int bc;       // the recurrence's batch chunk (16 / 32 / 64); 0: the listener does not fit next to the decoder
+  bool beside;  // the listener's stages run beside ONE decoder launch; otherwise the decoder is cut into segments around the GEMMs
+};
+PipePlan fast_pipeline_plan(const las_listener_dims* ld, const las_speller_dims* sd, int steps);
 int fast_pipeline_step(const las_decode_io* io, const SpellerF32Inputs& spl_f32, const void* spl_packed_fast, const las_speller_dims* sd,
                        int steps, int decode_mode, int relu, void* spl_ws_fast, const float* x, const int32_t* x_lengths, const void* lis_packed,
                        const las_listener_dims* ld, float* enc, int32_t* enc_lengths, void* lis_ws, bool f16, cudaStream_t st);

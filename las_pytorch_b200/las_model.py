@@ -341,9 +341,10 @@ class ServingResult:
 
 
 class ServingPipeline:
-    """Two batches in flight on one GPU: while batch i is being decoded (the persistent decoder owns 128 of the 148 SMs at paper
-    size and is latency-bound), batch i+1 is being encoded -- its recurrences on the SMs the decoder leaves free, its
-    input-projection GEMMs between the decoder's segments (include/las_b200.h `las_pipeline_step`, csrc/fast_pipeline.cu).
+    """Two batches in flight on one GPU: while batch i is being decoded (the persistent decoder owns 96 of the 148 SMs at paper
+    size and is latency-bound), batch i+1 is being encoded on the SMs the decoder leaves free -- its recurrences and, where they
+    fit, its input-projection GEMMs too, otherwise the GEMMs between the decoder's segments (include/las_b200.h
+    `las_pipeline_step`, csrc/fast_pipeline.cu).
 
         pipe = las.serve()
         for x in batches:                 # [B,T,F] device tensors
